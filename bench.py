@@ -621,6 +621,31 @@ def repl_loop_gpu(eng, name_defs):
     return out
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, search):
+    """What the timed path hands its caller after the last timed step, one float64 DIR/<name>.npy per array (exact for every
+    integer it holds): each chain's current and best support rows (one word per grid row, bit x = column x), support count, best
+    count, step and score counters, and the portfolio's best count and best layout (x, y, def_w, def_h, rotated; row-major order).
+    Beyond DUMP_BYTES in all, a fixed sample of the chains (seed 0) is written; chain_index names the chains of every chain_* file."""
+    st = search.read_chains()
+    h = search.grid.height
+    chains = {"chain_supports": st["S"][:, :h], "chain_best_supports": st["bestS"][:, :h], "chain_count": st["k"], "chain_best_count": st["best"],
+              "chain_step": st["step"], "chain_scored": st["scored"], "chain_index": np.arange(search.n_chains)}
+    per_chain = 8 * sum(a[0].size for a in chains.values())
+    keep = (DUMP_BYTES - (1 << 20)) // per_chain        # 1 MiB left for the best layout, the best count and the .npy headers
+    if search.n_chains > keep:
+        idx = np.sort(np.random.default_rng(0).choice(search.n_chains, keep, replace=False))
+        chains = {k: v[idx] for k, v in chains.items()}
+    best = search.best_count()
+    layout = [] if best is None else sorted(((p.x, p.y, p.definition.width, p.definition.height, int(p.rotated))
+                                             for p in search.best_layout().platforms().values()), key=lambda p: (p[1], p[0]))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dict(chains, best_count=[-1 if best is None else best], best_layout=np.reshape(layout, (-1, 5))).items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -636,7 +661,11 @@ def main():
     ap.add_argument("--batch-steps", type=int, default=2000, help="c5: SLS steps per chain")
     ap.add_argument("--phase-steps", type=int, default=4000, help="c4: SLS steps per window-decomposition phase")
     ap.add_argument("--c4-phases", type=int, default=15, help="c4 side measurement of the default line: timed phases")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (rank 0's chains, the best count "
+                                                          "and layout) as DIR/<name>.npy, float64, at most 64 MB (c2 on the GPU arm)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "c2"):
+        ap.error("--dump-outputs: only the c2 workload on the GPU arm")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "c5":
@@ -718,6 +747,8 @@ def main():
     sampler.join()
     best = search.best_count()
     s1 = eng.stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, search)
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     tot = torch.tensor([float(s1[k] - s0[k]) for k in ("sls_flips", "candidates_scored", "sls_steps", "kernel_launches")], dtype=torch.float64, device="cuda")
     tmax = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")

@@ -1055,8 +1055,6 @@ def test_fractional_lower_bound_on_the_gui_weight_objective(eng, fixtures):
 @pytest.mark.parametrize("name", ["ex1", "ex3", "ex2", "readme", "rect16", "rand20x14", "rect24"])
 @pytest.mark.parametrize("pset", ["1x1", "default8"])
 def test_fractional_lower_bound_certificate(eng, fixtures, readme, name, pset):
-    if name == "rect24" and pset == "default8":
-        pytest.skip("7 488 placements to re-derive with the oracle: the 1x1 case covers the grid-wide simplex on the GUI's default grid size")
     g = {"rect16": np.ones((16, 16), np.uint8), "rect24": np.ones((24, 24), np.uint8), "rand20x14": synth_terrain(20, 14, seed=3, t=1), "readme": readme[0]}.get(name)
     if g is None:
         g = fixtures[name]
