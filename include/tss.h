@@ -79,7 +79,7 @@ typedef struct tss_stats {
 
 /* ------------------------------------------------------------------------------------------------ engine */
 int tss_version(void);
-/* Bounds-checked build only (nvcc -DTSS_CHECKED, profiles/checked_build.py): shared-memory accesses of the thread-per-chain SLS kernel
+/* Bounds-checked build only (nvcc -DTSS_CHECKED, profiles/checked_build.py): shared-memory accesses of the thread-per-chain SLS kernels
  * that left their board since the library was loaded; -1 in the shipped build, which carries no checks. */
 int tss_debug_smem_violations(void);
 /* device < 0: current device.  Fails with TSS_E_CUDA when no CUDA device is usable (no CPU fallback). */
@@ -207,12 +207,13 @@ typedef struct tss_search_params {
     int32_t kernel;        /* TSS_KERNEL_*: which of the equivalent SLS kernels runs (same step rule, same trajectories); 0 = auto */
 } tss_search_params;
 
-/* SLS kernel variants for grids up to 32x32 with 1x1 supports.  All three execute the published step rule bit for bit
+/* SLS kernel variants for grids up to 32x32 with 1x1 supports.  All four execute the published step rule bit for bit
  * (tests replay each against the CPU model); they differ in how a chain is mapped to the hardware. */
 #define TSS_KERNEL_AUTO 0
 #define TSS_KERNEL_WARP 1      /* one chain per warp, any grid up to 32x32 */
 #define TSS_KERNEL_HALF_WARP 2 /* two chains per warp, grids of at most 16 rows */
 #define TSS_KERNEL_THREAD 3    /* one chain per thread, grids of at most 16 rows x 26 columns */
+#define TSS_KERNEL_PAIR 4      /* one chain per thread, two grid rows per word, grids of at most 16x16 */
 
 /* Creates a portfolio on one terrain.  defs must contain 1x1 (encoder.rs:564-566). */
 int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,

@@ -1,4 +1,5 @@
-"""compute-sanitizer is closed on this pool: the kernel that aliases shared-memory boards on purpose (csrc/sls_t16.cu) checks itself.
+"""compute-sanitizer is closed on this pool: the kernels that alias shared-memory boards on purpose (csrc/sls_t16.cu, csrc/sls_p16.cu)
+check themselves.
 Builds libtss with -DTSS_CHECKED (every shared-memory access of the step loop verified: loads inside the CTA's Smem block, stores
 in a row of the grid of the board they mean) into build/libtss_checked.so; run the trajectory / warm-start / optimum tests and a
 randomized campaign against it with TSS_LIB pointing there, then read tss_debug_smem_violations().
@@ -40,24 +41,27 @@ else:
         if rng.random() < 0.4:      # dense warm starts drive all five count planes and rows at the grid's edge
             warm = np.zeros((n_chains, 32, 32), np.uint8)
             warm[:, :h, :w] = rng.random((n_chains, h, w)) < rng.choice([0.1, 0.5, 1.0])
-        s = eng.search(T.WorldGrid(grid), seed=seed, n_chains=n_chains, kernel=T.KERNEL_THREAD)
-        if warm is not None:
-            s.write_chains((warm.astype(np.uint32) << np.arange(32, dtype=np.uint32)).sum(2, dtype=np.uint32))
-        for steps, _, target in epochs:
-            s.run(steps, target)
-        got = s.read_chains()
-        if n_chains <= 24:          # and the results are still the model's
-            want = O.sls_model(grid, n_chains, epochs, seed=seed, init_S=warm)
-            assert np.array_equal(got["k"], want["k"]) and np.array_equal(got["best"], want["best"]) and np.array_equal(got["scored"], want["scored"])
-        s.close()
-        runs += 1
+        want = None
+        for kernel in (T.KERNEL_THREAD, T.KERNEL_PAIR) if w <= 16 else (T.KERNEL_THREAD,):   # row pairs: grids of at most 16x16
+            s = eng.search(T.WorldGrid(grid), seed=seed, n_chains=n_chains, kernel=kernel)
+            if warm is not None:
+                s.write_chains((warm.astype(np.uint32) << np.arange(32, dtype=np.uint32)).sum(2, dtype=np.uint32))
+            for steps, _, target in epochs:
+                s.run(steps, target)
+            got = s.read_chains()
+            if n_chains <= 24:          # and the results are still the model's
+                want = want or O.sls_model(grid, n_chains, epochs, seed=seed, init_S=warm)
+                assert np.array_equal(got["k"], want["k"]) and np.array_equal(got["best"], want["best"]) and np.array_equal(got["scored"], want["scored"])
+            s.close()
+            runs += 1
     g16 = T.WorldGrid(np.ones((16, 16), np.uint8))
-    s = eng.search(g16, seed=1, kernel=T.KERNEL_THREAD)        # the bench's configuration: the device filled with chains
-    for _ in range(3):
-        s.run(2048, 0)
-    assert s.best_count() == 15
-    s.close()
+    for kernel in (T.KERNEL_THREAD, T.KERNEL_PAIR):
+        s = eng.search(g16, seed=1, kernel=kernel)        # the bench's configuration: the device filled with chains
+        for _ in range(3):
+            s.run(2048, 0)
+        assert s.best_count() == 15
+        s.close()
     v = lib.tss_debug_smem_violations()
-    print(f"checked build: {runs} randomized runs of sls_t16_kernel (grids up to 26x16, 1-300 chains, dense warm starts) + the bench configuration: "
-          f"{v} shared-memory violations")
+    print(f"checked build: {runs} randomized runs of sls_t16_kernel (grids up to 26x16) and sls_p16_kernel (grids up to 16x16), 1-300 chains, "
+          f"dense warm starts, + the bench configuration on both: {v} shared-memory violations")
     assert v == 0

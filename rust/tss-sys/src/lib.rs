@@ -9,6 +9,10 @@ pub const TSS_SAT: c_int = 10; // IPASIR / rustsat SolverResult::Sat
 pub const TSS_UNSAT: c_int = 20; // only from tss_solve_instance, when the limit lies below a certified lower bound
 pub const TSS_UNKNOWN: c_int = 0; // SolverResult::Interrupted
 pub const TSS_KERNEL_AUTO: i32 = 0;
+pub const TSS_KERNEL_WARP: i32 = 1; // one chain per warp, any grid up to 32x32
+pub const TSS_KERNEL_HALF_WARP: i32 = 2; // two chains per warp, grids of at most 16 rows
+pub const TSS_KERNEL_THREAD: i32 = 3; // one chain per thread, grids of at most 16 rows x 26 columns
+pub const TSS_KERNEL_PAIR: i32 = 4; // one chain per thread, two grid rows per word, grids of at most 16x16
 
 #[repr(C)]
 #[derive(Copy, Clone, Default, Debug, PartialEq, Eq)]

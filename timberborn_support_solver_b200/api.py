@@ -24,7 +24,7 @@ from ._lib import Dims as _Dims
 from ._lib import Platform as _Platform
 
 SAT, UNSAT, INTERRUPTED = "Sat", "Unsat", "Interrupted"  # rustsat SolverResult
-KERNEL_AUTO, KERNEL_WARP, KERNEL_HALF_WARP, KERNEL_THREAD = 0, 1, 2, 3  # tss.h TSS_KERNEL_*: equivalent SLS kernels
+KERNEL_AUTO, KERNEL_WARP, KERNEL_HALF_WARP, KERNEL_THREAD, KERNEL_PAIR = 0, 1, 2, 3, 4  # tss.h TSS_KERNEL_*: equivalent SLS kernels
 
 
 class TssError(RuntimeError):
@@ -439,7 +439,8 @@ class Search:
     """A device-resident SLS portfolio on one terrain (kernel (b))."""
 
     def __init__(self, engine: "Engine", grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], seed=0, n_chains=0, chain_offset=0, noise_pct=-1, kernel=0):
-        """kernel: KERNEL_AUTO / KERNEL_WARP / KERNEL_HALF_WARP / KERNEL_THREAD (tss.h TSS_KERNEL_*): equivalent SLS kernels."""
+        """kernel: KERNEL_AUTO / KERNEL_WARP / KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR (tss.h TSS_KERNEL_*): equivalent SLS kernels
+        (KERNEL_PAIR: one chain per thread with two grid rows per word, grids of at most 16x16)."""
         self.engine, self.grid = engine, grid
         self._h = C.c_void_p()
         params = _lib.SearchParams(seed, n_chains, chain_offset, noise_pct, kernel)
@@ -626,6 +627,8 @@ class Engine:
 
     # ---- kernel (b)
     def search(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], **kw) -> Search:
+        """A device-resident SLS portfolio; kw: seed, n_chains, chain_offset, noise_pct, kernel (KERNEL_AUTO, or one of KERNEL_WARP /
+        KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR to pin a variant; a variant that does not fit the grid raises TssError)."""
         return Search(self, grid, defs, **kw)
 
     def solve_upper_bound(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], card_limit: Optional[int] = None, seed=0, budget_ms=0, max_steps=0):

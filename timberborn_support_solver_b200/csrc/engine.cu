@@ -31,6 +31,13 @@ size_t sls_t16_list_words(int n_chains);
 int sls_run_t16(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, sls::ChainState* states, uint32_t* site_lists, int n_chains,
                 int chains_per_terrain, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev, int target,
                 int noise_pct, unsigned long long* totals_dev);
+// sls_p16.cu — one chain per thread, two grid rows per word, for grids of at most 16x16 (same site lists as sls_t16.cu)
+bool sls_p16_fits(int w, int h);
+int sls_p16_cta_chains();
+int sls_p16_smem_violations();
+int sls_run_p16(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, sls::ChainState* states, uint32_t* site_lists, int n_chains,
+                int chains_per_terrain, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev, int target,
+                int noise_pct, unsigned long long* totals_dev);
 int sls_run_h16_oneshot(tss_engine* e, const uint32_t* rows32_host, int bound, uint32_t* rows_dev, uint2* tabs_dev, sls::ChainState* states,
                         int n_chains, uint64_t seed, long long steps, int* bounds_dev, int2* best_dev, unsigned long long* key_dev,
                         unsigned int* ticket_dev, int target, int noise_pct, unsigned long long* totals_dev, uint32_t* result_host_mapped);
@@ -213,7 +220,7 @@ extern "C" {
 
 int tss_version(void) { return TSS_VERSION; }
 
-int tss_debug_smem_violations(void) { return sls_t16_checked_build() ? sls_t16_smem_violations() : -1; }
+int tss_debug_smem_violations(void) { return sls_t16_checked_build() ? sls_t16_smem_violations() + sls_p16_smem_violations() : -1; }
 
 int tss_engine_create(int device, tss_engine** out) {
     if (!out) return TSS_E_INVALID;
@@ -620,9 +627,10 @@ static void build_keys(const tss_dims* defs, int n_defs, std::vector<int2>& key_
 }
 
 // Chains that fill the device: 32 warps per SM for the warp kernels (two chains per warp on grids of <= 16 rows),
-// 3 CTAs of 128 threads per SM for the thread-per-chain kernel.
+// 3 CTAs of 128 threads per SM for the thread-per-chain kernels.
 static int default_chains(const tss_engine* e, int w, int h, int kernel) {
-    const bool thread_default = sls_t16_fits(w, h) && (kernel == TSS_KERNEL_AUTO || kernel == TSS_KERNEL_THREAD);
+    const bool thread_default = (sls_t16_fits(w, h) && (kernel == TSS_KERNEL_AUTO || kernel == TSS_KERNEL_THREAD)) ||
+                                (sls_p16_fits(w, h) && kernel == TSS_KERNEL_PAIR);
     const int per_sm = thread_default ? 3 * sls_t16_cta_chains() : (h <= 16 ? 64 : 32);
     return e->prop.multiProcessorCount * per_sm;
 }
@@ -665,8 +673,8 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
     // default: 32 warps per SM (8 CTAs of 4 warps); grids of <= 16 rows run two chains per warp
     // (thread-per-chain kernel: 3 CTAs of 128 chains per SM)
     s->kernel = params ? params->kernel : TSS_KERNEL_AUTO;
-    if (s->kernel < TSS_KERNEL_AUTO || s->kernel > TSS_KERNEL_THREAD || (s->kernel == TSS_KERNEL_HALF_WARP && h > 16) ||
-        (s->kernel == TSS_KERNEL_THREAD && !sls_t16_fits(w, h))) {
+    if (s->kernel < TSS_KERNEL_AUTO || s->kernel > TSS_KERNEL_PAIR || (s->kernel == TSS_KERNEL_HALF_WARP && h > 16) ||
+        (s->kernel == TSS_KERNEL_THREAD && !sls_t16_fits(w, h)) || (s->kernel == TSS_KERNEL_PAIR && !sls_p16_fits(w, h))) {
         int k = s->kernel;
         delete s;
         return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: kernel variant %d does not support a %dx%d grid", k, w, h);
@@ -763,17 +771,22 @@ void tss_sls_spec_probe(uint32_t* out) {
     out[5] = sls::step_hash(1u, 2u); out[6] = sls::tie_remove(3u, 40u) ^ sls::K3; out[7] = sls::chain_base(0x0123456789abcdefull, 5u); out[8] = sls::NO_BOUND;
 }
 
-// Which of the three equivalent SLS kernels (same spec, same trajectories) advances this portfolio.
+// Which of the four equivalent SLS kernels (same spec, same trajectories) advances this portfolio.
 static int search_kernel(const tss_search* s) {
     const int cpt = s->chains_per_terrain;
     const bool t16_ok = sls_t16_fits(s->w, s->h) && (cpt == 0 || cpt % sls_t16_cta_chains() == 0);
+    const bool p16_ok = sls_p16_fits(s->w, s->h) && (cpt == 0 || cpt % sls_p16_cta_chains() == 0);
     const bool h16_ok = s->h <= 16 && (cpt == 0 || cpt % 8 == 0);
+    if (s->kernel == TSS_KERNEL_PAIR && p16_ok) return TSS_KERNEL_PAIR;
     if (s->kernel == TSS_KERNEL_THREAD && t16_ok) return TSS_KERNEL_THREAD;
     if (s->kernel == TSS_KERNEL_WARP) return TSS_KERNEL_WARP;
     if (s->kernel == TSS_KERNEL_HALF_WARP && h16_ok) return TSS_KERNEL_HALF_WARP;
     // auto: a chain per thread pays off once the device is well filled — a thread-kernel warp steps its 32 chains in
     // ~2.4 us whatever the load, the half-warp kernel steps few chains in ~1.1 us (measured on rect 16x16,
     // profiles/crossover.py: equal at ~7000 chains; 2048 chains 48 vs 25 ms, 16384 chains 49 vs 102 ms per 20000 steps)
+    // (grids of at most 16x16: two grid rows per word issue fewer instructions per chain step than one row per word; rect
+    // 16x16, 56 832 chains: 30.3 against 24.7 G flips/s, profiles/r3_bench_alternation.jsonl)
+    if (s->kernel == TSS_KERNEL_AUTO && p16_ok && s->n_chains >= s->e->prop.multiProcessorCount * 48) return TSS_KERNEL_PAIR;
     if (s->kernel == TSS_KERNEL_AUTO && t16_ok && s->n_chains >= s->e->prop.multiProcessorCount * 48) return TSS_KERNEL_THREAD;
     return h16_ok ? TSS_KERNEL_HALF_WARP : TSS_KERNEL_WARP;
 }
@@ -812,13 +825,16 @@ int tss_search_run(tss_search* s, int64_t steps, int32_t target_count) {
     }
     int chains_per_group = s->n_groups == 1 ? s->n_chains : s->chains_per_terrain;
     const int variant = search_kernel(s);
-    if (variant == TSS_KERNEL_THREAD && !s->site_lists) TSS_CUDA(e, cudaMalloc(&s->site_lists, sizeof(uint32_t) * sls_t16_list_words(s->n_chains)));
+    if ((variant == TSS_KERNEL_THREAD || variant == TSS_KERNEL_PAIR) && !s->site_lists) TSS_CUDA(e, cudaMalloc(&s->site_lists, sizeof(uint32_t) * sls_t16_list_words(s->n_chains)));
     // an epoch is at most 32768 steps (the tabu stamps are 16 bit, sls_spec.hpp): longer runs are consecutive epochs
     for (long long left = steps; left > 0; left -= sls::MAX_EPOCH_STEPS) {
         const long long chunk = left < sls::MAX_EPOCH_STEPS ? left : sls::MAX_EPOCH_STEPS;
         const int target = target_count < 0 ? -1 : target_count;
         int rc;
-        if (variant == TSS_KERNEL_THREAD)
+        if (variant == TSS_KERNEL_PAIR)
+            rc = sls_run_p16(e, s->rows_dev, s->tabs_dev, s->states, s->site_lists, s->n_chains, s->chains_per_terrain, s->chain_offset, s->seed, chunk,
+                             s->bounds_dev, target, s->noise, s->totals_dev);
+        else if (variant == TSS_KERNEL_THREAD)
             rc = sls_run_t16(e, s->rows_dev, s->tabs_dev, s->states, s->site_lists, s->n_chains, s->chains_per_terrain, s->chain_offset, s->seed, chunk,
                              s->bounds_dev, target, s->noise, s->totals_dev);
         else
