@@ -4,10 +4,13 @@ with line info and counts the instructions attributed to each part of a chain st
 
     python profiles/sass_step_mix.py [OUTDIR]
 
-`flip` is inlined three times (list start-up, removal, addition) and reported per copy; the removal loop is unrolled by 4
-(plus a remainder copy) and reported per support scored, i.e. divided by 5; the addition block is one copy per step.
-Instructions attributed to small helpers defined outside these ranges (pick_rotated, the byte-pack functions) are not
-counted, so the figures compare parts of the two kernels, not whole steps."""
+`flip` is inlined three times (list start-up, removal, addition) and reported per copy; the addition block is one copy
+per step.  The removal scan is reported per support scored: t16's loop is unrolled by 4 (plus a remainder copy), so its
+instructions are divided by 5; p16 scans its CAP cached slots fully unrolled, divided by CAP (the loop over list entries
+past CAP, which only dense warm starts reach, is not counted).  The scan counts every instruction between its first and
+last one, the inlined helpers (anchor, byte packs, the loss) included; elsewhere instructions attributed to small helpers
+defined outside the ranges (pick_rotated, the byte-pack functions) are not counted, so the figures compare parts of the
+two kernels, not whole steps."""
 import collections
 import os
 import re
@@ -31,12 +34,17 @@ def ranges(src):
     shl = find(r"uint32_t shl_clamped\(")
     add_key = find(r"^template <int DX, int DY>")
     kern = find(r"^__global__ void")
-    rm0 = find(r"for \(int i = 0; i < k; i\+\+, mult", kern)
-    rm1 = find(r"const int best_i = ", rm0)
+    cap = re.search(r"constexpr int CAP = (\d+);", "\n".join(lines))
+    if cap:     # p16: the unrolled scan of the cached slots, up to the overflow loop
+        rm0 = find(r"for \(int i = 0; i < CAP; i\+\+\) \{", find(r"const int kw = ", kern))
+        rm1, rm_part = find(r"if \(kw > CAP\)", rm0), f"removal, per cached support (scan / {cap.group(1)})"
+    else:
+        rm0 = find(r"for \(int i = 0; i < k; i\+\+, mult", kern)
+        rm1, rm_part = find(r"const int best_i = ", rm0), "removal, per support (scan / 5)"
     ad0 = find(r"const int y = pick_rotated\(", rm1)
-    ad1 = find(r"flip<true>\(sm, tid, v, rowmask\)", ad0)
-    return {"flip (per copy)": (flip, shl, 3), "removal, per support (body / 5)": (rm0, rm1, 5),
-            "addition: 25 candidates (add_key/add_column)": (add_key, kern, 1), "addition: fetch, pick, tabu window, decode": (ad0, ad1, 1)}
+    ad1 = find(r"flip<true>\(sm, tid, v, ", ad0)
+    return {"flip (per copy)": (flip, shl, 3, False), rm_part: (rm0, rm1, int(cap.group(1)) if cap else 5, True),
+            "addition: 25 candidates (add_key/add_column)": (add_key, kern, 1, False), "addition: fetch, pick, tabu window, decode": (ad0, ad1, 1, False)}
 
 
 def mix(name, out):
@@ -49,6 +57,7 @@ def mix(name, out):
     sass = subprocess.run([os.path.join(CUDA, "bin", "nvdisasm"), "-g", "-c", cubin], capture_output=True, text=True, check=True).stdout
     rng = ranges(src)
     per = collections.defaultdict(collections.Counter)
+    ins = []   # (our source line or None, opcode) in address order
     line, ours = 0, False
     for l in sass.split("\n"):
         m = re.search(r'//## File "([^"]+)", line (\d+)', l)
@@ -56,13 +65,14 @@ def mix(name, out):
             ours, line = m.group(1).endswith(name + ".cu"), int(m.group(2))
             continue
         m = re.match(r"\s+/\*[0-9a-f]{4,}\*/\s+(?:@!?U?P\w+\s+)?([A-Z][A-Z0-9_]*)", l)
-        if not m or not ours:
-            continue
-        for part, (a, b, _) in rng.items():
-            if a <= line < b:
-                per[part][m.group(1)] += 1
+        if m:
+            ins.append((line if ours else None, m.group(1)))
+    for part, (a, b, _, span) in rng.items():
+        hit = [j for j, (ln, _) in enumerate(ins) if ln is not None and a <= ln < b]
+        for j in range(hit[0], hit[-1] + 1) if span else hit:
+            per[part][ins[j][1]] += 1
     print(f"{name}: {regs[0][1] if regs else '?'} registers, {regs[0][0] if regs else '?'} bytes spilled")
-    for part, (a, b, div) in rng.items():
+    for part, (a, b, div, _) in rng.items():
         c = per[part]
         top = ", ".join(f"{op} {n / div:.1f}" for op, n in c.most_common(8))
         print(f"  {part:48s} {sum(c.values()) / div:6.1f}   ({top})")

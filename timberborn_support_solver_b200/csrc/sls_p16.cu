@@ -22,7 +22,10 @@
 //     (8 loads, 7 PRMT with a selector chosen by y & 1): candidate (DX, DY) then starts at a static pair and half, and
 //     one slab per DX (pairs >> max(x+DX-3, 0)) serves all of its DYs.  The table alignment a candidate needs differs
 //     from its absolute one exactly when y is odd, hence the second table: the step picks the table base by y & 1.
-//     t's own window (candidate validity) and the tabu window stay in t16's byte-per-row format around (x-3, y-3).
+//     t's own window (candidate validity) and the tabu window stay in t16's byte-per-row format around (x-3, y-3);
+//   * the first CAP entries of the site list live in shared memory with their table windows ([slot][thread], bank =
+//     thread), so the removal scan reads a scored support with two conflict-free loads at immediate offsets instead of a
+//     global load and a bank-conflicting table read.  Entries at index >= CAP stay in the global list (dense warm starts).
 #include "engine.hpp"
 #include "sls_spec.hpp"
 
@@ -42,25 +45,36 @@ constexpr int TAB_N = 512 + 2 * TAB_PAD;
 // out-of-grid rows only ever meet zero window bits (reads) or a zero mask (no write)
 enum { B_C0 = 0, B_C1 = 1, B_C2 = 2, B_U = 3, B_O = 4, B_C3 = 5, B_C4 = 6, N_BOARDS = 7 };
 
+constexpr int CAP = 16;          // site-list entries per chain kept in shared memory (k stays at 14-15 on rect 16x16)
+
 struct Smem {
     uint2 tab[2][TAB_N];                   // [slot shift][site]: reach window of site v at tab[a][v + TAB_PAD], rows in slots s0 ^ a ..
+    uint2 cwin[CAP][NT];                   // [slot][thread]: tab[0] window of list entry `slot`
+    uint32_t cent[CAP][NT];                // [slot][thread]: list entry `slot` (format of `entry` below)
     uint32_t C[16];                        // terrain pairs; pair p at C[p + 2], zero outside the grid
     uint32_t rows[N_BOARDS * NP][NT];      // [board][pair][thread]: bank = thread, conflict free for any pair index
     uint16_t ring[32][NT];                 // site removed at step s in slot s & 31 (NONE if none)
 };
 constexpr int BOARD = NP * NT;             // words between the same pair of consecutive boards
-// Exactly 3 CTAs per SM (as t16): 444 CTAs of the default portfolio then fill the 148 SMs evenly.  The kernel itself
-// needs ~48 KB, which would let a 4th CTA in and schedule the default grid 4/4/.../2: the dynamic allocation is padded.
-constexpr size_t SMEM_BYTES = sizeof(Smem) > 64 * 1024 ? sizeof(Smem) : 64 * 1024;
+// Exactly 3 CTAs per SM (as t16): 444 CTAs of the default portfolio then fill the 148 SMs evenly (the SM has 228 KB, of
+// which 1 KB per resident CTA is reserved).
+constexpr size_t SMEM_BYTES = sizeof(Smem);
+static_assert(3 * (SMEM_BYTES + 1024) <= 228 * 1024 && 4 * (SMEM_BYTES + 1024) > 228 * 1024, "sls_p16 must fit exactly 3 CTAs per SM");
 
 // ---- bounds-checked build (-DTSS_CHECKED, profiles/checked_build.py), as in sls_t16.cu: every shared-memory access of the
 // step loop stays inside the CTA's Smem block, every store lands in a pair of the grid of the board it means.
 #ifdef TSS_CHECKED
 __device__ unsigned int g_smem_violations = 0;
-__device__ __forceinline__ const uint32_t* chk_ld(const Smem& sm, const uint32_t* p) {
+template <class T>
+__device__ __forceinline__ const T* chk_ld(const Smem& sm, const T* p) {
     const size_t off = (size_t)((const char*)p - (const char*)&sm);
-    if (off + 4 > sizeof(Smem) || (off & 3)) { atomicAdd(&g_smem_violations, 1u); return &sm.rows[0][0]; }
+    if (off + sizeof(T) > sizeof(Smem) || (off % sizeof(T))) { atomicAdd(&g_smem_violations, 1u); return reinterpret_cast<const T*>(&sm); }
     return p;
+}
+// a support-cache slot index (the slot's column is always the thread's own)
+__device__ __forceinline__ int chk_slot(int i) {
+    if ((unsigned)i >= (unsigned)CAP) { atomicAdd(&g_smem_violations, 1u); return 0; }
+    return i;
 }
 __device__ __forceinline__ const uint2* chk_tab(const Smem& sm, const uint2* p) {
     const ptrdiff_t off = p - &sm.tab[0][0];
@@ -76,10 +90,12 @@ __device__ __forceinline__ uint32_t* chk_st(Smem& sm, uint32_t* p, int board, in
 #define LD(p) (*chk_ld(sm, (p)))
 #define LDT(p) (*chk_tab(sm, (p)))
 #define ST(p, board) (*chk_st(sm, (p), (board), tid))
+#define SLOT(arr, i) (sm.arr[chk_slot(i)][tid])
 #else
 #define LD(p) (*(p))
 #define LDT(p) (*(p))
 #define ST(p, board) (*(p))
+#define SLOT(arr, i) (sm.arr[i][tid])
 #endif
 
 __device__ __forceinline__ int pick_rotated(uint32_t bits, uint32_t o) {
@@ -89,18 +105,33 @@ __device__ __forceinline__ int pick_rotated(uint32_t bits, uint32_t o) {
 
 // first pair of site v's window: floor((y - 3) / 2) for v = 32 y + x (x < 32 never carries into the quotient)
 __device__ __forceinline__ int first_pair(int v) { return (v - 96) >> 6; }
-__device__ __forceinline__ int anchor(int x) { return max(x - 3, 0); }
+__device__ __forceinline__ int anchor(int x) { return __viaddmax_s32_relu(x, -3, 0); }   // max(x - 3, 0), one VIADDMNMX
 // bytes 0 and 2 of four words as one word (row 2p / 2p+1 windows of four pairs: slots 0..7 -> two table words)
 __device__ __forceinline__ uint32_t pack_pairs(uint32_t a, uint32_t b) { return __byte_perm(a, b, 0x6420); }
 
-// adds (ADD) or removes the cover of site v on the five count planes and refreshes U, O and the non-empty-row mask.
+// site-list entry: site v (bits 0-8), first_pair(v) + 2 (bits 9-12) and the step it was added (bits 16-31).  Bits 9-12
+// are the byte offset of the window's first pair within a board, in units of one pair row (NT words = 512 bytes).  The
+// tabu test (stephi - e) < ten << 16 only sees bits 16-31: what the low half holds cannot borrow into them.
+static_assert(NT * sizeof(uint32_t) == 512, "entry() and removal_loss() take bits 9-12 of an entry as a byte offset of whole pair rows");
+__device__ __forceinline__ uint32_t entry(int v, uint32_t stamp) { return (uint32_t)v | (uint32_t)((v + 32) >> 6) << 9 | stamp << 16; }
+
+// removal loss of list entry e with window win: reach tiles that only its support covers
+__device__ __forceinline__ uint32_t removal_loss(const Smem& sm, int tid, uint32_t e, uint2 win) {
+    const int ax = anchor(e & 31);
+    const uint32_t* p = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(&sm.rows[B_O * NP - 2][0]) + ((e & 0x1e00u) | (uint32_t)tid << 2));
+    const uint32_t lo = pack_pairs(LD(p) >> ax, LD(p + NT) >> ax);
+    const uint32_t hi = pack_pairs(LD(p + 2 * NT) >> ax, LD(p + 3 * NT) >> ax);
+    return (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
+}
+
+// adds (ADD) or removes the cover of site v (window win = its tab[0] entry) on the five count planes and refreshes U, O
+// and the non-empty-row mask.
 // Branch free as in t16: pairs of the window without reach bits (m = 0) recompute what is already there; pairs outside
 // the grid read a neighbouring board (never written: the stores are predicated on m != 0) and meet C = 0.
 // rowmask is kept in padded coordinates: bit r + 4 = row r has an uncovered tile.
 template <bool ADD>
-__device__ __forceinline__ void flip(Smem& sm, int tid, int v, uint32_t& rowmask) {
+__device__ __forceinline__ void flip(Smem& sm, int tid, int v, uint2 win, uint32_t& rowmask) {
     const int ax = anchor(v & 31), p0 = first_pair(v);
-    const uint2 win = LDT(&sm.tab[0][v + TAB_PAD]);
     uint32_t* p = &sm.rows[0][tid] + p0 * NT;  // pair p0 of the first board
     uint32_t nz = 0;
 #pragma unroll
@@ -148,11 +179,12 @@ __device__ __forceinline__ constexpr int cell_index(int dx, int dy) { return cel
 __device__ __forceinline__ uint32_t shift_static(uint32_t v, int s) { return s >= 0 ? v << s : v >> (-s); }
 
 // rows of the support bitboard of a site list (rare path: recording a best layout, writing the state back)
-__device__ __noinline__ void list_to_rows(const uint32_t* sl, size_t stride, int k, uint32_t* out32) {
+// (entries below CAP in the thread's cache column `cached`, the rest in the global list)
+__device__ __noinline__ void list_to_rows(const uint32_t* cached, const uint32_t* sl, size_t stride, int k, uint32_t* out32) {
     uint32_t rows[16];
     for (int r = 0; r < 16; r++) rows[r] = 0;
     for (int i = 0; i < k; i++) {
-        const uint32_t v = sl[(size_t)i * stride] & 0x1ffu;
+        const uint32_t v = (i < CAP ? cached[i * NT] : sl[(size_t)i * stride]) & 0x1ffu;
         rows[v >> 5] |= 1u << (v & 31u);
     }
     for (int r = 0; r < 16; r++) out32[r] = rows[r];
@@ -239,6 +271,8 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
     for (int r = 0; r < N_BOARDS * NP; r++) sm.rows[r][tid] = 0;
 #pragma unroll
     for (int r = 0; r < 32; r++) sm.ring[r][tid] = (uint16_t)NONE;
+#pragma unroll
+    for (int i = 0; i < CAP; i++) { sm.cent[i][tid] = 0; sm.cwin[i][tid] = make_uint2(0u, 0u); }   // slots past k are loaded (not scored) by the removal scan
     __syncthreads();
 
     const bool exists = chain < n_chains;
@@ -256,20 +290,25 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
         const int tenure = tenure_of(chain_offset + (uint32_t)chain);
         uint32_t* sl = site_lists + chain;
         uint32_t* const Ub = &sm.rows[B_U * NP][tid];
-        const uint32_t* const Ob = &sm.rows[B_O * NP][tid];
+        const uint32_t* const cached = &sm.cent[0][tid];
         int best = st.best, k = 0;
         uint32_t step = st.step, rowmask = 0;
 
         {   // site list in row-major order (spec), stamps "half a period ago"; cover planes from the list
-            const uint32_t reset = (uint32_t)stamp_reset(step) << 16;
-            for (int y = 0; y < MAXH; y++)
-                for (uint32_t bits = st.S[y]; bits; bits &= bits - 1) sl[(size_t)(k++) * stride] = (uint32_t)(y * 32 + __ffs(bits) - 1) | reset;
             for (int p = 0; p < NP; p++) {
                 const uint32_t c = sm.C[p + 2];
                 Ub[p * NT] = c;
                 rowmask |= ((c & 0xffffu) ? 16u << (2 * p) : 0u) | ((c >> 16) ? 32u << (2 * p) : 0u);
             }
-            for (int i = 0; i < k; i++) flip<true>(sm, tid, (int)(sl[(size_t)i * stride] & 0x1ffu), rowmask);
+            const uint32_t reset = stamp_reset(step);
+            for (int y = 0; y < MAXH; y++)
+                for (uint32_t bits = st.S[y]; bits; bits &= bits - 1, k++) {
+                    const int v = y * 32 + __ffs(bits) - 1;
+                    const uint2 win = LDT(&sm.tab[0][v + TAB_PAD]);
+                    if (k < CAP) { SLOT(cent, k) = entry(v, reset); SLOT(cwin, k) = win; }
+                    else sl[(size_t)k * stride] = entry(v, reset);
+                    flip<true>(sm, tid, v, win, rowmask);
+                }
         }
 
         for (long long it = 0; it < steps; it++) {
@@ -282,7 +321,7 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
             sm.ring[step & 31u][tid] = (uint16_t)NONE;  // every consumed step owns its slot (stale entries are 32 steps old)
             if (!drop && rowmask == 0) {  // complete layout with k < limit supports
                 best = k;
-                list_to_rows(sl, stride, k, st.bestS);
+                list_to_rows(cached, sl, stride, k, st.bestS);
                 step++; my_steps++;
                 if (k <= target || k == 0) { done = 1; break; }
                 continue;
@@ -292,26 +331,59 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
                 // dropping).  key = young | loss | tie | list index: unique, so the minimum is the spec's (lowest index wins ties)
                 const uint32_t stephi = (step << 16) | 0xffffu;             // stephi - entry = (age << 16) + (0xffff - site): no borrow
                 const uint32_t young_below = drop ? 0u : (uint32_t)ten << 16;
-                uint32_t best_key = 0xffffffffu, mult = K3;                 // mult = (2i+1) * K3
-#pragma unroll 4
-                for (int i = 0; i < k; i++, mult += 2u * K3) {
-                    const uint32_t e = sl[(size_t)i * stride];
-                    const int v = (int)(e & 0x1ffu), ax = anchor(v & 31);
-                    const uint2 win = LDT(&sm.tab[0][v + TAB_PAD]);
-                    const uint32_t* p = Ob + first_pair(v) * NT;
-                    const uint32_t lo = pack_pairs(LD(p) >> ax, LD(p + NT) >> ax);
-                    const uint32_t hi = pack_pairs(LD(p + 2 * NT) >> ax, LD(p + 3 * NT) >> ax);
-                    const uint32_t loss = (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
-                    const uint32_t tie = ((hs * mult) >> 7) & 0x1fffe00u;  // tie_remove(hs, i) << 9
+                uint32_t best_key = 0xffffffffu;
+                // cached slots: the warp scans them in groups of SCAN up to its largest k (a thread scores only its own k).  No
+                // branch inside a group, so the loads of its slots overlap: with 3 warps per scheduler the scan is latency bound
+                // when every slot waits for the one before it.
+                // kw only has to be >= this thread's own k: threads that arrive here apart from the rest of the warp reduce over a
+                // partial mask and scan for their own group, which is still exact
+                const int kw = __reduce_max_sync(__activemask(), k);
+                constexpr int SCAN = 8;
+#pragma unroll
+                for (int i = 0; i < CAP; i++) {
+                    if (i % SCAN == 0 && i >= kw) break;
+                    const uint32_t e = SLOT(cent, i);
+                    const uint32_t loss = removal_loss(sm, tid, e, SLOT(cwin, i));
+                    const uint32_t tie = ((hs * ((2u * i + 1u) * K3)) >> 7) & 0x1fffe00u;  // tie_remove(hs, i) << 9
                     const uint32_t young = (stephi - e) < young_below ? TABU_BIT : 0u;
-                    best_key = min(best_key, (young | tie | (uint32_t)i) + loss * (1u << 25));
+                    const uint32_t key = (young | tie | (uint32_t)i) + loss * (1u << 25);
+                    best_key = i < k ? min(best_key, key) : best_key;   // compiles to a select: no branch inside a group
                 }
-                const int best_i = (int)(best_key & 0x1ffu);
-                const int u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
-                const uint32_t last = sl[(size_t)(k - 1) * stride];
-                sl[(size_t)best_i * stride] = last;
+                if (kw > CAP) {   // the rest of the list (dense warm starts): global entries, windows from the table
+                    uint32_t mult = (2u * CAP + 1u) * K3;                   // mult = (2i+1) * K3
+                    for (int i = CAP; i < k; i++, mult += 2u * K3) {
+                        const uint32_t e = sl[(size_t)i * stride];
+                        const uint32_t loss = removal_loss(sm, tid, e, LDT(&sm.tab[0][(e & 0x1ffu) + TAB_PAD]));
+                        const uint32_t tie = ((hs * mult) >> 7) & 0x1fffe00u;
+                        const uint32_t young = (stephi - e) < young_below ? TABU_BIT : 0u;
+                        best_key = min(best_key, (young | tie | (uint32_t)i) + loss * (1u << 25));
+                    }
+                }
+                const int best_i = (int)(best_key & 0x1ffu), last = k - 1;
+                int u;
+                uint2 win;
+                if (best_i < CAP) {
+                    u = (int)(SLOT(cent, best_i) & 0x1ffu);
+                    win = SLOT(cwin, best_i);
+                } else {
+                    u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
+                    win = LDT(&sm.tab[0][u + TAB_PAD]);
+                }
+                // swap-remove: entry k-1 (with its window) moves into slot best_i
+                if (last < CAP) {
+                    SLOT(cent, best_i) = SLOT(cent, last);
+                    SLOT(cwin, best_i) = SLOT(cwin, last);
+                } else {
+                    const uint32_t e = sl[(size_t)last * stride];
+                    if (best_i < CAP) {
+                        SLOT(cent, best_i) = e;
+                        SLOT(cwin, best_i) = LDT(&sm.tab[0][(e & 0x1ffu) + TAB_PAD]);
+                    } else {
+                        sl[(size_t)best_i * stride] = e;
+                    }
+                }
                 sm.ring[step & 31u][tid] = (uint16_t)u;
-                flip<false>(sm, tid, u, rowmask);
+                flip<false>(sm, tid, u, win, rowmask);
                 scored += (unsigned)k;
                 k--;
                 flips++;
@@ -361,8 +433,10 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
                 const int r = (cell >= 1) + (cell >= 4) + (cell >= 9) + (cell >= 16) + (cell >= 21) + (cell >= 24);
                 const int dy = r - 3, dx = cell - cell_start(r) - (3 - abs(dy));
                 const int v = (y + dy) * 32 + x + dx;
-                flip<true>(sm, tid, v, rowmask);
-                sl[(size_t)k * stride] = (uint32_t)v | (step << 16);
+                const uint2 win = LDT(&sm.tab[0][v + TAB_PAD]);
+                flip<true>(sm, tid, v, win, rowmask);
+                if (k < CAP) { SLOT(cent, k) = entry(v, step); SLOT(cwin, k) = win; }
+                else sl[(size_t)k * stride] = entry(v, step);
                 if (!noise) scored += (unsigned)(__popc(wt.x) + __popc(wt.y));
                 k++;
                 flips++;
@@ -370,7 +444,7 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
             step++; my_steps++;
         }
 
-        list_to_rows(sl, stride, k, st.S);
+        list_to_rows(cached, sl, stride, k, st.S);
         st.k = k; st.best = best; st.step = step; st.done = done;
         const unsigned long long tot = ((unsigned long long)st.scored_hi << 32 | st.scored_lo) + scored;
         st.scored_lo = (uint32_t)tot; st.scored_hi = (uint32_t)(tot >> 32);
