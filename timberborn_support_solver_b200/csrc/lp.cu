@@ -187,6 +187,11 @@ __device__ __forceinline__ double fast_rcp(double x) {
     return r;
 }
 
+// Devex pricing key d^2 / w.  The reference weights only grow (past 2^120 on full rectangles of 16x16 and more).  Beyond that the single-precision
+// seed of fast_rcp flushes to zero (--use_fast_math), which priced improving columns at 0 and ended the simplex short of the optimum
+// with the optimal flag set (full 32x32 grid, 1x1 supports: 45.70 of 46.90).  Such weights take an exact division.
+__device__ __forceinline__ double devex_key(double d, double w) { return d * d * (w < 0x1p120 ? fast_rcp(w) : 1.0 / w); }
+
 // Exact warp argmin over non-negative doubles (lowest index on ties) in three 32-bit REDUX instructions instead of five shuffle
 // rounds on (double, int) pairs: non-negative doubles order like their bit patterns, so reduce the high words, then the low words
 // among the lanes that hold the minimum high word, then the indices among the lanes that hold both.  Lanes without a candidate
@@ -261,8 +266,10 @@ lp_simplex_cluster_kernel(const double* __restrict__ T, int m, int n, const int*
         for (int j = tid; j < n; j += blockDim.x) {
             const double d = obj[j];
             if (d < -EPS) {
-                const double key = d * d * fast_rcp(devex[j]);
-                if (key > e.v) e = ArgD{key, j};            // (columns ascend: the first of equal keys stays)
+                const double key = devex_key(d, devex[j]);
+                // (columns ascend: the first of equal keys stays; every improving column is a candidate, even at key 0, so that
+                // "no candidate" means no reduced cost below -EPS)
+                if (key > e.v || e.i == 0x7fffffff) e = ArgD{key, j};
             }
         }
         e = warp_argmax_nonneg(e);
@@ -377,8 +384,8 @@ lp_simplex_grid_kernel(double* __restrict__ T, int m, int n, const int* __restri
         for (int j = tid; j < n; j += blockDim.x) {
             const double d = obj[j];
             if (d < -EPS) {
-                const double key = d * d * fast_rcp(devex[j]);
-                if (key > e.v) e = ArgD{key, j};
+                const double key = devex_key(d, devex[j]);
+                if (key > e.v || e.i == 0x7fffffff) e = ArgD{key, j};
             }
         }
         e = warp_argmax_nonneg(e);
