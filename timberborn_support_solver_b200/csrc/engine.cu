@@ -22,9 +22,9 @@ int sls_run(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, sls:
 int sls_best_reduce(tss_engine* e, const sls::ChainState* states, int chains_per_group, int n_chains, int n_groups, int2* out_dev,
                     int* bounds_dev, unsigned long long* key_dev);
 // sls_h16.cu — two chains per warp for grids of at most 16 rows (chains_per_terrain must be 0 or a multiple of 8)
+int sls_thread_cta_chains();   // chains per CTA of both thread-per-chain kernels (sls_thread.cuh)
 // sls_t16.cu — one chain per thread for grids of at most 16 rows x 26 columns (chains_per_terrain 0 or a multiple of the CTA size)
 bool sls_t16_fits(int w, int h);
-int sls_t16_cta_chains();
 int sls_t16_smem_violations();
 int sls_t16_checked_build();
 size_t sls_t16_list_words(int n_chains);
@@ -33,7 +33,6 @@ int sls_run_t16(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, 
                 int noise_pct, unsigned long long* totals_dev);
 // sls_p16.cu — one chain per thread, two grid rows per word, for grids of at most 16x16 (same site lists as sls_t16.cu)
 bool sls_p16_fits(int w, int h);
-int sls_p16_cta_chains();
 int sls_p16_smem_violations();
 int sls_run_p16(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, sls::ChainState* states, uint32_t* site_lists, int n_chains,
                 int chains_per_terrain, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev, int target,
@@ -631,7 +630,7 @@ static void build_keys(const tss_dims* defs, int n_defs, std::vector<int2>& key_
 static int default_chains(const tss_engine* e, int w, int h, int kernel) {
     const bool thread_default = (sls_t16_fits(w, h) && (kernel == TSS_KERNEL_AUTO || kernel == TSS_KERNEL_THREAD)) ||
                                 (sls_p16_fits(w, h) && kernel == TSS_KERNEL_PAIR);
-    const int per_sm = thread_default ? 3 * sls_t16_cta_chains() : (h <= 16 ? 64 : 32);
+    const int per_sm = thread_default ? 3 * sls_thread_cta_chains() : (h <= 16 ? 64 : 32);
     return e->prop.multiProcessorCount * per_sm;
 }
 
@@ -774,8 +773,8 @@ void tss_sls_spec_probe(uint32_t* out) {
 // Which of the four equivalent SLS kernels (same spec, same trajectories) advances this portfolio.
 static int search_kernel(const tss_search* s) {
     const int cpt = s->chains_per_terrain;
-    const bool t16_ok = sls_t16_fits(s->w, s->h) && (cpt == 0 || cpt % sls_t16_cta_chains() == 0);
-    const bool p16_ok = sls_p16_fits(s->w, s->h) && (cpt == 0 || cpt % sls_p16_cta_chains() == 0);
+    const bool t16_ok = sls_t16_fits(s->w, s->h) && (cpt == 0 || cpt % sls_thread_cta_chains() == 0);
+    const bool p16_ok = sls_p16_fits(s->w, s->h) && (cpt == 0 || cpt % sls_thread_cta_chains() == 0);
     const bool h16_ok = s->h <= 16 && (cpt == 0 || cpt % 8 == 0);
     if (s->kernel == TSS_KERNEL_PAIR && p16_ok) return TSS_KERNEL_PAIR;
     if (s->kernel == TSS_KERNEL_THREAD && t16_ok) return TSS_KERNEL_THREAD;

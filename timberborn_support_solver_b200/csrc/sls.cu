@@ -11,75 +11,12 @@
 // two hashes per step, no divisions, no selects on the shift direction.
 #include "engine.hpp"
 #include "sls_spec.hpp"
+#include "sls_warp.cuh"
 
 namespace tss {
 namespace sls {
 
 constexpr int WARPS = 4;  // chains per CTA
-constexpr unsigned FULL = 0xffffffffu;
-
-struct Lane {
-    uint32_t C, S, c0, c1, c2, c3, c4, U, O;
-};
-
-__device__ __forceinline__ void derive(Lane& L) {
-    uint32_t hi = L.c1 | L.c2 | L.c3 | L.c4;
-    L.U = L.C & ~(L.c0 | hi);
-    L.O = L.c0 & ~hi & L.C;  // (in WINDOW mode tiles covered by frozen supports are not a loss)
-}
-
-// Reach windows are 7 rows x 7 columns; window row dy is grid row y-3+dy, window column 0 is grid column
-// ax = max(x-3, 0) (anchoring at 0 near the left edge keeps every extraction a single right shift).
-__device__ __forceinline__ int anchor(int x) { return max(x - 3, 0); }
-
-// Row `lane` of the reach mask of site (x, y) in grid coordinates.
-__device__ __forceinline__ uint32_t row_mask(uint2 win, int x, int y, int lane) {
-    int dy = lane - y + 3;
-    int d = min(max(dy, 0), 6);
-    uint32_t m = d < 4 ? (win.x >> (7 * d)) : (win.y >> (7 * (d - 4)));
-    m = dy == d ? (m & 0x7fu) : 0u;
-    return m << anchor(x);
-}
-
-__device__ __forceinline__ void planes_add(Lane& L, uint32_t m) {
-    uint32_t t;
-    t = L.c0 & m; L.c0 ^= m; m = t;
-    t = L.c1 & m; L.c1 ^= m; m = t;
-    t = L.c2 & m; L.c2 ^= m; m = t;
-    t = L.c3 & m; L.c3 ^= m; m = t;
-    L.c4 ^= m;
-}
-__device__ __forceinline__ void planes_sub(Lane& L, uint32_t m) {
-    uint32_t t;
-    t = ~L.c0 & m; L.c0 ^= m; m = t;
-    t = ~L.c1 & m; L.c1 ^= m; m = t;
-    t = ~L.c2 & m; L.c2 ^= m; m = t;
-    t = ~L.c3 & m; L.c3 ^= m; m = t;
-    L.c4 ^= m;
-}
-
-// popcount(B & R(site at (x, y))) where B is a row-distributed bitboard (lane r holds row r) and `win` the site's
-// reach window.  Every lane scores its own site; all 32 lanes must call.
-__device__ __forceinline__ int score(uint32_t B, int x, int y, uint2 win) {
-    const int ax = anchor(x);
-    uint32_t lo = 0, hi = 0;
-#pragma unroll
-    for (int j = 6; j >= 4; j--) {  // shfl uses the low 5 bits of the source lane; rows outside the grid meet zero window bits
-        uint32_t row = __shfl_sync(FULL, B, y - 3 + j);
-        hi = hi * 128u + ((row >> ax) & 0x7fu);
-    }
-#pragma unroll
-    for (int j = 3; j >= 0; j--) {
-        uint32_t row = __shfl_sync(FULL, B, y - 3 + j);
-        lo = lo * 128u + ((row >> ax) & 0x7fu);
-    }
-    return __popc(lo & win.x) + __popc(hi & win.y);
-}
-
-__device__ __forceinline__ int pick_rotated(uint32_t bits, uint32_t o) {  // a set bit of `bits`, searching from offset o
-    uint32_t rot = __funnelshift_r(bits, bits, o);
-    return (int)((__ffs(rot) - 1 + o) & 31u);
-}
 
 // Reach windows: one thread per tile, three masked dilations inside the tile's own 7x7 window (geodesic paths of
 // length <= 3 never leave it).  rows: [n_terrains][32] ; out: [n_terrains][1024].

@@ -9,6 +9,7 @@
 //   the step is fully predicated (drop / record / swap flags per half) so both halves stay convergent for the shuffles.
 #include "engine.hpp"
 #include "sls_spec.hpp"
+#include "sls_warp.cuh"
 
 namespace tss {
 namespace sls16 {
@@ -17,57 +18,7 @@ using namespace tss::sls;
 
 constexpr int WARPS = 4;          // 8 chains per CTA
 constexpr int MAX_SITES16 = 512;  // tiles of a 32x16 grid
-constexpr unsigned FULL = 0xffffffffu;
 
-struct Lane {
-    uint32_t C, S, c0, c1, c2, c3, c4, U, O;
-};
-__device__ __forceinline__ void derive(Lane& L) {
-    uint32_t hi = L.c1 | L.c2 | L.c3 | L.c4;
-    L.U = L.C & ~(L.c0 | hi);
-    L.O = L.c0 & ~hi & L.C;
-}
-__device__ __forceinline__ int anchor(int x) { return max(x - 3, 0); }
-__device__ __forceinline__ uint32_t row_mask(uint2 win, int x, int y, int row) {
-    int dy = row - y + 3;
-    int d = min(max(dy, 0), 6);
-    uint32_t m = d < 4 ? (win.x >> (7 * d)) : (win.y >> (7 * (d - 4)));
-    m = dy == d ? (m & 0x7fu) : 0u;
-    return m << anchor(x);
-}
-__device__ __forceinline__ void planes_add(Lane& L, uint32_t m) {
-    uint32_t t;
-    t = L.c0 & m; L.c0 ^= m; m = t;
-    t = L.c1 & m; L.c1 ^= m; m = t;
-    t = L.c2 & m; L.c2 ^= m; m = t;
-    t = L.c3 & m; L.c3 ^= m; m = t;
-    L.c4 ^= m;
-}
-__device__ __forceinline__ void planes_sub(Lane& L, uint32_t m) {
-    uint32_t t;
-    t = ~L.c0 & m; L.c0 ^= m; m = t;
-    t = ~L.c1 & m; L.c1 ^= m; m = t;
-    t = ~L.c2 & m; L.c2 ^= m; m = t;
-    t = ~L.c3 & m; L.c3 ^= m; m = t;
-    L.c4 ^= m;
-}
-// popcount(B & R(site)) with B row-distributed inside each half-warp (width-16 shuffles: row index modulo 16; rows that
-// wrap around meet zero window bits because the grid has at most 16 rows)
-__device__ __forceinline__ int score16(uint32_t B, int x, int y, uint2 win) {
-    const int ax = anchor(x);
-    uint32_t lo = 0, hi = 0;
-#pragma unroll
-    for (int j = 6; j >= 4; j--) {
-        uint32_t row = __shfl_sync(FULL, B, y - 3 + j, 16);
-        hi = hi * 128u + ((row >> ax) & 0x7fu);
-    }
-#pragma unroll
-    for (int j = 3; j >= 0; j--) {
-        uint32_t row = __shfl_sync(FULL, B, y - 3 + j, 16);
-        lo = lo * 128u + ((row >> ax) & 0x7fu);
-    }
-    return __popc(lo & win.x) + __popc(hi & win.y);
-}
 __device__ __forceinline__ uint32_t half_min(uint32_t v) {
 #pragma unroll
     for (int o = 8; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(FULL, v, o, 16));
@@ -77,16 +28,6 @@ __device__ __forceinline__ uint32_t half_max(uint32_t v) {
 #pragma unroll
     for (int o = 8; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(FULL, v, o, 16));
     return v;
-}
-__device__ __forceinline__ int pick_rotated16(uint32_t bits16, uint32_t o) {  // spec: rotate the 32-bit row mask; rows >= 16 are empty
-    uint32_t rot = __funnelshift_r(bits16, bits16, o);
-    return (int)((__ffs(rot) - 1 + o) & 31u);
-}
-__device__ __forceinline__ void diamond_cell(int i, int& dx, int& dy) {
-    int r = (i >= 1) + (i >= 4) + (i >= 9) + (i >= 16) + (i >= 21) + (i >= 24);
-    int start = r <= 4 ? r * r : (r == 5 ? 21 : 24);
-    dy = r - 3;
-    dx = (i - start) - (3 - abs(dy));
 }
 
 // ONESHOT = the whole first epoch of a one-shot solve in ONE launch (tss_solve_upper_bound, latency mode): the terrain
@@ -216,7 +157,7 @@ __global__ void __launch_bounds__(WARPS * 32, 8) sls_h16_kernel(const uint32_t* 
                 const int i = b + row;
                 const bool valid = i < kk;
                 const int v = valid ? sites[i] : 0;
-                const int loss = score16(L.O, v & 31, v >> 5, tab[v]);
+                const int loss = score<16>(L.O, v & 31, v >> 5, tab[v]);
                 const uint32_t tie = tie_remove(hs, (uint32_t)i);
                 const uint32_t young = (!drop && is_tabu(step, stamps[v], ten)) ? TABU_BIT : 0u;
                 const uint32_t key = valid ? (young | ((uint32_t)loss << 16) | tie) : 0xffffffffu;
@@ -241,9 +182,9 @@ __global__ void __launch_bounds__(WARPS * 32, 8) sls_h16_kernel(const uint32_t* 
         if (__any_sync(FULL, do_add)) {
             const uint32_t rowmask = (__ballot_sync(FULL, L.U != 0) >> hshift) & 0xffffu;
             const bool adding = do_add && rowmask != 0;   // (rowmask is never empty for an adding chain)
-            const int y = adding ? pick_rotated16(rowmask, hs & 31u) : 0;
+            const int y = adding ? pick_rotated(rowmask, hs & 31u) : 0;
             const uint32_t Urow = __shfl_sync(FULL, L.U, y, 16);
-            const int x = adding ? pick_rotated16(Urow, (hs >> 5) & 31u) : 0;
+            const int x = adding ? pick_rotated(Urow, (hs >> 5) & 31u) : 0;
             const uint2 wt = tab[y * 32 + x];
             const int xoff = min(x, 3);
             // pass 0: cells 0..15, pass 1: cells 16..24
@@ -258,8 +199,8 @@ __global__ void __launch_bounds__(WARPS * 32, 8) sls_h16_kernel(const uint32_t* 
             const uint32_t t0 = tie_add(hs, (uint32_t)row), t1 = tie_add(hs, (uint32_t)(16 + row));
             uint32_t key0, key1;
             if (__any_sync(FULL, adding && !noise)) {
-                const int g0 = score16(L.U, cv0 & 31, cv0 >> 5, tab[cv0]);
-                const int g1 = score16(L.U, cv1 & 31, cv1 >> 5, tab[cv1]);
+                const int g0 = score<16>(L.U, cv0 & 31, cv0 >> 5, tab[cv0]);
+                const int g1 = score<16>(L.U, cv1 & 31, cv1 >> 5, tab[cv1]);
                 const uint32_t f0 = is_tabu(step, stamps[cv0], ten) ? 0u : TABU_BIT, f1 = is_tabu(step, stamps[cv1], ten) ? 0u : TABU_BIT;
                 key0 = noise ? (0x10000u | t0) : (f0 | ((uint32_t)(g0 + 1) << 16) | t0);
                 key1 = noise ? (0x10000u | t1) : (f1 | ((uint32_t)(g1 + 1) << 16) | t1);

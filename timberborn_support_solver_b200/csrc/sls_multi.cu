@@ -169,10 +169,7 @@ __device__ __forceinline__ int remove_min_loss(Lane& L, const Ctx& c, int& k, ui
     return code;
 }
 
-__device__ __forceinline__ int pick_rotated(uint32_t bits, uint32_t o) {
-    uint32_t rot = __funnelshift_r(bits, bits, o);
-    return (int)((__ffs(rot) - 1 + o) & 31u);
-}
+using sls::pick_rotated;
 
 // ONESHOT = the first epoch of a one-shot solve in ONE launch (tss_solve_upper_bound, first-model mode, workspace of the same
 // platform set cached): terrain rows and bound arrive as kernel parameters, chains start empty in registers (no init

@@ -90,6 +90,22 @@ struct ChainState {
 static_assert(sizeof(ChainState) == 288, "ChainState layout");
 
 #if defined(__CUDACC__)
+// The random uncovered tile of an addition: the first set bit of a row mask (then of the row) at or above offset o,
+// wrapping around (bits rotated right by o).
+__device__ __forceinline__ int pick_rotated(uint32_t bits, uint32_t o) {
+    uint32_t rot = __funnelshift_r(bits, bits, o);
+    return (int)((__ffs(rot) - 1 + o) & 31u);
+}
+
+// The 25-tile diamond |dx| + |dy| <= 3 of add candidates around t, cell index i in row-major order: window row r = dy + 3
+// holds cells cell_start(r) .. cell_start(r + 1) - 1.
+__device__ __forceinline__ constexpr int cell_start(int r) { return r <= 4 ? r * r : (r == 5 ? 21 : 24); }
+__device__ __forceinline__ void diamond_cell(int i, int& dx, int& dy) {
+    const int r = (i >= 1) + (i >= 4) + (i >= 9) + (i >= 16) + (i >= 21) + (i >= 24);
+    dy = r - 3;
+    dx = i - cell_start(r) - (3 - abs(dy));
+}
+
 // Reach window of site v = (x, y) on a terrain given as 32 row words: validate()'s three ceiling-masked dilations
 // (src/encoder/platform_layout.rs:127-141) run inside the site's own 7x7 window (geodesic paths of length <= 3 never
 // leave it).  Window row dy is grid row y-3+dy, window column 0 is grid column max(x-3, 0).

@@ -3,27 +3,18 @@
 // ncu on the warp-per-chain kernels (profiles/r1_sls_kernel.md, r1_sls_h16_kernel.md) shows the ALU pipe as the limiter
 // with ~276 warp instructions per chain step, most of them cross-lane plumbing (indexed shuffles to fetch window rows,
 // ballots, min/max butterflies) and per-chain "uniform" work that all lanes of a (half-)warp repeat.  Here a chain is
-// one thread: its bitboards live in shared memory as [row][thread] words (bank = thread, conflict free for any row
-// index), every candidate layout is scored by that thread alone (7 row loads, shift/mask/pack, 2 AND+POPC), there are
-// no shuffles, ballots or reductions in the step loop, and a warp instruction advances 32 layouts.
+// one thread (sls_thread.cuh: the step, the keys, the site list and the removal ring shared with sls_p16.cu): every
+// candidate layout is scored by that thread alone (7 row loads, shift/mask/pack, 2 AND+POPC), there are no shuffles,
+// ballots or reductions in the step loop, and a warp instruction advances 32 layouts.
 //
 // The step rule, RNG and tie-breaks are EXACTLY those of sls_spec.hpp: the parity tests replay this kernel against the
-// same CPU model as sls.cu / sls_h16.cu (bit-identical trajectories).  Implementation choices that differ:
+// same CPU model as sls.cu / sls_h16.cu (bit-identical trajectories).  The representation:
 //   * columns are stored shifted left by 3 and the reach windows re-anchored at x-3 when the table is loaded, so a
 //     window row is always `(row >> x) & 0x7f` (no anchor clamp); the boards sit back to back and a row is one LDS at an
 //     immediate offset from the site's row: rows outside the grid alias a neighbouring board, which is harmless because
 //     they only ever meet zero window bits (reads) or a zero mask (no write);
-//   * the site list lives in global memory as [index][chain] words (coalesced across the warp, L1 resident) and carries
-//     the step at which each support was added — for a current support that IS its last flip, so the "young support"
-//     test of the spec needs no per-site stamp array;
-//   * "recently removed" (the tabu test of add candidates, which are never current supports) is answered from a ring
-//     of the sites removed in the last 32 steps (one slot per step), folded once per step into a 7x7 window mask
-//     around the chosen uncovered tile.  Equivalent to the spec's 16-bit stamps for epochs of at most 32768 steps —
-//     the engine never launches longer ones (tss_search_run splits them).
 //   * add candidates: the 13x13 neighbourhood of the uncovered tile is fetched once into registers; per column offset a
-//     7-bit slab is masked once and the 25 diamond cells are scored with static shifts, packing on the FMA pipe;
-//   * selection keys carry the candidate's index in their low bits, so min / max are single instructions, independent of
-//     the evaluation order, and ties go to the lowest index as the spec demands.
+//     7-bit slab is masked once and the 25 diamond cells are scored with static shifts, packing on the FMA pipe.
 // ncu (profiles/r1_sls_t16_kernel.md): 73 warp instructions per chain step, ALU pipe 75 %, issue slots 72 %, shared-memory
 // wavefronts 17.8 per chain step (a third of them bank-conflict replays of the random 8-byte reach-table reads).
 // r2: windows as one byte per row assembled with PRMT (the per-row `& 0x7f` and the multiply-packs are gone): 73 -> 65 warp
@@ -32,21 +23,14 @@
 // Tried and dropped: the two high count planes in global memory for 4 CTAs per SM (r1: 277 vs 335 G candidates/s; r2, with a
 // per-chain "never carried into them" flag so that they are not even read: 22.2 G flips/s at 3 CTAs, 20.4 G at 4 CTAs vs 24.6 G);
 // skipping their shared-memory loads until some count reaches 8 (326 vs 334 G: the branches cost more than the loads).
-#include "engine.hpp"
-#include "sls_spec.hpp"
+#include "sls_thread.cuh"
 
 namespace tss {
 namespace slst {
 
-using namespace tss::sls;
+using namespace tss::slsth;
 
-constexpr int NT = 128;          // chains per CTA
 constexpr int MAXW = 26;         // 3 + w + 3 <= 32 bits
-constexpr uint32_t NONE = 0xffffu;
-constexpr int TAB_PAD = 128;     // table entries before / after the 512 real ones (candidate sites outside the grid index there)
-// boards, 16 rows each, back to back: rows outside [0, 16) of a board alias its neighbours — harmless, because out-of-grid
-// rows only ever meet zero window bits (reads) or a zero mask (no write)
-enum { B_C0 = 0, B_C1 = 1, B_C2 = 2, B_U = 3, B_O = 4, B_C3 = 5, B_C4 = 6, N_BOARDS = 7 };
 
 struct Smem {
     uint2 tab[512 + 2 * TAB_PAD];          // reach windows of the 16x32 sites, anchored at x-3; entry of site v at v + TAB_PAD
@@ -56,38 +40,7 @@ struct Smem {
 };
 constexpr int BOARD = 16 * NT;             // words between the same row of consecutive boards
 
-// ---- bounds-checked build (-DTSS_CHECKED, profiles/checked_build.py): compute-sanitizer is closed on the B200 pool, and this kernel
-// aliases neighbouring boards on purpose (rows outside the grid), so the claim "every access stays inside the CTA's Smem block,
-// every STORE lands in a row of the grid of the board it means" is checked by the kernel itself: each shared-memory access of the
-// step loop goes through these two functions, violations are counted in a device global (tss_debug_smem_violations()).
-#ifdef TSS_CHECKED
-__device__ unsigned int g_smem_violations = 0;
-__device__ __forceinline__ const uint32_t* chk_ld(const Smem& sm, const uint32_t* p) {
-    const size_t off = (size_t)((const char*)p - (const char*)&sm);
-    if (off + 4 > sizeof(Smem) || (off & 3)) { atomicAdd(&g_smem_violations, 1u); return &sm.rows[0][0]; }
-    return p;
-}
-// a store into row `row` (0..15) of board `board` for thread tid, and nowhere else
-__device__ __forceinline__ uint32_t* chk_st(Smem& sm, uint32_t* p, int board, int tid) {
-    const ptrdiff_t off = p - &sm.rows[board * 16][0];
-    if (off < 0 || off >= 16 * NT || (off % NT) != tid) { atomicAdd(&g_smem_violations, 1u); return &sm.rows[board * 16][tid]; }
-    return p;
-}
-#define LD(p) (*chk_ld(sm, (p)))
-#define ST(p, board) (*chk_st(sm, (p), (board), tid))
-#else
-#define LD(p) (*(p))
-#define ST(p, board) (*(p))
-#endif
-
-__device__ __forceinline__ int pick_rotated(uint32_t bits, uint32_t o) {
-    uint32_t rot = __funnelshift_r(bits, bits, o);
-    return (int)((__ffs(rot) - 1 + o) & 31u);
-}
-
 // adds (ADD) or removes the cover of site v on the five count planes and refreshes U, O and the non-empty-row mask.
-// Branch free: rows of the window without reach bits (m = 0) recompute what is already there; rows outside the grid read
-// a neighbouring board (never written: the stores are predicated on m != 0) and meet C = 0.
 // rowmask is kept in padded coordinates: bit r + 3 = row r has an uncovered tile.
 template <bool ADD>
 __device__ __forceinline__ void flip(Smem& sm, int tid, int v, uint32_t& rowmask) {
@@ -98,45 +51,12 @@ __device__ __forceinline__ void flip(Smem& sm, int tid, int v, uint32_t& rowmask
 #pragma unroll
     for (int j = 0; j < 7; j++) {
         const uint32_t m7 = (j < 4 ? win.x >> (8 * j) : win.y >> (8 * (j - 4))) & 0xffu;
-        const int off = (j - 3) * NT;
-        uint32_t m = m7 << x;
-        uint32_t a0 = LD(p + B_C0 * BOARD + off), a1 = LD(p + B_C1 * BOARD + off), a2 = LD(p + B_C2 * BOARD + off), t;
-        uint32_t a3 = LD(p + B_C3 * BOARD + off), a4 = LD(p + B_C4 * BOARD + off);
-        if (ADD) {
-            t = a0 & m; a0 ^= m; m = t;
-            t = a1 & m; a1 ^= m; m = t;
-            t = a2 & m; a2 ^= m; m = t;
-        } else {
-            t = ~a0 & m; a0 ^= m; m = t;
-            t = ~a1 & m; a1 ^= m; m = t;
-            t = ~a2 & m; a2 ^= m; m = t;
-        }
-        if (m) {  // a count crossing 7 <-> 8: rare
-            if (ADD) { t = a3 & m; a3 ^= m; a4 ^= t; } else { t = ~a3 & m; a3 ^= m; a4 ^= t; }
-            ST(p + B_C3 * BOARD + off, B_C3) = a3; ST(p + B_C4 * BOARD + off, B_C4) = a4;
-        }
-        const uint32_t hi = a1 | a2 | a3 | a4, C = sm.C[y + j];  // C[r + 3] = row r
-        const uint32_t Un = C & ~(a0 | hi);
-        if (m7) {
-            ST(p + B_C0 * BOARD + off, B_C0) = a0; ST(p + B_C1 * BOARD + off, B_C1) = a1; ST(p + B_C2 * BOARD + off, B_C2) = a2;
-            ST(p + B_U * BOARD + off, B_U) = Un;
-            ST(p + B_O * BOARD + off, B_O) = a0 & ~hi & C;
-        }
+        const uint32_t Un = flip_word<ADD, BOARD>(sm, tid, p, (j - 3) * NT, m7 << x, m7, y + j);  // C[r + 3] = row r
         nz |= Un ? 1u << j : 0u;
     }
     rowmask = (rowmask & ~(0x7fu << y)) | (nz << y);
 }
 
-__device__ __forceinline__ uint32_t shl_clamped(uint32_t v, int n) {  // PTX shl: shift counts above 31 (incl. "negative" ones) give 0
-    uint32_t r;
-    asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
-    return r;
-}
-
-__device__ __forceinline__ constexpr int cell_start(int r) { return r <= 4 ? r * r : (r == 5 ? 21 : 24); }   // first diamond cell of window row r
-__device__ __forceinline__ constexpr int iabs(int a) { return a < 0 ? -a : a; }
-__device__ __forceinline__ constexpr int cell_index(int dx, int dy) { return cell_start(dy + 3) + dx + (3 - iabs(dy)); }
-__device__ __forceinline__ uint32_t shift_static(uint32_t v, int s) { return s >= 0 ? v << s : v >> (-s); }
 // low bytes of four / three words as one word (the fourth byte of pack3 is a copy of a's: it only ever meets a zero table byte)
 __device__ __forceinline__ uint32_t pack4(uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
     return __byte_perm(__byte_perm(a, b, 0x0040), __byte_perm(c, d, 0x0040), 0x5410);
@@ -154,224 +74,124 @@ __device__ __noinline__ void list_to_rows(const uint32_t* sl, size_t stride, int
     for (int r = 0; r < 16; r++) out32[r] = rows[r];
 }
 
-// One ADD candidate: the site at offset (DX, DY) from the uncovered tile.  P = the 7-bit column slab of U for this DX
-// (P[j] = columns x+DX-3 .. x+DX+3 of row y-6+j).  Keys are unique per cell (the cell index sits in the low bits), so
-// the maximum is independent of the evaluation order and ties go to the lowest cell as the spec demands.
-template <int DX, int DY>
-__device__ __forceinline__ uint32_t add_key(const Smem& sm, const uint32_t (&P)[13], const uint2* tabt, uint2 wt, uint32_t fresh_lo, uint32_t fresh_hi,
-                                            uint32_t hs, uint32_t gmul) {
-    constexpr int cell = cell_index(DX, DY), bit = 8 * (DY + 3) + DX + 3;   // position in the byte-per-row window (rows 0-3 / 4-6)
-    const uint2 win = tabt[DY * 32 + DX];
-    const uint32_t lo = pack4(P[DY + 3], P[DY + 4], P[DY + 5], P[DY + 6]);
-    const uint32_t hi = pack3(P[DY + 7], P[DY + 8], P[DY + 9]);
-    const uint32_t g = (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
-    const uint32_t tie = ((hs * ((2u * cell + 1u) * K2)) >> 11) & 0x1fffe0u;             // tie_add(hs, cell) << 5
-    const uint32_t fresh = shift_static(bit < 32 ? fresh_lo : fresh_hi, 30 - (bit < 32 ? bit : bit - 32)) & TABU_BIT;  // (all zero in a noise step)
-    const uint32_t key = (fresh | tie) + g * gmul + ((1u << 21) | (31u - cell));   // gmul = 1 << 21, or 0 in a noise step
-    const bool valid = ((bit < 32 ? wt.x >> bit : wt.y >> (bit - 32)) & 1u) != 0;
-    return valid ? key : 0u;
-}
-
-template <int DX>
-__device__ __forceinline__ uint32_t add_column(const Smem& sm, const uint32_t (&R)[13], const uint2* tabt, uint2 wt, uint32_t fresh_lo, uint32_t fresh_hi,
-                                               uint32_t hs, uint32_t gmul) {
-    constexpr int M = 3 - iabs(DX);
-    uint32_t P[13];
+// U around the uncovered tile t = (x, y) of an addition: R[j] = row y-6+j, bit b = tile column b + x - 6
+struct Nbhd {
+    int x, y;
+    const uint2* tabt;   // t's table entry
+    uint2 wt;            // t's window
+    uint32_t R[13];
+    // the 7-bit column slab of U for column offset DX: P[j] = columns x+DX-3 .. x+DX+3 of row y-6+j
+    using Slab = uint32_t[13];
+    template <int DX, int M>
+    __device__ __forceinline__ void slab(Slab& P) const {
 #pragma unroll
-    for (int j = 3 - M; j <= 9 + M; j++) P[j] = R[j] >> (DX + 3);   // (only the low byte is used; its bit 7 meets a zero table bit)
-    uint32_t mx = add_key<DX, 0>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul);
-    if (M >= 1) {
-        mx = max(mx, add_key<DX, (M >= 1 ? -1 : 0)>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-        mx = max(mx, add_key<DX, (M >= 1 ? 1 : 0)>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
+        for (int j = 3 - M; j <= 9 + M; j++) P[j] = R[j] >> (DX + 3);   // (only the low byte is used; its bit 7 meets a zero table bit)
     }
-    if (M >= 2) {
-        mx = max(mx, add_key<DX, (M >= 2 ? -2 : 0)>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-        mx = max(mx, add_key<DX, (M >= 2 ? 2 : 0)>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
+    template <int DY>
+    static __device__ __forceinline__ uint32_t gain(const Slab& P, uint2 win) {
+        const uint32_t lo = pack4(P[DY + 3], P[DY + 4], P[DY + 5], P[DY + 6]);
+        const uint32_t hi = pack3(P[DY + 7], P[DY + 8], P[DY + 9]);
+        return (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
     }
-    if (M >= 3) {
-        mx = max(mx, add_key<DX, (M >= 3 ? -3 : 0)>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-        mx = max(mx, add_key<DX, (M >= 3 ? 3 : 0)>(sm, P, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
+};
+
+// the board representation of sls_t16_kernel for run_chains (sls_thread.cuh)
+struct Rows {
+    using Smem = slst::Smem;
+    Smem& sm;
+    const int tid;
+    uint32_t* const sl;
+    const size_t stride;
+    uint32_t* const Ub;
+    const uint32_t* const Ob;
+
+    __device__ __forceinline__ Rows(Smem& sm, int tid, uint32_t* sl, size_t stride)
+        : sm(sm), tid(tid), sl(sl), stride(stride), Ub(&sm.rows[B_U * 16][tid]), Ob(&sm.rows[B_O * 16][tid]) {}
+
+    static __device__ __forceinline__ void load(Smem& sm, int tid, const uint32_t* terrain_rows, const uint2* rtabs, int terrain) {
+        for (int i = tid; i < 512 + 2 * TAB_PAD; i += NT) {
+            const int v = i - TAB_PAD;
+            uint2 s = make_uint2(0u, 0u);
+            if (v >= 0 && v < 512) {
+                s = rtabs[(size_t)terrain * 1024 + v];
+                const int x = v & 31, sh = x < 3 ? 3 - x : 0;  // table windows are anchored at max(x-3, 0): re-anchor at x-3
+                s = byte_rows(make_uint2(s.x << sh, s.y << sh));
+            }
+            sm.tab[i] = s;
+        }
+        if (tid < 24) sm.C[tid] = (tid >= 3 && tid < 19) ? terrain_rows[(size_t)terrain * 32 + tid - 3] << 3 : 0u;
+#pragma unroll 8
+        for (int r = 0; r < N_BOARDS * 16; r++) sm.rows[r][tid] = 0;
+#pragma unroll
+        for (int r = 0; r < 32; r++) sm.ring[r][tid] = (uint16_t)NONE;
     }
-    return mx;
-}
+
+    __device__ __forceinline__ int start(const uint32_t* S, uint32_t step, uint32_t& rowmask) {
+        int k = 0;
+        const uint32_t reset = (uint32_t)stamp_reset(step) << 16;
+        for (int y = 0; y < 16; y++)
+            for (uint32_t bits = S[y]; bits; bits &= bits - 1) sl[(size_t)(k++) * stride] = (uint32_t)(y * 32 + __ffs(bits) - 1) | reset;
+        for (int r = 0; r < 16; r++) { const uint32_t c = sm.C[r + 3]; Ub[r * NT] = c; rowmask |= c ? 8u << r : 0u; }
+        for (int i = 0; i < k; i++) flip<true>(sm, tid, (int)(sl[(size_t)i * stride] & 0x1ffu), rowmask);
+        return k;
+    }
+
+    __device__ __forceinline__ void remove(uint32_t hs, uint32_t step, uint32_t stephi, uint32_t young_below, int k, uint32_t& rowmask) {
+        uint32_t best_key = 0xffffffffu, mult = K3;                 // mult = (2i+1) * K3
+#pragma unroll 4
+        for (int i = 0; i < k; i++, mult += 2u * K3) {
+            const uint32_t e = sl[(size_t)i * stride];
+            const int v = (int)(e & 0x1ffu), x = v & 31;
+            const uint2 win = sm.tab[v + TAB_PAD];
+            const uint32_t* p = Ob + (v >> 5) * NT;
+            uint32_t r7[7];
+#pragma unroll
+            for (int j = 0; j < 7; j++) r7[j] = ld(sm, p + (j - 3) * NT) >> x;
+            const uint32_t lo = pack4(r7[0], r7[1], r7[2], r7[3]);
+            const uint32_t hi = pack3(r7[4], r7[5], r7[6]);
+            const uint32_t loss = (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
+            best_key = min(best_key, remove_key(e, i, loss, hs * mult, stephi, young_below));
+        }
+        const int best_i = (int)(best_key & 0x1ffu);
+        const int u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
+        sl[(size_t)best_i * stride] = sl[(size_t)(k - 1) * stride];
+        sm.ring[step & 31u][tid] = (uint16_t)u;
+        flip<false>(sm, tid, u, rowmask);
+    }
+
+    __device__ __forceinline__ Nbhd fetch(uint32_t rowmask, uint32_t hs) const {
+        Nbhd N;
+        N.y = pick_rotated(rowmask >> 3, hs & 31u);
+        const uint32_t* Up = Ub + N.y * NT;
+        N.x = pick_rotated(Up[0] >> 3, (hs >> 5) & 31u);
+        N.tabt = &sm.tab[N.y * 32 + N.x + TAB_PAD];
+        N.wt = N.tabt[0];
+#pragma unroll
+        for (int j = 0; j < 13; j++) N.R[j] = (ld(sm, Up + (j - 6) * NT) << 3) >> N.x;
+        return N;
+    }
+
+    __device__ __forceinline__ void add(int v, uint32_t step, int k, uint32_t& rowmask) {
+        flip<true>(sm, tid, v, rowmask);
+        sl[(size_t)k * stride] = (uint32_t)v | (step << 16);
+    }
+
+    __device__ __forceinline__ void list_to_rows(int k, uint32_t* out32) const { slst::list_to_rows(sl, stride, k, out32); }
+};
 
 __global__ void __launch_bounds__(NT, 3) sls_t16_kernel(const uint32_t* __restrict__ terrain_rows, const uint2* __restrict__ rtabs,
                                                        ChainState* __restrict__ states, uint32_t* __restrict__ site_lists, size_t stride,
                                                        int n_chains, int chains_per_terrain, uint32_t chain_offset, uint64_t seed,
                                                        long long steps, const int* __restrict__ bounds, int target, int noise_pct,
                                                        const volatile int* interrupt, unsigned long long* __restrict__ totals) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
-    const int tid = threadIdx.x;
-    const int chain = blockIdx.x * NT + tid;
-    const int terrain = chains_per_terrain > 0 ? (blockIdx.x * NT) / chains_per_terrain : 0;
-    // a layout within the target is already known for this terrain (found in an earlier epoch): nothing to do.  Lets a host
-    // queue several epochs back to back without a round trip in between (one-shot solves, sls_spec.hpp).
-    if (target >= 0 && bounds[chains_per_terrain > 0 ? terrain : 0] <= target) return;
-    for (int i = tid; i < 512 + 2 * TAB_PAD; i += NT) {
-        const int v = i - TAB_PAD;
-        uint2 s = make_uint2(0u, 0u);
-        if (v >= 0 && v < 512) {
-            s = rtabs[(size_t)terrain * 1024 + v];
-            const int x = v & 31, sh = x < 3 ? 3 - x : 0;  // table windows are anchored at max(x-3, 0): re-anchor at x-3
-            s = make_uint2(s.x << sh, s.y << sh);
-            // ... and spread the 7-bit rows to one BYTE per row (rows 0-3 in .x, rows 4-6 in .y): windows cut out of the boards
-            // are then assembled with byte permutes, and bit 7 of every byte (zero here) masks whatever the cut left there
-            s = make_uint2((s.x & 0x7fu) | ((s.x & 0x3f80u) << 1) | ((s.x & 0x1fc000u) << 2) | ((s.x & 0xfe00000u) << 3),
-                           (s.y & 0x7fu) | ((s.y & 0x3f80u) << 1) | ((s.y & 0x1fc000u) << 2));
-        }
-        sm.tab[i] = s;
-    }
-    if (tid < 24) sm.C[tid] = (tid >= 3 && tid < 19) ? terrain_rows[(size_t)terrain * 32 + tid - 3] << 3 : 0u;
-#pragma unroll 8
-    for (int r = 0; r < N_BOARDS * 16; r++) sm.rows[r][tid] = 0;
-#pragma unroll
-    for (int r = 0; r < 32; r++) sm.ring[r][tid] = (uint16_t)NONE;
-    __syncthreads();
-
-    const bool exists = chain < n_chains;
-    ChainState& st = states[exists ? chain : 0];
-    int done = exists ? st.done : 1;
-    const bool run = !done;
-    unsigned long long scored = 0;
-    long long my_steps = 0;
-    uint32_t flips = 0;   // supports added + removed
-
-    if (run) {
-        const int epoch_bound = bounds[chains_per_terrain > 0 ? terrain : 0];
-        const uint32_t base = chain_base(seed, chain_offset + (uint32_t)chain);
-        const uint32_t nq7 = noise_q7(noise_pct);
-        const int tenure = tenure_of(chain_offset + (uint32_t)chain);
-        uint32_t* sl = site_lists + chain;
-        uint32_t* const Ub = &sm.rows[B_U * 16][tid];
-        const uint32_t* const Ob = &sm.rows[B_O * 16][tid];
-        int best = st.best, k = 0;
-        uint32_t step = st.step, rowmask = 0;
-
-        {   // site list in row-major order (spec), stamps "half a period ago"; cover planes from the list
-            const uint32_t reset = (uint32_t)stamp_reset(step) << 16;
-            for (int y = 0; y < 16; y++)
-                for (uint32_t bits = st.S[y]; bits; bits &= bits - 1) sl[(size_t)(k++) * stride] = (uint32_t)(y * 32 + __ffs(bits) - 1) | reset;
-            for (int r = 0; r < 16; r++) { const uint32_t c = sm.C[r + 3]; Ub[r * NT] = c; rowmask |= c ? 8u << r : 0u; }
-            for (int i = 0; i < k; i++) flip<true>(sm, tid, (int)(sl[(size_t)i * stride] & 0x1ffu), rowmask);
-        }
-
-        for (long long it = 0; it < steps; it++) {
-            if ((it & 1023) == 1023 && *interrupt) break;
-            const int limit = min(epoch_bound, best);
-            const uint32_t hs = step_hash(base, step);
-            const int ten = effective_tenure(tenure, k);
-            const bool drop = k >= limit;
-            if (drop && k == 0) { done = 1; break; }
-            sm.ring[step & 31u][tid] = (uint16_t)NONE;  // every consumed step owns its slot (stale entries are 32 steps old)
-            if (!drop && rowmask == 0) {  // complete layout with k < limit supports
-                best = k;
-                list_to_rows(sl, stride, k, st.bestS);
-                step++; my_steps++;
-                if (k <= target || k == 0) { done = 1; break; }
-                continue;
-            }
-            if (drop || (k == limit - 1 && k > 0)) {
-                // ---- removal: min-loss support, random ties; supports younger than the tenure only as a last resort (not when
-                // dropping).  key = young | loss | tie | list index: unique, so the minimum is the spec's (lowest index wins ties)
-                const uint32_t stephi = (step << 16) | 0xffffu;             // stephi - entry = (age << 16) + (0xffff - site): no borrow
-                const uint32_t young_below = drop ? 0u : (uint32_t)ten << 16;
-                uint32_t best_key = 0xffffffffu, mult = K3;                 // mult = (2i+1) * K3
-#pragma unroll 4
-                for (int i = 0; i < k; i++, mult += 2u * K3) {
-                    const uint32_t e = sl[(size_t)i * stride];
-                    const int v = (int)(e & 0x1ffu), x = v & 31;
-                    const uint2 win = sm.tab[v + TAB_PAD];
-                    const uint32_t* p = Ob + (v >> 5) * NT;
-                    uint32_t r7[7];
-#pragma unroll
-                    for (int j = 0; j < 7; j++) r7[j] = LD(p + (j - 3) * NT) >> x;
-                    const uint32_t lo = pack4(r7[0], r7[1], r7[2], r7[3]);
-                    const uint32_t hi = pack3(r7[4], r7[5], r7[6]);
-                    const uint32_t loss = (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
-                    const uint32_t tie = ((hs * mult) >> 7) & 0x1fffe00u;  // tie_remove(hs, i) << 9
-                    const uint32_t young = (stephi - e) < young_below ? TABU_BIT : 0u;
-                    best_key = min(best_key, (young | tie | (uint32_t)i) + loss * (1u << 25));
-                }
-                const int best_i = (int)(best_key & 0x1ffu);
-                const int u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
-                const uint32_t last = sl[(size_t)(k - 1) * stride];
-                sl[(size_t)best_i * stride] = last;
-                sm.ring[step & 31u][tid] = (uint16_t)u;
-                flip<false>(sm, tid, u, rowmask);
-                scored += (unsigned)k;
-                k--;
-                flips++;
-            }
-            if (!drop) {
-                // ---- addition at a random uncovered tile t: best-gain site of R(t)
-                const int y = pick_rotated(rowmask >> 3, hs & 31u);
-                const uint32_t* Up = Ub + y * NT;
-                const int x = pick_rotated(Up[0] >> 3, (hs >> 5) & 31u);
-                const uint2* tabt = &sm.tab[y * 32 + x + TAB_PAD];
-                const uint2 wt = tabt[0];
-                uint32_t R[13];  // rows y-6 .. y+6 of U; bit b of R[j] = tile column b + x - 6
-#pragma unroll
-                for (int j = 0; j < 13; j++) R[j] = (LD(Up + (j - 6) * NT) << 3) >> x;
-                const bool noise = ((hs >> 10) & 127u) < nq7;
-                uint32_t tw_lo = 0, tw_hi = 0;  // sites removed fewer than `ten` steps ago, as a byte-per-row window around t (rows 0-3 / 4-6)
-                for (int j = 0; j < ten; j++) {
-                    const uint32_t e = sm.ring[(step - (uint32_t)j) & 31u][tid];
-                    const int dx3 = (int)(e & 31u) - x + 3, dy3 = (int)(e >> 5) - y + 3;
-                    if ((unsigned)dx3 < 7u && (unsigned)dy3 < 7u) {
-                        const int bit = 8 * dy3 + dx3;       // byte-per-row window, like the reach table
-                        tw_lo |= shl_clamped(1u, bit);
-                        tw_hi |= shl_clamped(1u, bit - 32);
-                    }
-                }
-                const uint32_t fresh_lo = noise ? 0u : ~tw_lo, fresh_hi = noise ? 0u : ~tw_hi;
-                const uint32_t gmul = noise ? 0u : 1u << 21;
-                uint32_t mx = add_column<0>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul);
-                mx = max(mx, add_column<-1>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-                mx = max(mx, add_column<1>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-                mx = max(mx, add_column<-2>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-                mx = max(mx, add_column<2>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-                mx = max(mx, add_column<-3>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-                mx = max(mx, add_column<3>(sm, R, tabt, wt, fresh_lo, fresh_hi, hs, gmul));
-                // the winning cell from the key's low bits
-                const int cell = 31 - (int)(mx & 31u);
-                const int r = (cell >= 1) + (cell >= 4) + (cell >= 9) + (cell >= 16) + (cell >= 21) + (cell >= 24);
-                const int dy = r - 3, dx = cell - cell_start(r) - (3 - abs(dy));
-                const int v = (y + dy) * 32 + x + dx;
-                flip<true>(sm, tid, v, rowmask);
-                sl[(size_t)k * stride] = (uint32_t)v | (step << 16);
-                if (!noise) scored += (unsigned)(__popc(wt.x) + __popc(wt.y));
-                k++;
-                flips++;
-            }
-            step++; my_steps++;
-        }
-
-        list_to_rows(sl, stride, k, st.S);
-        st.k = k; st.best = best; st.step = step; st.done = done;
-        const unsigned long long tot = ((unsigned long long)st.scored_hi << 32 | st.scored_lo) + scored;
-        st.scored_lo = (uint32_t)tot; st.scored_hi = (uint32_t)(tot >> 32);
-        st.steps_done += (uint32_t)my_steps;
-    }
-    // one pair of atomics per warp
-    unsigned long long a = scored, b = (unsigned long long)my_steps, c = (unsigned long long)flips;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { a += __shfl_xor_sync(0xffffffffu, a, o); b += __shfl_xor_sync(0xffffffffu, b, o); c += __shfl_xor_sync(0xffffffffu, c, o); }
-    if ((tid & 31) == 0 && (a | b)) { atomicAdd(&totals[0], a); atomicAdd(&totals[1], b); atomicAdd(&totals[2], c); }
+    run_chains<Rows>(threadIdx.x, terrain_rows, rtabs, states, site_lists, stride, n_chains, chains_per_terrain, chain_offset, seed, steps, bounds, target,
+                     noise_pct, interrupt, totals);
 }
 
 }  // namespace slst
 
 // violations counted by a -DTSS_CHECKED build since the library was loaded (always 0 in the shipped build, which has no checks)
-int sls_t16_smem_violations() {
-#ifdef TSS_CHECKED
-    unsigned int v = 0;
-    if (cudaMemcpyFromSymbol(&v, slst::g_smem_violations, sizeof v) != cudaSuccess) return -1;
-    return (int)v;
-#else
-    return 0;
-#endif
-}
+int sls_t16_smem_violations() { return slst::smem_violations(); }
 int sls_t16_checked_build() {
 #ifdef TSS_CHECKED
     return 1;
@@ -380,22 +200,14 @@ int sls_t16_checked_build() {
 #endif
 }
 bool sls_t16_fits(int w, int h) { return h <= 16 && w <= slst::MAXW; }
-int sls_t16_cta_chains() { return slst::NT; }
+int sls_thread_cta_chains() { return slsth::NT; }
 size_t sls_t16_list_words(int n_chains) { return (size_t)16 * slst::MAXW * (((size_t)n_chains + 31) & ~(size_t)31); }
 
 int sls_run_t16(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, sls::ChainState* states, uint32_t* site_lists, int n_chains,
                 int chains_per_terrain, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev, int target,
                 int noise_pct, unsigned long long* totals_dev) {
-    // (idempotent and cheap; several engines / host threads may get here at once, so no "already set" cache)
-    TSS_CUDA(e, cudaFuncSetAttribute(slst::sls_t16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(slst::Smem)));
-    const size_t stride = ((size_t)n_chains + 31) & ~(size_t)31;
-    const int blocks = (n_chains + slst::NT - 1) / slst::NT;
-    slst::sls_t16_kernel<<<blocks, slst::NT, sizeof(slst::Smem), e->stream>>>(rows_dev, tabs_dev, states, site_lists, stride, n_chains,
-                                                                             chains_per_terrain, chain_offset, seed, steps, bounds_dev, target,
-                                                                             noise_pct, e->interrupt_dev, totals_dev);
-    TSS_CHECK_LAUNCH(e);
-    e->stats.kernel_launches++;
-    return TSS_OK;
+    return slsth::launch(slst::sls_t16_kernel, sizeof(slst::Smem), e, rows_dev, tabs_dev, states, site_lists, n_chains, chains_per_terrain,
+                         chain_offset, seed, steps, bounds_dev, target, noise_pct, totals_dev);
 }
 
 }  // namespace tss
