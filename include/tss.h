@@ -204,7 +204,8 @@ typedef struct tss_search_params {
     int32_t n_chains;      /* independent layouts searched in parallel (one per warp); 0 = fill the device */
     int32_t chain_offset;  /* global index of this engine's first chain (rank * n_chains in a multi-GPU portfolio) */
     int32_t noise_pct;     /* probability (percent) of a random instead of greedy add move; < 0 = default */
-    int32_t kernel;        /* TSS_KERNEL_*: which of the equivalent SLS kernels runs (same step rule, same trajectories); 0 = auto */
+    int32_t kernel;        /* TSS_KERNEL_*: which of the equivalent SLS kernels runs (same step rule, same trajectories); 0 = auto.
+                            * TSS_KERNEL_WINDOW_PLACEMENTS selects a different search on grids larger than 32x32 (see there) */
 } tss_search_params;
 
 /* SLS kernel variants for grids up to 32x32 with 1x1 supports.  All four execute the published step rule bit for bit
@@ -214,6 +215,14 @@ typedef struct tss_search_params {
 #define TSS_KERNEL_HALF_WARP 2 /* two chains per warp, grids of at most 16 rows */
 #define TSS_KERNEL_THREAD 3    /* one chain per thread, grids of at most 16 rows x 26 columns */
 #define TSS_KERNEL_PAIR 4      /* one chain per thread, two grid rows per word, grids of at most 16x16 */
+/* The window-decomposed placement search: grids wider or taller than 32 with a platform set beyond {1x1} (at most 16 dims
+ * keys, each at most 6x6), on one rank.  The global layout starts as the greedy placement cover and only improves: each
+ * tss_search_run phase (MAX_EPOCH_STEPS steps at most, longer runs are several phases) runs the placement search on 32x32
+ * windows with the platforms near window borders frozen, and keeps each window's best (its target_count is not used:
+ * the windows search without a target).  n_chains = chains per window
+ * (rounded up to a multiple of 4; 0 = 8..16).  Otherwise (AUTO) those grids run the 1x1 window decomposition with a
+ * host post-pass.  tss_search_create answers TSS_E_UNSUPPORTED where it does not apply. */
+#define TSS_KERNEL_WINDOW_PLACEMENTS 5
 
 /* Creates a portfolio on one terrain.  defs must contain 1x1 (encoder.rs:564-566). */
 int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
@@ -230,11 +239,12 @@ int tss_search_set_bound(tss_search* s, int32_t count);
 /* The bound the next epoch searches below: min(best counts of this search, bounds set from outside, and — with a
  * communicator on the engine — the best counts of every rank's search); -1 if none yet.  (synchronises the stream) */
 int tss_search_global_best(tss_search* s, int32_t* count);
-/* Best layout (re-validated by kernel (a) before it is returned). */
+/* Best layout (re-validated by kernel (a) before it is returned).  TSS_KERNEL_WINDOW_PLACEMENTS: the global layout, before
+ * the first run the start layout (the greedy placement cover). */
 int tss_search_best_layout(tss_search* s, tss_platform* out, int32_t cap, int32_t* n_out);
 int tss_search_n_chains(const tss_search* s);
-/* Which TSS_KERNEL_* variant advances this portfolio (what TSS_KERNEL_AUTO resolved to); 0 for the window-decomposed and the
- * placement search, which have a single kernel each. */
+/* Which TSS_KERNEL_* variant advances this portfolio (what TSS_KERNEL_AUTO resolved to); 0 for the 1x1 window decomposition
+ * and the placement search, which have a single kernel each; TSS_KERNEL_WINDOW_PLACEMENTS for that search. */
 int tss_search_kernel(const tss_search* s);
 /* Introspection for the parity tests (the CPU model in oracle/sls_model.cpp replays the same trajectories): per-chain
  * state after the last epoch.  S / best_S: support rows u32[n_chains][32]; any pointer may be NULL. */
@@ -253,7 +263,8 @@ int tss_search_write_chains(tss_search* s, const uint32_t* S);
 /* GUI objective (crates/gui/src/app.rs:53-62,235-245): minimise PlatformLayout::total_weight (platform_layout.rs:174-183)
  * instead of the platform count.  weights = records (def_w, def_h, weight) keyed by canonical def dims, exactly the
  * PlatformLimits.weights map; call before the first tss_search_run.  Afterwards tss_search_best_count /
- * tss_search_set_bound speak total weight.  Needs a platform set beyond {1x1} on a grid up to 32x32. */
+ * tss_search_set_bound speak total weight.  Needs a platform set beyond {1x1} on a grid up to 32x32, or a search created
+ * with TSS_KERNEL_WINDOW_PLACEMENTS. */
 int tss_search_set_weights(tss_search* s, const int32_t* weights, int32_t n_weights);
 
 /* Values of the SLS specification's hash / tie-break functions (csrc/sls_spec.hpp) at fixed probe points, so the

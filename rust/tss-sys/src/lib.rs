@@ -13,6 +13,7 @@ pub const TSS_KERNEL_WARP: i32 = 1; // one chain per warp, any grid up to 32x32
 pub const TSS_KERNEL_HALF_WARP: i32 = 2; // two chains per warp, grids of at most 16 rows
 pub const TSS_KERNEL_THREAD: i32 = 3; // one chain per thread, grids of at most 16 rows x 26 columns
 pub const TSS_KERNEL_PAIR: i32 = 4; // one chain per thread, two grid rows per word, grids of at most 16x16
+pub const TSS_KERNEL_WINDOW_PLACEMENTS: i32 = 5; // window-decomposed placement search, grids larger than 32x32
 
 #[repr(C)]
 #[derive(Copy, Clone, Default, Debug, PartialEq, Eq)]

@@ -5,7 +5,7 @@ library's interface for the feasibility-and-bound path, bound to it through ctyp
 the built library; creating an Engine needs a CUDA device.  There is no CPU fallback.
 """
 from ._lib import LIB_PATH, SIGNATURES, load  # noqa: F401
-from .api import (INTERRUPTED, KERNEL_AUTO, KERNEL_HALF_WARP, KERNEL_PAIR, KERNEL_THREAD, KERNEL_WARP, PLATFORMS_DEFAULT, SAT, UNSAT, Cnf, DeviceCnf, Encoding, EncodingVars, Engine,  # noqa: F401
+from .api import (INTERRUPTED, KERNEL_AUTO, KERNEL_HALF_WARP, KERNEL_PAIR, KERNEL_THREAD, KERNEL_WARP, KERNEL_WINDOW_PLACEMENTS, PLATFORMS_DEFAULT, SAT, UNSAT, Cnf, DeviceCnf, Encoding, EncodingVars, Engine,  # noqa: F401
                   GpuBoundSolver, Platform, PlatformDef, PlatformLayout, PlatformLimits, Project, Search, TssError,
                   ValidationResult, World, WorldGrid, render_world, solver_loop, weight_loop)
 

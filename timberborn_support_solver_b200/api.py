@@ -25,6 +25,7 @@ from ._lib import Platform as _Platform
 
 SAT, UNSAT, INTERRUPTED = "Sat", "Unsat", "Interrupted"  # rustsat SolverResult
 KERNEL_AUTO, KERNEL_WARP, KERNEL_HALF_WARP, KERNEL_THREAD, KERNEL_PAIR = 0, 1, 2, 3, 4  # tss.h TSS_KERNEL_*: equivalent SLS kernels
+KERNEL_WINDOW_PLACEMENTS = 5  # tss.h: the window-decomposed placement search on grids larger than 32x32
 
 
 class TssError(RuntimeError):
@@ -440,7 +441,9 @@ class Search:
 
     def __init__(self, engine: "Engine", grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], seed=0, n_chains=0, chain_offset=0, noise_pct=-1, kernel=0):
         """kernel: KERNEL_AUTO / KERNEL_WARP / KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR (tss.h TSS_KERNEL_*): equivalent SLS kernels
-        (KERNEL_PAIR: one chain per thread with two grid rows per word, grids of at most 16x16)."""
+        (KERNEL_PAIR: one chain per thread with two grid rows per word, grids of at most 16x16).  KERNEL_WINDOW_PLACEMENTS: the
+        window-decomposed placement search on grids larger than 32x32 with platforms beyond 1x1 (n_chains = chains per window); each
+        run() is a phase that can only improve the global layout, best_layout() returns it (before the first run: the greedy cover)."""
         self.engine, self.grid = engine, grid
         self._h = C.c_void_p()
         params = _lib.SearchParams(seed, n_chains, chain_offset, noise_pct, kernel)
@@ -628,7 +631,8 @@ class Engine:
     # ---- kernel (b)
     def search(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], **kw) -> Search:
         """A device-resident SLS portfolio; kw: seed, n_chains, chain_offset, noise_pct, kernel (KERNEL_AUTO, or one of KERNEL_WARP /
-        KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR to pin a variant; a variant that does not fit the grid raises TssError)."""
+        KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR to pin a variant, or KERNEL_WINDOW_PLACEMENTS for the placement search on
+        grids larger than 32x32; a kernel that does not fit the grid or platform set raises TssError)."""
         return Search(self, grid, defs, **kw)
 
     def solve_upper_bound(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], card_limit: Optional[int] = None, seed=0, budget_ms=0, max_steps=0):

@@ -60,6 +60,17 @@ int lns_layout(tss_engine* e, LnsSearch* s, std::vector<uint32_t>& rows);
 int lns_count(const LnsSearch* s);
 unsigned long long lns_total(const LnsSearch* s, int i);
 int lns_chains(const LnsSearch* s);
+// lns_placements.cu — window-decomposed placement search for grids larger than 32x32 (TSS_KERNEL_WINDOW_PLACEMENTS)
+struct LnspSearch;
+int lnsp_create(tss_engine* e, const uint8_t* grid, int w, int h, const uint8_t* anchors, const int2* keys_dev, const int* costs_dev, const int* order_dev,
+                int n_keys, int seeds, uint64_t seed, uint32_t chain_offset, int noise, LnspSearch** out);
+void lnsp_destroy(LnspSearch* s);
+int lnsp_phase(tss_engine* e, LnspSearch* s, long long steps);
+int lnsp_objective(tss_engine* e, LnspSearch* s);
+int lnsp_anchors(tss_engine* e, LnspSearch* s, std::vector<uint8_t>& anchors);
+int lnsp_value(const LnspSearch* s);
+unsigned long long lnsp_total(const LnspSearch* s, int i);
+int lnsp_chains(const LnspSearch* s);
 // sls_multi.cu — placements of several platform types
 size_t slsm_state_bytes();
 int slsm_max_keys();
@@ -181,6 +192,7 @@ struct tss_search {
     bool share = false;                        // all-reduce-min the bound over the engine's communicator after every epoch
     int cap_terrains = 0, cap_chains = 0;      // allocated capacity of a batch workspace (tss_solve_batch reuses it)
     tss::LnsSearch* lns = nullptr;             // grids larger than 32x32: window decomposition (lns.cu)
+    tss::LnspSearch* lnsp = nullptr;           // ... with TSS_KERNEL_WINDOW_PLACEMENTS: over placements (lns_placements.cu, keys_dev / costs_dev below)
     int external_bound = tss::sls::NO_BOUND;
     // platform sets beyond {1x1} on grids up to 32x32: placement search (sls_multi.cu)
     bool multi = false;
@@ -557,6 +569,7 @@ int tss_layout_to_assignment_impl(tss_engine* e, const Encoding& enc, const uint
 static void search_free(tss_search* s) {
     if (!s) return;
     if (s->lns) lns_destroy(s->lns);
+    if (s->lnsp) lnsp_destroy(s->lnsp);
     cudaFree(s->keys_dev);
     cudaFree(s->costs_dev);
     cudaFree(s->mstates);
@@ -625,6 +638,16 @@ static void build_keys(const tss_dims* defs, int n_defs, std::vector<int2>& key_
         }
 }
 
+// keys by area, largest first (stable): the second candidate pass of the placement search draws from the front
+static std::vector<int> keys_by_area(const std::vector<int2>& key_dims) {
+    std::vector<int> order(key_dims.size());
+    for (size_t i = 0; i < order.size(); i++) order[i] = (int)i;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return key_dims[a].x * key_dims[a].y > key_dims[b].x * key_dims[b].y; });
+    return order;
+}
+
+static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds);
+
 // Chains that fill the device: 32 warps per SM for the warp kernels (two chains per warp on grids of <= 16 rows),
 // 3 CTAs of 128 threads per SM for the thread-per-chain kernels.
 static int default_chains(const tss_engine* e, int w, int h, int kernel) {
@@ -662,6 +685,12 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
         int fill = (e->prop.multiProcessorCount * 32 / n_win) / 4 * 4;
         fill = fill < 8 ? 8 : (fill > 16 ? 16 : fill);
         int seeds = (params && params->n_chains > 0) ? ((params->n_chains + 3) / 4) * 4 : fill;
+        if (params && params->kernel == TSS_KERNEL_WINDOW_PLACEMENTS) {
+            int rc = window_placements_create(e, s, defs, n_defs, seeds);
+            if (rc != TSS_OK) { search_free(s); return rc; }
+            *out = s;
+            return TSS_OK;
+        }
         int rc = lns_create(e, grid, w, h, seeds, s->seed, s->chain_offset, s->noise, &s->lns);
         if (rc != TSS_OK) { delete s; return rc; }
         build_keys(defs, n_defs, s->key_dims, s->key_proto);   // (platform sets beyond {1x1}: the 1x1 layout is merged afterwards, merge_supports)
@@ -676,6 +705,8 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
         (s->kernel == TSS_KERNEL_THREAD && !sls_t16_fits(w, h)) || (s->kernel == TSS_KERNEL_PAIR && !sls_p16_fits(w, h))) {
         int k = s->kernel;
         delete s;
+        if (k == TSS_KERNEL_WINDOW_PLACEMENTS)
+            return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: the window placement search needs a grid wider or taller than 32 (got %dx%d)", w, h);
         return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: kernel variant %d does not support a %dx%d grid", k, w, h);
     }
     s->n_chains = (params && params->n_chains > 0) ? params->n_chains : default_chains(e, w, h, s->kernel);
@@ -732,9 +763,7 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
         if (err == cudaSuccess) err = cudaMemcpyAsync(s->rows_dev, rows, sizeof rows, cudaMemcpyHostToDevice, e->stream);
         if (err == cudaSuccess) err = cudaMemcpyAsync(s->keys_dev, s->key_dims.data(), sizeof(int2) * s->key_dims.size(), cudaMemcpyHostToDevice, e->stream);
         if (err == cudaSuccess) err = cudaMemcpyAsync(s->costs_dev, s->key_costs.data(), sizeof(int) * s->key_costs.size(), cudaMemcpyHostToDevice, e->stream);
-        std::vector<int> order(s->key_dims.size());   // keys by area, largest first (stable): the second candidate pass draws from the front
-        for (size_t i = 0; i < order.size(); i++) order[i] = (int)i;
-        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return s->key_dims[a].x * s->key_dims[a].y > s->key_dims[b].x * s->key_dims[b].y; });
+        const std::vector<int> order = keys_by_area(s->key_dims);
         if (err == cudaSuccess) err = cudaMemcpyAsync(s->costs_dev + slsm_max_keys(), order.data(), sizeof(int) * order.size(), cudaMemcpyHostToDevice, e->stream);
         if (err == cudaSuccess) err = cudaMemcpyAsync(s->bounds_dev, &nb, sizeof nb, cudaMemcpyHostToDevice, e->stream);
         if (err == cudaSuccess) err = cudaMemsetAsync(s->totals_dev, 0, sizeof(unsigned long long) * 3, e->stream);
@@ -790,7 +819,9 @@ static int search_kernel(const tss_search* s) {
     return h16_ok ? TSS_KERNEL_HALF_WARP : TSS_KERNEL_WARP;
 }
 
-int tss_search_kernel(const tss_search* s) { return !s ? TSS_E_INVALID : ((s->lns || s->multi) ? 0 : search_kernel(s)); }
+int tss_search_kernel(const tss_search* s) {
+    return !s ? TSS_E_INVALID : (s->lnsp ? TSS_KERNEL_WINDOW_PLACEMENTS : ((s->lns || s->multi) ? 0 : search_kernel(s)));
+}
 
 int tss_search_run(tss_search* s, int64_t steps, int32_t target_count) {
     if (!s) return TSS_E_INVALID;
@@ -798,9 +829,10 @@ int tss_search_run(tss_search* s, int64_t steps, int32_t target_count) {
     if (steps <= 0) return e->fail(TSS_E_INVALID, "tss_search_run: steps must be positive");
     TSS_CUDA(e, cudaSetDevice(e->device));
     TSS_CUDA(e, cudaEventRecord(e->ev0, e->stream));
-    if (s->lns) {  // one phase of the window decomposition (a phase is one epoch per window: at most MAX_EPOCH_STEPS, see below)
+    if (s->lns || s->lnsp) {  // one phase of the window decomposition (a phase is one epoch per window: at most MAX_EPOCH_STEPS, see below)
         for (long long left = steps; left > 0; left -= sls::MAX_EPOCH_STEPS) {
-            int rc = lns_phase(e, s->lns, left < sls::MAX_EPOCH_STEPS ? left : sls::MAX_EPOCH_STEPS, s->share);
+            const long long chunk = left < sls::MAX_EPOCH_STEPS ? left : sls::MAX_EPOCH_STEPS;
+            int rc = s->lns ? lns_phase(e, s->lns, chunk, s->share) : lnsp_phase(e, s->lnsp, chunk);
             if (rc) return rc;
         }
         TSS_CUDA(e, cudaEventRecord(e->ev1, e->stream));
@@ -863,8 +895,8 @@ static int search_sync(tss_search* s) {
         e->stats.device_ms = ms;
         s->timed = false;
     }
-    const unsigned long long t0 = s->lns ? lns_total(s->lns, 0) : s->totals_host[0], t1 = s->lns ? lns_total(s->lns, 1) : s->totals_host[1];
-    const unsigned long long t2 = s->lns ? lns_total(s->lns, 2) : s->totals_host[2];
+    auto total = [s](int i) { return s->lns ? lns_total(s->lns, i) : (s->lnsp ? lnsp_total(s->lnsp, i) : s->totals_host[i]); };
+    const unsigned long long t0 = total(0), t1 = total(1), t2 = total(2);
     e->stats.candidates_scored += t0 - s->totals_seen[0];
     e->stats.sls_steps += t1 - s->totals_seen[1];
     e->stats.sls_flips += t2 - s->totals_seen[2];
@@ -879,8 +911,8 @@ int tss_search_best_count(tss_search* s, int32_t* count) {
     if (!s || !count) return TSS_E_INVALID;
     int rc = search_sync(s);
     if (rc) return rc;
-    if (s->lns) {  // the global layout is always complete; a bound given from outside hides counts that do not beat it
-        int c = lns_count(s->lns);
+    if (s->lns || s->lnsp) {  // the global layout is always complete; a bound given from outside hides counts that do not beat it
+        int c = s->lns ? lns_count(s->lns) : lnsp_value(s->lnsp);
         *count = c < s->external_bound ? c : -1;
         s->e->stats.best_count = *count;
         return TSS_OK;
@@ -897,7 +929,7 @@ int tss_search_global_best(tss_search* s, int32_t* count) {
     tss_engine* e = s->e;
     int rc = search_sync(s);
     if (rc) return rc;
-    if (s->lns) return tss_search_best_count(s, count);
+    if (s->lns || s->lnsp) return tss_search_best_count(s, count);
     int b = sls::NO_BOUND;
     TSS_CUDA(e, cudaMemcpy(&b, s->bounds_dev, sizeof(int), cudaMemcpyDeviceToHost));
     *count = b >= sls::NO_BOUND ? -1 : b;
@@ -910,7 +942,7 @@ int tss_search_set_bound(tss_search* s, int32_t count) {
     if (count < 0) return e->fail(TSS_E_INVALID, "tss_search_set_bound: negative bound");
     int rc = search_sync(s);
     if (rc) return rc;
-    if (s->lns) { s->external_bound = count < s->external_bound ? count : s->external_bound; return TSS_OK; }
+    if (s->lns || s->lnsp) { s->external_bound = count < s->external_bound ? count : s->external_bound; return TSS_OK; }
     TSS_CUDA(e, cudaSetDevice(e->device));
     bound_min_kernel<<<(s->n_groups + 255) / 256, 256, 0, e->stream>>>(s->bounds_dev, s->n_groups, count, false);   // in-stream, before the next epoch
     TSS_CHECK_LAUNCH(e);
@@ -922,7 +954,7 @@ int tss_search_set_bound(tss_search* s, int32_t count) {
 int tss_search_read_chains(tss_search* s, uint32_t* S, uint32_t* best_S, int32_t* k, int32_t* best, uint32_t* step, uint64_t* scored) {
     if (!s) return TSS_E_INVALID;
     tss_engine* e = s->e;
-    if (s->lns || s->multi) return e->fail(TSS_E_UNSUPPORTED, "tss_search_read_chains: only the 1x1 search on grids up to 32x32 exposes per-chain state");
+    if (s->lns || s->lnsp || s->multi) return e->fail(TSS_E_UNSUPPORTED, "tss_search_read_chains: only the 1x1 search on grids up to 32x32 exposes per-chain state");
     int rc = search_sync(s);
     if (rc) return rc;
     std::vector<sls::ChainState> st((size_t)s->n_chains);
@@ -955,7 +987,7 @@ int tss_search_write_chains(tss_search* s, const uint32_t* S) {
     if (!s) return TSS_E_INVALID;
     tss_engine* e = s->e;
     if (!S) return e->fail(TSS_E_INVALID, "tss_search_write_chains: null layout");
-    if (s->lns || s->multi) return e->fail(TSS_E_UNSUPPORTED, "tss_search_write_chains: only the 1x1 search on grids up to 32x32 takes a warm start");
+    if (s->lns || s->lnsp || s->multi) return e->fail(TSS_E_UNSUPPORTED, "tss_search_write_chains: only the 1x1 search on grids up to 32x32 takes a warm start");
     int rc = search_sync(s);
     if (rc) return rc;
     const uint32_t colmask = s->w >= 32 ? 0xffffffffu : ((1u << s->w) - 1u);
@@ -1085,6 +1117,61 @@ static void merge_supports(int w, int h, const std::vector<int2>& key_dims, cons
     plats.swap(merged);
 }
 
+// The greedy placement cover of the terrain (greedy.cu) as platforms, redundant ones pruned (platform sets of at most 16 dims
+// keys, each at most 6x6).  greedy.cu emits placements in the order its threads finish and prune_redundant keeps the first of
+// equally large redundant platforms, so `anchor_order` sorts the placements row-major first: the same layout on every run.
+static int greedy_layout(tss_engine* e, const tss_search* s, bool anchor_order, std::vector<tss_platform>& out) {
+    BitGrid bg = BitGrid::from_bytes(s->grid.data(), s->w, s->h);
+    std::vector<int4> placed;
+    int rc = greedy_cover(e, bg.rows.data(), s->w, s->h, s->key_dims, placed);
+    if (rc) return rc;
+    if (anchor_order) std::sort(placed.begin(), placed.end(), [](const int4& a, const int4& b) { return a.y != b.y ? a.y < b.y : a.x < b.x; });
+    out.clear();
+    for (auto& q : placed) {
+        tss_platform pl = s->key_proto[(size_t)q.z];
+        pl.x = q.x; pl.y = q.y;
+        out.push_back(pl);
+    }
+    prune_redundant(s->grid, s->w, s->h, out);
+    return TSS_OK;
+}
+
+// TSS_KERNEL_WINDOW_PLACEMENTS on a grid larger than 32x32: dims keys, costs and the start layout — the greedy placement cover,
+// redundant platforms pruned, as an anchor grid — on the device, then the search (lns_placements.cu).  seeds = chains per window.
+static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds) {
+    build_keys(defs, n_defs, s->key_dims, s->key_proto);
+    bool fits = s->key_dims.size() > 1 && (int)s->key_dims.size() <= slsm_max_keys();
+    for (auto& kd : s->key_dims) fits = fits && kd.x <= 6 && kd.y <= 6;
+    if (!fits)
+        return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: the window placement search needs a platform set beyond {1x1} with at most %d dims keys, each at most 6x6",
+                       slsm_max_keys());
+    if (e->comm && comm_world(e->comm) > 1) return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: the window placement search runs on a single rank");
+    s->kernel = TSS_KERNEL_WINDOW_PLACEMENTS;
+    s->key_costs.assign(s->key_dims.size(), 1);
+    std::vector<tss_platform> start;
+    int rc = greedy_layout(e, s, true, start);
+    if (rc) return rc;
+    std::vector<uint8_t> anchors((size_t)s->w * s->h, 0);
+    for (auto& p : start) {
+        const Dims d = platform_dims(p);
+        for (size_t k = 0; k < s->key_dims.size(); k++)
+            if (s->key_dims[k].x == d.w && s->key_dims[k].y == d.h) anchors[(size_t)p.y * s->w + p.x] = (uint8_t)(k + 1);
+    }
+    const std::vector<int> order = keys_by_area(s->key_dims);
+    const size_t nk = s->key_dims.size();
+    cudaError_t err = cudaMalloc(&s->keys_dev, sizeof(int2) * (size_t)slsm_max_keys());
+    if (err == cudaSuccess) err = cudaMalloc(&s->costs_dev, sizeof(int) * 2 * (size_t)slsm_max_keys());   // costs | keys ordered by area
+    if (err == cudaSuccess) err = cudaMemcpy(s->keys_dev, s->key_dims.data(), sizeof(int2) * nk, cudaMemcpyHostToDevice);
+    if (err == cudaSuccess) err = cudaMemcpy(s->costs_dev, s->key_costs.data(), sizeof(int) * nk, cudaMemcpyHostToDevice);
+    if (err == cudaSuccess) err = cudaMemcpy(s->costs_dev + slsm_max_keys(), order.data(), sizeof(int) * nk, cudaMemcpyHostToDevice);
+    if (err != cudaSuccess) return e->fail(TSS_E_CUDA, "tss_search_create: %s", cudaGetErrorString(err));
+    rc = lnsp_create(e, s->grid.data(), s->w, s->h, anchors.data(), s->keys_dev, s->costs_dev, s->costs_dev + slsm_max_keys(), (int)nk, seeds, s->seed,
+                     s->chain_offset, s->noise, &s->lnsp);
+    if (rc) return rc;
+    s->n_chains = lnsp_chains(s->lnsp);
+    return TSS_OK;
+}
+
 int tss_layout_merge_supports(const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, tss_platform* plats, int32_t n,
                               int32_t cap) {
     if (!grid || w <= 0 || h <= 0 || n < 0 || (n > 0 && !plats) || (n_defs > 0 && !defs)) return TSS_E_INVALID;
@@ -1131,21 +1218,29 @@ int tss_search_best_layout(tss_search* s, tss_platform* out, int32_t cap, int32_
                 bool fits = true;
                 for (auto& kd : s->key_dims) fits = fits && kd.x <= 6 && kd.y <= 6;
                 if (fits && (int)s->key_dims.size() <= 16) {
-                    BitGrid bg = BitGrid::from_bytes(s->grid.data(), s->w, s->h);
-                    std::vector<int4> placed;
-                    rc = greedy_cover(e, bg.rows.data(), s->w, s->h, s->key_dims, placed);
+                    rc = greedy_layout(e, s, false, s->greedy_plats);
                     if (rc) return rc;
-                    for (auto& q : placed) {
-                        tss_platform pl = s->key_proto[(size_t)q.z];
-                        pl.x = q.x; pl.y = q.y;
-                        s->greedy_plats.push_back(pl);
-                    }
-                    prune_redundant(s->grid, s->w, s->h, s->greedy_plats);
                 }
                 s->greedy_done = true;
             }
             if (!s->greedy_plats.empty() && s->greedy_plats.size() < plats.size()) plats = s->greedy_plats;
         }
+        best = make_int2((int)plats.size(), 0);
+    } else if (s->lnsp) {
+        std::vector<uint8_t> anchors;
+        rc = lnsp_anchors(e, s->lnsp, anchors);
+        if (rc) return rc;
+        int cost = 0;
+        for (int y = 0; y < s->h; y++)
+            for (int x = 0; x < s->w; x++) {
+                const int a = anchors[(size_t)y * s->w + x];
+                if (!a) continue;
+                tss_platform p = s->key_proto[(size_t)a - 1];
+                p.x = x; p.y = y;
+                plats.push_back(p);
+                cost += s->key_costs[(size_t)a - 1];
+            }
+        if (cost != lnsp_value(s->lnsp)) return e->fail(TSS_E_CUDA, "internal error: layout costs %d, the search reported %d", cost, lnsp_value(s->lnsp));
         best = make_int2((int)plats.size(), 0);
     } else if (s->multi) {
         best = s->best_host[0];
@@ -1190,7 +1285,8 @@ int tss_search_set_weights(tss_search* s, const int32_t* weights, int32_t n_weig
     if (!s) return TSS_E_INVALID;
     tss_engine* e = s->e;
     if (n_weights < 0 || (n_weights > 0 && !weights)) return e->fail(TSS_E_INVALID, "tss_search_set_weights: bad arguments");
-    if (!s->multi) return e->fail(TSS_E_UNSUPPORTED, "tss_search_set_weights: the weight objective needs a platform set beyond {1x1} on a grid up to 32x32");
+    if (!s->multi && !s->lnsp)
+        return e->fail(TSS_E_UNSUPPORTED, "tss_search_set_weights: the weight objective needs a platform set beyond {1x1} on a grid up to 32x32, or the window placement search");
     int rc = search_sync(s);
     if (rc) return rc;
     // cost of a platform = sum of the weights of every def contained in its def (platform_layout.rs:174-183)
@@ -1203,6 +1299,11 @@ int tss_search_set_weights(tss_search* s, const int32_t* weights, int32_t n_weig
         s->key_costs[k] = (int)cost;
     }
     TSS_CUDA(e, cudaMemcpy(s->costs_dev, s->key_costs.data(), sizeof(int) * s->key_costs.size(), cudaMemcpyHostToDevice));
+    if (s->lnsp) {   // the objective of the current layout under the new costs
+        rc = lnsp_objective(e, s->lnsp);
+        if (rc) return rc;
+        s->dirty = true;
+    }
     return TSS_OK;
 }
 

@@ -12,6 +12,7 @@
 // Completeness is invariant: every tile belongs to exactly one window and stays covered by frozen + core supports.
 // Phases alternate the offset between 0 and -16 per axis so that every site is movable in some phase.
 #include "engine.hpp"
+#include "lns_window.cuh"
 #include "sls_spec.hpp"
 
 namespace tss {
@@ -37,26 +38,6 @@ __global__ void gap_supports_kernel(const uint32_t* __restrict__ S, const uint32
     int y = i / wpr;
     uint32_t core = core_row(y, oy) ? colmask : 0u;
     F[i] = S[i] & ~core & C[i];  // only supports under a ceiling tile support anything (platform_layout.rs:116-119)
-}
-
-__global__ void dilate_global_kernel(const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, const uint32_t* __restrict__ C, int nw, int wpr) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nw) return;
-    int col = i % wpr;
-    uint32_t x = src[i], l = x << 1, r = x >> 1;
-    if (col > 0) l |= src[i - 1] >> 31;
-    if (col + 1 < wpr) r |= src[i + 1] << 31;
-    uint32_t up = i >= wpr ? src[i - wpr] : 0u, down = i + wpr < nw ? src[i + wpr] : 0u;
-    dst[i] = (x | l | r | up | down) & C[i];
-}
-
-// 32 bits of row gy of a bit-packed grid starting at column gx0 (may be negative / beyond the grid: zeros)
-__device__ __forceinline__ uint32_t fetch32(const uint32_t* __restrict__ X, int gy, int gx0, int h, int wpr) {
-    if (gy < 0 || gy >= h) return 0u;
-    int wq = gx0 >> 5, sh = gx0 & 31;  // arithmetic shift: floor division also for negative gx0
-    uint32_t lo = (wq >= 0 && wq < wpr) ? X[gy * wpr + wq] : 0u;
-    uint32_t hi = (wq + 1 >= 0 && wq + 1 < wpr) ? X[gy * wpr + wq + 1] : 0u;
-    return __funnelshift_r(lo, hi, sh);
 }
 
 // one warp per window: window rows, need mask, core supports -> chain states

@@ -25,6 +25,7 @@
 // generalises "k == L-1 -> swap" to "no candidate is affordable (W + min cost >= L) -> remove first", candidates must be
 // affordable (W + cost < L) and are ranked by gain per cost.
 #include "engine.hpp"
+#include "sls_multi.hpp"
 #include "sls_spec.hpp"
 
 namespace tss {
@@ -32,27 +33,17 @@ namespace slsm {
 
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int WARPS = 4;
-constexpr int MAX_ITEMS = 1024;
-constexpr int MAX_KEYS = 16;
 constexpr int WIN = 12;  // window rows / columns: footprint (<= 6) + 3 on each side
-
-struct MultiState {  // persistent per-chain state in HBM
-    uint16_t items[MAX_ITEMS];       // key << 10 | y << 5 | x
-    uint16_t best_items[MAX_ITEMS];
-    int32_t k, best;      // platforms now; best OBJECTIVE value found (platform count, or total weight in weight mode)
-    uint32_t step;
-    int32_t tabu_add, tabu_rem, done;
-    int32_t best_k;       // number of platforms in best_items
-    uint32_t pad[1];
-};
 
 struct Lane {
     uint32_t C, Occ, c0, c1, c2, c3, c4, U, O;
+    uint32_t N;   // WINDOW: the tiles this window still has to cover (ceiling not covered by the frozen platforms)
 };
+template <bool WINDOW>
 __device__ __forceinline__ void derive(Lane& L) {
     uint32_t hi = L.c1 | L.c2 | L.c3 | L.c4;
-    L.U = L.C & ~(L.c0 | hi);
-    L.O = L.c0 & ~hi;
+    L.U = (WINDOW ? L.N : L.C) & ~(L.c0 | hi);
+    L.O = WINDOW ? (L.N & L.c0 & ~hi) : (L.c0 & ~hi);
 }
 __device__ __forceinline__ void planes_add(Lane& L, uint32_t m) {
     uint32_t t;
@@ -140,6 +131,7 @@ __device__ __forceinline__ void unpack(const Ctx& c, int code, int& x, int& y, i
     w = d.x; h = d.y;
 }
 
+template <bool WINDOW>
 __device__ __forceinline__ int remove_min_loss(Lane& L, const Ctx& c, int& k, uint32_t hl, int exclude) {
     uint32_t best_key = 0xffffffffu;
     int best_i = 0;
@@ -164,7 +156,7 @@ __device__ __forceinline__ int remove_min_loss(Lane& L, const Ctx& c, int& k, ui
     uint32_t foot, reach;
     placement_rows(L.C, c.lane, x, y, w, h, foot, reach);
     planes_sub(L, reach);
-    derive(L);
+    derive<WINDOW>(L);
     L.Occ &= ~foot;
     return code;
 }
@@ -189,15 +181,20 @@ struct OneShotM {
                                   // from word 16: the n placement codes as u16
 };
 
-template <bool ONESHOT>
-__global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* __restrict__ terrain_rows, int W, int H,
+// WINDOW = the window-decomposed placement search on grids larger than 32x32 (lns_placements.cu, see WindowM): chain c works
+// on window c / seeds, `terrain_rows` holds 32 ceiling rows per window and the epoch bound is bounds[window].
+// (WINDOW: at most 4 CTAs per SM, i.e. up to 128 registers — the window's need rows and box do not fit the 96 registers the
+// compiler settles for otherwise without spilling; a phase on 256x256 launches ~1300 chains, 2-3 CTAs per SM)
+template <bool ONESHOT, bool WINDOW>
+__global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(const uint32_t* __restrict__ terrain_rows, int W, int H,
                                                               const int2* __restrict__ keys_g, const int* __restrict__ costs_g,
                                                               const int* __restrict__ order_g, int n_keys,
                                                               MultiState* __restrict__ states,
                                                               int n_chains, uint32_t chain_offset, uint64_t seed, long long steps,
                                                               const int* __restrict__ bounds, int target, int noise_pct,
                                                               const volatile int* interrupt, unsigned long long* __restrict__ totals,
-                                                              const OneShotM os) {
+                                                              const OneShotM os, const WindowM wm) {
+    static_assert(!(ONESHOT && WINDOW), "a one-shot solve never runs on windows");
     __shared__ uint16_t items_all[WARPS][MAX_ITEMS];
     __shared__ int2 keys[MAX_KEYS];
     __shared__ int costs[MAX_KEYS];
@@ -206,12 +203,15 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
     const int chain = blockIdx.x * WARPS + warp;
     // a layout within the target is already known for this terrain (found in an earlier epoch): nothing to do.  Lets a host
     // queue several epochs back to back without a round trip in between (one-shot solves, sls_spec.hpp).
-    if (!ONESHOT && target >= 0 && bounds[0] <= target) return;
+    // (windows: the warps of a CTA may belong to different windows, so this test waits until after the barrier)
+    if (!ONESHOT && !WINDOW && target >= 0 && bounds[0] <= target) return;
     if (threadIdx.x < n_keys) { keys[threadIdx.x] = keys_g[threadIdx.x]; costs[threadIdx.x] = costs_g[threadIdx.x]; order[threadIdx.x] = order_g[threadIdx.x]; }
     __syncthreads();
     int cmin = costs[0];
     for (int i = 1; i < n_keys; i++) cmin = min(cmin, costs[i]);
     if (!ONESHOT && chain >= n_chains) return;   // (a one-shot launch has whole CTAs of chains: everyone takes part in the ticket)
+    const int win = WINDOW ? chain / wm.seeds : 0;
+    if (WINDOW && target >= 0 && bounds[win] <= target) return;
     MultiState& st = states[chain];
     if (!ONESHOT && st.done) return;
     if (ONESHOT && blockIdx.x == 0 && threadIdx.x < 32) {
@@ -219,13 +219,15 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
         if (threadIdx.x == 0) os.bounds_out[0] = os.bound;
     }
 
-    const int epoch_bound = ONESHOT ? os.bound : bounds[0];
+    const int epoch_bound = ONESHOT ? os.bound : bounds[win];
     const uint32_t base = sls::chain_base(seed, chain_offset + (uint32_t)chain);
     const uint32_t nq7 = sls::noise_q7(noise_pct);
     Ctx c{items_all[warp], keys, lane, W, H};
     Lane L;
-    L.C = ONESHOT ? os.rows[lane] : terrain_rows[lane];
-    L.Occ = 0;
+    L.C = ONESHOT ? os.rows[lane] : terrain_rows[win * 32 + lane];
+    L.Occ = WINDOW ? wm.occ[win * 32 + lane] : 0u;
+    if (WINDOW) L.N = wm.need[win * 32 + lane];
+    const int4 box = WINDOW ? wm.box[win] : make_int4(0, 0, W, H);
     L.c0 = L.c1 = L.c2 = L.c3 = L.c4 = 0;
     int k = ONESHOT ? 0 : st.k, best = ONESHOT ? sls::NO_BOUND : st.best, tabu_add = ONESHOT ? -1 : st.tabu_add, tabu_rem = ONESHOT ? -1 : st.tabu_rem, done = 0;
     uint32_t step = ONESHOT ? 0u : st.step;
@@ -244,7 +246,7 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
         L.Occ |= foot;
         Wt += costs[c.items[i] >> 10];
     }
-    derive(L);
+    derive<WINDOW>(L);
 
     long long it = 0;
     for (; it < steps; it++, step++) {
@@ -255,7 +257,7 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
         if (Wt >= limit) {  // too expensive for an improvement: drop a platform
             if (k == 0) { done = 1; break; }
             scored += (unsigned)k;
-            tabu_add = remove_min_loss(L, c, k, hl, -1);
+            tabu_add = remove_min_loss<WINDOW>(L, c, k, hl, -1);
             Wt -= costs[tabu_add >> 10];
             flips++;
             continue;
@@ -269,7 +271,7 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
         }
         if (Wt + cmin >= limit && k > 0) {  // nothing is affordable: swap = remove + add
             scored += (unsigned)k;
-            tabu_add = remove_min_loss(L, c, k, hl, tabu_rem);
+            tabu_add = remove_min_loss<WINDOW>(L, c, k, hl, tabu_rem);
             Wt -= costs[tabu_add >> 10];
             flips++;
         }
@@ -290,7 +292,8 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
             // footprint intersects the 7x7 box around t: x in [tx-3-(w-1), tx+3], y in [ty-3-(h-1), ty+3]
             const int x = tx - 3 - (d.x - 1) + (int)((((r >> 16) & 0xffu) * (uint32_t)(d.x + 6)) >> 8);
             const int y = ty - 3 - (d.y - 1) + (int)(((r >> 24) * (uint32_t)(d.y + 6)) >> 8);
-            const bool inb = x >= 0 && y >= 0 && x + d.x <= W && y + d.y <= H;   // out-of-bounds placements are never valid
+            const bool inb = WINDOW ? (x >= box.x && y >= box.y && x + d.x <= box.z && y + d.y <= box.w)   // inside the window's box
+                                    : (x >= 0 && y >= 0 && x + d.x <= W && y + d.y <= H);   // out-of-bounds placements are never valid
             const int code = inb ? ((key << 10) | (y << 5) | x) : 0;
             bool ov;
             int g = score_placement(L.C, L.U, L.Occ, inb ? x : 0, inb ? y : 0, d.x, d.y, ov);
@@ -312,7 +315,7 @@ __global__ void __launch_bounds__(WARPS * 32) sls_multi_kernel(const uint32_t* _
         uint32_t foot, reach;
         placement_rows(L.C, lane, x, y, w, h, foot, reach);
         planes_add(L, reach);
-        derive(L);
+        derive<WINDOW>(L);
         L.Occ |= foot;
         if (lane == 0) c.items[k] = (uint16_t)best_code;
         __syncwarp();
@@ -440,9 +443,9 @@ int slsm_run(tss_engine* e, const uint32_t* rows_dev, int W, int H, const int2* 
              uint32_t chain_offset, uint64_t seed, long long steps, int* bounds_dev, int target, int noise_pct, unsigned long long* totals_dev,
              int2* best_dev) {
     int blocks = (n_chains + slsm::WARPS - 1) / slsm::WARPS;
-    slsm::sls_multi_kernel<false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states, n_chains,
-                                                                            chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
-                                                                            totals_dev, slsm::OneShotM{});
+    slsm::sls_multi_kernel<false, false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states, n_chains,
+                                                                                   chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
+                                                                                   totals_dev, slsm::OneShotM{}, slsm::WindowM{});
     TSS_CHECK_LAUNCH(e);
     slsm::multi_best_kernel<<<1, 256, 0, e->stream>>>((const slsm::MultiState*)states, n_chains, best_dev, bounds_dev);
     TSS_CHECK_LAUNCH(e);
@@ -460,9 +463,22 @@ int slsm_run_oneshot(tss_engine* e, const uint32_t* rows32_host, int bound, uint
     for (int r = 0; r < 32; r++) os.rows[r] = rows32_host[r];
     os.bound = bound; os.rows_out = rows_dev; os.bounds_out = bounds_dev; os.best_out = best_dev; os.key = key_dev; os.ticket = ticket_dev;
     os.result_host = result_host_mapped;
-    slsm::sls_multi_kernel<true><<<n_chains / slsm::WARPS, slsm::WARPS * 32, 0, e->stream>>>(nullptr, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states,
-                                                                                            n_chains, 0u, seed, steps, nullptr, target, noise_pct, e->interrupt_dev,
-                                                                                            totals_dev, os);
+    slsm::sls_multi_kernel<true, false><<<n_chains / slsm::WARPS, slsm::WARPS * 32, 0, e->stream>>>(nullptr, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states,
+                                                                                                   n_chains, 0u, seed, steps, nullptr, target, noise_pct, e->interrupt_dev,
+                                                                                                   totals_dev, os, slsm::WindowM{});
+    TSS_CHECK_LAUNCH(e);
+    e->stats.kernel_launches++;
+    return TSS_OK;
+}
+// One epoch of every window's chains (the window-decomposed placement search, lns_placements.cu); chains are numbered
+// window * wm.seeds + j.  No best-reduce here: the caller picks a winner per window.
+int slsm_run_windows(tss_engine* e, const uint32_t* rows_dev, const slsm::WindowM& wm, const int2* keys_dev, const int* costs_dev, const int* order_dev,
+                     int n_keys, slsm::MultiState* states, int n_chains, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev,
+                     int target, int noise_pct, unsigned long long* totals_dev) {
+    const int blocks = (n_chains + slsm::WARPS - 1) / slsm::WARPS;
+    slsm::sls_multi_kernel<false, true><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, 32, 32, keys_dev, costs_dev, order_dev, n_keys, states, n_chains,
+                                                                                  chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
+                                                                                  totals_dev, slsm::OneShotM{}, wm);
     TSS_CHECK_LAUNCH(e);
     e->stats.kernel_launches++;
     return TSS_OK;
