@@ -27,6 +27,9 @@ from timberborn_support_solver_b200 import build as B  # noqa: E402
 
 CUDA = os.path.dirname(os.path.dirname(os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")))
 FLAGS = [f for f in B.NVCC_FLAGS if f not in ("-shared", "-cudart", "static", "-ldl")]
+# opcodes issued to the integer-ALU pipe (the "ALU" column): the pipe that bounds both kernels, one warp instruction every
+# 2 clocks per scheduler (DESIGN.md).  IMAD, POPC and the memory instructions issue elsewhere.
+ALU = {"LOP3", "SHF", "PRMT", "ISETP", "SEL", "VIMNMX", "VIADDMNMX", "IADD3", "LEA", "R2P", "PLOP3"}
 
 
 def read(path):
@@ -107,10 +110,12 @@ def mix(name, out):
         for j in range(hit[0], hit[-1] + 1) if span else hit:
             per[part][ins[j][1]] += 1
     print(f"{name}: {regs[0][1] if regs else '?'} registers, {regs[0][0] if regs else '?'} bytes spilled")
+    print(f"  {'':48s} {'all':>6s} {'ALU':>6s}")
     for part, (_, div, _) in rng.items():
         c = per[part]
+        alu = sum(n for op, n in c.items() if op in ALU)
         top = ", ".join(f"{op} {n / div:.1f}" for op, n in c.most_common(8))
-        print(f"  {part:48s} {sum(c.values()) / div:6.1f}   ({top})")
+        print(f"  {part:48s} {sum(c.values()) / div:6.1f} {alu / div:6.1f}   ({top})")
 
 
 if __name__ == "__main__":

@@ -83,6 +83,23 @@ __device__ __forceinline__ uint32_t removal_loss(const Smem& sm, int tid, uint32
     return (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
 }
 
+// Removal key of list entry e (index i, loss `loss`) in remove_key's order (young, loss, tie, index), one byte per field
+// most significant first: young * 64 + loss (a reach window has at most 25 tiles), tie_remove(hs, i) in bytes 1-2, which are bytes 2-3 of
+// hsm = hs * (2i+1) * K3, and i (a 16x16 list has at most 256 entries).  One IMAD and one PRMT instead of remove_key's
+// shift, mask and merge on the integer-ALU pipe.
+static_assert(MAXW * MAXH <= 256, "removal_key keeps a list index in one byte: a list holds at most one entry per site");
+__device__ __forceinline__ uint32_t removal_key(uint32_t e, int i, uint32_t loss, uint32_t hsm, uint32_t stephi, uint32_t young_below) {
+    const uint32_t x = loss * (1u << 24) + ((stephi - e) < young_below ? TABU_BIT | (uint32_t)i : (uint32_t)i);
+    return __byte_perm(hsm, x, 0x7324);
+}
+
+// the least of N keys as a tree of mins: log2(N) dependent steps instead of N
+template <int N>
+__device__ __forceinline__ uint32_t tree_min(const uint32_t* key) {
+    if constexpr (N == 1) return key[0];
+    else return min(tree_min<N / 2>(key), tree_min<N / 2>(key + N / 2));
+}
+
 // adds (ADD) or removes the cover of site v (window win = its tab[0] entry) on the five count planes and refreshes U, O
 // and the non-empty-row mask.
 // rowmask is kept in padded coordinates: bit r + 4 = row r has an uncovered tile.
@@ -201,30 +218,35 @@ struct Pairs {
 
     __device__ __forceinline__ void remove(uint32_t hs, uint32_t step, uint32_t stephi, uint32_t young_below, int k, uint32_t& rowmask) {
         uint32_t best_key = 0xffffffffu;
-        // cached slots: the warp scans them in groups of SCAN up to its largest k (a thread scores only its own k).  No
-        // branch inside a group, so the loads of its slots overlap: with 3 warps per scheduler the scan is latency bound
-        // when every slot waits for the one before it.
+        // cached slots: the warp scans a first group of SCAN slots, then the rest in pairs, up to its largest k (a thread
+        // scores only its own k).  No branch inside a group, so the loads of its slots overlap: with 3 warps per scheduler
+        // the scan is latency bound when every slot waits for the one before it.  The first group serves grids whose k
+        // stays at 8 or below (ex3: 3-5) with one branch; past it, pairs score at most one slot beyond kw (groups of 8 would
+        // score 16 slots at the bench's k = 14).
         // kw only has to be >= this thread's own k: threads that arrive here apart from the rest of the warp reduce over a
         // partial mask and scan for their own group, which is still exact
         const int kw = __reduce_max_sync(__activemask(), k);
         constexpr int SCAN = 8;
+        uint32_t key[CAP];
 #pragma unroll
         for (int i = 0; i < CAP; i++) {
-            if (i % SCAN == 0 && i >= kw) break;
+            if ((i < SCAN ? i == 0 : i % 2 == 0) && i >= kw) break;
             const uint32_t e = sm.cent[slot(i)][tid];
             const uint32_t loss = removal_loss(sm, tid, e, sm.cwin[slot(i)][tid]);
-            const uint32_t key = remove_key(e, i, loss, hs * ((2u * i + 1u) * K3), stephi, young_below);
-            best_key = i < k ? min(best_key, key) : best_key;   // compiles to a select: no branch inside a group
+            key[i] = i < k ? removal_key(e, i, loss, hs * ((2u * i + 1u) * K3), stephi, young_below) : 0xffffffffu;
+            // a group's keys are masked first and then reduced as a tree, not folded into one chain of slot-by-slot mins
+            if (i == SCAN - 1) best_key = min(best_key, tree_min<SCAN>(&key[0]));
+            else if (i > SCAN && i % 2 == 1) best_key = min(best_key, tree_min<2>(&key[i - 1]));
         }
         if (kw > CAP) {   // the rest of the list (dense warm starts): global entries, windows from the table
             uint32_t mult = (2u * CAP + 1u) * K3;                   // mult = (2i+1) * K3
             for (int i = CAP; i < k; i++, mult += 2u * K3) {
                 const uint32_t e = sl[(size_t)i * stride];
                 const uint32_t loss = removal_loss(sm, tid, e, ld_tab(sm, &sm.tab[0][(e & 0x1ffu) + TAB_PAD]));
-                best_key = min(best_key, remove_key(e, i, loss, hs * mult, stephi, young_below));
+                best_key = min(best_key, removal_key(e, i, loss, hs * mult, stephi, young_below));
             }
         }
-        const int best_i = (int)(best_key & 0x1ffu), last = k - 1;
+        const int best_i = (int)(best_key & 0xffu), last = k - 1;
         int u;
         uint2 win;
         if (best_i < CAP) {

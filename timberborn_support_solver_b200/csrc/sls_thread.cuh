@@ -126,27 +126,29 @@ __device__ __forceinline__ uint32_t flip_word(Smem& sm, int tid, uint32_t* p, in
 
 // Removal key of list entry e (index i, loss `loss`): young | loss | tie | index, unique, so the minimum is the spec's
 // (lowest index wins ties).  hsm = hs * (2i+1) * K3; stephi - e = (age << 16) + (0xffff - low half): no borrow.
+// sls_p16.cu encodes the same order with one byte per field (its removal_key): its lists have at most 256 entries.
 __device__ __forceinline__ uint32_t remove_key(uint32_t e, int i, uint32_t loss, uint32_t hsm, uint32_t stephi, uint32_t young_below) {
     const uint32_t tie = (hsm >> 7) & 0x1fffe00u;  // tie_remove(hs, i) << 9
     const uint32_t young = (stephi - e) < young_below ? TABU_BIT : 0u;
     return (young | tie | (uint32_t)i) + loss * (1u << 25);
 }
 
-__device__ __forceinline__ uint32_t shift_static(uint32_t v, int s) { return s >= 0 ? v << s : v >> (-s); }
-
 // One ADD candidate: the site at offset (DX, DY) from the uncovered tile.  S = the kernel's slab of U for this DX, from
 // which Nbhd::gain takes the candidate's gain with its reach window; tabt = the table entry of the tile, wt = the tile's
 // own window in byte-per-row format around (x-3, y-3) (candidate validity).  Keys are unique per cell (the cell index sits
 // in the low bits), so the maximum is independent of the evaluation order and ties go to the lowest cell as the spec demands.
+// One byte per field, most significant first: fresh * 64 + gain + 1 (a gain is at most 25 tiles; 1 in a noise step),
+// tie_add(hs, cell) in bytes 1-2, which are bytes 2-3 of the tie product, and 31 - cell.  The fields are built on the FMA
+// pipe (one IMAD) and merged with one PRMT, off the integer-ALU pipe that bounds both kernels.
 template <int DX, int DY, class Nbhd, class Smem>
 __device__ __forceinline__ uint32_t add_key(const Smem& sm, const typename Nbhd::Slab& S, const uint2* tabt, uint2 wt, uint32_t fresh_lo,
                                             uint32_t fresh_hi, uint32_t hs, uint32_t gmul) {
     constexpr int cell = cell_index(DX, DY), bit = 8 * (DY + 3) + DX + 3;   // position in t's byte-per-row window (rows 0-3 / 4-6)
     const uint2 win = ld_tab(sm, tabt + DY * 32 + DX);
     const uint32_t g = Nbhd::template gain<DY>(S, win);
-    const uint32_t tie = ((hs * ((2u * cell + 1u) * K2)) >> 11) & 0x1fffe0u;             // tie_add(hs, cell) << 5
-    const uint32_t fresh = shift_static(bit < 32 ? fresh_lo : fresh_hi, 30 - (bit < 32 ? bit : bit - 32)) & TABU_BIT;  // (all zero in a noise step)
-    const uint32_t key = (fresh | tie) + g * gmul + ((1u << 21) | (31u - cell));   // gmul = 1 << 21, or 0 in a noise step
+    const bool fresh = ((bit < 32 ? fresh_lo >> bit : fresh_hi >> (bit - 32)) & 1u) != 0;   // (all zero in a noise step)
+    const uint32_t lo = (fresh ? 0x41000000u : 0x01000000u) | (31u - cell);
+    const uint32_t key = __byte_perm(hs * ((2u * cell + 1u) * K2), g * gmul + lo, 0x7324);   // gmul = 1 << 24, or 0 in a noise step
     const bool valid = ((bit < 32 ? wt.x >> bit : wt.y >> (bit - 32)) & 1u) != 0;
     return valid ? key : 0u;
 }
@@ -189,7 +191,7 @@ __device__ __forceinline__ int add_site(const Smem& sm, int tid, const Nbhd& N, 
         }
     }
     const uint32_t fresh_lo = noise ? 0u : ~tw_lo, fresh_hi = noise ? 0u : ~tw_hi;
-    const uint32_t gmul = noise ? 0u : 1u << 21;
+    const uint32_t gmul = noise ? 0u : 1u << 24;
     uint32_t mx = add_column<0>(sm, N, fresh_lo, fresh_hi, hs, gmul);
     mx = max(mx, add_column<-1>(sm, N, fresh_lo, fresh_hi, hs, gmul));
     mx = max(mx, add_column<1>(sm, N, fresh_lo, fresh_hi, hs, gmul));
