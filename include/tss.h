@@ -308,7 +308,14 @@ int tss_lower_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, co
  * tile, *out_total = their sum, *out_max_load = the largest sum over the reach of any placement, recomputed from the reach
  * bitboards, and *out_bound = min over placements of ceil(total * cost / load) (= ceil(total / max_load) with unit costs) —
  * valid whatever the floating point solve did.  It dominates tss_lower_bound up to rounding (README terrain, 1x1 supports:
- * 12 -> 14 = the optimum).  out_info[3] (optional) = pivots, 1 if the simplex reached optimality, constraints.  Grids up to 32x32. */
+ * 12 -> 14 = the optimum).  out_info[3] (optional) = pivots, 1 if the simplex reached optimality, constraints.  Grids up to 32x32
+ * take that simplex.  Grids larger than 32x32, up to 256x256, take a first-order method instead (csrc/lp_big.cu: optimistic
+ * multiplicative weights on the zero-sum game of the LP, no tableau) with the same certificate over every in-bounds placement:
+ * any platform set of at most 16 dims keys, each at most 6x6 (what the window placement search takes, or 1x1 alone), count or
+ * weights; anything else returns TSS_E_UNSUPPORTED.  There `max_pivots` caps the ITERATIONS (<= 0: 3 000), `target` > 0 stops
+ * as soon as the integer-certified bound reaches `target` (checked every 250 iterations), tiles in the reach of a platform that
+ * costs nothing are fixed at 0, and out_info = iterations, 0 (the method never proves optimality), constraints (placements whose
+ * reach holds ceiling and that cost something).  Two calls on the same device give the same weights. */
 int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* weights,
                        int32_t n_weights, int32_t max_pivots, int64_t target, int32_t* out_weights, int64_t* out_total, int64_t* out_max_load,
                        int64_t* out_bound, int32_t* out_info);

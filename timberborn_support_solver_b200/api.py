@@ -673,6 +673,9 @@ class Engine:
         """Fractional packing lower bound (tss_lower_bound_lp), certified in integers: on the platform count, or with `weights`
         ({PlatformDef: weight}, the PlatformLimits.weights map) on PlatformLayout::total_weight.  target > 0: the simplex stops as
         soon as the bound reaches it (every iterate is feasible; enough for "is there nothing within target - 1?").
+        On grids larger than 32x32 (up to 256x256; at most 16 dims keys, each at most 6x6) a first-order method replaces the
+        simplex under the same certificate: `max_pivots` caps its iterations (0: 3 000) and the result's `pivots` counts them,
+        `target` is checked on the certified bound every 250 iterations, and `optimal` is always False.
         -> dict(bound, weights int32[h, w], total, max_load, pivots, optimal, constraints)."""
         defs = list(defs)
         wts = np.zeros((grid.height, grid.width), np.int32)

@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libtss.so")
-SOURCES = ["engine.cu", "eval.cu", "eval_thread.cu", "cnf.cu", "sls.cu", "sls_h16.cu", "sls_t16.cu", "sls_p16.cu", "sls_multi.cu", "lns.cu", "lns_placements.cu", "greedy.cu", "lb.cu", "lp.cu", "comm.cu", "peaks.cu", "capi_host.cpp", "host_model.cpp", "instance.cpp"]
+SOURCES = ["engine.cu", "eval.cu", "eval_thread.cu", "cnf.cu", "sls.cu", "sls_h16.cu", "sls_t16.cu", "sls_p16.cu", "sls_multi.cu", "lns.cu", "lns_placements.cu", "greedy.cu", "lb.cu", "lp.cu", "lp_big.cu", "comm.cu", "peaks.cu", "capi_host.cpp", "host_model.cpp", "instance.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math",
               "-Xcompiler", "-fPIC,-Wall,-Wno-unknown-pragmas", "-shared", "-cudart", "static", "-ldl"]
 

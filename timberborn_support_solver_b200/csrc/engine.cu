@@ -47,6 +47,9 @@ int run_peaks(tss_engine* e, double* out, int n_out);
 // lp.cu — fractional packing lower bound
 int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs, int max_pivots,
            long long target, int* out_weights, unsigned long long* totals, int* info);
+// lp_big.cu — the same bound on grids larger than 32x32 (first-order method, same certificate)
+int lp_big_run(tss_engine* e, const uint32_t* rows_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs, int max_iters,
+               long long target, int* out_weights, unsigned long long* totals, int* info);
 // lb.cu — packing lower bound
 int lb_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::vector<int2>& key_dims, uint64_t seed, int restarts,
            uint32_t* out_rows32, int* out_count);
@@ -1676,7 +1679,6 @@ int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h,
     if (out_bound) *out_bound = 0;
     if (!grid || !out_bound || w <= 0 || h <= 0 || (!defs && n_defs > 0) || n_weights < 0 || (n_weights > 0 && !weights))
         return e->fail(TSS_E_INVALID, "tss_lower_bound_lp: bad arguments");
-    if (w > 32 || h > 32) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: grids larger than 32x32 are not supported");
     bool has_1x1 = n_defs == 0;
     for (int i = 0; i < n_defs; i++) {
         if (defs[i].w <= 0 || defs[i].h <= 0) return e->fail(TSS_E_INVALID, "tss_lower_bound_lp: empty platform dimensions");
@@ -1700,6 +1702,20 @@ int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h,
             if (cost < 0 || cost > 4096) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: platform costs must be in 0..4096 (got %ld for %dx%d)", cost, def.w, def.h);
             key_costs[k] = (int)cost;
         }
+    if (w > 32 || h > 32) {   // first-order method on the whole grid (lp_big.cu), the same certificate
+        BitGrid bg = BitGrid::from_bytes(grid, w, h);
+        std::vector<int> wts((size_t)w * h);
+        int info[3];
+        unsigned long long totals[3];
+        int rc = lp_big_run(e, bg.rows.data(), w, h, key_dims, key_costs, max_pivots, target, wts.data(), totals, info);
+        if (rc) return rc;
+        if (out_weights) std::copy(wts.begin(), wts.end(), out_weights);
+        if (out_total) *out_total = (int64_t)totals[0];
+        if (out_max_load) *out_max_load = (int64_t)totals[1];
+        if (out_info) { out_info[0] = info[0]; out_info[1] = info[1]; out_info[2] = info[2]; }
+        *out_bound = (totals[1] > 0 && totals[2] != ~0ull) ? (int64_t)totals[2] : 0;
+        return TSS_OK;
+    }
     uint32_t rows[32] = {0};
     for (int y = 0; y < h; y++)
         for (int x = 0; x < w; x++)
