@@ -65,13 +65,16 @@ def ranges(name):
         rm1, rm_part = find(L, r"const int best_i = ", rm0), "removal, per support (scan / 5)"
     add0 = find(L, r"__device__ __forceinline__ void add\(")
     run = find(H, r"void run_chains\(")
+    # the tabu window's ring slots that a step loads ahead of its removal, and its fold (r10 on)
+    pre = [(hdr, r, r + 3) for r in [find(H, r"uint32_t recent\[RECENT\];", run)]] + [(hdr, *body(H, r"void tabu_bit\("))] \
+        if any("uint32_t recent[RECENT];" in l for l in H) else []
     return {"flip (per copy)": ([(src, *body(L, r"__device__ __forceinline__ void flip\("))], 3, False),
             rm_part: ([(src, rm0, rm1)], int(cap.group(1)) if cap else 5, True),
             "addition: 25 candidates (add_key/add_column)": ([(hdr, *body(H, r"uint32_t add_key\(")), (hdr, *body(H, r"uint32_t add_column\(")),
                                                               (src, *body(L, r"void slab\(")), (src, *body(L, r"uint32_t gain\("))], 1, False),
             "addition: fetch, pick, tabu window, decode": ([(src, *body(L, r"Nbhd fetch\(")), (src, add0, find(L, r"flip<true>\(sm, tid, v, ", add0)),
                                                             (hdr, find(H, r"const auto N = R\.fetch\(", run), find(H, r"const int v = add_site\(", run) + 1),
-                                                            (hdr, *body(H, r"int add_site\(")), (spec, *body(S, r"void diamond_cell\("))], 1, False)}
+                                                            (hdr, *body(H, r"int add_site\(")), (spec, *body(S, r"void diamond_cell\(")), *pre], 1, False)}
 
 
 def transparent(name):

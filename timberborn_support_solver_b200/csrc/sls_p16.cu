@@ -216,8 +216,19 @@ struct Pairs {
         return k;
     }
 
-    __device__ __forceinline__ void remove(uint32_t hs, uint32_t step, uint32_t stephi, uint32_t young_below, int k, uint32_t& rowmask) {
+    __device__ __forceinline__ int remove(uint32_t hs, uint32_t stephi, uint32_t young_below, int k, uint32_t& rowmask, Prof& pf) {
         uint32_t best_key = 0xffffffffu;
+        // swap-remove: entry k-1 (with its window) moves into the removed one's slot; its index is known before the scan
+        const int last = k - 1;
+        uint32_t e_last;
+        uint2 w_last;
+        if (last < CAP) {
+            e_last = sm.cent[slot(last)][tid];
+            w_last = sm.cwin[slot(last)][tid];
+        } else {
+            e_last = sl[(size_t)last * stride];
+            w_last = ld_tab(sm, &sm.tab[0][(e_last & 0x1ffu) + TAB_PAD]);
+        }
         // cached slots: the warp scans a first group of SCAN slots, then the rest in pairs, up to its largest k (a thread
         // scores only its own k).  No branch inside a group, so the loads of its slots overlap: with 3 warps per scheduler
         // the scan is latency bound when every slot waits for the one before it.  The first group serves grids whose k
@@ -246,7 +257,8 @@ struct Pairs {
                 best_key = min(best_key, removal_key(e, i, loss, hs * mult, stephi, young_below));
             }
         }
-        const int best_i = (int)(best_key & 0xffu), last = k - 1;
+        pf.mark(PH_SCAN);
+        const int best_i = (int)(best_key & 0xffu);
         int u;
         uint2 win;
         if (best_i < CAP) {
@@ -256,21 +268,14 @@ struct Pairs {
             u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
             win = ld_tab(sm, &sm.tab[0][u + TAB_PAD]);
         }
-        // swap-remove: entry k-1 (with its window) moves into slot best_i
-        if (last < CAP) {
-            sm.cent[slot(best_i)][tid] = sm.cent[slot(last)][tid];
-            sm.cwin[slot(best_i)][tid] = sm.cwin[slot(last)][tid];
+        if (best_i < CAP) {
+            sm.cent[slot(best_i)][tid] = e_last;
+            sm.cwin[slot(best_i)][tid] = w_last;
         } else {
-            const uint32_t e = sl[(size_t)last * stride];
-            if (best_i < CAP) {
-                sm.cent[slot(best_i)][tid] = e;
-                sm.cwin[slot(best_i)][tid] = ld_tab(sm, &sm.tab[0][(e & 0x1ffu) + TAB_PAD]);
-            } else {
-                sl[(size_t)best_i * stride] = e;
-            }
+            sl[(size_t)best_i * stride] = e_last;
         }
-        sm.ring[step & 31u][tid] = (uint16_t)u;
         flip<false>(sm, tid, u, win, rowmask);
+        return u;
     }
 
     __device__ __forceinline__ Nbhd fetch(uint32_t rowmask, uint32_t hs) const {
@@ -319,6 +324,10 @@ __global__ void __launch_bounds__(NT, 3) sls_p16_kernel(const uint32_t* __restri
 
 // violations counted by a -DTSS_CHECKED build since the library was loaded (always 0 in the shipped build, which has no checks)
 int sls_p16_smem_violations() { return slsp::smem_violations(); }
+#ifdef TSS_SLS_PROF
+// the phase-profiling build's totals (sls_thread.cuh, profiles/sls_phases.py): cycles per phase, then thread steps; cleared
+extern "C" int tss_debug_sls_p16_phases(unsigned long long* out) { return slsp::read_phases(out); }
+#endif
 bool sls_p16_fits(int w, int h) { return h <= slsp::MAXH && w <= slsp::MAXW; }
 
 // site lists: the caller allocates sls_t16_list_words (416 entries per chain >= the 256 sites of a 16x16 grid)

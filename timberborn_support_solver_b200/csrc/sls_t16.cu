@@ -136,7 +136,7 @@ struct Rows {
         return k;
     }
 
-    __device__ __forceinline__ void remove(uint32_t hs, uint32_t step, uint32_t stephi, uint32_t young_below, int k, uint32_t& rowmask) {
+    __device__ __forceinline__ int remove(uint32_t hs, uint32_t stephi, uint32_t young_below, int k, uint32_t& rowmask, Prof& pf) {
         uint32_t best_key = 0xffffffffu, mult = K3;                 // mult = (2i+1) * K3
 #pragma unroll 4
         for (int i = 0; i < k; i++, mult += 2u * K3) {
@@ -152,11 +152,12 @@ struct Rows {
             const uint32_t loss = (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
             best_key = min(best_key, remove_key(e, i, loss, hs * mult, stephi, young_below));
         }
+        pf.mark(PH_SCAN);
         const int best_i = (int)(best_key & 0x1ffu);
         const int u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
         sl[(size_t)best_i * stride] = sl[(size_t)(k - 1) * stride];
-        sm.ring[step & 31u][tid] = (uint16_t)u;
         flip<false>(sm, tid, u, rowmask);
+        return u;
     }
 
     __device__ __forceinline__ Nbhd fetch(uint32_t rowmask, uint32_t hs) const {

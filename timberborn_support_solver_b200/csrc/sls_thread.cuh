@@ -78,6 +78,42 @@ static inline int smem_violations() {
 static inline int smem_violations() { return 0; }   // the shipped build has no checks
 #endif
 
+// ---- phase-profiling build (-DTSS_SLS_PROF, profiles/sls_phases.py): clock64() between the parts of a step, summed per
+// thread and added into a device global once per warp at the end of the launch (read by the kernel file's
+// sls_*_phases()).  A load is charged to the phase that first waits for it, so the figures say where a warp waits, not
+// where an instruction was issued.  In the shipped build Prof is empty and every mark compiles to nothing.
+enum { PH_SCAN, PH_RFLIP, PH_FETCH, PH_CAND, PH_AFLIP, PH_FRAME, N_PHASES };
+#ifdef TSS_SLS_PROF
+static __device__ unsigned long long g_phases[N_PHASES + 1];   // cycles per phase summed over threads, then thread steps
+struct Prof {
+    unsigned long long c[N_PHASES] = {};
+    long long t = 0;
+    __device__ __forceinline__ void start() { t = clock64(); }
+    __device__ __forceinline__ void mark(int ph) { const long long n = clock64(); c[ph] += (unsigned long long)(n - t); t = n; }
+    __device__ __forceinline__ void flush(unsigned long long steps) {
+#pragma unroll
+        for (int i = 0; i <= N_PHASES; i++) {
+            unsigned long long a = i < N_PHASES ? c[i] : steps;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+            if ((threadIdx.x & 31) == 0) atomicAdd(&g_phases[i], a);
+        }
+    }
+};
+// copies the totals to out[0 .. N_PHASES] and clears them
+static inline int read_phases(unsigned long long* out) {
+    static const unsigned long long zero[N_PHASES + 1] = {};
+    if (cudaMemcpyFromSymbol(out, g_phases, sizeof zero) != cudaSuccess) return -1;
+    return cudaMemcpyToSymbol(g_phases, zero, sizeof zero) == cudaSuccess ? N_PHASES : -1;
+}
+#else
+struct Prof {
+    __device__ __forceinline__ void start() {}
+    __device__ __forceinline__ void mark(int) {}
+    __device__ __forceinline__ void flush(unsigned long long) {}
+};
+#endif
+
 __device__ __forceinline__ uint32_t shl_clamped(uint32_t v, int n) {  // PTX shl: shift counts above 31 (incl. "negative" ones) give 0
     uint32_t r;
     asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
@@ -138,8 +174,10 @@ __device__ __forceinline__ uint32_t remove_key(uint32_t e, int i, uint32_t loss,
 // own window in byte-per-row format around (x-3, y-3) (candidate validity).  Keys are unique per cell (the cell index sits
 // in the low bits), so the maximum is independent of the evaluation order and ties go to the lowest cell as the spec demands.
 // One byte per field, most significant first: fresh * 64 + gain + 1 (a gain is at most 25 tiles; 1 in a noise step),
-// tie_add(hs, cell) in bytes 1-2, which are bytes 2-3 of the tie product, and 31 - cell.  The fields are built on the FMA
-// pipe (one IMAD) and merged with one PRMT, off the integer-ALU pipe that bounds both kernels.
+// tie_add(hs, cell) in bytes 1-2, which are bytes 2-3 of the tie product, and (3 - DY) * 32 + (3 - DX) in byte 0: it falls
+// as the cell index grows (cells are numbered by DY, then DX), and the site is (y + 3) * 32 + x + 3 minus it, with no
+// decode of the cell.  The fields are built on the FMA pipe (one IMAD) and merged with one PRMT, off the integer-ALU pipe
+// that bounds both kernels.
 template <int DX, int DY, class Nbhd, class Smem>
 __device__ __forceinline__ uint32_t add_key(const Smem& sm, const typename Nbhd::Slab& S, const uint2* tabt, uint2 wt, uint32_t fresh_lo,
                                             uint32_t fresh_hi, uint32_t hs, uint32_t gmul) {
@@ -147,7 +185,7 @@ __device__ __forceinline__ uint32_t add_key(const Smem& sm, const typename Nbhd:
     const uint2 win = ld_tab(sm, tabt + DY * 32 + DX);
     const uint32_t g = Nbhd::template gain<DY>(S, win);
     const bool fresh = ((bit < 32 ? fresh_lo >> bit : fresh_hi >> (bit - 32)) & 1u) != 0;   // (all zero in a noise step)
-    const uint32_t lo = (fresh ? 0x41000000u : 0x01000000u) | (31u - cell);
+    const uint32_t lo = (fresh ? 0x41000000u : 0x01000000u) | (uint32_t)((3 - DY) * 32 + 3 - DX);
     const uint32_t key = __byte_perm(hs * ((2u * cell + 1u) * K2), g * gmul + lo, 0x7324);   // gmul = 1 << 24, or 0 in a noise step
     const bool valid = ((bit < 32 ? wt.x >> bit : wt.y >> (bit - 32)) & 1u) != 0;
     return valid ? key : 0u;
@@ -175,21 +213,35 @@ __device__ __forceinline__ uint32_t add_column(const Smem& sm, const Nbhd& N, ui
     return mx;
 }
 
-// The addition at the uncovered tile (N.x, N.y) that the kernel's fetch picked: the site of the best of the 25 candidates.
-// Sites removed fewer than `ten` steps ago are tabu; in a noise step every valid candidate ties on gain and freshness.
-template <class Smem, class Nbhd>
-__device__ __forceinline__ int add_site(const Smem& sm, int tid, const Nbhd& N, uint32_t hs, uint32_t step, int ten, bool noise) {
-    const int x = N.x, y = N.y;
-    uint32_t tw_lo = 0, tw_hi = 0;  // sites removed fewer than `ten` steps ago, as a byte-per-row window around t (rows 0-3 / 4-6)
-    for (int j = 0; j < ten; j++) {
-        const uint32_t e = sm.ring[(step - (uint32_t)j) & 31u][tid];
-        const int dx3 = (int)(e & 31u) - x + 3, dy3 = (int)(e >> 5) - y + 3;
-        if ((unsigned)dx3 < 7u && (unsigned)dy3 < 7u) {
-            const int bit = 8 * dy3 + dx3;       // byte-per-row window, like wt
-            tw_lo |= shl_clamped(1u, bit);
-            tw_hi |= shl_clamped(1u, bit - 32);
-        }
+// Removal-ring slots of the steps before this one that every step reads: a tenure is at least 2, and at most 4 at k <= 14
+// (effective_tenure), the 16x16 optimum plateau.  They do not depend on the step's own results, so the step loads them first.
+constexpr int RECENT = 3;
+
+// site e (NONE: none) into the tabu window around t = (x, y): a byte-per-row window like wt (rows 0-3 in lo, 4-6 in hi)
+__device__ __forceinline__ void tabu_bit(uint32_t e, int x, int y, uint32_t& lo, uint32_t& hi) {
+    const int dx3 = (int)(e & 31u) - x + 3, dy3 = (int)(e >> 5) - y + 3;
+    if ((unsigned)dx3 < 7u && (unsigned)dy3 < 7u) {
+        const int bit = 8 * dy3 + dx3;
+        lo |= shl_clamped(1u, bit);
+        hi |= shl_clamped(1u, bit - 32);
     }
+}
+
+// The addition at the uncovered tile (N.x, N.y) that the kernel's fetch picked: the site of the best of the 25 candidates.
+// Sites removed fewer than `ten` steps ago are tabu: `removed` in this step, recent[j] j + 1 steps ago, older ones in the
+// ring.  In a noise step every valid candidate ties on gain and freshness.
+template <class Smem, class Nbhd>
+__device__ __forceinline__ int add_site(const Smem& sm, int tid, const Nbhd& N, uint32_t hs, uint32_t step, int ten, bool noise, uint32_t removed,
+                                        const uint32_t (&recent)[RECENT], Prof& pf) {
+    const int x = N.x, y = N.y;
+    uint32_t tw_lo = 0, tw_hi = 0;
+    tabu_bit(removed, x, y, tw_lo, tw_hi);
+#pragma unroll
+    for (int j = 0; j < RECENT; j++)
+        if (j + 1 < ten) tabu_bit(recent[j], x, y, tw_lo, tw_hi);
+#pragma unroll 1
+    for (int j = RECENT + 1; j < ten; j++) tabu_bit(sm.ring[(step - (uint32_t)j) & 31u][tid], x, y, tw_lo, tw_hi);
+    pf.mark(PH_FETCH);
     const uint32_t fresh_lo = noise ? 0u : ~tw_lo, fresh_hi = noise ? 0u : ~tw_hi;
     const uint32_t gmul = noise ? 0u : 1u << 24;
     uint32_t mx = add_column<0>(sm, N, fresh_lo, fresh_hi, hs, gmul);
@@ -199,16 +251,14 @@ __device__ __forceinline__ int add_site(const Smem& sm, int tid, const Nbhd& N, 
     mx = max(mx, add_column<2>(sm, N, fresh_lo, fresh_hi, hs, gmul));
     mx = max(mx, add_column<-3>(sm, N, fresh_lo, fresh_hi, hs, gmul));
     mx = max(mx, add_column<3>(sm, N, fresh_lo, fresh_hi, hs, gmul));
-    int dx, dy;
-    diamond_cell(31 - (int)(mx & 31u), dx, dy);   // the winning cell from the key's low bits
-    return (y + dy) * 32 + x + dx;
+    return (y + 3) * 32 + x + 3 - (int)(mx & 0xffu);   // the winning site from the key's low byte
 }
 
 // The kernel body.  K is the board representation:
 //   K::Smem, K::load(sm, tid, terrain_rows, rtabs, terrain)  shared memory and its set-up (table, terrain, boards, ring)
 //   K(sm, tid, sl, stride)                                    the chain's view of it and of its global site list `sl`
 //   start(S, step, rowmask) -> k                              site list and cover planes of the layout S
-//   remove(hs, step, stephi, young_below, k, rowmask)         the removal: scan, swap-remove, ring slot, flip
+//   remove(hs, stephi, young_below, k, rowmask, pf)           the removal: scan, swap-remove, flip; returns the removed site
 //   fetch(rowmask, hs) -> Nbhd                                the uncovered tile of an addition and U around it
 //   add(v, step, k, rowmask)                                  the addition of site v as list entry k
 //   list_to_rows(k, out)                                      the support rows of the list (rare path)
@@ -237,6 +287,8 @@ __device__ __forceinline__ void run_chains(const int tid, const uint32_t* __rest
     unsigned long long scored = 0;
     long long my_steps = 0;
     uint32_t flips = 0;   // supports added + removed
+    Prof pf;
+    pf.start();
 
     if (run) {
         const int epoch_bound = bounds[chains_per_terrain > 0 ? terrain : 0];
@@ -247,43 +299,59 @@ __device__ __forceinline__ void run_chains(const int tid, const uint32_t* __rest
         int best = st.best;
         uint32_t step = st.step, rowmask = 0;
         int k = R.start(st.S, step, rowmask);   // site list in row-major order (spec), stamps "half a period ago"
+        int limit = min(epoch_bound, best);
+        uint32_t hs = step_hash(base, step);
 
         for (long long it = 0; it < steps; it++) {
             if ((it & 1023) == 1023 && *interrupt) break;
-            const int limit = min(epoch_bound, best);
-            const uint32_t hs = step_hash(base, step);
             const int ten = effective_tenure(tenure, k);
             const bool drop = k >= limit;
             if (drop && k == 0) { done = 1; break; }
-            sm.ring[step & 31u][tid] = (uint16_t)NONE;  // every consumed step owns its slot (stale entries are 32 steps old)
+            // the ring slots of earlier steps and the next step's hash depend on nothing this step computes: issued first, their
+            // latency overlaps the removal scan instead of waiting in the addition's (and the next step's) dependent chain
+            uint32_t recent[RECENT];
+#pragma unroll
+            for (int j = 0; j < RECENT; j++) recent[j] = sm.ring[(step - 1u - (uint32_t)j) & 31u][tid];
+            const uint32_t hs_next = step_hash(base, step + 1u);
             if (!drop && rowmask == 0) {  // complete layout with k < limit supports
+                sm.ring[step & 31u][tid] = (uint16_t)NONE;  // every consumed step owns its slot (stale entries are 32 steps old)
                 best = k;
+                limit = min(epoch_bound, best);
                 R.list_to_rows(k, st.bestS);
                 step++; my_steps++;
+                hs = hs_next;
                 if (k <= target || k == 0) { done = 1; break; }
                 continue;
             }
+            uint32_t removed = NONE;
             if (drop || (k > 0 && k == limit - 1)) {
                 // ---- removal: min-loss support, random ties; supports younger than the tenure only as a last resort (not when
                 // dropping)
                 const uint32_t stephi = (step << 16) | 0xffffu;
                 const uint32_t young_below = drop ? 0u : (uint32_t)ten << 16;
-                R.remove(hs, step, stephi, young_below, k, rowmask);
+                pf.mark(PH_FRAME);
+                removed = (uint32_t)R.remove(hs, stephi, young_below, k, rowmask, pf);
+                pf.mark(PH_RFLIP);
                 scored += (unsigned)k;
                 k--;
                 flips++;
             }
+            sm.ring[step & 31u][tid] = (uint16_t)removed;
             if (!drop) {
                 // ---- addition at a random uncovered tile t: best-gain site of R(t)
+                pf.mark(PH_FRAME);
                 const auto N = R.fetch(rowmask, hs);
                 const bool noise = ((hs >> 10) & 127u) < nq7;
-                const int v = add_site(sm, tid, N, hs, step, ten, noise);
+                const int v = add_site(sm, tid, N, hs, step, ten, noise, removed, recent, pf);
+                pf.mark(PH_CAND);
                 R.add(v, step, k, rowmask);
+                pf.mark(PH_AFLIP);
                 if (!noise) scored += (unsigned)(__popc(N.wt.x) + __popc(N.wt.y));
                 k++;
                 flips++;
             }
             step++; my_steps++;
+            hs = hs_next;
         }
 
         R.list_to_rows(k, st.S);
@@ -292,6 +360,7 @@ __device__ __forceinline__ void run_chains(const int tid, const uint32_t* __rest
         st.scored_lo = (uint32_t)tot; st.scored_hi = (uint32_t)(tot >> 32);
         st.steps_done += (uint32_t)my_steps;
     }
+    pf.flush((unsigned long long)my_steps);
     // one pair of atomics per warp
     unsigned long long a = scored, b = (unsigned long long)my_steps, c = (unsigned long long)flips;
 #pragma unroll
