@@ -336,7 +336,8 @@ int tss_solve_batch(tss_engine* e, const uint8_t* grids, int32_t w, int32_t h, i
 typedef struct tss_instance_info {
     int32_t w, h, n_defs;            /* terrain size and platform set of the encoding */
     int32_t card_limit_1x1;          /* n of "at most n platforms" (PlatformLimits.card_limits[1x1], main.rs:346), -1 if none */
-    int32_t n_other_card_limits;     /* card limits on other platform types (the search does not steer by those) */
+    int32_t n_other_card_limits;     /* card limits on other platform types (per-type limits: tss_solve_instance steers the search by
+                                        them on grids up to 32x32 when the handle came from tss_instance_find) */
     int32_t has_weight_limit;
     int64_t weight_limit;            /* PlatformLimits.weight_limit (crates/gui/src/app.rs:235-245) */
     int32_t n_weights;
@@ -382,6 +383,36 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
  * out[0] LOP3 Gop/s (thread-ops), out[1] POPC Gop/s, out[2] SHFL Gop/s, out[3] shared-memory GB/s, out[4] SM clock MHz
  * observed (cycles / elapsed). */
 int tss_measure_peaks(tss_engine* e, double* out, int32_t n_out);
+
+/* ------------------------------------------------------------------------------------------ per-type platform limits */
+/* The REPL's `solve -l k:v[,k:v]` (PlatformLimits.card_limits beyond 1x1, crates/repl/src/main.rs:85-101), as
+ * Encoding::with_limits lowers a limit on type d: one literal per anchor, set by a platform of any dims key q that contains d or
+ * its transpose (d's CLASS: the keys q with dims_le(k, q) for a key k in {d, d^T}).  A platform counts at most once towards a
+ * class.  A record whose d and d^T are both absent from the platform set constrains nothing, nor does a limit of 1024 or more:
+ * such records are VACUOUS and ignored.  Records are (def_w, def_h, limit), the `card` argument of tss_encoding_with_limits.
+ *
+ * The classes themselves, host only: key_mask[k] (capacity 16) = classes of dims key k in the engine's key order (defs order,
+ * unflipped then flipped, duplicates dropped; tss_search_read_placements reports it), bit j = class j; class_limit[j]
+ * (capacity 16).  1x1 records (the platform count) and vacuous records make no class; records with the same class merge into
+ * the smaller limit. */
+int tss_card_limit_classes(const tss_dims* defs, int32_t n_defs, const int32_t* card, int32_t n_card, int32_t* key_mask, int32_t* class_limit,
+                           int32_t* n_keys, int32_t* n_classes);
+/* Steers a placement search by per-type limits: an addition that would take a class beyond its limit is no candidate, so every
+ * current and best layout of every chain keeps every limit (a limit of 0 blocks its class from the start).  Call before the
+ * first tss_search_run.  TSS_E_INVALID for a 1x1 record (the platform count is the search's bound: tss_search_set_bound), a
+ * negative limit, or after the first run; vacuous records are ignored (on a {1x1}-only set every record is); TSS_E_UNSUPPORTED
+ * for a record that is not vacuous on a search other than the placement search on a grid up to 32x32 (the window searches:
+ * their windows pick winners independently, which could jointly exceed a limit). */
+int tss_search_set_card_limits(tss_search* s, const int32_t* card, int32_t n_card);
+/* The PlatformLimits-shaped one-shot solve: card = records (def_w, def_h, limit) including the platform count (1x1); with
+ * weights (n_weights > 0) the objective is the total weight, bounded by weight_limit (< 0: unbounded), and a 1x1 record is
+ * TSS_E_UNSUPPORTED (one objective per search).  Defs in a class with limit 0 are dropped from the set first (as --platforms
+ * would), positive limits steer the placement search (tss_search_set_card_limits; grids up to 32x32).  Budgets and the return
+ * contract are tss_solve_upper_bound's: TSS_SAT with the layout and *out_objective (optional) = its count or weight, TSS_UNKNOWN
+ * if none was found, never TSS_UNSAT. */
+int tss_solve_with_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
+                          int32_t n_card, const int32_t* weights, int32_t n_weights, int64_t weight_limit, uint64_t seed, int32_t budget_ms,
+                          int64_t max_steps, tss_platform* out, int32_t cap, int32_t* n_out, int64_t* out_objective);
 
 #ifdef __cplusplus
 }

@@ -212,6 +212,16 @@ unsafe extern "C" {
         n_keys: *mut i32,
     ) -> c_int;
     pub fn tss_search_set_weights(s: *mut tss_search, weights: *const i32, n_weights: i32) -> c_int;
+    pub fn tss_search_set_card_limits(s: *mut tss_search, card: *const i32, n_card: i32) -> c_int;
+    pub fn tss_card_limit_classes(
+        defs: *const tss_dims, n_defs: i32, card: *const i32, n_card: i32, key_mask: *mut i32, class_limit: *mut i32, n_keys: *mut i32,
+        n_classes: *mut i32,
+    ) -> c_int;
+    pub fn tss_solve_with_limits(
+        e: *mut tss_engine, grid: *const u8, w: i32, h: i32, defs: *const tss_dims, n_defs: i32, card: *const i32, n_card: i32,
+        weights: *const i32, n_weights: i32, weight_limit: i64, seed: u64, budget_ms: i32, max_steps: i64, out: *mut tss_platform, cap: i32,
+        n_out: *mut i32, out_objective: *mut i64,
+    ) -> c_int;
     pub fn tss_sls_spec_probe(out: *mut u32);
     pub fn tss_solve_batch(
         e: *mut tss_engine, grids: *const u8, w: i32, h: i32, n: i64, seed: u64, steps: i64, chains_per_terrain: i32, out_counts: *mut i32,

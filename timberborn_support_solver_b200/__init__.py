@@ -6,7 +6,7 @@ the built library; creating an Engine needs a CUDA device.  There is no CPU fall
 """
 from ._lib import LIB_PATH, SIGNATURES, load  # noqa: F401
 from .api import (INTERRUPTED, KERNEL_AUTO, KERNEL_HALF_WARP, KERNEL_PAIR, KERNEL_THREAD, KERNEL_WARP, KERNEL_WINDOW_PLACEMENTS, PLATFORMS_DEFAULT, SAT, UNSAT, Cnf, DeviceCnf, Encoding, EncodingVars, Engine,  # noqa: F401
-                  GpuBoundSolver, Platform, PlatformDef, PlatformLayout, PlatformLimits, Project, Search, TssError,
+                  GpuBoundSolver, Platform, PlatformDef, PlatformLayout, PlatformLimits, Project, Search, TssError, card_limit_classes,
                   ValidationResult, World, WorldGrid, render_world, solver_loop, weight_loop)
 
 load()  # fail loudly at import time if libtss.so is missing or does not export every declared symbol

@@ -103,6 +103,9 @@ SIGNATURES = {
     "tss_search_set_weights": (C.c_int, [_vp, _i32p, _i32]),
     "tss_solve_min_weight": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i64, _u64, _i32, _i64, _P(Platform), _i32, _i32p, _i64p]),
     "tss_solve_upper_bound": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32, _u64, _i32, _i64, _P(Platform), _i32, _i32p]),
+    "tss_card_limit_classes": (C.c_int, [_P(Dims), _i32, _i32p, _i32, _i32p, _i32p, _i32p, _i32p]),
+    "tss_search_set_card_limits": (C.c_int, [_vp, _i32p, _i32]),
+    "tss_solve_with_limits": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32p, _i32, _i64, _u64, _i32, _i64, _P(Platform), _i32, _i32p, _i64p]),
     "tss_lower_bound": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _u64, _i32, _i32p, _i32, _i32p]),
     "tss_lower_bound_lp": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32, _i64, _i32p, _i64p, _i64p, _i64p, _i32p]),
     "tss_solve_batch": (C.c_int, [_vp, _u8p, _i32, _i32, _i64, _u64, _i64, _i32, _i32p, _u32p]),

@@ -436,6 +436,31 @@ class DeviceCnf:
         return a if rc == 10 else None
 
 
+def _card_records(limits: dict) -> np.ndarray:
+    return np.array([[d.width, d.height, v] for d, v in limits.items()], np.int32).reshape(-1, 3)
+
+
+def card_limit_classes(defs, limits: dict):
+    """The classes per-type limits constrain, as Encoding::with_limits lowers them (tss_card_limit_classes; host only):
+    limits {PlatformDef: limit} -> (key_dims [(w, h)] in the engine's key order, key_mask [int] per key (bit j = class j),
+    class_limit [int]).  1x1 and vacuous entries make no class."""
+    defs = list(defs)
+    card = _card_records(limits)
+    mask, lim = (C.c_int32 * 16)(), (C.c_int32 * 16)()
+    nk, nc = C.c_int32(), C.c_int32()
+    lib = _lib.load()
+    rc = lib.tss_card_limit_classes(_defs_array(defs), len(defs), _ptr(card, C.c_int32) if len(card) else None, len(card), mask, lim, C.byref(nk), C.byref(nc))
+    if rc < 0:
+        raise TssError(rc, "tss_card_limit_classes")
+    keys = []
+    for d in defs:
+        for k in ((d.width, d.height), (d.height, d.width)):
+            if k not in keys:
+                keys.append(k)
+    assert len(keys) == nk.value
+    return keys, [int(mask[i]) for i in range(nk.value)], [int(lim[j]) for j in range(nc.value)]
+
+
 class Search:
     """A device-resident SLS portfolio on one terrain (kernel (b))."""
 
@@ -496,6 +521,14 @@ class Search:
         """GUI objective (crates/gui/src/app.rs:53-62): {PlatformDef: weight}; the search then minimises total_weight."""
         wts = np.array([[d.width, d.height, v] for d, v in weights.items()], np.int32).reshape(-1, 3)
         self.engine._check(self.engine.lib.tss_search_set_weights(self._h, _ptr(wts, C.c_int32), len(wts)))
+
+    def set_card_limits(self, limits: dict):
+        """Per-type platform limits (`solve -l k:v`, PlatformLimits.card_limits without 1x1): {PlatformDef: limit}.  Additions that
+        would take a limit's class (card_limit_classes) beyond it are no candidates, so every layout of every chain keeps every
+        limit.  Call before the first run(); TssError for a 1x1 entry or a negative limit, and for a limit that is not vacuous on
+        anything but the placement search on a grid up to 32x32."""
+        card = _card_records(limits)
+        self.engine._check(self.engine.lib.tss_search_set_card_limits(self._h, _ptr(card, C.c_int32) if len(card) else None, len(card)))
 
     def read_placements(self) -> dict:
         """Per-chain state of the placement search (platform sets beyond {1x1}) after the last epoch."""
@@ -659,6 +692,23 @@ class Engine:
             return SAT, PlatformLayout(Platform._from_c(out[i]) for i in range(n.value)), wt.value
         return INTERRUPTED, None, None
 
+    def solve_with_limits(self, grid: WorldGrid, defs, limits: PlatformLimits, seed=0, budget_ms=0, max_steps=0):
+        """The PlatformLimits-shaped solve (tss_solve_with_limits): card_limits including the platform count (1x1) and per-type
+        limits; with weights the objective is the total weight, bounded by weight_limit (weights and a 1x1 limit together raise
+        TssError).  Budgets as solve_upper_bound.  -> (SAT | INTERRUPTED, PlatformLayout | None, objective | None)."""
+        defs = list(defs)
+        card = _card_records(limits.card_limits)
+        wts = _card_records(limits.weights)
+        out = (_Platform * (grid.data.size + 1))()
+        n, obj = C.c_int32(), C.c_int64()
+        wl = -1 if limits.weight_limit is None else limits.weight_limit
+        rc = self._check(self.lib.tss_solve_with_limits(self._h, _ptr(grid.data, C.c_uint8), grid.width, grid.height, _defs_array(defs), len(defs),
+                                                        _ptr(card, C.c_int32) if len(card) else None, len(card), _ptr(wts, C.c_int32) if len(wts) else None,
+                                                        len(wts), wl, seed, budget_ms, max_steps, out, len(out), C.byref(n), C.byref(obj)))
+        if rc == _lib.TSS_SAT:
+            return SAT, PlatformLayout(Platform._from_c(out[i]) for i in range(n.value)), obj.value
+        return INTERRUPTED, None, None
+
     def lower_bound(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], seed=0, restarts=0):
         """Packing lower bound (tss_lower_bound): -> list of (x, y) ceiling tiles no two of which one platform of `defs` can
         support; its length bounds the platform count of every complete layout from below."""
@@ -728,14 +778,19 @@ class GpuBoundSolver:
     def solve(self) -> str:  # Solve::solve
         """SAT with a CNF-verified witness, or INTERRUPTED = "the GPU could not answer within its budget" (which is also what a
         real interrupt returns).  The search is steered by the 1x1 card limit (= the platform count, what the REPL tightens,
-        main.rs:346) or by the weight limit (the GUI's objective, app.rs:235-245); limits on other platform types alone are
-        only enforced by the CNF check below, so such instances go to the exact solver."""
+        main.rs:346) or by the weight limit (the GUI's objective, app.rs:235-245), and by limits on other platform types
+        (`solve -l k:v`) on grids up to 32x32; elsewhere such instances go to the exact solver."""
         one = PlatformDef(1, 1)
         bound = self.limits.card_limits.get(one)
         self.engine.clear_interrupt()      # the flag is sticky by design (InterruptSolver::interrupt may fire before solve starts a kernel): one solve, one flag
+        weighted = bool(self.limits.weights) and (self.limits.weight_limit is not None or bound is None)
         if any(d != one for d in self.limits.card_limits):
-            return INTERRUPTED             # card limits the search cannot steer by: leave the instance to the exact solver
-        if self.limits.weights and (self.limits.weight_limit is not None or bound is None):
+            g = self.encoding._grid
+            if g.width > 32 or g.height > 32 or (weighted and bound is not None):
+                return INTERRUPTED         # limits the search cannot steer by here: leave the instance to the exact solver
+            lim = self.limits if weighted else PlatformLimits(dict(self.limits.card_limits), {}, None)
+            res, layout, _ = self.engine.solve_with_limits(g, self.encoding.defs, lim, self.seed, self.budget_ms, self.max_steps)
+        elif weighted:
             # the GUI's instances: weights always, a weight limit from the second iteration on (app.rs:235-245)
             res, layout, _ = self.engine.solve_min_weight(self.encoding._grid, self.encoding.defs, self.limits.weights, self.limits.weight_limit,
                                                           self.seed, self.budget_ms, self.max_steps)

@@ -28,6 +28,9 @@ struct tss_encoding_data {
 // a handle is a shared reference: the registry keeps encodings alive after the caller destroyed its own handle
 struct tss_encoding {
     std::shared_ptr<const tss_encoding_data> d;
+    // a handle from tss_instance_find: the recorded PlatformLimits.card_limits as (def_w, def_h, limit) records, 1x1 included
+    bool has_card_limits = false;
+    std::vector<int32_t> card_limits;
 };
 
 namespace tss {

@@ -80,7 +80,7 @@ int slsm_max_keys();
 int slsm_init(tss_engine* e, void* states, int n);
 int slsm_run(tss_engine* e, const uint32_t* rows_dev, int W, int H, const int2* keys_dev, const int* costs_dev, const int* order_dev, int n_keys, void* states, int n_chains,
              uint32_t chain_offset, uint64_t seed, long long steps, int* bounds_dev, int target, int noise_pct, unsigned long long* totals_dev,
-             int2* best_dev);
+             int2* best_dev, const int* limits_dev, int n_classes);
 int slsm_read_best(tss_engine* e, const void* states, int chain, std::vector<uint16_t>& codes);
 int slsm_run_oneshot(tss_engine* e, const uint32_t* rows32_host, int bound, uint32_t* rows_dev, int W, int H, const int2* keys_dev, const int* costs_dev,
                      const int* order_dev, int n_keys, void* states, int n_chains, uint64_t seed, long long steps, int* bounds_dev, int2* best_dev,
@@ -203,7 +203,9 @@ struct tss_search {
     std::vector<tss_platform> key_proto;       // def dims + rotated flag per key
     std::vector<int> key_costs;                // objective cost per key: 1 = platform count; GUI weights via tss_search_set_weights
     int2* keys_dev = nullptr;
-    int* costs_dev = nullptr;
+    int* costs_dev = nullptr;                  // [4][MAX_KEYS]: costs | keys by area | class mask per key | limit per class
+    int n_classes = 0;                         // per-type limits (tss_search_set_card_limits): classes in costs_dev; 0 = none
+    bool started = false;                      // tss_search_run was called
     void* mstates = nullptr;
     // in-stream witness of one-shot solves: codes u16[1024], (x, y, w, h) records, misc = offsets[2] + evaluator result[4]
     std::vector<tss_platform> greedy_plats;    // grids > 32x32, platform sets beyond {1x1}: the greedy placement cover (computed once, it only depends on the terrain)
@@ -649,6 +651,42 @@ static std::vector<int> keys_by_area(const std::vector<int2>& key_dims) {
     return order;
 }
 
+// The classes of per-type platform limits (PlatformLimits.card_limits beyond 1x1), as Encoding::with_limits
+// (host_model.cpp, encoder.rs:619-667) lowers them: a limit on type d counts one literal per anchor, set by the plat var of
+// key d (square d) or implied by those of keys d and its transpose (rectangular d); a platform sets the plat var of every key
+// contained in its dims (tss_layout_to_assignment).  So class C_d = the keys q with dims_le(k, q) for some key k in {d, d^T},
+// closed under rotation, and a platform counts at most once towards it.  A record with neither d nor d^T among the keys emits
+// no constraint, nor does a limit of MAX_ITEMS or more: both are vacuous and skipped.  1x1 records (the platform count, whose
+// class is every key) are skipped as well: their callers treat them on their own.  Records with the same class merge into one
+// with the smaller limit.  -> key_mask[k] = classes of key k (bit j = class j), class_limit[j]; at most MAX_KEYS classes.
+static int card_limit_classes(const std::vector<int2>& key_dims, const int32_t* card, int n_card, std::vector<uint32_t>& key_mask,
+                              std::vector<int>& class_limit) {
+    key_mask.assign(key_dims.size(), 0u);
+    class_limit.clear();
+    std::vector<uint32_t> members;   // keys of each class (bit k)
+    for (int i = 0; i < n_card; i++) {
+        const int dw = card[3 * i], dh = card[3 * i + 1], lim = card[3 * i + 2];
+        if (dw <= 0 || dh <= 0 || lim < 0) return TSS_E_INVALID;
+        if ((dw == 1 && dh == 1) || lim >= slsm_max_items()) continue;
+        uint32_t m = 0;
+        for (size_t k = 0; k < key_dims.size(); k++) {
+            if (!((key_dims[k].x == dw && key_dims[k].y == dh) || (key_dims[k].x == dh && key_dims[k].y == dw))) continue;
+            for (size_t q = 0; q < key_dims.size(); q++)
+                if (dims_le(Dims{key_dims[k].x, key_dims[k].y}, Dims{key_dims[q].x, key_dims[q].y})) m |= 1u << q;
+        }
+        if (!m) continue;
+        const size_t j = std::find(members.begin(), members.end(), m) - members.begin();
+        if (j < members.size()) { class_limit[j] = std::min(class_limit[j], lim); continue; }
+        if ((int)members.size() == slsm_max_keys()) return TSS_E_UNSUPPORTED;
+        members.push_back(m);
+        class_limit.push_back(lim);
+    }
+    for (size_t j = 0; j < members.size(); j++)
+        for (size_t k = 0; k < key_dims.size(); k++)
+            if ((members[j] >> k) & 1u) key_mask[k] |= 1u << j;
+    return TSS_OK;
+}
+
 static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds);
 
 // Chains that fill the device: 32 warps per SM for the warp kernels (two chains per warp on grids of <= 16 rows),
@@ -742,7 +780,7 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
         } else {
             err = cudaMalloc(&s->rows_dev, sizeof rows);
             if (err == cudaSuccess) err = cudaMalloc(&s->keys_dev, sizeof(int2) * (size_t)slsm_max_keys());
-            if (err == cudaSuccess) err = cudaMalloc(&s->costs_dev, sizeof(int) * 2 * (size_t)slsm_max_keys());   // costs | keys ordered by area
+            if (err == cudaSuccess) err = cudaMalloc(&s->costs_dev, sizeof(int) * 4 * (size_t)slsm_max_keys());   // costs | keys by area | limit classes
             if (err == cudaSuccess) err = cudaMalloc(&s->mstates, slsm_state_bytes() * (size_t)s->n_chains);
             if (err == cudaSuccess) err = cudaMalloc(&s->totals_dev, sizeof(unsigned long long) * 3);
             if (err == cudaSuccess) err = cudaMalloc(&s->best_dev, sizeof(int2));
@@ -831,6 +869,7 @@ int tss_search_run(tss_search* s, int64_t steps, int32_t target_count) {
     tss_engine* e = s->e;
     if (steps <= 0) return e->fail(TSS_E_INVALID, "tss_search_run: steps must be positive");
     TSS_CUDA(e, cudaSetDevice(e->device));
+    s->started = true;
     TSS_CUDA(e, cudaEventRecord(e->ev0, e->stream));
     if (s->lns || s->lnsp) {  // one phase of the window decomposition (a phase is one epoch per window: at most MAX_EPOCH_STEPS, see below)
         for (long long left = steps; left > 0; left -= sls::MAX_EPOCH_STEPS) {
@@ -846,7 +885,7 @@ int tss_search_run(tss_search* s, int64_t steps, int32_t target_count) {
     }
     if (s->multi) {
         int rc = slsm_run(e, s->rows_dev, s->w, s->h, s->keys_dev, s->costs_dev, s->costs_dev + slsm_max_keys(), (int)s->key_dims.size(), s->mstates, s->n_chains, s->chain_offset, s->seed, steps,
-                          s->bounds_dev, target_count < 0 ? -1 : target_count, s->noise, s->totals_dev, s->best_dev);
+                          s->bounds_dev, target_count < 0 ? -1 : target_count, s->noise, s->totals_dev, s->best_dev, s->costs_dev + 2 * slsm_max_keys(), s->n_classes);
         if (rc == TSS_OK && e->comm && s->share) rc = comm_allreduce_min(e, e->comm, s->bounds_dev, 1);
         if (rc) return rc;
         TSS_CUDA(e, cudaEventRecord(e->ev1, e->stream));
@@ -1310,6 +1349,51 @@ int tss_search_set_weights(tss_search* s, const int32_t* weights, int32_t n_weig
     return TSS_OK;
 }
 
+int tss_card_limit_classes(const tss_dims* defs, int32_t n_defs, const int32_t* card, int32_t n_card, int32_t* key_mask, int32_t* class_limit,
+                           int32_t* n_keys, int32_t* n_classes) {
+    if ((n_defs > 0 && !defs) || n_defs < 0 || n_card < 0 || (n_card > 0 && !card) || !key_mask || !class_limit || !n_keys || !n_classes) return TSS_E_INVALID;
+    std::vector<int2> kd;
+    std::vector<tss_platform> kp;
+    build_keys(defs, n_defs, kd, kp);
+    if ((int)kd.size() > slsm_max_keys()) return TSS_E_UNSUPPORTED;
+    std::vector<uint32_t> mask;
+    std::vector<int> lim;
+    const int rc = card_limit_classes(kd, card, n_card, mask, lim);
+    if (rc) return rc;
+    for (size_t k = 0; k < kd.size(); k++) key_mask[k] = (int32_t)mask[k];
+    for (size_t j = 0; j < lim.size(); j++) class_limit[j] = lim[j];
+    *n_keys = (int32_t)kd.size();
+    *n_classes = (int32_t)lim.size();
+    return TSS_OK;
+}
+
+int tss_search_set_card_limits(tss_search* s, const int32_t* card, int32_t n_card) {
+    if (!s) return TSS_E_INVALID;
+    tss_engine* e = s->e;
+    if (n_card < 0 || (n_card > 0 && !card)) return e->fail(TSS_E_INVALID, "tss_search_set_card_limits: bad arguments");
+    if (s->started) return e->fail(TSS_E_INVALID, "tss_search_set_card_limits: call it before the first tss_search_run");
+    for (int i = 0; i < n_card; i++) {
+        if (card[3 * i] == 1 && card[3 * i + 1] == 1)
+            return e->fail(TSS_E_INVALID, "tss_search_set_card_limits: the platform count (1x1) is the search's bound, not a per-type limit");
+        if (card[3 * i + 2] < 0) return e->fail(TSS_E_INVALID, "tss_search_set_card_limits: negative limit for %dx%d", card[3 * i], card[3 * i + 1]);
+    }
+    std::vector<uint32_t> mask;
+    std::vector<int> lim;
+    int rc = card_limit_classes(s->key_dims, card, n_card, mask, lim);
+    if (rc) return e->fail(rc, "tss_search_set_card_limits: bad limit records");
+    if (lim.empty()) return TSS_OK;   // every record vacuous (e.g. on a {1x1}-only set)
+    if (!s->multi)
+        return e->fail(TSS_E_UNSUPPORTED, "tss_search_set_card_limits: per-type limits need the placement search (a platform set beyond {1x1} on a grid up to 32x32)");
+    rc = search_sync(s);
+    if (rc) return rc;
+    std::vector<int> dev(2 * (size_t)slsm_max_keys(), 0);
+    for (size_t k = 0; k < mask.size(); k++) dev[k] = (int)mask[k];
+    for (size_t j = 0; j < lim.size(); j++) dev[(size_t)slsm_max_keys() + j] = lim[j];
+    TSS_CUDA(e, cudaMemcpy(s->costs_dev + 2 * slsm_max_keys(), dev.data(), sizeof(int) * dev.size(), cudaMemcpyHostToDevice));
+    s->n_classes = (int)lim.size();
+    return TSS_OK;
+}
+
 int tss_solve_min_weight(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
                          const int32_t* weights, int32_t n_weights, int64_t weight_limit, uint64_t seed, int32_t budget_ms,
                          int64_t max_steps, tss_platform* out, int32_t cap, int32_t* n_out, int64_t* out_weight) {
@@ -1359,11 +1443,27 @@ int tss_solve_min_weight(tss_engine* e, const uint8_t* grid, int32_t w, int32_t 
     return rc != TSS_OK ? rc : result;
 }
 
-int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
-                          int32_t card_limit, uint64_t seed, int32_t budget_ms, int64_t max_steps, tss_platform* out,
-                          int32_t cap, int32_t* n_out) {
+// The one-shot solve behind tss_solve_upper_bound and tss_solve_with_limits: a layout whose objective (platform count, or total
+// weight with `weights`) is at most `limit` (< 0: unbounded) and that keeps the per-type limits `card` (records without 1x1,
+// see tss_search_set_card_limits).  *out_objective = the objective of the layout returned.
+static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, int64_t limit,
+                        const int32_t* weights, int32_t n_weights, const int32_t* card, int32_t n_card, uint64_t seed, int32_t budget_ms,
+                        int64_t max_steps, tss_platform* out, int32_t cap, int32_t* n_out, int64_t* out_objective) {
     if (!e) return TSS_E_INVALID;
     if (n_out) *n_out = 0;
+    const int32_t card_limit = limit < 0 ? -1 : (int32_t)std::min<int64_t>(limit, sls::NO_BOUND - 1);
+    // weights and limits live in the search's own buffers: only the plain count objective may take the fused first epochs
+    bool limited = false;
+    if (n_card > 0) {
+        std::vector<int2> kd;
+        std::vector<tss_platform> kp;
+        std::vector<uint32_t> mask;
+        std::vector<int> lim;
+        build_keys(defs, n_defs, kd, kp);
+        if (card_limit_classes(kd, card, n_card, mask, lim) != TSS_OK) return e->fail(TSS_E_INVALID, "tss_solve_with_limits: bad limit records");
+        limited = !lim.empty();
+    }
+    const bool plain = n_weights <= 0 && !limited;
     // One SAT-like call (no budget, no step count: return the first model within the bound) is latency bound: few
     // chains per SM step fastest (measured on rect 16x16, profiles/tto_sweep.py: 16 chains per SM on the half-warp kernel
     // 0.23 ms, 64 per SM 0.34 ms, 128 per SM 0.50 ms per call).  A call with an effort budget is throughput bound: the
@@ -1390,7 +1490,7 @@ int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t
     }
     int64_t fused_steps = 0;   // steps already executed by the fused first epoch
     int fused_best = -1;
-    if (e->cached_search && grid && w > 0 && h > 0 && w <= 32 && h <= 32 && only_1x1) {
+    if (e->cached_search && grid && w > 0 && h > 0 && w <= 32 && h <= 32 && only_1x1 && plain) {
         // reuse the engine's workspace: same buffers, fresh terrain / reach table / chain states (no allocation)
         TSS_CUDA(e, cudaSetDevice(e->device));   // (before the workspace is detached: an early return must not leak it)
         s = e->cached_search;
@@ -1452,7 +1552,7 @@ int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t
             }
         }
         if (rc != TSS_OK) { search_free(s); return rc; }
-    } else if (!only_1x1 && multi_chains > 0 && grid && defs && w > 0 && h > 0 && e->cached_multi && e->cached_multi->n_chains == multi_chains &&
+    } else if (!only_1x1 && plain && multi_chains > 0 && grid && defs && w > 0 && h > 0 && e->cached_multi && e->cached_multi->n_chains == multi_chains &&
                !e->interrupted()) {
         // placement search, first-model mode, workspace of the SAME platform set cached (keys, costs and their order are
         // already on the device): the first epoch as one fused launch (sls_multi.cu OneShotM)
@@ -1517,7 +1617,9 @@ int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t
         if (rc) return rc;
     }
     s->share = false;  // a one-shot solve runs a rank-local number of epochs: no collective inside
-    if (card_limit >= 0 && fused_steps == 0) rc = tss_search_set_bound(s, card_limit + 1);   // (the fused epoch took its bound as a parameter)
+    if (n_weights > 0) rc = tss_search_set_weights(s, weights, n_weights);
+    if (rc == TSS_OK && limited) rc = tss_search_set_card_limits(s, card, n_card);
+    if (rc == TSS_OK && card_limit >= 0 && fused_steps == 0) rc = tss_search_set_bound(s, card_limit + 1);   // (the fused epoch took its bound as a parameter)
     const double t0 = now_ms();
     // no budget given: behave like one SAT call (return the first model within the bound), but give up after a
     // default effort — the engine cannot prove UNSAT, so "no model found" must not turn into an endless search
@@ -1564,6 +1666,7 @@ int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t
         if (budget_ms > 0 && now_ms() - t0 >= budget_ms) break;
     }
     e->stats.last_solve_steps = done_steps;
+    if (rc == TSS_OK && best >= 0 && out_objective) *out_objective = best;
     int result = TSS_UNKNOWN;
     if (rc == TSS_OK && best >= 0 && in_stream_witness) {
         // the witness of the last epoch, already validated on the device (witness_kernel / the fused epoch's last CTA):
@@ -1617,11 +1720,56 @@ int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t
         e->cached_search = s;  // keep the workspace for the next call
     } else if (s->multi && !e->cached_multi && rc == TSS_OK) {
         cudaStreamSynchronize(e->stream);
+        s->n_classes = 0;      // (a later solve without limits may run on this workspace as it stands: the fused path above)
         e->cached_multi = s;   // (tss_search_create adopts its buffers)
     } else {
         tss_search_destroy(s);
     }
     return rc != TSS_OK ? rc : result;
+}
+
+int tss_solve_upper_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
+                          int32_t card_limit, uint64_t seed, int32_t budget_ms, int64_t max_steps, tss_platform* out,
+                          int32_t cap, int32_t* n_out) {
+    return solve_search(e, grid, w, h, defs, n_defs, card_limit, nullptr, 0, nullptr, 0, seed, budget_ms, max_steps, out, cap, n_out, nullptr);
+}
+
+int tss_solve_with_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
+                          int32_t n_card, const int32_t* weights, int32_t n_weights, int64_t weight_limit, uint64_t seed, int32_t budget_ms,
+                          int64_t max_steps, tss_platform* out, int32_t cap, int32_t* n_out, int64_t* out_objective) {
+    if (!e) return TSS_E_INVALID;
+    if (n_out) *n_out = 0;
+    if (!grid || w <= 0 || h <= 0 || n_defs < 0 || (n_defs > 0 && !defs) || n_card < 0 || (n_card > 0 && !card) || n_weights < 0 || (n_weights > 0 && !weights))
+        return e->fail(TSS_E_INVALID, "tss_solve_with_limits: bad arguments");
+    int32_t count_limit = -1;   // PlatformLimits.card_limits[1x1]: the platform count
+    std::vector<int32_t> other;
+    for (int i = 0; i < n_card; i++) {
+        if (card[3 * i + 2] < 0) return e->fail(TSS_E_INVALID, "tss_solve_with_limits: negative limit for %dx%d", card[3 * i], card[3 * i + 1]);
+        if (card[3 * i] == 1 && card[3 * i + 1] == 1) count_limit = count_limit < 0 ? card[3 * i + 2] : std::min(count_limit, card[3 * i + 2]);
+        else other.insert(other.end(), card + 3 * i, card + 3 * i + 3);
+    }
+    if (n_weights > 0 && count_limit >= 0)
+        return e->fail(TSS_E_UNSUPPORTED, "tss_solve_with_limits: the search minimises one objective: total weight or the platform count, not both");
+    // A limit of 0 removes its class from the platform set, exactly as a smaller --platforms would: the reduced set runs the
+    // kernels of that set (down to the 1x1 search), and only positive limits reach the placement search's class counters.
+    std::vector<int2> kd;
+    std::vector<tss_platform> kp;
+    std::vector<uint32_t> mask;
+    std::vector<int> lim;
+    build_keys(defs, n_defs, kd, kp);
+    const int n_other = (int)other.size() / 3;
+    int rc = card_limit_classes(kd, other.data(), n_other, mask, lim);
+    if (rc) return e->fail(rc, "tss_solve_with_limits: bad limit records");
+    uint32_t zero = 0;   // classes with limit 0
+    for (size_t j = 0; j < lim.size(); j++) zero |= lim[j] == 0 ? 1u << j : 0u;
+    std::vector<tss_dims> kept;
+    for (int i = 0; i < n_defs; i++) {
+        bool drop = false;
+        for (size_t k = 0; k < kd.size(); k++) drop = drop || (kd[k].x == defs[i].w && kd[k].y == defs[i].h && (mask[k] & zero));
+        if (!drop) kept.push_back(defs[i]);
+    }
+    return solve_search(e, grid, w, h, kept.data(), (int32_t)kept.size(), n_weights > 0 ? weight_limit : (int64_t)count_limit, weights, n_weights,
+                        other.data(), n_other, seed, budget_ms, max_steps, out, cap, n_out, out_objective);
 }
 
 int tss_lower_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, uint64_t seed,

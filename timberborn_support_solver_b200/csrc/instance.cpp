@@ -81,6 +81,8 @@ int tss_instance_find(const int32_t* lits, const uint32_t* offsets, int32_t n_cl
     tss_encoding* enc = new (std::nothrow) tss_encoding();
     if (!enc) return TSS_E_INVALID;
     enc->d = hit->d;
+    enc->has_card_limits = true;
+    for (const auto& c : hit->limits.card_limits) enc->card_limits.insert(enc->card_limits.end(), {c.def.w, c.def.h, (int32_t)std::min(c.value, (long)INT32_MAX)});
     *enc_out = enc;
     info->w = hit->d->enc.w;
     info->h = hit->d->enc.h;
@@ -152,8 +154,11 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
                        uint64_t seed, int64_t give_up_steps, uint8_t* assignment) {
     if (!e) return TSS_E_INVALID;
     if (!c || !enc || !info || !assignment) return e->fail(TSS_E_INVALID, "tss_solve_instance: bad arguments");
-    if (info->n_other_card_limits > 0) return TSS_UNKNOWN;   // limits the search cannot steer by: leave the instance to the exact solver
     const Encoding& E = enc->d->enc;
+    // per-type limits: the placement search steers by the limits recorded on a handle of tss_instance_find, on grids up to 32x32,
+    // with one objective (the platform count or the total weight); anything else is left to the exact solver
+    const bool per_type = info->n_other_card_limits > 0;
+    if (per_type && (!enc->has_card_limits || E.w > 32 || E.h > 32 || (info->has_weight_limit && info->card_limit_1x1 >= 0))) return TSS_UNKNOWN;
     std::vector<tss_dims> defs;
     for (const Dims& d : E.defs) defs.push_back(tss_dims{d.w, d.h});
     // A limit below a CERTIFIED lower bound has no model: answer UNSAT without searching.  Only when the platform count is the
@@ -183,7 +188,13 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
     int32_t n = 0;
     auto search = [&](int64_t give_up, uint64_t sd) -> int {   // a SAT-like call with a give-up point (tss.h)
         int r;
-        if (info->has_weight_limit && info->n_weights > 0 && weights) {
+        if (per_type) {
+            const bool weighted = info->has_weight_limit && info->n_weights > 0 && weights;
+            int64_t obj = 0;
+            r = tss_solve_with_limits(e, enc->d->grid.data(), E.w, E.h, defs.data(), (int32_t)defs.size(), enc->card_limits.data(),
+                                      (int32_t)(enc->card_limits.size() / 3), weighted ? weights : nullptr, weighted ? info->n_weights : 0,
+                                      weighted ? info->weight_limit : -1, sd, 0, give_up > 0 ? -give_up : 0, plats.data(), (int32_t)plats.size(), &n, &obj);
+        } else if (info->has_weight_limit && info->n_weights > 0 && weights) {
             int64_t wt = 0;
             r = tss_solve_min_weight(e, enc->d->grid.data(), E.w, E.h, defs.data(), (int32_t)defs.size(), weights, info->n_weights, info->weight_limit, sd, 0,
                                      give_up > 0 ? give_up : 0, plats.data(), (int32_t)plats.size(), &n, &wt);

@@ -181,20 +181,34 @@ struct OneShotM {
                                   // from word 16: the n placement codes as u16
 };
 
+// LIMITS = per-type platform limits (`solve -l k:v`, PlatformLimits.card_limits beyond 1x1; tss_search_set_card_limits): class j
+// of the limits holds the keys whose platforms count towards limit j (tss::card_limit_classes), mask[key] is the set of classes
+// of a key.  Lane j keeps n_j, the platforms of the current layout in class j (recounted from the item list at every launch),
+// and `full` = { j : n_j >= limit[j] } is one ballot after every flip.  An addition whose key lies in a full class is not a
+// candidate, and the swap trigger takes its minimum cost over the keys that are not blocked.  Chains start empty, so every
+// current and every best layout keeps every limit.
+struct LimitsM {
+    const int* mask;              // [n_keys] classes of each key (bit j = class j)
+    const int* limit;             // [n_classes] at most limit[j] platforms in class j (>= 1)
+    int n_classes;                // <= MAX_KEYS
+};
+
 // WINDOW = the window-decomposed placement search on grids larger than 32x32 (lns_placements.cu, see WindowM): chain c works
 // on window c / seeds, `terrain_rows` holds 32 ceiling rows per window and the epoch bound is bounds[window].
 // (WINDOW: at most 4 CTAs per SM, i.e. up to 128 registers — the window's need rows and box do not fit the 96 registers the
-// compiler settles for otherwise without spilling; a phase on 256x256 launches ~1300 chains, 2-3 CTAs per SM)
-template <bool ONESHOT, bool WINDOW>
-__global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(const uint32_t* __restrict__ terrain_rows, int W, int H,
+// compiler settles for otherwise without spilling; a phase on 256x256 launches ~1300 chains, 2-3 CTAs per SM.  LIMITS: the
+// same, for the class counters; an epoch launches 16 chains = 4 CTAs per SM)
+template <bool ONESHOT, bool WINDOW, bool LIMITS>
+__global__ void __launch_bounds__(WARPS * 32, (WINDOW || LIMITS) ? 4 : 0) sls_multi_kernel(const uint32_t* __restrict__ terrain_rows, int W, int H,
                                                               const int2* __restrict__ keys_g, const int* __restrict__ costs_g,
                                                               const int* __restrict__ order_g, int n_keys,
                                                               MultiState* __restrict__ states,
                                                               int n_chains, uint32_t chain_offset, uint64_t seed, long long steps,
                                                               const int* __restrict__ bounds, int target, int noise_pct,
                                                               const volatile int* interrupt, unsigned long long* __restrict__ totals,
-                                                              const OneShotM os, const WindowM wm) {
+                                                              const OneShotM os, const WindowM wm, const LimitsM lm) {
     static_assert(!(ONESHOT && WINDOW), "a one-shot solve never runs on windows");
+    static_assert(!LIMITS || (!ONESHOT && !WINDOW), "per-type limits run on the epoch kernel only");
     __shared__ uint16_t items_all[WARPS][MAX_ITEMS];
     __shared__ int2 keys[MAX_KEYS];
     __shared__ int costs[MAX_KEYS];
@@ -237,6 +251,11 @@ __global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(c
     for (int i = lane; i < k; i += 32) c.items[i] = st.items[i];
     __syncwarp();
     int Wt = 0;  // total cost of the current layout
+    // LIMITS: lane i < n_keys holds key i's class mask and cost, lane j < n_classes holds n_j and limit[j]
+    const uint32_t kmask = LIMITS && lane < n_keys ? (uint32_t)lm.mask[lane] : 0u;
+    const int kcost = LIMITS && lane < n_keys ? costs[lane] : 0x7fffffff;
+    const int climit = LIMITS && lane < lm.n_classes ? lm.limit[lane] : 0x7fffffff;
+    int ncls = 0;
     for (int i = 0; i < k; i++) {
         int x, y, w, h;
         unpack(c, c.items[i], x, y, w, h);
@@ -245,8 +264,18 @@ __global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(c
         planes_add(L, reach);
         L.Occ |= foot;
         Wt += costs[c.items[i] >> 10];
+        if (LIMITS) ncls += (__shfl_sync(FULL, kmask, c.items[i] >> 10) >> lane) & 1u;
     }
     derive<WINDOW>(L);
+    uint32_t full = 0;   // LIMITS: classes at their limit
+    int cfree = cmin;    // LIMITS: smallest cost of a key in no full class (1x1 is in none: always defined)
+    auto count_flip = [&](int code, int sign) {
+        if (!LIMITS) return;
+        ncls += sign * (int)((__shfl_sync(FULL, kmask, code >> 10) >> lane) & 1u);
+        full = __ballot_sync(FULL, ncls >= climit);
+        cfree = (int)__reduce_min_sync(FULL, (kmask & full) ? 0x7fffffffu : (uint32_t)kcost);
+    };
+    if (LIMITS) count_flip(0, 0);
 
     long long it = 0;
     for (; it < steps; it++, step++) {
@@ -259,6 +288,7 @@ __global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(c
             scored += (unsigned)k;
             tabu_add = remove_min_loss<WINDOW>(L, c, k, hl, -1);
             Wt -= costs[tabu_add >> 10];
+            count_flip(tabu_add, -1);
             flips++;
             continue;
         }
@@ -269,10 +299,11 @@ __global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(c
             if (Wt <= target || k == 0) { done = 1; it++; step++; break; }
             continue;
         }
-        if (Wt + cmin >= limit && k > 0) {  // nothing is affordable: swap = remove + add
+        if (Wt + (LIMITS ? cfree : cmin) >= limit && k > 0) {  // nothing is affordable: swap = remove + add
             scored += (unsigned)k;
             tabu_add = remove_min_loss<WINDOW>(L, c, k, hl, tabu_rem);
             Wt -= costs[tabu_add >> 10];
+            count_flip(tabu_add, -1);
             flips++;
         }
         // a random uncovered tile, then two passes of 32 random placements near it
@@ -298,7 +329,8 @@ __global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(c
             bool ov;
             int g = score_placement(L.C, L.U, L.Occ, inb ? x : 0, inb ? y : 0, d.x, d.y, ov);
             const int cost = costs[key];
-            const bool ok = inb && !ov && g > 0 && code != tabu_add && Wt + cost < limit;
+            const bool blocked = LIMITS && (__shfl_sync(FULL, kmask, key) & full) != 0u;
+            const bool ok = inb && !ov && g > 0 && code != tabu_add && Wt + cost < limit && !blocked;
             const uint32_t rank = cost == 1 ? (uint32_t)g : ((uint32_t)g * 64u) / (uint32_t)cost;  // gain per cost (< 2^14)
             uint32_t kk = ok ? ((noise ? 0x10000u : (rank << 16)) | (r >> 16 ^ (r & 0xffffu))) : 0u;
             kk = ok ? (kk | 1u) : 0u;
@@ -321,6 +353,7 @@ __global__ void __launch_bounds__(WARPS * 32, WINDOW ? 4 : 0) sls_multi_kernel(c
         __syncwarp();
         k++;
         Wt += costs[best_code >> 10];
+        count_flip(best_code, +1);
         tabu_rem = best_code;
         flips++;
     }
@@ -439,13 +472,20 @@ int slsm_init(tss_engine* e, void* states, int n) {
     e->stats.kernel_launches++;
     return TSS_OK;
 }
+// limits_dev: class masks per key [MAX_KEYS] then limits per class [MAX_KEYS] (see slsm::LimitsM); n_classes == 0: no limits
 int slsm_run(tss_engine* e, const uint32_t* rows_dev, int W, int H, const int2* keys_dev, const int* costs_dev, const int* order_dev, int n_keys, void* states, int n_chains,
              uint32_t chain_offset, uint64_t seed, long long steps, int* bounds_dev, int target, int noise_pct, unsigned long long* totals_dev,
-             int2* best_dev) {
+             int2* best_dev, const int* limits_dev, int n_classes) {
     int blocks = (n_chains + slsm::WARPS - 1) / slsm::WARPS;
-    slsm::sls_multi_kernel<false, false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states, n_chains,
-                                                                                   chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
-                                                                                   totals_dev, slsm::OneShotM{}, slsm::WindowM{});
+    if (n_classes > 0)
+        slsm::sls_multi_kernel<false, false, true><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states,
+                                                                                             n_chains, chain_offset, seed, steps, bounds_dev, target, noise_pct,
+                                                                                             e->interrupt_dev, totals_dev, slsm::OneShotM{}, slsm::WindowM{},
+                                                                                             slsm::LimitsM{limits_dev, limits_dev + slsm::MAX_KEYS, n_classes});
+    else
+        slsm::sls_multi_kernel<false, false, false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states,
+                                                                                              n_chains, chain_offset, seed, steps, bounds_dev, target, noise_pct,
+                                                                                              e->interrupt_dev, totals_dev, slsm::OneShotM{}, slsm::WindowM{}, slsm::LimitsM{});
     TSS_CHECK_LAUNCH(e);
     slsm::multi_best_kernel<<<1, 256, 0, e->stream>>>((const slsm::MultiState*)states, n_chains, best_dev, bounds_dev);
     TSS_CHECK_LAUNCH(e);
@@ -463,9 +503,10 @@ int slsm_run_oneshot(tss_engine* e, const uint32_t* rows32_host, int bound, uint
     for (int r = 0; r < 32; r++) os.rows[r] = rows32_host[r];
     os.bound = bound; os.rows_out = rows_dev; os.bounds_out = bounds_dev; os.best_out = best_dev; os.key = key_dev; os.ticket = ticket_dev;
     os.result_host = result_host_mapped;
-    slsm::sls_multi_kernel<true, false><<<n_chains / slsm::WARPS, slsm::WARPS * 32, 0, e->stream>>>(nullptr, W, H, keys_dev, costs_dev, order_dev, n_keys, (slsm::MultiState*)states,
-                                                                                                   n_chains, 0u, seed, steps, nullptr, target, noise_pct, e->interrupt_dev,
-                                                                                                   totals_dev, os, slsm::WindowM{});
+    slsm::sls_multi_kernel<true, false, false><<<n_chains / slsm::WARPS, slsm::WARPS * 32, 0, e->stream>>>(nullptr, W, H, keys_dev, costs_dev, order_dev, n_keys,
+                                                                                                          (slsm::MultiState*)states, n_chains, 0u, seed, steps, nullptr,
+                                                                                                          target, noise_pct, e->interrupt_dev, totals_dev, os,
+                                                                                                          slsm::WindowM{}, slsm::LimitsM{});
     TSS_CHECK_LAUNCH(e);
     e->stats.kernel_launches++;
     return TSS_OK;
@@ -476,9 +517,9 @@ int slsm_run_windows(tss_engine* e, const uint32_t* rows_dev, const slsm::Window
                      int n_keys, slsm::MultiState* states, int n_chains, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev,
                      int target, int noise_pct, unsigned long long* totals_dev) {
     const int blocks = (n_chains + slsm::WARPS - 1) / slsm::WARPS;
-    slsm::sls_multi_kernel<false, true><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, 32, 32, keys_dev, costs_dev, order_dev, n_keys, states, n_chains,
-                                                                                  chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
-                                                                                  totals_dev, slsm::OneShotM{}, wm);
+    slsm::sls_multi_kernel<false, true, false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, 32, 32, keys_dev, costs_dev, order_dev, n_keys, states, n_chains,
+                                                                                         chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
+                                                                                         totals_dev, slsm::OneShotM{}, wm, slsm::LimitsM{});
     TSS_CHECK_LAUNCH(e);
     e->stats.kernel_launches++;
     return TSS_OK;
