@@ -449,10 +449,12 @@ def lns_model(grid, seeds, phases, phase_steps, seed=0, chain_offset=0, noise_pc
     return out
 
 
-def slsm_model(grid, key_dims, costs, n_chains, epochs, seed=0, chain_offset=0, noise_pct=20, share_bound=True):
+def slsm_model(grid, key_dims, costs, n_chains, epochs, seed=0, chain_offset=0, noise_pct=20, share_bound=True, count_flips=False):
     """Replays the placement search (platform sets beyond {1x1}) on the CPU.  key_dims: [(w, h)] effective dims per key in
     the engine's key order, costs: objective cost per key, epochs: [(steps, bound, target)].
-    -> dict(items uint16[n,1024], k, best_items, best_k, best, step, scored_total, steps_total)"""
+    -> dict(items uint16[n,1024], k, best_items, best_k, best, step, scored_total, steps_total), plus flips_total with
+    count_flips (the totals are the engine's tss_stats candidates_scored / sls_steps / sls_flips: flips = platforms added +
+    removed).  Without count_flips the dict has the keys callers compare key by key against other replays of the step rule."""
     g = _grid(grid)
     kd = np.ascontiguousarray(key_dims, np.int32).reshape(-1, 2)
     cs = np.ascontiguousarray(costs, np.int32)
@@ -461,9 +463,12 @@ def slsm_model(grid, key_dims, costs, n_chains, epochs, seed=0, chain_offset=0, 
     best_items = np.zeros((n_chains, 1024), np.uint16)
     k, best_k, best = np.zeros(n_chains, np.int32), np.zeros(n_chains, np.int32), np.zeros(n_chains, np.int32)
     step = np.zeros(n_chains, np.uint32)
-    totals = np.zeros(2, np.uint64)
+    totals = np.zeros(3, np.uint64)
     rc = lib().tsso_slsm_model(_p(g, C.c_uint8), g.shape[1], g.shape[0], _p(kd), _p(cs), len(cs), n_chains, C.c_uint32(chain_offset), C.c_uint64(seed),
                                noise_pct, _p(ep, C.c_longlong), len(ep), int(share_bound), _p(items, C.c_uint16), _p(k), _p(best_items, C.c_uint16),
                                _p(best_k), _p(best), _p(step, C.c_uint32), _p(totals, C.c_uint64))
     assert rc == 0
-    return dict(items=items, k=k, best_items=best_items, best_k=best_k, best=best, step=step, scored_total=int(totals[0]), steps_total=int(totals[1]))
+    out = dict(items=items, k=k, best_items=best_items, best_k=best_k, best=best, step=step, scored_total=int(totals[0]), steps_total=int(totals[1]))
+    if count_flips:
+        out["flips_total"] = int(totals[2])
+    return out

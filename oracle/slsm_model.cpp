@@ -83,7 +83,7 @@ struct Runner {
     Chain& c;
     uint32_t base;
     uint8_t cnt[1024], occ[1024];
-    uint64_t scored = 0, steps_done = 0;
+    uint64_t scored = 0, steps_done = 0, flips = 0;   // flips = platforms added + removed
 
     Runner(const Terrain& t, const int* k, const int* cs, int nk, Chain& ch, uint32_t b) : T(t), keys(k), costs(cs), n_keys(nk), c(ch), base(b) {
         order.resize(nk);
@@ -126,6 +126,7 @@ struct Runner {
         c.items.pop_back();
         c.k--;
         apply(code, -1);
+        flips++;
         return code;
     }
 
@@ -195,7 +196,7 @@ struct Runner {
                     const int g = count_in_reach(x, y, w, h, 0), cost = costs[key];
                     const bool ok = !overlaps(x, y, w, h) && g > 0 && code != c.tabu_add && Wt + cost < limit;
                     if (!ok) continue;
-                    const uint32_t rank = cost == 1 ? (uint32_t)g : ((uint32_t)g * 64u) / (uint32_t)cost;
+                    const uint32_t rank = ((uint32_t)g * 64u) / (uint32_t)cost;
                     const uint32_t kk = ((noise ? 0x10000u : (rank << 16)) | ((r >> 16) ^ (r & 0xffffu))) | 1u;
                     if (kk > mx) { mx = kk; mx_code = code; }
                 }
@@ -208,6 +209,7 @@ struct Runner {
             c.k++;
             Wt += costs[best_code >> 10];
             c.tabu_rem = best_code;
+            flips++;
         }
         steps_done += (uint64_t)it;
     }
@@ -219,8 +221,9 @@ extern "C" {
 
 // keys: (w, h) effective dims per key, costs per key.  epochs: (steps, bound, target) records; with share_bound the bound
 // of epoch e+1 is min(given, best objective over all chains after epoch e) — the engine's multi_best_kernel.
-// Outputs per chain: items / best_items as u16[1024] (key << 10 | y << 5 | x), k, best, best_k, step; totals[2] =
-// candidates scored, steps executed (summed over chains and epochs, the engine's tss_stats counters).
+// Outputs per chain: items / best_items as u16[1024] (key << 10 | y << 5 | x), k, best, best_k, step; totals[3] =
+// candidates scored, steps executed, platforms added + removed (summed over chains and epochs, the engine's tss_stats
+// counters candidates_scored, sls_steps and sls_flips).
 int tsso_slsm_model(const uint8_t* grid, int w, int h, const int* keys, const int* costs, int n_keys, int n_chains, uint32_t chain_offset,
                     uint64_t seed, int noise_pct, const long long* epochs, int n_epochs, int share_bound, uint16_t* out_items, int* out_k,
                     uint16_t* out_best_items, int* out_best_k, int* out_best, uint32_t* out_step, uint64_t* totals) {
@@ -232,7 +235,7 @@ int tsso_slsm_model(const uint8_t* grid, int w, int h, const int* keys, const in
         for (int x = 0; x < w; x++) T.ceil[y][x] = grid[y * w + x] != 0;
     std::vector<Chain> chains(n_chains);
     int shared = NO_BOUND;
-    totals[0] = totals[1] = 0;
+    totals[0] = totals[1] = totals[2] = 0;
     for (int e = 0; e < n_epochs; e++) {
         long long steps = epochs[3 * e];
         int bound = (int)epochs[3 * e + 1], target = (int)epochs[3 * e + 2];
@@ -242,6 +245,7 @@ int tsso_slsm_model(const uint8_t* grid, int w, int h, const int* keys, const in
             r.run(steps, bound, target, noise_pct);
             totals[0] += r.scored;
             totals[1] += r.steps_done;
+            totals[2] += r.flips;
         }
         for (auto& c : chains) shared = std::min(shared, c.best);
     }

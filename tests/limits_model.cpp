@@ -107,7 +107,7 @@ struct LimitedRunner : Runner {
                     const bool blocked = ((uint32_t)mask[key] & full) != 0;
                     const bool ok = !overlaps(x, y, w, h) && g > 0 && code != c.tabu_add && Wt + cost < limit && !blocked;
                     if (!ok) continue;
-                    const uint32_t rank = cost == 1 ? (uint32_t)g : ((uint32_t)g * 64u) / (uint32_t)cost;
+                    const uint32_t rank = ((uint32_t)g * 64u) / (uint32_t)cost;
                     const uint32_t kk = ((noise ? 0x10000u : (rank << 16)) | ((r >> 16) ^ (r & 0xffffu))) | 1u;
                     if (kk > mx) { mx = kk; mx_code = code; }
                 }
@@ -121,6 +121,7 @@ struct LimitedRunner : Runner {
             Wt += costs[best_code >> 10];
             count(best_code, +1);
             c.tabu_rem = best_code;
+            flips++;
         }
         steps_done += (uint64_t)it;
     }
@@ -142,7 +143,7 @@ int limits_model(const uint8_t* grid, int w, int h, const int* keys, const int* 
         for (int x = 0; x < w; x++) T.ceil[y][x] = grid[y * w + x] != 0;
     std::vector<Chain> chains(n_chains);
     int shared = NO_BOUND;
-    totals[0] = totals[1] = 0;
+    totals[0] = totals[1] = totals[2] = 0;
     for (int e = 0; e < n_epochs; e++) {
         long long steps = epochs[3 * e];
         int bound = (int)epochs[3 * e + 1], target = (int)epochs[3 * e + 2];
@@ -152,6 +153,7 @@ int limits_model(const uint8_t* grid, int w, int h, const int* keys, const int* 
             r.run(steps, bound, target, noise_pct);
             totals[0] += r.scored;
             totals[1] += r.steps_done;
+            totals[2] += r.flips;
         }
         for (auto& c : chains) shared = std::min(shared, c.best);
     }

@@ -40,9 +40,10 @@ def _p(a, t=C.c_int):
     return a.ctypes.data_as(C.POINTER(t))
 
 
-def limits_model(grid, key_dims, costs, key_mask, class_limit, n_chains, epochs, seed=0, chain_offset=0, noise_pct=20, share_bound=True):
+def limits_model(grid, key_dims, costs, key_mask, class_limit, n_chains, epochs, seed=0, chain_offset=0, noise_pct=20, share_bound=True,
+                 count_flips=False):
     """oracle.slsm_model with per-type limits: key_mask[k] = classes of key k (bit j = class j), class_limit[j] = at most that
-    many platforms in class j.  -> the same dict as oracle.slsm_model."""
+    many platforms in class j.  -> the same dict as oracle.slsm_model (flips_total with count_flips)."""
     g = np.ascontiguousarray(grid, dtype=np.uint8)
     kd = np.ascontiguousarray(key_dims, np.int32).reshape(-1, 2)
     cs = np.ascontiguousarray(costs, np.int32)
@@ -54,9 +55,12 @@ def limits_model(grid, key_dims, costs, key_mask, class_limit, n_chains, epochs,
     best_items = np.zeros((n_chains, 1024), np.uint16)
     k, best_k, best = np.zeros(n_chains, np.int32), np.zeros(n_chains, np.int32), np.zeros(n_chains, np.int32)
     step = np.zeros(n_chains, np.uint32)
-    totals = np.zeros(2, np.uint64)
+    totals = np.zeros(3, np.uint64)
     rc = lib().limits_model(_p(g, C.c_uint8), g.shape[1], g.shape[0], _p(kd), _p(cs), len(cs), _p(mk), _p(lm), len(lm), n_chains, C.c_uint32(chain_offset),
                             C.c_uint64(seed), noise_pct, _p(ep, C.c_longlong), len(ep), int(share_bound), _p(items, C.c_uint16), _p(k),
                             _p(best_items, C.c_uint16), _p(best_k), _p(best), _p(step, C.c_uint32), _p(totals, C.c_uint64))
     assert rc == 0
-    return dict(items=items, k=k, best_items=best_items, best_k=best_k, best=best, step=step, scored_total=int(totals[0]), steps_total=int(totals[1]))
+    out = dict(items=items, k=k, best_items=best_items, best_k=best_k, best=best, step=step, scored_total=int(totals[0]), steps_total=int(totals[1]))
+    if count_flips:
+        out["flips_total"] = int(totals[2])
+    return out

@@ -79,7 +79,7 @@ struct Runner {
     Chain& c;
     uint32_t base;
     uint8_t cnt[1024], occ[1024];
-    uint64_t scored = 0, steps_done = 0;
+    uint64_t scored = 0, steps_done = 0, flips = 0;   // flips = platforms added + removed
     // WINDOW mode (the window-decomposed placement search, csrc/lns_placements.cu): `need` = the tiles still to be covered
     // (replaces the ceiling in the uncovered / covered-once tests), `occ0` = the frozen footprints every run starts from, and
     // additions must lie inside `box` = (x0, y0, x1, y1).  Outside WINDOW mode: the ceiling, no occupancy, the grid.
@@ -130,6 +130,7 @@ struct Runner {
         c.items.pop_back();
         c.k--;
         apply(code, -1);
+        flips++;
         return code;
     }
 
@@ -200,7 +201,7 @@ struct Runner {
                     const int g = count_in_reach(x, y, w, h, 0), cost = costs[key];
                     const bool ok = !overlaps(x, y, w, h) && g > 0 && code != c.tabu_add && Wt + cost < limit;
                     if (!ok) continue;
-                    const uint32_t rank = cost == 1 ? (uint32_t)g : ((uint32_t)g * 64u) / (uint32_t)cost;
+                    const uint32_t rank = ((uint32_t)g * 64u) / (uint32_t)cost;
                     const uint32_t kk = ((noise ? 0x10000u : (rank << 16)) | ((r >> 16) ^ (r & 0xffffu))) | 1u;
                     if (kk > mx) { mx = kk; mx_code = code; }
                 }
@@ -213,6 +214,7 @@ struct Runner {
             c.k++;
             Wt += costs[best_code >> 10];
             c.tabu_rem = best_code;
+            flips++;
         }
         steps_done += (uint64_t)it;
     }
@@ -226,7 +228,7 @@ extern "C" {
 // `terrain` = the window's ceiling u8[32*32] (reach is derived from it), `need` the tiles still to be covered, `occ` the frozen
 // footprints, `box` = (x0, y0, x1, y1) the additions must lie in.  Every chain starts from the same placements `items`
 // (window-local codes) with best = `best` and step = `step`, and runs ONE epoch of `steps` steps without a bound or target.
-// Outputs per chain: best_items u16[1024], best_k, best; totals[2] += candidates scored, steps executed.
+// Outputs per chain: best_items u16[1024], best_k, best; totals[3] += candidates scored, steps executed, platforms added + removed.
 int tsso_slsm_window_model(const uint8_t* terrain, const uint8_t* need, const uint8_t* occ, const int* box, const int* keys, const int* costs, int n_keys,
                            int n_chains, uint32_t chain_offset, uint64_t seed, int noise_pct, long long steps, const uint16_t* items, int n_items,
                            int best, uint32_t step, uint16_t* out_best_items, int* out_best_k, int* out_best, uint64_t* totals) {
@@ -249,6 +251,7 @@ int tsso_slsm_window_model(const uint8_t* terrain, const uint8_t* need, const ui
         r.run(steps, NO_BOUND, -1, noise_pct);
         totals[0] += r.scored;
         totals[1] += r.steps_done;
+        totals[2] += r.flips;
         std::memset(out_best_items + (size_t)i * MAX_ITEMS, 0, sizeof(uint16_t) * MAX_ITEMS);
         std::copy(c.best_items.begin(), c.best_items.end(), out_best_items + (size_t)i * MAX_ITEMS);
         out_best_k[i] = c.best_k;

@@ -55,7 +55,7 @@ def lns_placements_model(grid, key_dims, costs, start, seeds, phases, phase_step
     in its window's [3, 29)^2, every other platform is frozen; in every window `seeds` chains of the WINDOW-mode step rule
     (tests/window_model.cpp) start from the window's movable platforms in row-major anchor order, and the chain with the
     lowest best (lowest chain on ties) replaces them.  phase_steps <= 32768 (one epoch per phase).
-    -> dict(layouts=[sorted [(x, y, key)] after every phase], objectives=[...], scored_total, steps_total)"""
+    -> dict(layouts=[sorted [(x, y, key)] after every phase], objectives=[...], scored_total, steps_total, flips_total)"""
     assert phase_steps <= 32768
     C_ = _grid(grid).astype(np.uint8)
     h, w = C_.shape
@@ -65,7 +65,7 @@ def lns_placements_model(grid, key_dims, costs, start, seeds, phases, phase_step
     OFF = [(0, 0), (-16, -16), (0, -16), (-16, 0)]
     anchors = {(int(x), int(y)): int(k) for x, y, k in start}
     layouts, objectives = [], []
-    totals = np.zeros(2, np.uint64)
+    totals = np.zeros(3, np.uint64)
     L = lib()
     for phase in range(phases):
         ox, oy = OFF[phase & 3]
@@ -115,4 +115,5 @@ def lns_placements_model(grid, key_dims, costs, start, seeds, phases, phase_step
         anchors = new
         layouts.append(sorted((x, y, k) for (x, y), k in anchors.items()))
         objectives.append(int(sum(int(cs[k]) for k in anchors.values())))
-    return dict(layouts=layouts, objectives=objectives, scored_total=int(totals[0]), steps_total=int(totals[1]))
+    return dict(layouts=layouts, objectives=objectives, scored_total=int(totals[0]), steps_total=int(totals[1]),
+                flips_total=int(totals[2]))

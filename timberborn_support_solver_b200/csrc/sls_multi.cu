@@ -331,7 +331,7 @@ __global__ void __launch_bounds__(WARPS * 32, (WINDOW || LIMITS) ? 4 : 0) sls_mu
             const int cost = costs[key];
             const bool blocked = LIMITS && (__shfl_sync(FULL, kmask, key) & full) != 0u;
             const bool ok = inb && !ov && g > 0 && code != tabu_add && Wt + cost < limit && !blocked;
-            const uint32_t rank = cost == 1 ? (uint32_t)g : ((uint32_t)g * 64u) / (uint32_t)cost;  // gain per cost (< 2^14)
+            const uint32_t rank = ((uint32_t)g * 64u) / (uint32_t)cost;  // gain per cost (< 2^14)
             uint32_t kk = ok ? ((noise ? 0x10000u : (rank << 16)) | (r >> 16 ^ (r & 0xffffu))) : 0u;
             kk = ok ? (kk | 1u) : 0u;
             uint32_t mx = __reduce_max_sync(FULL, kk);
