@@ -614,6 +614,70 @@ static int search_alloc(tss_engine* e, tss_search* s, const uint32_t* rows32_hos
     return TSS_OK;
 }
 
+// the placement search's buffers (sls_multi.cu) for one terrain and s->n_chains chains
+static cudaError_t multi_alloc(tss_engine* e, tss_search* s) {
+    cudaError_t err = cudaMalloc(&s->rows_dev, sizeof(uint32_t) * 32);
+    if (err == cudaSuccess) err = cudaMalloc(&s->keys_dev, sizeof(int2) * (size_t)slsm_max_keys());
+    if (err == cudaSuccess) err = cudaMalloc(&s->costs_dev, sizeof(int) * 4 * (size_t)slsm_max_keys());   // costs | keys by area | limit classes
+    if (err == cudaSuccess) err = cudaMalloc(&s->mstates, slsm_state_bytes() * (size_t)s->n_chains);
+    if (err == cudaSuccess) err = cudaMalloc(&s->totals_dev, sizeof(unsigned long long) * 3);
+    if (err == cudaSuccess) err = cudaMalloc(&s->best_dev, sizeof(int2));
+    if (err == cudaSuccess) err = cudaMalloc(&s->bounds_dev, sizeof(int));
+    if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->best_host, sizeof(int2), cudaHostAllocDefault);
+    if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->totals_host, sizeof(unsigned long long) * 3, cudaHostAllocDefault);
+    if (err == cudaSuccess) err = cudaMalloc(&s->mw_codes_dev, sizeof(uint16_t) * (size_t)slsm_max_items());
+    if (err == cudaSuccess) err = cudaMalloc(&s->mw_plats_dev, sizeof(int4) * (size_t)slsm_max_items());
+    if (err == cudaSuccess) err = cudaMalloc(&s->mw_misc_dev, sizeof(uint32_t) * 8);
+    if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->mw_codes_host, sizeof(uint16_t) * (size_t)slsm_max_items(), cudaHostAllocDefault);
+    if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->mw_misc_host, sizeof(uint32_t) * 8, cudaHostAllocDefault);
+    if (err == cudaSuccess) err = cudaMalloc(&s->reduce_key_dev, sizeof(unsigned long long));
+    if (err == cudaSuccess) err = cudaMalloc(&s->ticket_dev, sizeof(unsigned int));
+    if (err == cudaSuccess) err = cudaMemsetAsync(s->reduce_key_dev, 0xff, sizeof(unsigned long long), e->stream);
+    if (err == cudaSuccess) err = cudaMemsetAsync(s->ticket_dev, 0, sizeof(unsigned int), e->stream);
+    if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->oneshot_host, sizeof(uint32_t) * (16 + (size_t)slsm_max_items() / 2), cudaHostAllocMapped);
+    if (err == cudaSuccess) err = cudaHostGetDevicePointer((void**)&s->oneshot_host_dev, s->oneshot_host, 0);
+    return err;
+}
+
+// a cached workspace takes the terrain of a new call: its grid and seed, the default chain offset and noise, no outside bound
+static void reuse_for_terrain(tss_search* s, const uint8_t* grid, int w, int h, uint64_t seed) {
+    s->w = w; s->h = h; s->seed = seed; s->chain_offset = 0; s->noise = sls::DEFAULT_NOISE_PCT;
+    s->grid.assign(grid, grid + (size_t)w * h);
+    s->external_bound = sls::NO_BOUND;
+}
+
+// u8 grid -> one u32 per row (w, h <= 32; rows >= h are zero), the host side of pack_rows32_kernel
+static void pack_rows32(const uint8_t* grid, int w, int h, uint32_t rows[32]) {
+    for (int y = 0; y < 32; y++) rows[y] = 0;
+    for (int y = 0; y < h; y++)
+        for (int x = 0; x < w; x++)
+            if (grid[(size_t)y * w + x]) rows[y] |= 1u << x;
+}
+
+// A platform set every entry point takes: no empty def, and 1x1 among the defs (none at all stands for {1x1}).  `fn` names the
+// caller in the message.  *only_1x1 (may be null) = every def is 1x1.
+static int check_defs(tss_engine* e, const tss_dims* defs, int n_defs, const char* fn, bool* only_1x1) {
+    bool has_1x1 = n_defs == 0, only = true;
+    for (int i = 0; i < n_defs; i++) {
+        if (defs[i].w <= 0 || defs[i].h <= 0) return e->fail(TSS_E_INVALID, "%s: empty platform dimensions", fn);
+        has_1x1 = has_1x1 || (defs[i].w == 1 && defs[i].h == 1);
+        only = only && defs[i].w == 1 && defs[i].h == 1;
+    }
+    if (!has_1x1) return e->fail(TSS_E_INVALID, "the platform set must contain 1x1 (src/encoder.rs:564-566)");
+    if (only_1x1) *only_1x1 = only;
+    return TSS_OK;
+}
+
+// what a platform of a key costs under GUI weights: the sum of the weights of every def contained in its def, exactly what
+// PlatformLayout::total_weight charges it (platform_layout.rs:174-183); weights = (w, h, weight) records
+static long key_cost(const tss_platform& proto, const int32_t* weights, int n_weights) {
+    const Dims def{proto.def_w, proto.def_h};
+    long cost = 0;
+    for (int i = 0; i < n_weights; i++)
+        if (dims_le(Dims{weights[3 * i], weights[3 * i + 1]}, def)) cost += weights[3 * i + 2];
+    return cost;
+}
+
 static int search_init_device(tss_engine* e, tss_search* s, int n_terrains) {
     TSS_CUDA(e, cudaMemsetAsync(s->totals_dev, 0, sizeof(unsigned long long) * 3, e->stream));
     TSS_CUDA(e, cudaMemsetAsync(s->reduce_key_dev, 0xff, sizeof(unsigned long long), e->stream));
@@ -702,12 +766,7 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
                       const tss_search_params* params, tss_search** out) {
     if (!e) return TSS_E_INVALID;
     if (!grid || !out || w <= 0 || h <= 0 || (!defs && n_defs > 0)) return e->fail(TSS_E_INVALID, "tss_search_create: bad arguments");
-    bool has_1x1 = n_defs == 0;
-    for (int i = 0; i < n_defs; i++) {
-        if (defs[i].w <= 0 || defs[i].h <= 0) return e->fail(TSS_E_INVALID, "tss_search_create: empty platform dimensions");
-        has_1x1 = has_1x1 || (defs[i].w == 1 && defs[i].h == 1);
-    }
-    if (!has_1x1) return e->fail(TSS_E_INVALID, "the platform set must contain 1x1 (src/encoder.rs:564-566)");
+    if (int rc = check_defs(e, defs, n_defs, "tss_search_create", nullptr)) return rc;
     if ((size_t)h * ((w + 31) / 32) * 20 > 200 * 1024) return e->fail(TSS_E_UNSUPPORTED, "tss_search: grid %dx%d exceeds the validator's shared-memory planes", w, h);
     TSS_CUDA(e, cudaSetDevice(e->device));
     tss_search* s = new tss_search();
@@ -753,10 +812,8 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
     s->n_chains = (params && params->n_chains > 0) ? params->n_chains : default_chains(e, w, h, s->kernel);
     s->n_groups = 1;
     s->chains_per_terrain = 0;
-    uint32_t rows[32] = {0};
-    for (int y = 0; y < h; y++)
-        for (int x = 0; x < w; x++)
-            if (grid[(size_t)y * w + x]) rows[y] |= 1u << x;
+    uint32_t rows[32];
+    pack_rows32(grid, w, h, rows);
     // more than the single 1x1 key -> placement search
     build_keys(defs, n_defs, s->key_dims, s->key_proto);
     bool fits = (int)s->key_dims.size() <= slsm_max_keys();
@@ -764,41 +821,26 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
     if (s->key_dims.size() > 1 && fits) {
         s->multi = true;
         if (!(params && params->n_chains > 0)) s->n_chains = e->prop.multiProcessorCount * 16;
-        s->key_costs.assign(s->key_dims.size(), 1);
         cudaError_t err = cudaSuccess;
-        tss_search* old = e->cached_multi;  // workspace of an earlier one-shot solve: same buffers, no allocation
-        if (old && old->n_chains == s->n_chains) {
+        tss_search* c = e->cached_multi;
+        if (c && c->n_chains == s->n_chains) {
+            // the workspace of an earlier one-shot solve: its buffers (no allocation) with the host state of this call.  (What is
+            // not reset here — n_groups, chains_per_terrain, the 1x1 and window buffers — is the same in every placement search.)
             e->cached_multi = nullptr;
-            s->rows_dev = old->rows_dev; s->keys_dev = old->keys_dev; s->costs_dev = old->costs_dev; s->mstates = old->mstates;
-            s->totals_dev = old->totals_dev; s->best_dev = old->best_dev; s->bounds_dev = old->bounds_dev;
-            s->best_host = old->best_host; s->totals_host = old->totals_host;
-            s->mw_codes_dev = old->mw_codes_dev; s->mw_plats_dev = old->mw_plats_dev; s->mw_misc_dev = old->mw_misc_dev;
-            s->mw_codes_host = old->mw_codes_host; s->mw_misc_host = old->mw_misc_host;
-            s->reduce_key_dev = old->reduce_key_dev; s->ticket_dev = old->ticket_dev;
-            s->oneshot_host = old->oneshot_host; s->oneshot_host_dev = old->oneshot_host_dev;
-            delete old;
+            reuse_for_terrain(c, grid, w, h, s->seed);
+            c->chain_offset = s->chain_offset; c->noise = s->noise; c->share = s->share; c->kernel = s->kernel;
+            c->key_dims.swap(s->key_dims);
+            c->key_proto.swap(s->key_proto);
+            c->started = c->timed = c->dirty = false;
+            c->n_classes = 0;
+            c->greedy_plats.clear();
+            c->greedy_done = false;
+            delete s;
+            s = c;
         } else {
-            err = cudaMalloc(&s->rows_dev, sizeof rows);
-            if (err == cudaSuccess) err = cudaMalloc(&s->keys_dev, sizeof(int2) * (size_t)slsm_max_keys());
-            if (err == cudaSuccess) err = cudaMalloc(&s->costs_dev, sizeof(int) * 4 * (size_t)slsm_max_keys());   // costs | keys by area | limit classes
-            if (err == cudaSuccess) err = cudaMalloc(&s->mstates, slsm_state_bytes() * (size_t)s->n_chains);
-            if (err == cudaSuccess) err = cudaMalloc(&s->totals_dev, sizeof(unsigned long long) * 3);
-            if (err == cudaSuccess) err = cudaMalloc(&s->best_dev, sizeof(int2));
-            if (err == cudaSuccess) err = cudaMalloc(&s->bounds_dev, sizeof(int));
-            if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->best_host, sizeof(int2), cudaHostAllocDefault);
-            if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->totals_host, sizeof(unsigned long long) * 3, cudaHostAllocDefault);
-            if (err == cudaSuccess) err = cudaMalloc(&s->mw_codes_dev, sizeof(uint16_t) * (size_t)slsm_max_items());
-            if (err == cudaSuccess) err = cudaMalloc(&s->mw_plats_dev, sizeof(int4) * (size_t)slsm_max_items());
-            if (err == cudaSuccess) err = cudaMalloc(&s->mw_misc_dev, sizeof(uint32_t) * 8);
-            if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->mw_codes_host, sizeof(uint16_t) * (size_t)slsm_max_items(), cudaHostAllocDefault);
-            if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->mw_misc_host, sizeof(uint32_t) * 8, cudaHostAllocDefault);
-            if (err == cudaSuccess) err = cudaMalloc(&s->reduce_key_dev, sizeof(unsigned long long));
-            if (err == cudaSuccess) err = cudaMalloc(&s->ticket_dev, sizeof(unsigned int));
-            if (err == cudaSuccess) err = cudaMemsetAsync(s->reduce_key_dev, 0xff, sizeof(unsigned long long), e->stream);
-            if (err == cudaSuccess) err = cudaMemsetAsync(s->ticket_dev, 0, sizeof(unsigned int), e->stream);
-            if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->oneshot_host, sizeof(uint32_t) * (16 + (size_t)slsm_max_items() / 2), cudaHostAllocMapped);
-            if (err == cudaSuccess) err = cudaHostGetDevicePointer((void**)&s->oneshot_host_dev, s->oneshot_host, 0);
+            err = multi_alloc(e, s);
         }
+        s->key_costs.assign(s->key_dims.size(), 1);
         s->totals_seen[0] = s->totals_seen[1] = s->totals_seen[2] = 0;
         const int nb = sls::NO_BOUND;
         if (err == cudaSuccess) err = cudaMemcpyAsync(s->rows_dev, rows, sizeof rows, cudaMemcpyHostToDevice, e->stream);
@@ -927,6 +969,16 @@ int tss_search_run(tss_search* s, int64_t steps, int32_t target_count) {
     return TSS_OK;
 }
 
+// the search's running totals (candidates scored, steps, flips) into the engine's counters: what they grew since last seen
+static void fold_totals(tss_engine* e, tss_search* s, unsigned long long t0, unsigned long long t1, unsigned long long t2) {
+    e->stats.candidates_scored += t0 - s->totals_seen[0];
+    e->stats.sls_steps += t1 - s->totals_seen[1];
+    e->stats.sls_flips += t2 - s->totals_seen[2];
+    s->totals_seen[0] = t0;
+    s->totals_seen[1] = t1;
+    s->totals_seen[2] = t2;
+}
+
 static int search_sync(tss_search* s) {
     tss_engine* e = s->e;
     if (!s->dirty) return TSS_OK;
@@ -938,13 +990,7 @@ static int search_sync(tss_search* s) {
         s->timed = false;
     }
     auto total = [s](int i) { return s->lns ? lns_total(s->lns, i) : (s->lnsp ? lnsp_total(s->lnsp, i) : s->totals_host[i]); };
-    const unsigned long long t0 = total(0), t1 = total(1), t2 = total(2);
-    e->stats.candidates_scored += t0 - s->totals_seen[0];
-    e->stats.sls_steps += t1 - s->totals_seen[1];
-    e->stats.sls_flips += t2 - s->totals_seen[2];
-    s->totals_seen[0] = t0;
-    s->totals_seen[1] = t1;
-    s->totals_seen[2] = t2;
+    fold_totals(e, s, total(0), total(1), total(2));
     s->dirty = false;
     return TSS_OK;
 }
@@ -1236,6 +1282,16 @@ int tss_layout_merge_supports(const uint8_t* grid, int32_t w, int32_t h, const t
     return (int)supports.size();
 }
 
+// placement codes of the placement search (key << 10 | y << 5 | x, sls_multi.cu) -> platforms
+static void codes_to_platforms(const tss_search* s, const uint16_t* codes, int n, tss_platform* out) {
+    for (int i = 0; i < n; i++) {
+        tss_platform p = s->key_proto[codes[i] >> 10];
+        p.x = codes[i] & 31;
+        p.y = (codes[i] >> 5) & 31;
+        out[i] = p;
+    }
+}
+
 int tss_search_best_layout(tss_search* s, tss_platform* out, int32_t cap, int32_t* n_out) {
     if (!s || !n_out) return TSS_E_INVALID;
     tss_engine* e = s->e;
@@ -1294,12 +1350,8 @@ int tss_search_best_layout(tss_search* s, tss_platform* out, int32_t cap, int32_
         for (uint16_t code : codes) cost += s->key_costs[code >> 10];
         if (cost != best.x) return e->fail(TSS_E_CUDA, "internal error: best layout costs %d, chain reported %d", cost, best.x);
         best.x = (int)codes.size();
-        for (uint16_t code : codes) {
-            tss_platform p = s->key_proto[code >> 10];
-            p.x = code & 31;
-            p.y = (code >> 5) & 31;
-            plats.push_back(p);
-        }
+        plats.resize(codes.size());
+        codes_to_platforms(s, codes.data(), (int)codes.size(), plats.data());
     } else {
         best = s->best_host[0];
         if (best.x >= sls::NO_BOUND || best.y < 0) { *n_out = 0; return e->fail(TSS_E_INVALID, "tss_search_best_layout: no complete layout found yet"); }
@@ -1331,13 +1383,10 @@ int tss_search_set_weights(tss_search* s, const int32_t* weights, int32_t n_weig
         return e->fail(TSS_E_UNSUPPORTED, "tss_search_set_weights: the weight objective needs a platform set beyond {1x1} on a grid up to 32x32, or the window placement search");
     int rc = search_sync(s);
     if (rc) return rc;
-    // cost of a platform = sum of the weights of every def contained in its def (platform_layout.rs:174-183)
     for (size_t k = 0; k < s->key_dims.size(); k++) {
-        Dims def{s->key_proto[k].def_w, s->key_proto[k].def_h};
-        long cost = 0;
-        for (int i = 0; i < n_weights; i++)
-            if (dims_le(Dims{weights[3 * i], weights[3 * i + 1]}, def)) cost += weights[3 * i + 2];
-        if (cost <= 0 || cost > 4096) return e->fail(TSS_E_UNSUPPORTED, "tss_search_set_weights: platform costs must be in 1..4096 (got %ld for %dx%d)", cost, def.w, def.h);
+        const long cost = key_cost(s->key_proto[k], weights, n_weights);
+        if (cost <= 0 || cost > 4096)
+            return e->fail(TSS_E_UNSUPPORTED, "tss_search_set_weights: platform costs must be in 1..4096 (got %ld for %dx%d)", cost, s->key_proto[k].def_w, s->key_proto[k].def_h);
         s->key_costs[k] = (int)cost;
     }
     TSS_CUDA(e, cudaMemcpy(s->costs_dev, s->key_costs.data(), sizeof(int) * s->key_costs.size(), cudaMemcpyHostToDevice));
@@ -1394,6 +1443,44 @@ int tss_search_set_card_limits(tss_search* s, const int32_t* card, int32_t n_car
     return TSS_OK;
 }
 
+// The end of a one-shot solve that succeeded: a 1x1 search of one terrain group is kept for the next call (cached_search),
+// so is a placement search, without the call's per-type limits (cached_multi: the next solve's fused first epoch runs on it as
+// it stands, tss_search_create adopts it).  Everything else, and a workspace whose slot is taken, is destroyed.
+static void keep_or_destroy(tss_engine* e, tss_search* s, int rc) {
+    if (!s->lns && !s->lnsp && !s->multi && s->n_groups == 1 && !e->cached_search && rc == TSS_OK) {
+        cudaStreamSynchronize(e->stream);
+        e->cached_search = s;
+    } else if (s->multi && !e->cached_multi && rc == TSS_OK) {
+        cudaStreamSynchronize(e->stream);
+        s->n_classes = 0;
+        e->cached_multi = s;
+    } else {
+        tss_search_destroy(s);
+    }
+}
+
+// The fused first epoch of a one-shot solve on a cached workspace (sls_h16.cu OneShot, sls_multi.cu OneShotM) between
+// fused_epoch_begin and fused_epoch_end: the caller enqueues the one launch in between and reads its result block after.
+static int fused_epoch_begin(tss_engine* e, tss_search* s) {
+    const int rc = search_sync(s);   // (nothing in flight on a cached workspace; folds counters if there was)
+    if (rc == TSS_OK) cudaEventRecord(e->ev0, e->stream);
+    return rc;
+}
+
+// rc = the launch's: one synchronisation, then the epoch's device time, and the epoch counts as a solve
+static int fused_epoch_end(tss_engine* e, int rc) {
+    cudaEventRecord(e->ev1, e->stream);
+    if (rc == TSS_OK && cudaStreamSynchronize(e->stream) != cudaSuccess)
+        rc = e->fail(TSS_E_CUDA, "tss_solve_upper_bound: fused epoch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (rc == TSS_OK) {
+        float ms = 0;
+        if (cudaEventElapsedTime(&ms, e->ev0, e->ev1) != cudaSuccess) cudaGetLastError();
+        e->stats.device_ms = ms;
+        e->stats.n_solves++;
+    }
+    return rc;
+}
+
 int tss_solve_min_weight(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
                          const int32_t* weights, int32_t n_weights, int64_t weight_limit, uint64_t seed, int32_t budget_ms,
                          int64_t max_steps, tss_platform* out, int32_t cap, int32_t* n_out, int64_t* out_weight) {
@@ -1434,12 +1521,7 @@ int tss_solve_min_weight(tss_engine* e, const uint8_t* grid, int32_t w, int32_t 
         if (out_weight) *out_weight = best;
         if (rc == TSS_OK) result = TSS_SAT;
     }
-    if (s->multi && !e->cached_multi && rc == TSS_OK) {
-        cudaStreamSynchronize(e->stream);
-        e->cached_multi = s;   // the GUI tightens weight_limit call after call (app.rs:235-245): the next tss_search_create adopts these buffers
-    } else {
-        tss_search_destroy(s);
-    }
+    keep_or_destroy(e, s, rc);   // the GUI tightens weight_limit call after call (app.rs:235-245): the next tss_search_create adopts the workspace
     return rc != TSS_OK ? rc : result;
 }
 
@@ -1495,44 +1577,25 @@ static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h
         TSS_CUDA(e, cudaSetDevice(e->device));   // (before the workspace is detached: an early return must not leak it)
         s = e->cached_search;
         e->cached_search = nullptr;
-        s->w = w; s->h = h; s->seed = seed; s->chain_offset = 0; s->noise = sls::DEFAULT_NOISE_PCT;
+        reuse_for_terrain(s, grid, w, h, seed);
         s->kernel = kernel;
-        s->grid.assign(grid, grid + (size_t)w * h);
-        s->external_bound = sls::NO_BOUND;
         uint32_t rows_now[32];
-        for (int y = 0; y < 32; y++) rows_now[y] = 0;
-        for (int y = 0; y < h; y++)
-            for (int x = 0; x < w; x++)
-                if (grid[(size_t)y * w + x]) rows_now[y] |= 1u << x;
+        pack_rows32(grid, w, h, rows_now);
         if (latency_mode && s->n_chains % 8 == 0 && !e->interrupted()) {
             // the whole first epoch in ONE launch and ONE synchronisation (sls_h16.cu OneShot): rows travel as kernel
             // parameters, the reach table is derived per CTA, chains start in registers, the last CTA publishes the winner
             // and its validation into mapped host memory
             fused_steps = 32;   // (profiles/steps_to_optimum.py: the fastest of SM x 16 chains needs 16-32 steps on rect 16x16 and test/ex2)
-            rc = search_sync(s);   // (nothing in flight on a cached workspace; folds counters if there was)
-            if (rc == TSS_OK) {
-                cudaEventRecord(e->ev0, e->stream);
-                rc = sls_run_h16_oneshot(e, rows_now, card_limit >= 0 ? card_limit + 1 : sls::NO_BOUND, s->rows_dev, s->tabs_dev, s->states, s->n_chains, seed,
-                                         fused_steps, s->bounds_dev, s->best_dev, s->reduce_key_dev, s->ticket_dev,
-                                         card_limit >= 0 ? card_limit : sls::NO_BOUND - 1, s->noise, s->totals_dev, s->oneshot_host_dev);
-                cudaEventRecord(e->ev1, e->stream);
-            }
-            if (rc == TSS_OK && cudaStreamSynchronize(e->stream) != cudaSuccess) rc = e->fail(TSS_E_CUDA, "tss_solve_upper_bound: fused epoch failed: %s", cudaGetErrorString(cudaGetLastError()));
-            if (rc == TSS_OK) {
+            rc = fused_epoch_begin(e, s);
+            if (rc == TSS_OK)
+                rc = fused_epoch_end(e, sls_run_h16_oneshot(e, rows_now, card_limit >= 0 ? card_limit + 1 : sls::NO_BOUND, s->rows_dev, s->tabs_dev, s->states,
+                                                            s->n_chains, seed, fused_steps, s->bounds_dev, s->best_dev, s->reduce_key_dev, s->ticket_dev,
+                                                            card_limit >= 0 ? card_limit : sls::NO_BOUND - 1, s->noise, s->totals_dev, s->oneshot_host_dev));
+            if (rc == TSS_OK) {   // (OneShot's result block, sls_h16.cu: [34] best, [35] chain, [36..41] totals)
                 const volatile uint32_t* r = s->oneshot_host;
-                float ms = 0;
-                if (cudaEventElapsedTime(&ms, e->ev0, e->ev1) != cudaSuccess) cudaGetLastError();
-                e->stats.device_ms = ms;
-                e->stats.n_solves++;
-                const unsigned long long t0 = ((unsigned long long)r[37] << 32) | r[36], t1 = ((unsigned long long)r[39] << 32) | r[38];
-                const unsigned long long t2 = ((unsigned long long)r[41] << 32) | r[40];
-                e->stats.candidates_scored += t0 - s->totals_seen[0];
-                e->stats.sls_steps += t1 - s->totals_seen[1];
-                e->stats.sls_flips += t2 - s->totals_seen[2];
-                s->totals_seen[0] = t0; s->totals_seen[1] = t1; s->totals_seen[2] = t2;
-                s->totals_host[0] = t0; s->totals_host[1] = t1; s->totals_host[2] = t2;
+                for (int i = 0; i < 3; i++) s->totals_host[i] = ((unsigned long long)r[37 + 2 * i] << 32) | r[36 + 2 * i];
+                fold_totals(e, s, s->totals_host[0], s->totals_host[1], s->totals_host[2]);
                 s->best_host[0] = make_int2((int)r[34], (int)r[35]);
-                s->dirty = false;
                 if ((int)r[34] < sls::NO_BOUND) {
                     fused_best = (int)r[34];
                     e->stats.best_count = fused_best;
@@ -1565,40 +1628,21 @@ static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h
         if (same) {
             s = c;
             e->cached_multi = nullptr;
-            s->w = w; s->h = h; s->seed = seed; s->chain_offset = 0; s->noise = sls::DEFAULT_NOISE_PCT;
-            s->grid.assign(grid, grid + (size_t)w * h);
-            s->external_bound = sls::NO_BOUND;
+            reuse_for_terrain(s, grid, w, h, seed);
             uint32_t rows_now[32];
-            for (int y = 0; y < 32; y++) rows_now[y] = 0;
-            for (int y = 0; y < h; y++)
-                for (int x = 0; x < w; x++)
-                    if (grid[(size_t)y * w + x]) rows_now[y] |= 1u << x;
+            pack_rows32(grid, w, h, rows_now);
             fused_steps = 16;
-            rc = cudaSetDevice(e->device) == cudaSuccess ? search_sync(s) : e->fail(TSS_E_CUDA, "tss_solve_upper_bound: cudaSetDevice failed");
-            if (rc == TSS_OK) {
-                cudaEventRecord(e->ev0, e->stream);
-                rc = slsm_run_oneshot(e, rows_now, card_limit >= 0 ? card_limit + 1 : sls::NO_BOUND, s->rows_dev, w, h, s->keys_dev, s->costs_dev,
-                                      s->costs_dev + slsm_max_keys(), (int)s->key_dims.size(), s->mstates, s->n_chains, seed, fused_steps, s->bounds_dev,
-                                      s->best_dev, s->reduce_key_dev, s->ticket_dev, card_limit >= 0 ? card_limit : sls::NO_BOUND - 1, s->noise,
-                                      s->totals_dev, s->oneshot_host_dev);
-                cudaEventRecord(e->ev1, e->stream);
-            }
-            if (rc == TSS_OK && cudaStreamSynchronize(e->stream) != cudaSuccess) rc = e->fail(TSS_E_CUDA, "tss_solve_upper_bound: fused epoch failed: %s", cudaGetErrorString(cudaGetLastError()));
-            if (rc == TSS_OK) {
+            rc = cudaSetDevice(e->device) == cudaSuccess ? fused_epoch_begin(e, s) : e->fail(TSS_E_CUDA, "tss_solve_upper_bound: cudaSetDevice failed");
+            if (rc == TSS_OK)
+                rc = fused_epoch_end(e, slsm_run_oneshot(e, rows_now, card_limit >= 0 ? card_limit + 1 : sls::NO_BOUND, s->rows_dev, w, h, s->keys_dev, s->costs_dev,
+                                                         s->costs_dev + slsm_max_keys(), (int)s->key_dims.size(), s->mstates, s->n_chains, seed, fused_steps,
+                                                         s->bounds_dev, s->best_dev, s->reduce_key_dev, s->ticket_dev, card_limit >= 0 ? card_limit : sls::NO_BOUND - 1,
+                                                         s->noise, s->totals_dev, s->oneshot_host_dev));
+            if (rc == TSS_OK) {   // (OneShotM's result block, sls_multi.cu: [0] best, [1] chain, [2] n, [3..5] validation, [6..11] totals, codes from word 16)
                 const volatile uint32_t* r = s->oneshot_host;
-                float ms = 0;
-                if (cudaEventElapsedTime(&ms, e->ev0, e->ev1) != cudaSuccess) cudaGetLastError();
-                e->stats.device_ms = ms;
-                e->stats.n_solves++;
-                const unsigned long long t0 = ((unsigned long long)r[7] << 32) | r[6], t1 = ((unsigned long long)r[9] << 32) | r[8];
-                const unsigned long long t2 = ((unsigned long long)r[11] << 32) | r[10];
-                e->stats.candidates_scored += t0 - s->totals_seen[0];
-                e->stats.sls_steps += t1 - s->totals_seen[1];
-                e->stats.sls_flips += t2 - s->totals_seen[2];
-                s->totals_seen[0] = t0; s->totals_seen[1] = t1; s->totals_seen[2] = t2;
-                s->totals_host[0] = t0; s->totals_host[1] = t1; s->totals_host[2] = t2;
+                for (int i = 0; i < 3; i++) s->totals_host[i] = ((unsigned long long)r[7 + 2 * i] << 32) | r[6 + 2 * i];
+                fold_totals(e, s, s->totals_host[0], s->totals_host[1], s->totals_host[2]);
                 s->best_host[0] = make_int2((int)r[0], (int)r[1]);
-                s->dirty = false;
                 if ((int)r[0] < sls::NO_BOUND) {   // hand the witness to the common tail in the layout of the in-stream witness buffers
                     fused_best = (int)r[0];
                     e->stats.best_count = fused_best;
@@ -1700,13 +1744,7 @@ static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h
             if (n > cap || !out) rc = e->fail(TSS_E_CAPACITY, "tss_solve_upper_bound: need room for %d platforms", n);
         }
         if (rc == TSS_OK) {
-            for (int i = 0; i < n; i++) {
-                const uint16_t code = s->mw_codes_host[i];
-                tss_platform pl = s->key_proto[code >> 10];
-                pl.x = code & 31;
-                pl.y = (code >> 5) & 31;
-                out[i] = pl;
-            }
+            codes_to_platforms(s, s->mw_codes_host, n, out);
             result = TSS_SAT;
         }
     } else if (rc == TSS_OK && best >= 0) {
@@ -1715,16 +1753,7 @@ static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h
         if (n_out) *n_out = n;
         if (rc == TSS_OK) result = TSS_SAT;
     }
-    if (!s->lns && !s->multi && s->n_groups == 1 && !e->cached_search && rc == TSS_OK) {
-        cudaStreamSynchronize(e->stream);
-        e->cached_search = s;  // keep the workspace for the next call
-    } else if (s->multi && !e->cached_multi && rc == TSS_OK) {
-        cudaStreamSynchronize(e->stream);
-        s->n_classes = 0;      // (a later solve without limits may run on this workspace as it stands: the fused path above)
-        e->cached_multi = s;   // (tss_search_create adopts its buffers)
-    } else {
-        tss_search_destroy(s);
-    }
+    keep_or_destroy(e, s, rc);
     return rc != TSS_OK ? rc : result;
 }
 
@@ -1777,13 +1806,8 @@ int tss_lower_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, co
     if (!e) return TSS_E_INVALID;
     if (n_out) *n_out = 0;
     if (!grid || !n_out || w <= 0 || h <= 0 || (!defs && n_defs > 0) || cap < 0 || (cap > 0 && !out_xy)) return e->fail(TSS_E_INVALID, "tss_lower_bound: bad arguments");
-    bool has_1x1 = n_defs == 0, only_1x1 = true;
-    for (int i = 0; i < n_defs; i++) {
-        if (defs[i].w <= 0 || defs[i].h <= 0) return e->fail(TSS_E_INVALID, "tss_lower_bound: empty platform dimensions");
-        has_1x1 = has_1x1 || (defs[i].w == 1 && defs[i].h == 1);
-        only_1x1 = only_1x1 && defs[i].w == 1 && defs[i].h == 1;
-    }
-    if (!has_1x1) return e->fail(TSS_E_INVALID, "the platform set must contain 1x1 (src/encoder.rs:564-566)");
+    bool only_1x1 = true;
+    if (int rc = check_defs(e, defs, n_defs, "tss_lower_bound", &only_1x1)) return rc;
     TSS_CUDA(e, cudaSetDevice(e->device));
     if (w > 32 || h > 32) {   // whole-board packing in parallel rounds (lb.cu), 1x1 supports
         if (!only_1x1) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound: grids larger than 32x32 are supported with 1x1 supports only");
@@ -1804,10 +1828,8 @@ int tss_lower_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, co
     std::vector<tss_platform> key_proto;
     const tss_dims one{1, 1};
     build_keys(n_defs ? defs : &one, n_defs ? n_defs : 1, key_dims, key_proto);
-    uint32_t rows[32] = {0}, pack[32];
-    for (int y = 0; y < h; y++)
-        for (int x = 0; x < w; x++)
-            if (grid[(size_t)y * w + x]) rows[y] |= 1u << x;
+    uint32_t rows[32], pack[32];
+    pack_rows32(grid, w, h, rows);
     int count = 0;
     int rc = lb_run(e, rows, w, h, key_dims, seed, restarts, pack, &count);
     if (rc) return rc;
@@ -1827,27 +1849,18 @@ int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h,
     if (out_bound) *out_bound = 0;
     if (!grid || !out_bound || w <= 0 || h <= 0 || (!defs && n_defs > 0) || n_weights < 0 || (n_weights > 0 && !weights))
         return e->fail(TSS_E_INVALID, "tss_lower_bound_lp: bad arguments");
-    bool has_1x1 = n_defs == 0;
-    for (int i = 0; i < n_defs; i++) {
-        if (defs[i].w <= 0 || defs[i].h <= 0) return e->fail(TSS_E_INVALID, "tss_lower_bound_lp: empty platform dimensions");
-        has_1x1 = has_1x1 || (defs[i].w == 1 && defs[i].h == 1);
-    }
-    if (!has_1x1) return e->fail(TSS_E_INVALID, "the platform set must contain 1x1 (src/encoder.rs:564-566)");
+    if (int rc = check_defs(e, defs, n_defs, "tss_lower_bound_lp", nullptr)) return rc;
     TSS_CUDA(e, cudaSetDevice(e->device));
     std::vector<int2> key_dims;
     std::vector<tss_platform> key_proto;
     const tss_dims one{1, 1};
     build_keys(n_defs ? defs : &one, n_defs ? n_defs : 1, key_dims, key_proto);
-    // what a platform of each key costs: 1 (the platform count) or, with weights, the sum of the weights of every def contained in
-    // its def — exactly what PlatformLayout::total_weight charges it (platform_layout.rs:174-183)
-    std::vector<int> key_costs(key_dims.size(), 1);
+    std::vector<int> key_costs(key_dims.size(), 1);   // 1: the platform count
     if (n_weights > 0)
         for (size_t k = 0; k < key_dims.size(); k++) {
-            const Dims def{key_proto[k].def_w, key_proto[k].def_h};
-            long cost = 0;
-            for (int i = 0; i < n_weights; i++)
-                if (dims_le(Dims{weights[3 * i], weights[3 * i + 1]}, def)) cost += weights[3 * i + 2];
-            if (cost < 0 || cost > 4096) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: platform costs must be in 0..4096 (got %ld for %dx%d)", cost, def.w, def.h);
+            const long cost = key_cost(key_proto[k], weights, n_weights);
+            if (cost < 0 || cost > 4096)
+                return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: platform costs must be in 0..4096 (got %ld for %dx%d)", cost, key_proto[k].def_w, key_proto[k].def_h);
             key_costs[k] = (int)cost;
         }
     if (w > 32 || h > 32) {   // first-order method on the whole grid (lp_big.cu), the same certificate
@@ -1864,10 +1877,8 @@ int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h,
         *out_bound = (totals[1] > 0 && totals[2] != ~0ull) ? (int64_t)totals[2] : 0;
         return TSS_OK;
     }
-    uint32_t rows[32] = {0};
-    for (int y = 0; y < h; y++)
-        for (int x = 0; x < w; x++)
-            if (grid[(size_t)y * w + x]) rows[y] |= 1u << x;
+    uint32_t rows[32];
+    pack_rows32(grid, w, h, rows);
     int wts[1024], info[3];
     unsigned long long totals[3];
     int rc = lp_run(e, rows, w, h, key_dims, key_costs, max_pivots, target, wts, totals, info);
