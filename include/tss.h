@@ -366,15 +366,21 @@ int tss_witness_for_cnf(tss_engine* e, const tss_cnf* c, const tss_encoding* enc
 int tss_cnf_complete(tss_engine* e, const tss_cnf* c, uint8_t* assignment, int32_t* out_conflict, int32_t* out_n_falsified);
 /* Solve::solve as the GPU answers it: ONE SAT-like search within the instance's limit (platform count, or total weight when
  * the instance carries a weight limit) that gives up after `give_up_steps` SLS steps per chain (<= 0: the engine default),
- * then tss_witness_for_cnf.  TSS_SAT with a verified model in `assignment`; TSS_UNSAT when the instance's only limit (platform
+ * then tss_witness_for_cnf.  TSS_SAT with a verified model in `assignment`; TSS_UNSAT when the instance's objective limit (platform
  * count, or total weight) lies below a certified lower bound (the integral packing, checked before searching; the fractional
  * LP, computed once per instance after a search came back empty — a first search on an eighth of the give-up budget while that
  * bound is still to be computed, the whole budget only if the bound does not settle the question; grids up to 32x32) — the
  * unmodified bound-tightening loops
  * (crates/repl/src/main.rs:331-334, crates/gui/src/app.rs:212-249) then end proven optimal without their exact solver;
- * TSS_UNKNOWN otherwise: the caller asks its exact solver, which stays the only prover of UNSAT by search.
- * tss_engine_certified_unsat switches the bound-based UNSAT answers off (0) or on (non-zero, the default). */
+ * TSS_UNKNOWN otherwise: the caller asks its exact solver, which stays the only prover of UNSAT by search.  Bounds of the whole
+ * platform set hold for instances with per-type limits too (a limit only removes layouts); with tss_engine_limit_bounds on,
+ * such instances (grids up to 32x32) take the class-aware LP (tss_lower_bound_lp_limits) instead of the plain one, which is what
+ * ends a `solve -l k:v` loop whose optimum the limits moved above the plain bounds.  Each LP bound is cached on the encoding,
+ * keyed by the per-type records and the weights.
+ * tss_engine_certified_unsat switches the bound-based UNSAT answers off (0) or on (non-zero, the default);
+ * tss_engine_limit_bounds switches the class-aware LP on (non-zero) or off (0, the default). */
 int tss_engine_certified_unsat(tss_engine* e, int enabled);
+int tss_engine_limit_bounds(tss_engine* e, int enabled);
 int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc, const tss_instance_info* info, const int32_t* weights,
                        uint64_t seed, int64_t give_up_steps, uint8_t* assignment);
 
@@ -413,6 +419,20 @@ int tss_search_set_card_limits(tss_search* s, const int32_t* card, int32_t n_car
 int tss_solve_with_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
                           int32_t n_card, const int32_t* weights, int32_t n_weights, int64_t weight_limit, uint64_t seed, int32_t budget_ms,
                           int64_t max_steps, tss_platform* out, int32_t cap, int32_t* n_out, int64_t* out_objective);
+/* tss_lower_bound_lp with per-type limits kept (the class-aware LP): card = the records of tss_solve_with_limits (1x1 and vacuous
+ * records make no class).  Defs in a class with limit 0 are dropped from the set first, as tss_solve_with_limits does; each class
+ * j that is left (tss_card_limit_classes on the reduced set, at most 16) with limit L_j adds a dual variable z_j >= 0:
+ *     maximise sum_t y_t - sum_j L_j z_j   s.t.   sum_{t in reach(p)} y_t - sum_{j: key(p) in class j} z_j <= cost(p),   y, z >= 0.
+ * Certified in integers like tss_lower_bound_lp: k_t = floor(y_t * scale) in out_weights[w*h] (optional), zeta_j = floor(z_j *
+ * scale) in out_class_weights[16] (optional, zero past the last class), *out_total = V = sum k_t - sum_j L_j zeta_j (may be
+ * negative), *out_max_load = the largest NET load sum_{reach(p)} k_t - sum_{j: key(p) in class j} zeta_j, *out_bound = min over
+ * placements with a positive net load of ceil(V * cost / load), 0 if V <= 0.  Every layout within the limits costs at least that
+ * (csrc/lp.cu derives it).  Weights, max_pivots, target and out_info as in tss_lower_bound_lp; without a class it computes exactly
+ * what tss_lower_bound_lp does.  Grids larger than 32x32 take lp_big when every record is vacuous and return TSS_E_UNSUPPORTED
+ * otherwise; a negative limit is TSS_E_INVALID. */
+int tss_lower_bound_lp_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
+                              int32_t n_card, const int32_t* weights, int32_t n_weights, int32_t max_pivots, int64_t target, int32_t* out_weights,
+                              int32_t* out_class_weights, int64_t* out_total, int64_t* out_max_load, int64_t* out_bound, int32_t* out_info);
 
 #ifdef __cplusplus
 }

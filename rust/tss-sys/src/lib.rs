@@ -149,6 +149,7 @@ unsafe extern "C" {
     pub fn tss_witness_for_cnf(e: *mut tss_engine, c: *const tss_cnf, enc: *const tss_encoding, plats: *const tss_platform, n: i32, assignment: *mut u8) -> c_int;
     pub fn tss_cnf_complete(e: *mut tss_engine, c: *const tss_cnf, assignment: *mut u8, out_conflict: *mut i32, out_n_falsified: *mut i32) -> c_int;
     pub fn tss_engine_certified_unsat(e: *mut tss_engine, enabled: c_int) -> c_int;
+    pub fn tss_engine_limit_bounds(e: *mut tss_engine, enabled: c_int) -> c_int;
     pub fn tss_solve_instance(
         e: *mut tss_engine, c: *const tss_cnf, enc: *const tss_encoding, info: *const tss_instance_info, weights: *const i32, seed: u64,
         give_up_steps: i64, assignment: *mut u8,
@@ -162,6 +163,11 @@ unsafe extern "C" {
     pub fn tss_lower_bound_lp(
         e: *mut tss_engine, grid: *const u8, w: i32, h: i32, defs: *const tss_dims, n_defs: i32, weights: *const i32, n_weights: i32, max_pivots: i32,
         target: i64, out_weights: *mut i32, out_total: *mut i64, out_max_load: *mut i64, out_bound: *mut i64, out_info: *mut i32,
+    ) -> c_int;
+    pub fn tss_lower_bound_lp_limits(
+        e: *mut tss_engine, grid: *const u8, w: i32, h: i32, defs: *const tss_dims, n_defs: i32, card: *const i32, n_card: i32, weights: *const i32,
+        n_weights: i32, max_pivots: i32, target: i64, out_weights: *mut i32, out_class_weights: *mut i32, out_total: *mut i64, out_max_load: *mut i64,
+        out_bound: *mut i64, out_info: *mut i32,
     ) -> c_int;
     pub fn tss_encoding_terrain(enc: *const tss_encoding, grid: *mut u8, cap: usize, w: *mut i32, h: *mut i32) -> c_int;
     pub fn tss_encoding_defs(enc: *const tss_encoding, defs: *mut tss_dims, cap: i32, n: *mut i32) -> c_int;

@@ -108,6 +108,7 @@ SIGNATURES = {
     "tss_solve_with_limits": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32p, _i32, _i64, _u64, _i32, _i64, _P(Platform), _i32, _i32p, _i64p]),
     "tss_lower_bound": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _u64, _i32, _i32p, _i32, _i32p]),
     "tss_lower_bound_lp": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32, _i64, _i32p, _i64p, _i64p, _i64p, _i32p]),
+    "tss_lower_bound_lp_limits": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32p, _i32, _i32, _i64, _i32p, _i32p, _i64p, _i64p, _i64p, _i32p]),
     "tss_solve_batch": (C.c_int, [_vp, _u8p, _i32, _i32, _i64, _u64, _i64, _i32, _i32p, _u32p]),
     "tss_instance_find": (C.c_int, [_i32p, _u32p, _i32, _i32, _P(_vp), _P(InstanceInfo), _i32p, _i32]),
     "tss_encoding_terrain": (C.c_int, [_vp, _u8p, _sz, _i32p, _i32p]),
@@ -117,6 +118,7 @@ SIGNATURES = {
     "tss_solve_instance": (C.c_int, [_vp, _vp, _vp, _P(InstanceInfo), _i32p, _u64, _i64, _u8p]),
     "tss_cnf_complete": (C.c_int, [_vp, _vp, _u8p, _i32p, _i32p]),
     "tss_engine_certified_unsat": (C.c_int, [_vp, C.c_int]),
+    "tss_engine_limit_bounds": (C.c_int, [_vp, C.c_int]),
     "tss_measure_peaks": (C.c_int, [_vp, _P(C.c_double), _i32]),
 }
 

@@ -719,23 +719,42 @@ class Engine:
                                              _ptr(out, C.c_int32), len(out), C.byref(n)))
         return [(int(x), int(y)) for x, y in out[: n.value]]
 
-    def lower_bound_lp(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], max_pivots=0, weights: Optional[dict] = None, target=0):
+    def lower_bound_lp(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], max_pivots=0, weights: Optional[dict] = None, target=0,
+                       limits: Optional[dict] = None):
         """Fractional packing lower bound (tss_lower_bound_lp), certified in integers: on the platform count, or with `weights`
         ({PlatformDef: weight}, the PlatformLimits.weights map) on PlatformLayout::total_weight.  target > 0: the simplex stops as
         soon as the bound reaches it (every iterate is feasible; enough for "is there nothing within target - 1?").
         On grids larger than 32x32 (up to 256x256; at most 16 dims keys, each at most 6x6) a first-order method replaces the
         simplex under the same certificate: `max_pivots` caps its iterations (0: 3 000) and the result's `pivots` counts them,
         `target` is checked on the certified bound every 250 iterations, and `optimal` is always False.
-        -> dict(bound, weights int32[h, w], total, max_load, pivots, optimal, constraints)."""
+        limits ({PlatformDef: limit}, PlatformLimits.card_limits; 1x1 entries are ignored): the class-aware LP that keeps the
+        per-type limits (tss_lower_bound_lp_limits), a bound on every layout within them.  Defs in a class with limit 0 leave the
+        set first; `class_weights` (int64[16]) then holds the integer weight of class j of card_limit_classes on what is left,
+        and `total` is the weights' sum minus sum_j limit_j * class_weights[j].  Grids up to 32x32 unless every limit is vacuous.
+        -> dict(bound, weights int32[h, w], total, max_load, pivots, optimal, constraints[, class_weights])."""
         defs = list(defs)
         wts = np.zeros((grid.height, grid.width), np.int32)
         total, max_load, bound = C.c_int64(), C.c_int64(), C.c_int64()
         info = (C.c_int32 * 3)()
         rec = np.array([[d.width, d.height, v] for d, v in (weights or {}).items()], np.int32).reshape(-1, 3)
-        self._check(self.lib.tss_lower_bound_lp(self._h, _ptr(grid.data, C.c_uint8), grid.width, grid.height, _defs_array(defs), len(defs),
-                                                _ptr(rec, C.c_int32) if len(rec) else None, len(rec), max_pivots, int(target),
-                                                _ptr(wts, C.c_int32), C.byref(total), C.byref(max_load), C.byref(bound), info))
-        return dict(bound=bound.value, weights=wts, total=total.value, max_load=max_load.value, pivots=info[0], optimal=bool(info[1]), constraints=info[2])
+        common = (_ptr(grid.data, C.c_uint8), grid.width, grid.height, _defs_array(defs), len(defs))
+        w_args = (_ptr(rec, C.c_int32) if len(rec) else None, len(rec), max_pivots, int(target), _ptr(wts, C.c_int32))
+        out = dict()
+        if limits is None:
+            self._check(self.lib.tss_lower_bound_lp(self._h, *common, *w_args, C.byref(total), C.byref(max_load), C.byref(bound), info))
+        else:
+            card = _card_records(limits)
+            cw = np.zeros(16, np.int32)
+            self._check(self.lib.tss_lower_bound_lp_limits(self._h, *common, _ptr(card, C.c_int32) if len(card) else None, len(card), *w_args,
+                                                           _ptr(cw, C.c_int32), C.byref(total), C.byref(max_load), C.byref(bound), info))
+            out["class_weights"] = cw.astype(np.int64)
+        return dict(bound=bound.value, weights=wts, total=total.value, max_load=max_load.value, pivots=info[0], optimal=bool(info[1]),
+                    constraints=info[2], **out)
+
+    def limit_bounds(self, enabled: bool = True):
+        """tss_engine_limit_bounds: tss_solve_instance certifies the UNSAT of an instance with per-type limits with the class-aware
+        LP (grids up to 32x32) instead of the bounds of the whole set.  Off by default."""
+        self._check(self.lib.tss_engine_limit_bounds(self._h, 1 if enabled else 0))
 
     def solve_batch(self, grids, seed=0, steps=2048, want_layouts=False, chains_per_terrain=0):
         """grids: uint8[n, h, w] -> counts int32[n] (and packed support rows uint32[n, h] if asked)"""
@@ -817,7 +836,7 @@ class GpuBoundSolver:
 
 
 def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, engine: Engine, exact_solver=None, seed=0, budget_ms=None,
-                on_solution=None, use_lower_bound=True):
+                on_solution=None, use_lower_bound=True, limit_bounds=False):
     """crates/repl/src/main.rs:280-366 with the GPU engine as the SAT side and an optional exact solver
     (`exact_solver(cnf) -> (SAT|UNSAT|INTERRUPTED, assignment)`, Glucose in the reference) for the proof.
 
@@ -828,6 +847,9 @@ def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, en
 
     use_lower_bound: ask the engine for its packing lower bound first (tss_lower_bound); when the count reaches it the loop
     ends with `proved_optimal` and no exact-solver call.
+
+    limit_bounds: loops with per-type limits (`solve -l k:v`) use the bounds as well, the fractional one being the class-aware LP
+    that keeps the limits (Engine.lower_bound_lp(..., limits=...)); without it only loops whose sole limit is the count do.
 
     Returns dict(best=PlatformLayout|None, proved_optimal=bool, steps=[...], lower_bound=int|None)."""
     one = PlatformDef(1, 1)
@@ -841,7 +863,8 @@ def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, en
     # ms on a 21x16 terrain) only when the GPU has found nothing below a count the packing does not already certify.
     lower, lp_done = None, False
     g = encoding._grid
-    only_count = not limits.weights and limits.weight_limit is None and all(d == one for d in limits.card_limits)
+    per_type = {d: v for d, v in limits.card_limits.items() if d != one}
+    only_count = not limits.weights and limits.weight_limit is None and (limit_bounds or not per_type)
     use_lower_bound = use_lower_bound and only_count and g.width <= 32 and g.height <= 32
     if use_lower_bound:
         try:
@@ -871,7 +894,7 @@ def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, en
         if result != SAT and lp_pending:
             lp_done = True                                      # the GPU found nothing below the current count: can the fractional bound certify it?
             # (asked only "does the bound reach the count at hand?": the simplex stops as soon as it does)
-            lower = max(lower, engine.lower_bound_lp(g, encoding.defs, target=best.platform_count())["bound"])
+            lower = max(lower, engine.lower_bound_lp(g, encoding.defs, target=best.platform_count(), limits=per_type or None)["bound"])
             if limits.card_limits.get(one) is not None and limits.card_limits[one] < lower:
                 steps.append(dict(bound=limits.card_limits[one], result=UNSAT, source="lower bound"))
                 proved = True

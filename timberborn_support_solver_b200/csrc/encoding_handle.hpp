@@ -18,6 +18,9 @@ struct tss_encoding_data {
     mutable bool lp_count_final = false, lp_weight_final = false;   // the simplex ran to optimality (not stopped at a target): asking again cannot improve the bound
     mutable std::vector<int32_t> lp_weights;   // the weight table `lp_weight_bound` was computed for
     mutable long long lp_weight_bound = -1;    // tss_lower_bound_lp on the total weight
+    // the per-type records (def_w, def_h, limit; 1x1 excluded) each LP bound above was computed with (tss_lower_bound_lp_limits);
+    // empty: the plain LP of the whole set, which holds for every limit
+    mutable std::vector<int32_t> lp_count_card, lp_weight_card;
     // the CNF of the last tss_encoding_with_limits call: callers ask twice, once for the sizes and once for the clauses, and the
     // registry keeps the same object (no second lowering of the limits, no copy of the clauses)
     mutable std::mutex lowered_mutex;

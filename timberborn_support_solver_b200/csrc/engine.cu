@@ -45,8 +45,10 @@ int sls_run_h16(tss_engine* e, const uint32_t* rows_dev, const uint2* tabs_dev, 
                 int noise_pct, unsigned long long* totals_dev);
 int run_peaks(tss_engine* e, double* out, int n_out);
 // lp.cu — fractional packing lower bound
-int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs, int max_pivots,
-           long long target, int* out_weights, unsigned long long* totals, int* info);
+int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs,
+           const std::vector<uint32_t>& key_mask, const std::vector<int>& class_limit, int max_pivots, long long target, int* out_weights,
+           unsigned long long* totals, int* info);
+constexpr int kLpMaxClasses = 16;   // lp.cu: class columns of per-type limits; the weights buffer holds 1024 tile weights, then these
 // lp_big.cu — the same bound on grids larger than 32x32 (first-order method, same certificate)
 int lp_big_run(tss_engine* e, const uint32_t* rows_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs, int max_iters,
                long long target, int* out_weights, unsigned long long* totals, int* info);
@@ -1842,14 +1844,13 @@ int tss_lower_bound(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, co
     return TSS_OK;
 }
 
-int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* weights,
-                       int32_t n_weights, int32_t max_pivots, int64_t target, int32_t* out_weights, int64_t* out_total, int64_t* out_max_load,
-                       int64_t* out_bound, int32_t* out_info) {
-    if (!e) return TSS_E_INVALID;
-    if (out_bound) *out_bound = 0;
-    if (!grid || !out_bound || w <= 0 || h <= 0 || (!defs && n_defs > 0) || n_weights < 0 || (n_weights > 0 && !weights))
-        return e->fail(TSS_E_INVALID, "tss_lower_bound_lp: bad arguments");
-    if (int rc = check_defs(e, defs, n_defs, "tss_lower_bound_lp", nullptr)) return rc;
+// The fractional bound of tss_lower_bound_lp and tss_lower_bound_lp_limits: key_mask / class_limit = classes of per-type limits
+// on the keys of `defs` (card_limit_classes; empty: the plain LP, which is all grids larger than 32x32 take).
+static int lower_bound_lp(tss_engine* e, const char* fn, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
+                          const std::vector<uint32_t>& key_mask, const std::vector<int>& class_limit, const int32_t* weights, int32_t n_weights,
+                          int32_t max_pivots, int64_t target, int32_t* out_weights, int32_t* out_class_weights, int64_t* out_total,
+                          int64_t* out_max_load, int64_t* out_bound, int32_t* out_info) {
+    if (int rc = check_defs(e, defs, n_defs, fn, nullptr)) return rc;
     TSS_CUDA(e, cudaSetDevice(e->device));
     std::vector<int2> key_dims;
     std::vector<tss_platform> key_proto;
@@ -1860,9 +1861,10 @@ int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h,
         for (size_t k = 0; k < key_dims.size(); k++) {
             const long cost = key_cost(key_proto[k], weights, n_weights);
             if (cost < 0 || cost > 4096)
-                return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: platform costs must be in 0..4096 (got %ld for %dx%d)", cost, key_proto[k].def_w, key_proto[k].def_h);
+                return e->fail(TSS_E_UNSUPPORTED, "%s: platform costs must be in 0..4096 (got %ld for %dx%d)", fn, cost, key_proto[k].def_w, key_proto[k].def_h);
             key_costs[k] = (int)cost;
         }
+    if (out_class_weights) std::fill(out_class_weights, out_class_weights + kLpMaxClasses, 0);
     if (w > 32 || h > 32) {   // first-order method on the whole grid (lp_big.cu), the same certificate
         BitGrid bg = BitGrid::from_bytes(grid, w, h);
         std::vector<int> wts((size_t)w * h);
@@ -1879,23 +1881,76 @@ int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h,
     }
     uint32_t rows[32];
     pack_rows32(grid, w, h, rows);
-    int wts[1024], info[3];
+    int wts[1024 + kLpMaxClasses], info[3];
     unsigned long long totals[3];
-    int rc = lp_run(e, rows, w, h, key_dims, key_costs, max_pivots, target, wts, totals, info);
+    int rc = lp_run(e, rows, w, h, key_dims, key_costs, key_mask, class_limit, max_pivots, target, wts, totals, info);
     if (rc) return rc;
     if (target > 0 && !info[1] && !(totals[1] > 0 && totals[2] != ~0ull && (int64_t)totals[2] >= target)) {
         // stopped early on the floating-point objective, and the integer certificate falls short of the target: run to optimality
-        rc = lp_run(e, rows, w, h, key_dims, key_costs, max_pivots, 0, wts, totals, info);
+        rc = lp_run(e, rows, w, h, key_dims, key_costs, key_mask, class_limit, max_pivots, 0, wts, totals, info);
         if (rc) return rc;
     }
     if (out_weights)
         for (int y = 0; y < h; y++)
             for (int x = 0; x < w; x++) out_weights[(size_t)y * w + x] = wts[y * 32 + x];
-    if (out_total) *out_total = (int64_t)totals[0];
+    if (out_class_weights) std::copy(wts + 1024, wts + 1024 + kLpMaxClasses, out_class_weights);
+    if (out_total) *out_total = (int64_t)totals[0];   // (V: signed, negative when the classes outweigh the tiles)
     if (out_max_load) *out_max_load = (int64_t)totals[1];
     if (out_info) { out_info[0] = info[0]; out_info[1] = info[1]; out_info[2] = info[2]; }
-    *out_bound = (totals[1] > 0 && totals[2] != ~0ull) ? (int64_t)totals[2] : 0;   // min over placements of ceil(total * cost / load): exact
+    *out_bound = (totals[1] > 0 && totals[2] != ~0ull) ? (int64_t)totals[2] : 0;   // min over placements of ceil(V * cost / load): exact
     return TSS_OK;
+}
+
+int tss_lower_bound_lp(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* weights,
+                       int32_t n_weights, int32_t max_pivots, int64_t target, int32_t* out_weights, int64_t* out_total, int64_t* out_max_load,
+                       int64_t* out_bound, int32_t* out_info) {
+    if (!e) return TSS_E_INVALID;
+    if (out_bound) *out_bound = 0;
+    if (!grid || !out_bound || w <= 0 || h <= 0 || (!defs && n_defs > 0) || n_weights < 0 || (n_weights > 0 && !weights))
+        return e->fail(TSS_E_INVALID, "tss_lower_bound_lp: bad arguments");
+    return lower_bound_lp(e, "tss_lower_bound_lp", grid, w, h, defs, n_defs, {}, {}, weights, n_weights, max_pivots, target, out_weights, nullptr,
+                          out_total, out_max_load, out_bound, out_info);
+}
+
+int tss_lower_bound_lp_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
+                              int32_t n_card, const int32_t* weights, int32_t n_weights, int32_t max_pivots, int64_t target, int32_t* out_weights,
+                              int32_t* out_class_weights, int64_t* out_total, int64_t* out_max_load, int64_t* out_bound, int32_t* out_info) {
+    if (!e) return TSS_E_INVALID;
+    if (out_bound) *out_bound = 0;
+    if (!grid || !out_bound || w <= 0 || h <= 0 || (!defs && n_defs > 0) || n_card < 0 || (n_card > 0 && !card) || n_weights < 0 || (n_weights > 0 && !weights))
+        return e->fail(TSS_E_INVALID, "tss_lower_bound_lp_limits: bad arguments");
+    for (int i = 0; i < n_card; i++)
+        if (card[3 * i + 2] < 0) return e->fail(TSS_E_INVALID, "tss_lower_bound_lp_limits: negative limit for %dx%d", card[3 * i], card[3 * i + 1]);
+    if (int rc = check_defs(e, defs, n_defs, "tss_lower_bound_lp_limits", nullptr)) return rc;
+    // the classes on the whole set; a limit of 0 then removes its class from the set, as tss_solve_with_limits does, and the
+    // classes are taken again on what is left (the zero-limit records are vacuous there)
+    const tss_dims one{1, 1};
+    const tss_dims* all = n_defs ? defs : &one;
+    const int n_all = n_defs ? n_defs : 1;
+    std::vector<int2> kd;
+    std::vector<tss_platform> kp;
+    std::vector<uint32_t> mask;
+    std::vector<int> lim;
+    build_keys(all, n_all, kd, kp);
+    int rc = card_limit_classes(kd, card, n_card, mask, lim);
+    if (rc) return e->fail(rc, "tss_lower_bound_lp_limits: bad limit records");
+    if (!lim.empty() && (w > 32 || h > 32))
+        return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp_limits: per-type limits on grids larger than 32x32 are not supported (got %dx%d)", w, h);
+    uint32_t zero = 0;
+    for (size_t j = 0; j < lim.size(); j++) zero |= lim[j] == 0 ? 1u << j : 0u;
+    std::vector<tss_dims> kept;
+    for (int i = 0; i < n_all; i++) {
+        bool drop = false;
+        for (size_t k = 0; k < kd.size(); k++) drop = drop || (kd[k].x == all[i].w && kd[k].y == all[i].h && (mask[k] & zero));
+        if (!drop) kept.push_back(all[i]);
+    }
+    if (zero) {
+        build_keys(kept.data(), (int)kept.size(), kd, kp);
+        rc = card_limit_classes(kd, card, n_card, mask, lim);
+        if (rc) return e->fail(rc, "tss_lower_bound_lp_limits: bad limit records");
+    }
+    return lower_bound_lp(e, "tss_lower_bound_lp_limits", grid, w, h, kept.data(), (int32_t)kept.size(), mask, lim, weights, n_weights, max_pivots, target,
+                          out_weights, out_class_weights, out_total, out_max_load, out_bound, out_info);
 }
 
 int tss_solve_batch(tss_engine* e, const uint8_t* grids, int32_t w, int32_t h, int64_t n, uint64_t seed, int64_t steps,

@@ -150,6 +150,12 @@ int tss_engine_certified_unsat(tss_engine* e, int enabled) {
     return TSS_OK;
 }
 
+int tss_engine_limit_bounds(tss_engine* e, int enabled) {
+    if (!e) return TSS_E_INVALID;
+    e->limit_bounds = enabled != 0;
+    return TSS_OK;
+}
+
 int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc, const tss_instance_info* info, const int32_t* weights,
                        uint64_t seed, int64_t give_up_steps, uint8_t* assignment) {
     if (!e) return TSS_E_INVALID;
@@ -161,17 +167,23 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
     if (per_type && (!enc->has_card_limits || E.w > 32 || E.h > 32 || (info->has_weight_limit && info->card_limit_1x1 >= 0))) return TSS_UNKNOWN;
     std::vector<tss_dims> defs;
     for (const Dims& d : E.defs) defs.push_back(tss_dims{d.w, d.h});
-    // A limit below a CERTIFIED lower bound has no model: answer UNSAT without searching.  Only when the platform count is the
-    // sole limit (the REPL's loop); the integral packing first (~0.1 ms, computed once per instance), the fractional LP only after
-    // the search came back empty-handed.
+    // A limit below a CERTIFIED lower bound has no model: answer UNSAT without searching.  Only when one objective is limited
+    // (the platform count: the REPL's loop; the total weight: the GUI's); the integral packing first (~0.1 ms, computed once per
+    // instance), the fractional LP only after the search came back empty-handed.  Both are bounds of the whole platform set, valid
+    // under any per-type limit; with tss_engine_limit_bounds the LP of an instance with per-type limits keeps them (the class-aware
+    // LP), and its cached value only answers instances with the same per-type records.
     Trace tr;
     const bool small = e->certified_unsat && E.w <= 32 && E.h <= 32;
     const bool count_only = small && info->card_limit_1x1 >= 0 && !info->has_weight_limit;
     const bool weight_only = small && info->card_limit_1x1 < 0 && info->has_weight_limit && info->n_weights > 0 && weights;
+    std::vector<int32_t> lp_card;   // the per-type records the LP bound of this call keeps (empty: the plain LP)
+    if (per_type && e->limit_bounds && enc->has_card_limits)
+        for (size_t i = 0; i + 2 < enc->card_limits.size(); i += 3)
+            if (!(enc->card_limits[i] == 1 && enc->card_limits[i + 1] == 1)) lp_card.insert(lp_card.end(), enc->card_limits.begin() + i, enc->card_limits.begin() + i + 3);
     if (weight_only) {
         std::lock_guard<std::mutex> lock(enc->d->bounds_mutex);
         if (enc->d->lp_weight_bound >= 0 && enc->d->lp_weights == std::vector<int32_t>(weights, weights + 3 * (size_t)info->n_weights) &&
-            info->weight_limit < enc->d->lp_weight_bound)
+            enc->d->lp_weight_card == lp_card && info->weight_limit < enc->d->lp_weight_bound)
             return TSS_UNSAT;
     }
     if (count_only) {
@@ -182,7 +194,7 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
         }
         tr.lap("solve: packing bound");
         if (enc->d->packing_bound >= 0 && info->card_limit_1x1 < enc->d->packing_bound) return TSS_UNSAT;
-        if (enc->d->lp_count_bound >= 0 && info->card_limit_1x1 < enc->d->lp_count_bound) return TSS_UNSAT;
+        if (enc->d->lp_count_bound >= 0 && enc->d->lp_count_card == lp_card && info->card_limit_1x1 < enc->d->lp_count_bound) return TSS_UNSAT;
     }
     std::vector<tss_platform> plats((size_t)E.w * E.h + 1);
     int32_t n = 0;
@@ -209,9 +221,19 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
     // early; computed again, to the new target, only if a later call asks about a limit the cached bound does not settle and the
     // solve was not final.  true = the limit lies below the certified bound.
     const std::vector<int32_t> wv = weight_only ? std::vector<int32_t>(weights, weights + 3 * (size_t)info->n_weights) : std::vector<int32_t>();
-    auto count_pending = [&] { return enc->d->lp_count_bound == -1 || (enc->d->lp_count_bound >= 0 && !enc->d->lp_count_final && info->card_limit_1x1 >= enc->d->lp_count_bound); };
+    auto count_pending = [&] {
+        return enc->d->lp_count_bound == -1 || enc->d->lp_count_card != lp_card ||
+               (enc->d->lp_count_bound >= 0 && !enc->d->lp_count_final && info->card_limit_1x1 >= enc->d->lp_count_bound);
+    };
     auto weight_pending = [&] {
-        return enc->d->lp_weight_bound == -1 || enc->d->lp_weights != wv || (enc->d->lp_weight_bound >= 0 && !enc->d->lp_weight_final && info->weight_limit >= enc->d->lp_weight_bound);
+        return enc->d->lp_weight_bound == -1 || enc->d->lp_weights != wv || enc->d->lp_weight_card != lp_card ||
+               (enc->d->lp_weight_bound >= 0 && !enc->d->lp_weight_final && info->weight_limit >= enc->d->lp_weight_bound);
+    };
+    auto lp_bound = [&](const int32_t* w, int32_t n_w, int64_t target, int64_t* lb, int32_t* lp_info) {   // plain, or keeping the per-type limits
+        if (lp_card.empty())
+            return tss_lower_bound_lp(e, enc->d->grid.data(), E.w, E.h, defs.data(), (int32_t)defs.size(), w, n_w, 0, target, nullptr, nullptr, nullptr, lb, lp_info);
+        return tss_lower_bound_lp_limits(e, enc->d->grid.data(), E.w, E.h, defs.data(), (int32_t)defs.size(), lp_card.data(), (int32_t)(lp_card.size() / 3), w, n_w,
+                                         0, target, nullptr, nullptr, nullptr, nullptr, lb, lp_info);
     };
     auto lp_refutes = [&]() -> bool {
         std::lock_guard<std::mutex> lock(enc->d->bounds_mutex);
@@ -219,8 +241,8 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
         int32_t lp_info[3] = {0, 0, 0};
         if (count_only) {
             if (count_pending()) {
-                const int ok = tss_lower_bound_lp(e, enc->d->grid.data(), E.w, E.h, defs.data(), (int32_t)defs.size(), nullptr, 0, 0, (int64_t)info->card_limit_1x1 + 1,
-                                                  nullptr, nullptr, nullptr, &lb, lp_info);
+                const int ok = lp_bound(nullptr, 0, (int64_t)info->card_limit_1x1 + 1, &lb, lp_info);
+                enc->d->lp_count_card = lp_card;
                 enc->d->lp_count_bound = ok == TSS_OK ? lb : -2;
                 enc->d->lp_count_final = lp_info[1] != 0;
                 tr.lap("solve: fractional bound");
@@ -230,8 +252,8 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
         if (weight_only) {   // the same question about the GUI's weight limit (crates/gui/src/app.rs:235-239)
             if (weight_pending()) {
                 enc->d->lp_weights = wv;
-                const int ok = tss_lower_bound_lp(e, enc->d->grid.data(), E.w, E.h, defs.data(), (int32_t)defs.size(), weights, info->n_weights, 0, info->weight_limit + 1,
-                                                  nullptr, nullptr, nullptr, &lb, lp_info);
+                enc->d->lp_weight_card = lp_card;
+                const int ok = lp_bound(weights, info->n_weights, info->weight_limit + 1, &lb, lp_info);
                 enc->d->lp_weight_bound = ok == TSS_OK ? lb : -2;
                 enc->d->lp_weight_final = lp_info[1] != 0;
                 tr.lap("solve: fractional bound (weights)");

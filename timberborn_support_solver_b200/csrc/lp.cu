@@ -14,12 +14,26 @@
 // ceil(sum k / max load) — exact, whatever the simplex did (a primal simplex iterate is feasible at every pivot, so an
 // iteration cap only weakens the bound).
 //
+// PER-TYPE LIMITS (`solve -l k:v`, PlatformLimits.card_limits beyond 1x1) only remove layouts, so the LP above stays a bound, but
+// a weak one.  The class-aware LP keeps them: class j (card_limit_classes in engine.cu) is a set of dims keys of which a layout
+// holds at most L_j platforms, and its dual gets one variable z_j >= 0 per class:
+//
+//     maximise  sum_t y_t - sum_j L_j z_j   subject to   sum_{t in reach(p)} y_t - sum_{j ∋ key(p)} z_j <= cost(p)   for every p,   y, z >= 0
+//
+// The certificate takes integers k_t = floor(y_t * scale) and zeta_j = floor(z_j * scale) (any non-negative integers are valid):
+// V = sum_t k_t - sum_j L_j zeta_j and the NET load(p) = sum_{t in reach(p)} k_t - sum_{j ∋ key(p)} zeta_j.  For a complete layout L
+// within the limits
+//     sum_t k_t <= sum_{p in L} sum_{t in reach(p)} k_t = sum_{p in L} load(p) + sum_j zeta_j |L ∩ class j| <= sum_{p in L} load(p) + sum_j L_j zeta_j,
+// so V <= sum_{p in L} load(p) <= max_p (load(p) / cost(p)) * cost(L): the bound is min over placements with load(p) > 0 of
+// ceil(V * cost(p) / load(p)), and 0 if V <= 0.  Without classes it is the certificate above.  The class columns sit after the tile
+// columns of the tableau (col_site >= 1024: class slot col_site - 1024 of the weights buffer), so the simplex kernels are the same.
+//
 // Kernels: lp_reach_kernel (one warp per placement: footprint, dilations -> 32 row words), lp_init_kernel (dense condensed
 // tableau [m + 1][n + 1] in doubles: constraints x ceiling tiles, right-hand side, objective row), lp_simplex_kernel (ONE CTA
 // of 1024 threads: Devex pricing, ratio test, rank-1 update with the pivot row staged in shared memory; the
 // instances are a few hundred columns, launch-free pivoting beats a multi-CTA update with grid syncs), lp_simplex_cluster_kernel
 // (tableaus up to ~1.6 MB: rows resident in the shared memory of an 8-CTA thread-block cluster, exchange over distributed
-// shared memory), lp_certify_kernel (integer loads).
+// shared memory), lp_certify_kernel (integer loads, net of the class weights).
 #include <cooperative_groups.h>
 
 #include <algorithm>
@@ -35,7 +49,9 @@ namespace lp {
 constexpr uint32_t FULL = 0xffffffffu;
 constexpr int MAX_KEYS = 16;
 constexpr int THREADS = 1024;
-constexpr int MAX_COLS = 1024;                 // ceiling tiles of a 32x32 grid
+constexpr int MAX_CLASSES = 16;               // classes of per-type limits (card_limit_classes)
+constexpr int MAX_COLS = 1024 + MAX_CLASSES;   // ceiling tiles of a 32x32 grid, then the class columns
+constexpr int N_WEIGHTS = 1024 + MAX_CLASSES;  // weights buffer: k_t per site (index y * 32 + x), then zeta_j per class
 constexpr double EPS = 1e-9;
 // integer weights k_t = floor(y_t * scale); scale = 2^20 for costs up to 1024, smaller powers of two above (k_t fits an int)
 
@@ -43,6 +59,9 @@ struct Keys {
     int n;
     int w[MAX_KEYS], h[MAX_KEYS];
     int cost[MAX_KEYS];   // what a platform of this key costs: 1 for the platform count, the GUI's total_weight otherwise
+    uint32_t mask[MAX_KEYS];         // classes of per-type limits the key counts towards (bit j = class j)
+    int n_classes;
+    int limit[MAX_CLASSES];          // L_j
 };
 
 __device__ __forceinline__ uint32_t dilate(uint32_t X, uint32_t C, int lane) {
@@ -69,8 +88,9 @@ __global__ void __launch_bounds__(128) lp_reach_kernel(const uint32_t* __restric
     if (lane == 0) nonempty[p] = any ? 1 : 0;
 }
 
-// condensed tableau, row-major with leading dimension ld = n + 1: rows 0..m-1 = constraints (column j = tile col_site[j],
-// column n = right-hand side), row m = objective (-1 per tile, value 0)
+// condensed tableau, row-major with leading dimension ld = n + 1: rows 0..m-1 = constraints (column j = tile col_site[j], or class
+// col_site[j] - 1024 of the per-type limits: -1 where the placement's key is in the class; column n = right-hand side), row m =
+// objective (the negated coefficients: -1 per tile, +L_j per class, value 0)
 __global__ void lp_init_kernel(const uint32_t* __restrict__ reach, const int* __restrict__ cons, int m, const int* __restrict__ col_site, int n,
                                double* __restrict__ T, double perturb, Keys keys) {
     const int ld = n + 1;
@@ -78,11 +98,11 @@ __global__ void lp_init_kernel(const uint32_t* __restrict__ reach, const int* __
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
         const int i = (int)(idx / ld), j = (int)(idx % ld);
         double v;
-        if (i == m) v = j < n ? -1.0 : 0.0;
+        if (i == m) v = j == n ? 0.0 : col_site[j] < 1024 ? -1.0 : (double)keys.limit[col_site[j] - 1024];
         else if (j == n) v = (double)keys.cost[cons[i] >> 10] * (1.0 + perturb * (double)((i * 37) % 101) / 101.0);   // cost of the placement; tiny perturbation against degenerate ties (the certificate is exact anyway)
         else {
             const int s = col_site[j];
-            v = (double)((reach[(size_t)cons[i] * 32 + (s >> 5)] >> (s & 31)) & 1u);
+            v = s >= 1024 ? -(double)((keys.mask[cons[i] >> 10] >> (s - 1024)) & 1u) : (double)((reach[(size_t)cons[i] * 32 + (s >> 5)] >> (s & 31)) & 1u);
         }
         T[idx] = v;
     }
@@ -110,7 +130,7 @@ __device__ ArgD block_argmin(ArgD a, ArgD* red) {
 }
 
 // Primal simplex on the condensed tableau, all-slack start (y = 0 is feasible).  basis[i] = label of row i, nonbasis[j] =
-// label of column j; labels 0..n-1 are tiles, n.. are slacks.  info[0] = pivots, info[1] = 1 if optimal.
+// label of column j; labels 0..n-1 are tiles (then classes of per-type limits), n.. are slacks.  info[0] = pivots, info[1] = 1 if optimal.
 __global__ void __launch_bounds__(THREADS) lp_simplex_kernel(double* __restrict__ T, int m, int n, int* __restrict__ basis, int* __restrict__ nonbasis,
                                                             int max_pivots, double stop_at, int* __restrict__ info) {
     __shared__ double prow[MAX_COLS + 1];
@@ -138,7 +158,7 @@ __global__ void __launch_bounds__(THREADS) lp_simplex_kernel(double* __restrict_
             if (a > EPS) r = better_min(r, ArgD{T[(size_t)i * ld + n] / a, i});
         }
         r = block_argmin(r, red);
-        if (r.i == 0x7fffffff) break;   // unbounded: cannot happen (every tile lies in its own site's reach), never spin on it
+        if (r.i == 0x7fffffff) break;   // unbounded: only with limits that leave no layout covering every tile (without classes every tile lies in its own site's reach); never spin on it
         const int pr = r.i;
         const double piv = T[(size_t)pr * ld + q], inv = 1.0 / piv;
         __syncthreads();
@@ -238,7 +258,7 @@ __device__ __forceinline__ ArgD warp_argmin(ArgD a) {
 // Decisions are unchanged (same keys, same tie-breaks): the same pivot sequence and certificate as before.
 __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(CL_THREADS)
 lp_simplex_cluster_kernel(const double* __restrict__ T, int m, int n, const int* __restrict__ col_site, int max_pivots, double stop_at, int* __restrict__ info,
-                          int* __restrict__ weights /* [1024] zeroed */, double scale, long long* __restrict__ prof /* optional [8]: clock cycles per pivot stage */) {
+                          int* __restrict__ weights /* [N_WEIGHTS] zeroed */, double scale, long long* __restrict__ prof /* optional [8]: clock cycles per pivot stage */) {
     cg::cluster_group cluster = cg::this_cluster();
     const int rank = (int)cluster.block_rank(), tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, ld = n + 1;
     const int rows_per = (m + CLUSTER - 1) / CLUSTER, row0 = rank * rows_per, my_rows = max(0, min(rows_per, m - row0));
@@ -309,7 +329,7 @@ lp_simplex_cluster_kernel(const double* __restrict__ T, int m, int n, const int*
         cluster.sync();
         LP_LAP(2);
         const ArgD g = warp_argmin_nonneg(slots[par * CLUSTER + (lane & (CLUSTER - 1))]);   // the winner among the eight candidates
-        if (g.i == 0x7fffffff) break;                       // unbounded: cannot happen, never spin on it
+        if (g.i == 0x7fffffff) break;                       // unbounded: only with limits that leave no layout (see above), never spin on it
         const int pr = g.i, owner = pr / rows_per;
         const double* crow = cand + ((size_t)par * CLUSTER + owner) * ld;   // the pivot row before scaling: a local copy
         const double inv = fast_rcp(crow[q]);
@@ -362,7 +382,7 @@ constexpr int GRID_THREADS = 512;
 
 __global__ void __launch_bounds__(GRID_THREADS, 1)
 lp_simplex_grid_kernel(double* __restrict__ T, int m, int n, const int* __restrict__ col_site, int max_pivots, double stop_at, int* __restrict__ info,
-                       int* __restrict__ weights /* [1024] zeroed */, double scale, int* __restrict__ basis /* [m] */, int* __restrict__ nonbasis /* [n] */,
+                       int* __restrict__ weights /* [N_WEIGHTS] zeroed */, double scale, int* __restrict__ basis /* [m] */, int* __restrict__ nonbasis /* [n] */,
                        double* __restrict__ cand /* [2][gridDim.x][ld] */, ArgD* __restrict__ slots /* [2][gridDim.x] */) {
     cg::grid_group grid = cg::this_grid();
     const int G = (int)gridDim.x, rank = (int)blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, ld = n + 1;
@@ -420,7 +440,7 @@ lp_simplex_grid_kernel(double* __restrict__ T, int m, int n, const int* __restri
         ArgD g{__longlong_as_double(0x7ff0000000000000ll), 0x7fffffff};
         for (int c = lane; c < G; c += 32) g = better_min(g, ArgD{__ldcg(&slots[par * G + c].v), __ldcg(&slots[par * G + c].i)});   // (L2 reads: written by other SMs)
         g = warp_argmin_nonneg(g);
-        if (g.i == 0x7fffffff) break;                       // unbounded: cannot happen, never spin on it
+        if (g.i == 0x7fffffff) break;                       // unbounded: only with limits that leave no layout (see above), never spin on it
         const int pr = g.i, owner = pr / rows_per;
         const double* crow = cand + ((size_t)par * G + owner) * ld;   // the pivot row before scaling
         const double inv = fast_rcp(__ldcg(&crow[q]));
@@ -456,7 +476,7 @@ lp_simplex_grid_kernel(double* __restrict__ T, int m, int n, const int* __restri
 
 // y -> integer weights per site (floor(y * SCALE), never negative), zero for non-basic tiles
 __global__ void lp_weights_kernel(const double* __restrict__ T, int m, int n, const int* __restrict__ basis, const int* __restrict__ col_site,
-                                  int* __restrict__ weights /* [1024] zeroed */, double scale) {
+                                  int* __restrict__ weights /* [N_WEIGHTS] zeroed */, double scale) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= m) return;
     const int label = basis[i];
@@ -466,14 +486,16 @@ __global__ void lp_weights_kernel(const double* __restrict__ T, int m, int n, co
     weights[col_site[label]] = (int)(k > (1ll << 30) ? (1ll << 30) : k);
 }
 
-// exact certificate, all in 64-bit integers.  out[0] = sum of the weights k_t (lp_total_kernel).  For every in-bounds placement p (ALL
-// of them, not only the tableau's rows) with load(p) = sum of the weights in its reach: a layout L costs sum_{p in L} cost(p) and
-// covers every tile, so  total <= sum_{p in L} load(p) <= (max_p load(p) / cost(p)) * cost(L):  cost(L) >= total * cost(p) / load(p)
-// for the placement with the worst ratio.  out[1] = max load, out[2] = min over placements of ceil(total * cost(p) / load(p)) — the
-// bound.  With unit costs that is ceil(total / max load).
-__global__ void lp_total_kernel(const int* __restrict__ weights, unsigned long long* __restrict__ out) {
+// exact certificate, all in 64-bit integers.  out[0] = V = sum of the weights k_t minus sum_j L_j zeta_j (lp_total_kernel; signed,
+// it may be negative with classes).  For every in-bounds placement p (ALL of them, not only the tableau's rows) with the net
+// load(p) = sum of the weights in its reach minus the zeta of its key's classes: a layout L costs sum_{p in L} cost(p), covers every
+// tile and keeps every limit, so  V <= sum_{p in L} load(p) <= (max_p load(p) / cost(p)) * cost(L):  cost(L) >= V * cost(p) / load(p)
+// for the placement with the worst ratio.  out[1] = max load, out[2] = min over placements of ceil(V * cost(p) / load(p)) — the
+// bound, left at ~0 (no bound) when V <= 0.  With unit costs and no classes that is ceil(total / max load).
+__global__ void lp_total_kernel(const int* __restrict__ weights, Keys keys, unsigned long long* __restrict__ out) {
     long long s = 0;
     for (int t = threadIdx.x; t < 1024; t += 32) s += weights[t];
+    for (int j = threadIdx.x; j < keys.n_classes; j += 32) s -= (long long)keys.limit[j] * weights[1024 + j];
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(FULL, s, o);
     if (threadIdx.x == 0) out[0] = (unsigned long long)s;
 }
@@ -483,27 +505,37 @@ __global__ void __launch_bounds__(128) lp_certify_kernel(const uint32_t* __restr
     if (p >= n_placements) return;
     long long load = 0;
     for (uint32_t bits = reach[(size_t)p * 32 + lane]; bits; bits &= bits - 1) load += weights[lane * 32 + __ffs(bits) - 1];
+    if (lane < keys.n_classes && ((keys.mask[p >> 10] >> lane) & 1u)) load -= weights[1024 + lane];
     for (int o = 16; o > 0; o >>= 1) load += __shfl_xor_sync(FULL, load, o);
+    const long long total = (long long)out[0];
     if (lane == 0 && load > 0) {
-        const unsigned long long total = out[0], num = total * (unsigned long long)keys.cost[p >> 10];
         atomicMax(&out[1], (unsigned long long)load);
-        atomicMin(&out[2], (num + (unsigned long long)load - 1ull) / (unsigned long long)load);
+        if (total > 0) {
+            const unsigned long long num = (unsigned long long)total * (unsigned long long)keys.cost[p >> 10];
+            atomicMin(&out[2], (num + (unsigned long long)load - 1ull) / (unsigned long long)load);
+        }
     }
 }
 
 }  // namespace lp
 
-// rows32_host: terrain rows; key_dims: effective (w, h) per dims key.  out_weights (host, 1024 ints, index y * 32 + x),
-// key_costs: cost of a platform per key.  totals[0] = sum of the weights, totals[1] = largest placement load, totals[2] = the bound
-// (min over placements of ceil(total * cost / load); ~0 if no placement carries load), info[0] = pivots, info[1] = optimal, info[2] = constraints.
-int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs, int max_pivots,
-           long long target, int* out_weights, unsigned long long* totals, int* info) {
+// rows32_host: terrain rows; key_dims: effective (w, h) per dims key, key_costs: cost of a platform per key; key_mask / class_limit:
+// classes of per-type limits (card_limit_classes; empty: none).  out_weights (host, lp::N_WEIGHTS ints: index y * 32 + x, then
+// zeta_j at 1024 + j).  totals[0] = V (signed), totals[1] = largest net placement load, totals[2] = the bound (min over placements of
+// ceil(V * cost / load); ~0 if no placement carries load or V <= 0), info[0] = pivots, info[1] = optimal, info[2] = constraints.
+int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::vector<int2>& key_dims, const std::vector<int>& key_costs,
+           const std::vector<uint32_t>& key_mask, const std::vector<int>& class_limit, int max_pivots, long long target, int* out_weights,
+           unsigned long long* totals, int* info) {
     if ((int)key_dims.size() > lp::MAX_KEYS) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: more than %d dims keys", lp::MAX_KEYS);
+    if ((int)class_limit.size() > lp::MAX_CLASSES) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp_limits: more than %d classes", lp::MAX_CLASSES);
     lp::Keys keys;
     keys.n = (int)key_dims.size();
+    keys.n_classes = (int)class_limit.size();
+    for (int j = 0; j < lp::MAX_CLASSES; j++) keys.limit[j] = j < keys.n_classes ? class_limit[(size_t)j] : 0;
     int max_cost = 1;
     for (int i = 0; i < keys.n; i++) {
         keys.w[i] = key_dims[(size_t)i].x; keys.h[i] = key_dims[(size_t)i].y; keys.cost[i] = key_costs[(size_t)i];
+        keys.mask[i] = keys.n_classes ? key_mask[(size_t)i] : 0u;
         max_cost = key_costs[(size_t)i] > max_cost ? key_costs[(size_t)i] : max_cost;
     }
     double scale = (double)(1 << 20);            // y_t <= the largest cost: keep floor(y * scale) below 2^30
@@ -512,11 +544,13 @@ int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::
     std::vector<int> col_site;
     for (int s = 0; s < 1024; s++)
         if ((rows32_host[s >> 5] >> (s & 31)) & 1u) col_site.push_back(s);
+    const int tiles = (int)col_site.size();
+    for (int j = 0; j < keys.n_classes; j++) col_site.push_back(1024 + j);   // the class columns: z_j -> slot 1024 + j of the weights
     const int n = (int)col_site.size();
     totals[0] = totals[1] = totals[2] = 0;
     info[0] = info[1] = info[2] = 0;
-    for (int i = 0; i < 1024; i++) out_weights[i] = 0;
-    if (n == 0) return TSS_OK;
+    for (int i = 0; i < lp::N_WEIGHTS; i++) out_weights[i] = 0;
+    if (tiles == 0) return TSS_OK;
     // scratch slot 6: rows [32] | reach [n_place][32] | nonempty [n_place] bytes ; slot 7 is lb.cu's
     const size_t reach_words = (size_t)n_place * 32;
     uint32_t* buf = (uint32_t*)e->dev(6, sizeof(uint32_t) * (32 + reach_words) + (size_t)n_place);
@@ -537,16 +571,16 @@ int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::
     info[2] = m;
     const size_t cells = (size_t)(m + 1) * (n + 1);
     if (cells > ((size_t)1 << 27)) return e->fail(TSS_E_UNSUPPORTED, "tss_lower_bound_lp: tableau of %d x %d exceeds the supported size", m, n);
-    // scratch slot 5: tableau doubles | cons [m] | col_site [n] | basis [m] | nonbasis [n] | weights [1024] | info [4] | totals [2] u64
-    const size_t ints = (size_t)m + n + m + n + 1024 + 4;
+    // scratch slot 5: tableau doubles | cons [m] | col_site [n] | basis [m] | nonbasis [n] | weights [N_WEIGHTS] | info [4] | totals [3] u64
+    const size_t ints = (size_t)m + n + m + n + lp::N_WEIGHTS + 4;
     double* T = (double*)e->dev(5, sizeof(double) * cells + sizeof(int) * ints + 16 + 24);
     if (!T) return TSS_E_CUDA;
     int* cons_dev = (int*)(T + cells);
-    int *col_dev = cons_dev + m, *basis = col_dev + n, *nonbasis = basis + m, *weights = nonbasis + n, *info_dev = weights + 1024;
+    int *col_dev = cons_dev + m, *basis = col_dev + n, *nonbasis = basis + m, *weights = nonbasis + n, *info_dev = weights + lp::N_WEIGHTS;
     unsigned long long* totals_dev = (unsigned long long*)(((uintptr_t)(info_dev + 4) + 15) & ~(uintptr_t)15);
     TSS_CUDA(e, cudaMemcpyAsync(cons_dev, cons.data(), sizeof(int) * (size_t)m, cudaMemcpyHostToDevice, e->stream));
     TSS_CUDA(e, cudaMemcpyAsync(col_dev, col_site.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, e->stream));
-    TSS_CUDA(e, cudaMemsetAsync(weights, 0, sizeof(int) * (1024 + 4), e->stream));
+    TSS_CUDA(e, cudaMemsetAsync(weights, 0, sizeof(int) * (lp::N_WEIGHTS + 4), e->stream));
     TSS_CUDA(e, cudaMemsetAsync(totals_dev, 0, sizeof(unsigned long long) * 2, e->stream));
     TSS_CUDA(e, cudaMemsetAsync(totals_dev + 2, 0xff, sizeof(unsigned long long), e->stream));   // running minimum
     const int init_blocks = (int)((cells + 255) / 256 < (size_t)e->prop.multiProcessorCount * 8 ? (cells + 255) / 256 : (size_t)e->prop.multiProcessorCount * 8);
@@ -556,9 +590,11 @@ int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::
     const int pivots_cap = max_pivots > 0 ? max_pivots : 8 * (m + n);
     // target > 0: the caller only asks whether the bound reaches `target`.  Every iterate is feasible and the objective only grows,
     // so the simplex may stop once it exceeds target - 1 by more than the certificate loses to rounding (floor(y * scale) per
-    // tile: < n / scale in total; right-hand sides perturbed by 1e-7): the loop's question "nothing within target - 1?" is usually
-    // settled after 60-80 % of the pivots (ex2 / README terrain with 1x1 supports: 13.0 is passed long before the optimum 13.2 / 13.13)
-    const double stop_at = target > 0 ? (double)(target - 1) + 4.0 * (double)n / scale + 2e-3 : 0.0;
+    // tile: < tiles / scale in total; floor(z * scale) per class: a net load up to J units above cost * scale, which costs the
+    // bound up to J * target / scale; right-hand sides perturbed by 1e-7): the loop's question "nothing within target - 1?" is
+    // usually settled after 60-80 % of the pivots (ex2 / README terrain with 1x1 supports: 13.0 is passed long before the optimum
+    // 13.2 / 13.13).  Without classes n = tiles and the margin is 4 n / scale as it always was.
+    const double stop_at = target > 0 ? (double)(target - 1) + 4.0 * ((double)n + (double)keys.n_classes * (double)target) / scale + 2e-3 : 0.0;
     const int rows_per = (m + lp::CLUSTER - 1) / lp::CLUSTER, ld = n + 1;
     const size_t cl_smem = sizeof(double) * ((size_t)rows_per * ld + 2 * (size_t)ld + rows_per + 2 * (size_t)lp::CLUSTER * ld) + sizeof(lp::ArgD) * 2 * lp::CLUSTER +
                            sizeof(int) * ((size_t)m + n);
@@ -592,12 +628,12 @@ int lp_run(tss_engine* e, const uint32_t* rows32_host, int W, int H, const std::
             lp::lp_weights_kernel<<<(m + 255) / 256, 256, 0, e->stream>>>(T, m, n, basis, col_dev, weights, scale);
         }
     }
-    lp::lp_total_kernel<<<1, 32, 0, e->stream>>>(weights, totals_dev);
+    lp::lp_total_kernel<<<1, 32, 0, e->stream>>>(weights, keys, totals_dev);
     lp::lp_certify_kernel<<<(n_place + 3) / 4, 128, 0, e->stream>>>(reach, n_place, weights, keys, totals_dev);
     TSS_CHECK_LAUNCH(e);
     TSS_CUDA(e, cudaEventRecord(e->ev1, e->stream));
     e->stats.kernel_launches += 5;
-    TSS_CUDA(e, cudaMemcpyAsync(out_weights, weights, sizeof(int) * 1024, cudaMemcpyDeviceToHost, e->stream));
+    TSS_CUDA(e, cudaMemcpyAsync(out_weights, weights, sizeof(int) * lp::N_WEIGHTS, cudaMemcpyDeviceToHost, e->stream));
     TSS_CUDA(e, cudaMemcpyAsync(info, info_dev, sizeof(int) * 2, cudaMemcpyDeviceToHost, e->stream));
     TSS_CUDA(e, cudaMemcpyAsync(totals, totals_dev, sizeof(unsigned long long) * 3, cudaMemcpyDeviceToHost, e->stream));
     TSS_CUDA(e, cudaStreamSynchronize(e->stream));
