@@ -72,17 +72,21 @@ def ranges(name):
             rm_part: ([(src, rm0, rm1)], int(cap.group(1)) if cap else 5, True),
             "addition: 25 candidates (add_key/add_column)": ([(hdr, *body(H, r"uint32_t add_key\(")), (hdr, *body(H, r"uint32_t add_column\(")),
                                                               (src, *body(L, r"void slab\(")), (src, *body(L, r"uint32_t gain\("))], 1, False),
-            "addition: fetch, pick, tabu window, decode": ([(src, *body(L, r"Nbhd fetch\(")), (src, add0, find(L, r"flip<true>\(sm, tid, v, ", add0)),
+            "addition: fetch, pick, tabu window, decode": ([(src, *body(L, r"Nbhd fetch\(")), (src, add0, find(L, r"flip<true>\(sm, tid, [ev], ", add0)),
                                                             (hdr, find(H, r"const auto N = R\.fetch\(", run), find(H, r"const int v = add_site\(", run) + 1),
                                                             (hdr, *body(H, r"int add_site\(")), (spec, *body(S, r"void diamond_cell\(")), *pre], 1, False)}
 
 
 def transparent(name):
-    """sls_thread.cuh functions whose instructions count where they are called: the checked loads / stores (the macros of
-    earlier kernels) and the key and plane helpers that used to be written out at their call sites"""
-    hdr = os.path.join(B.CSRC, "sls_thread.cuh")
-    H = read(hdr)
-    return [(hdr, *body(H, pat)) for pat in (r" T ld\(", r"uint2 ld_tab\(", r"uint32_t& st\(", r"uint32_t flip_word\(", r"uint32_t remove_key\(")]
+    """functions whose instructions count where they are called: the checked loads / stores of sls_thread.cuh (the macros of
+    earlier kernels), its key and plane helpers that used to be written out at their call sites, and the one-instruction PTX
+    wrappers (and_b32, the kernel's min_u16x2)"""
+    hdr, src = os.path.join(B.CSRC, "sls_thread.cuh"), os.path.join(B.CSRC, name + ".cu")
+    H, L = read(hdr), read(src)
+    pats = [r" T ld\(", r"uint2 ld_tab\(", r"uint32_t& st\(", r"uint32_t flip_word\(", r"uint32_t remove_key\(", r"uint32_t and_b32\("]
+    # and the one-instruction PTX wrappers (r14 on)
+    return [(hdr, *body(H, pat)) for pat in pats if any(re.search(pat, l) for l in H)] + \
+        ([(src, *body(L, r"uint32_t min_u16x2\("))] if any("uint32_t min_u16x2(" in l for l in L) else [])
 
 
 def mix(name, out):

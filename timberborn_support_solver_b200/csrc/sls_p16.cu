@@ -62,24 +62,39 @@ __device__ __forceinline__ int slot(int i) {
     return i;
 }
 
-// first pair of site v's window: floor((y - 3) / 2) for v = 32 y + x (x < 32 never carries into the quotient)
-__device__ __forceinline__ int first_pair(int v) { return (v - 96) >> 6; }
 __device__ __forceinline__ int anchor(int x) { return __viaddmax_s32_relu(x, -3, 0); }   // max(x - 3, 0), one VIADDMNMX
+// the two 16-bit halves of a and b, each the lesser of its pair (one VIMNMX.U16x2): min16x2(w, 0x00010001) is 1 in each
+// half of w that is not zero
+__device__ __forceinline__ uint32_t min_u16x2(uint32_t a, uint32_t b) {
+    uint32_t r;
+    asm("min.u16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
+    return r;
+}
 // bytes 0 and 2 of four words as one word (row 2p / 2p+1 windows of four pairs: slots 0..7 -> two table words)
 __device__ __forceinline__ uint32_t pack_pairs(uint32_t a, uint32_t b) { return __byte_perm(a, b, 0x6420); }
 
-// site-list entry: site v (bits 0-8), first_pair(v) + 2 (bits 9-12) and the step it was added (bits 16-31).  Bits 9-12
-// are the byte offset of the window's first pair within a board, in units of one pair row (NT words = 512 bytes).  The
-// tabu test (stephi - e) < ten << 16 only sees bits 16-31: what the low half holds cannot borrow into them.
+// site-list entry of site v = 32 y + x: its window anchor ax = max(x - 3, 0) (bits 0-3, bit 4 zero), min(x, 3) (bits 5-6,
+// so x = ax + min(x, 3)), y + 1 (bits 8-12) and the step it was added (bits 16-31).
+//   * bits 0-4 are the shift count of the window's columns as they stand: a funnel shift takes its count mod 32, so the
+//     removal scan and the flips shift by the entry itself with no anchor derivation;
+//   * bits 9-12 are (y + 1) >> 1 = floor((y - 3) / 2) + 2, the window's first pair + 2, and as they stand the byte offset
+//     of that pair within a board in units of one pair row (NT words = 512 bytes);
+//   * the tabu test (stephi - e) < ten << 16 only sees bits 16-31: what the low half holds cannot borrow into them.
 static_assert(NT * sizeof(uint32_t) == 512, "entry() and removal_loss() take bits 9-12 of an entry as a byte offset of whole pair rows");
-__device__ __forceinline__ uint32_t entry(int v, uint32_t stamp) { return (uint32_t)v | (uint32_t)((v + 32) >> 6) << 9 | stamp << 16; }
+__device__ __forceinline__ uint32_t entry(int v, uint32_t stamp) {
+    const int x = v & 31, y = v >> 5;
+    return (uint32_t)anchor(x) | (uint32_t)min(x, 3) << 5 | (uint32_t)(y + 1) << 8 | stamp << 16;
+}
+// the site of entry e
+__device__ __forceinline__ int site(uint32_t e) { return (int)((e >> 8) & 31u) * 32 - 32 + (int)(e & 15u) + (int)((e >> 5) & 3u); }
+// w >> ax for entry e (a funnel shift with a zero high word takes bits 0-4 of e as the count)
+__device__ __forceinline__ uint32_t shr_anchor(uint32_t w, uint32_t e) { return __funnelshift_r(w, 0u, e); }
 
 // removal loss of list entry e with window win: reach tiles that only its support covers
 __device__ __forceinline__ uint32_t removal_loss(const Smem& sm, int tid, uint32_t e, uint2 win) {
-    const int ax = anchor(e & 31);
     const uint32_t* p = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(&sm.rows[B_O * NP - 2][0]) + ((e & 0x1e00u) | (uint32_t)tid << 2));
-    const uint32_t lo = pack_pairs(ld(sm, p) >> ax, ld(sm, p + NT) >> ax);
-    const uint32_t hi = pack_pairs(ld(sm, p + 2 * NT) >> ax, ld(sm, p + 3 * NT) >> ax);
+    const uint32_t lo = pack_pairs(shr_anchor(ld(sm, p), e), shr_anchor(ld(sm, p + NT), e));
+    const uint32_t hi = pack_pairs(shr_anchor(ld(sm, p + 2 * NT), e), shr_anchor(ld(sm, p + 3 * NT), e));
     return (uint32_t)(__popc(lo & win.x) + __popc(hi & win.y));
 }
 
@@ -100,21 +115,24 @@ __device__ __forceinline__ uint32_t tree_min(const uint32_t* key) {
     else return min(tree_min<N / 2>(key), tree_min<N / 2>(key + N / 2));
 }
 
-// adds (ADD) or removes the cover of site v (window win = its tab[0] entry) on the five count planes and refreshes U, O
-// and the non-empty-row mask.
+// adds (ADD) or removes the cover of list entry e (window win = its site's tab[0] entry) on the five count planes and
+// refreshes U, O and the non-empty-row mask.
 // rowmask is kept in padded coordinates: bit r + 4 = row r has an uncovered tile.
 template <bool ADD>
-__device__ __forceinline__ void flip(Smem& sm, int tid, int v, uint2 win, uint32_t& rowmask) {
-    const int ax = anchor(v & 31), p0 = first_pair(v);
-    uint32_t* p = &sm.rows[0][tid] + p0 * NT;  // pair p0 of the first board
+__device__ __forceinline__ void flip(Smem& sm, int tid, uint32_t e, uint2 win, uint32_t& rowmask) {
+    const int f = (int)((e >> 9) & 15u);        // first pair + 2
+    uint32_t* p = &sm.rows[0][tid] + (f - 2) * NT;  // first pair of the first board
+    // nz: bit 2j = the low row of pair f-2+j has an uncovered tile (bit 2j of the sum of min16x2(Un, 1) << 2j), bit 2j+1 =
+    // its high row (bit 16+2j of the sum, brought down by the shift by 15)
     uint32_t nz = 0;
 #pragma unroll
     for (int j = 0; j < 4; j++) {
         const uint32_t m8 = __byte_perm(j < 2 ? win.x : win.y, 0u, (j & 1) ? 0x4342 : 0x4140);   // slots 2j, 2j+1 at bits 0, 16
-        const uint32_t Un = flip_word<ADD, BOARD>(sm, tid, p, j * NT, m8 << ax, m8, p0 + j + 2);
-        nz |= ((Un & 0xffffu) ? 1u << (2 * j) : 0u) | ((Un >> 16) ? 2u << (2 * j) : 0u);
+        const uint32_t Un = flip_word<ADD, BOARD>(sm, tid, p, j * NT, __funnelshift_l(0u, m8, e), m8, f + j);   // m8 << ax
+        nz += min_u16x2(Un, 0x00010001u) * (1u << (2 * j));
     }
-    const int sh = 2 * p0 + 4;
+    nz = (nz | nz >> 15) & 0xffu;
+    const int sh = 2 * f;
     rowmask = (rowmask & ~(0xffu << sh)) | (nz << sh);
 }
 
@@ -124,7 +142,7 @@ __device__ __noinline__ void list_to_rows(const uint32_t* cached, const uint32_t
     uint32_t rows[16];
     for (int r = 0; r < 16; r++) rows[r] = 0;
     for (int i = 0; i < k; i++) {
-        const uint32_t v = (i < CAP ? cached[i * NT] : sl[(size_t)i * stride]) & 0x1ffu;
+        const int v = site(i < CAP ? cached[i * NT] : sl[(size_t)i * stride]);
         rows[v >> 5] |= 1u << (v & 31u);
     }
     for (int r = 0; r < 16; r++) out32[r] = rows[r];
@@ -209,9 +227,10 @@ struct Pairs {
             for (uint32_t bits = S[y]; bits; bits &= bits - 1, k++) {
                 const int v = y * 32 + __ffs(bits) - 1;
                 const uint2 win = ld_tab(sm, &sm.tab[0][v + TAB_PAD]);
-                if (k < CAP) { sm.cent[slot(k)][tid] = entry(v, reset); sm.cwin[slot(k)][tid] = win; }
-                else sl[(size_t)k * stride] = entry(v, reset);
-                flip<true>(sm, tid, v, win, rowmask);
+                const uint32_t e = entry(v, reset);
+                if (k < CAP) { sm.cent[slot(k)][tid] = e; sm.cwin[slot(k)][tid] = win; }
+                else sl[(size_t)k * stride] = e;
+                flip<true>(sm, tid, e, win, rowmask);
             }
         return k;
     }
@@ -227,7 +246,7 @@ struct Pairs {
             w_last = sm.cwin[slot(last)][tid];
         } else {
             e_last = sl[(size_t)last * stride];
-            w_last = ld_tab(sm, &sm.tab[0][(e_last & 0x1ffu) + TAB_PAD]);
+            w_last = ld_tab(sm, &sm.tab[0][site(e_last) + TAB_PAD]);
         }
         // cached slots: the warp scans a first group of SCAN slots, then the rest in pairs, up to its largest k (a thread
         // scores only its own k).  No branch inside a group, so the loads of its slots overlap: with 3 warps per scheduler
@@ -253,20 +272,20 @@ struct Pairs {
             uint32_t mult = (2u * CAP + 1u) * K3;                   // mult = (2i+1) * K3
             for (int i = CAP; i < k; i++, mult += 2u * K3) {
                 const uint32_t e = sl[(size_t)i * stride];
-                const uint32_t loss = removal_loss(sm, tid, e, ld_tab(sm, &sm.tab[0][(e & 0x1ffu) + TAB_PAD]));
+                const uint32_t loss = removal_loss(sm, tid, e, ld_tab(sm, &sm.tab[0][site(e) + TAB_PAD]));
                 best_key = min(best_key, removal_key(e, i, loss, hs * mult, stephi, young_below));
             }
         }
         pf.mark(PH_SCAN);
         const int best_i = (int)(best_key & 0xffu);
-        int u;
+        uint32_t e;
         uint2 win;
         if (best_i < CAP) {
-            u = (int)(sm.cent[slot(best_i)][tid] & 0x1ffu);
+            e = sm.cent[slot(best_i)][tid];
             win = sm.cwin[slot(best_i)][tid];
         } else {
-            u = (int)(sl[(size_t)best_i * stride] & 0x1ffu);
-            win = ld_tab(sm, &sm.tab[0][u + TAB_PAD]);
+            e = sl[(size_t)best_i * stride];
+            win = ld_tab(sm, &sm.tab[0][site(e) + TAB_PAD]);
         }
         if (best_i < CAP) {
             sm.cent[slot(best_i)][tid] = e_last;
@@ -274,8 +293,8 @@ struct Pairs {
         } else {
             sl[(size_t)best_i * stride] = e_last;
         }
-        flip<false>(sm, tid, u, win, rowmask);
-        return u;
+        flip<false>(sm, tid, e, win, rowmask);
+        return site(e);
     }
 
     __device__ __forceinline__ Nbhd fetch(uint32_t rowmask, uint32_t hs) const {
@@ -303,9 +322,10 @@ struct Pairs {
 
     __device__ __forceinline__ void add(int v, uint32_t step, int k, uint32_t& rowmask) {
         const uint2 win = ld_tab(sm, &sm.tab[0][v + TAB_PAD]);
-        flip<true>(sm, tid, v, win, rowmask);
-        if (k < CAP) { sm.cent[slot(k)][tid] = entry(v, step); sm.cwin[slot(k)][tid] = win; }
-        else sl[(size_t)k * stride] = entry(v, step);
+        const uint32_t e = entry(v, step);
+        flip<true>(sm, tid, e, win, rowmask);
+        if (k < CAP) { sm.cent[slot(k)][tid] = e; sm.cwin[slot(k)][tid] = win; }
+        else sl[(size_t)k * stride] = e;
     }
 
     __device__ __forceinline__ void list_to_rows(int k, uint32_t* out32) const { slsp::list_to_rows(cached, sl, stride, k, out32); }

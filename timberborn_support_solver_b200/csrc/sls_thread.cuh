@@ -7,8 +7,9 @@
 // A chain is one thread: its boards live in shared memory as [row][thread] words (bank = thread, conflict free for any row
 // index), every candidate layout is scored by that thread alone, and a warp instruction advances 32 layouts.
 //   * the site list lives in global memory as [index][chain] words (coalesced across the warp, L1 resident): site v in bits
-//     0-8, the step at which the support was added in bits 16-31 — for a current support that IS its last flip, so the
-//     "young support" test of the spec needs no per-site stamp array;
+//     0-8 (sls_p16.cu packs the site into the low half its own way, see its entry()), the step at which the support was
+//     added in bits 16-31 — for a current support that IS its last flip, so the "young support" test of the spec needs no
+//     per-site stamp array;
 //   * "recently removed" (the tabu test of add candidates, which are never current supports) is answered from a ring of
 //     the sites removed in the last 32 steps (one slot per step), folded once per step into a 7x7 window mask around the
 //     chosen uncovered tile.  Equivalent to the spec's 16-bit stamps for epochs of at most 32768 steps — the engine never
@@ -119,6 +120,12 @@ __device__ __forceinline__ uint32_t shl_clamped(uint32_t v, int n) {  // PTX shl
     asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
     return r;
 }
+// a & b as one AND that the compiler keeps: a product or a test of the result does not get the AND folded into it
+__device__ __forceinline__ uint32_t and_b32(uint32_t a, uint32_t b) {
+    uint32_t r;
+    asm("and.b32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
+    return r;
+}
 __device__ __forceinline__ constexpr int iabs(int a) { return a < 0 ? -a : a; }
 __device__ __forceinline__ constexpr int cell_index(int dx, int dy) { return cell_start(dy + 3) + dx + (3 - iabs(dy)); }
 
@@ -170,45 +177,45 @@ __device__ __forceinline__ uint32_t remove_key(uint32_t e, int i, uint32_t loss,
 }
 
 // One ADD candidate: the site at offset (DX, DY) from the uncovered tile.  S = the kernel's slab of U for this DX, from
-// which Nbhd::gain takes the candidate's gain with its reach window; tabt = the table entry of the tile, wt = the tile's
-// own window in byte-per-row format around (x-3, y-3) (candidate validity).  Keys are unique per cell (the cell index sits
-// in the low bits), so the maximum is independent of the evaluation order and ties go to the lowest cell as the spec demands.
+// which Nbhd::gain takes the candidate's gain with its reach window; tabt = the table entry of the tile; vf = validity and
+// freshness of the 25 candidates (add_site).  Keys are unique per cell (the cell index sits in the low bits), so the
+// maximum is independent of the evaluation order and ties go to the lowest cell as the spec demands.
 // One byte per field, most significant first: fresh * 64 + gain + 1 (a gain is at most 25 tiles; 1 in a noise step),
 // tie_add(hs, cell) in bytes 1-2, which are bytes 2-3 of the tie product, and (3 - DY) * 32 + (3 - DX) in byte 0: it falls
 // as the cell index grows (cells are numbered by DY, then DX), and the site is (y + 3) * 32 + x + 3 minus it, with no
-// decode of the cell.  The fields are built on the FMA pipe (one IMAD) and merged with one PRMT, off the integer-ALU pipe
-// that bounds both kernels.
+// decode of the cell.  The fields are built on the FMA pipe (IMADs) and merged with one PRMT, off the integer-ALU pipe
+// that bounds both kernels: one AND picks the candidate's two bits of vf, valid at bit a (lands in byte 1, which the PRMT
+// drops) and fresh at bit a + 16 (lands at bit 30, the 64 of byte 3), and the same AND decides validity.
 template <int DX, int DY, class Nbhd, class Smem>
-__device__ __forceinline__ uint32_t add_key(const Smem& sm, const typename Nbhd::Slab& S, const uint2* tabt, uint2 wt, uint32_t fresh_lo,
-                                            uint32_t fresh_hi, uint32_t hs, uint32_t gmul) {
-    constexpr int cell = cell_index(DX, DY), bit = 8 * (DY + 3) + DX + 3;   // position in t's byte-per-row window (rows 0-3 / 4-6)
+__device__ __forceinline__ uint32_t add_key(const Smem& sm, const typename Nbhd::Slab& S, const uint2* tabt, const uint32_t (&vf)[4],
+                                            uint32_t hs, uint32_t gmul) {
+    constexpr int cell = cell_index(DX, DY), a = 8 * ((DY + 3) & 1) + DX + 3;   // a: the candidate's validity bit in vf[(DY + 3) >> 1]
     const uint2 win = ld_tab(sm, tabt + DY * 32 + DX);
     const uint32_t g = Nbhd::template gain<DY>(S, win);
-    const bool fresh = ((bit < 32 ? fresh_lo >> bit : fresh_hi >> (bit - 32)) & 1u) != 0;   // (all zero in a noise step)
-    const uint32_t lo = (fresh ? 0x41000000u : 0x01000000u) | (uint32_t)((3 - DY) * 32 + 3 - DX);
-    const uint32_t key = __byte_perm(hs * ((2u * cell + 1u) * K2), g * gmul + lo, 0x7324);   // gmul = 1 << 24, or 0 in a noise step
-    const bool valid = ((bit < 32 ? wt.x >> bit : wt.y >> (bit - 32)) & 1u) != 0;
-    return valid ? key : 0u;
+    const uint32_t q = and_b32(vf[(DY + 3) >> 1], 1u << a | 1u << (a + 16));
+    const uint32_t lo = 0x01000000u | (uint32_t)((3 - DY) * 32 + 3 - DX);
+    const uint32_t key = __byte_perm(hs * ((2u * cell + 1u) * K2), g * gmul + lo + q * (1u << (14 - a)), 0x7324);   // gmul = 1 << 24, or 0 in a noise step
+    return q ? key : 0u;
 }
 
 // the best key of the candidates in column DX of the diamond: one slab of U serves all of them
 template <int DX, class Smem, class Nbhd>
-__device__ __forceinline__ uint32_t add_column(const Smem& sm, const Nbhd& N, uint32_t fresh_lo, uint32_t fresh_hi, uint32_t hs, uint32_t gmul) {
+__device__ __forceinline__ uint32_t add_column(const Smem& sm, const Nbhd& N, const uint32_t (&vf)[4], uint32_t hs, uint32_t gmul) {
     constexpr int M = 3 - iabs(DX);
     typename Nbhd::Slab S;
     N.template slab<DX, M>(S);
-    uint32_t mx = add_key<DX, 0, Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul);
+    uint32_t mx = add_key<DX, 0, Nbhd>(sm, S, N.tabt, vf, hs, gmul);
     if (M >= 1) {
-        mx = max(mx, add_key<DX, (M >= 1 ? -1 : 0), Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul));
-        mx = max(mx, add_key<DX, (M >= 1 ? 1 : 0), Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul));
+        mx = max(mx, add_key<DX, (M >= 1 ? -1 : 0), Nbhd>(sm, S, N.tabt, vf, hs, gmul));
+        mx = max(mx, add_key<DX, (M >= 1 ? 1 : 0), Nbhd>(sm, S, N.tabt, vf, hs, gmul));
     }
     if (M >= 2) {
-        mx = max(mx, add_key<DX, (M >= 2 ? -2 : 0), Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul));
-        mx = max(mx, add_key<DX, (M >= 2 ? 2 : 0), Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul));
+        mx = max(mx, add_key<DX, (M >= 2 ? -2 : 0), Nbhd>(sm, S, N.tabt, vf, hs, gmul));
+        mx = max(mx, add_key<DX, (M >= 2 ? 2 : 0), Nbhd>(sm, S, N.tabt, vf, hs, gmul));
     }
     if (M >= 3) {
-        mx = max(mx, add_key<DX, (M >= 3 ? -3 : 0), Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul));
-        mx = max(mx, add_key<DX, (M >= 3 ? 3 : 0), Nbhd>(sm, S, N.tabt, N.wt, fresh_lo, fresh_hi, hs, gmul));
+        mx = max(mx, add_key<DX, (M >= 3 ? -3 : 0), Nbhd>(sm, S, N.tabt, vf, hs, gmul));
+        mx = max(mx, add_key<DX, (M >= 3 ? 3 : 0), Nbhd>(sm, S, N.tabt, vf, hs, gmul));
     }
     return mx;
 }
@@ -242,15 +249,19 @@ __device__ __forceinline__ int add_site(const Smem& sm, int tid, const Nbhd& N, 
 #pragma unroll 1
     for (int j = RECENT + 1; j < ten; j++) tabu_bit(sm.ring[(step - (uint32_t)j) & 31u][tid], x, y, tw_lo, tw_hi);
     pf.mark(PH_FETCH);
-    const uint32_t fresh_lo = noise ? 0u : ~tw_lo, fresh_hi = noise ? 0u : ~tw_hi;
+    // vf[i]: rows 2i, 2i+1 of t's window N.wt (byte-per-row, validity) in bytes 0-1, the same rows of its valid and fresh
+    // candidates (not tabu; none in a noise step) in bytes 2-3
+    const uint32_t fv_lo = noise ? 0u : N.wt.x & ~tw_lo, fv_hi = noise ? 0u : N.wt.y & ~tw_hi;
+    const uint32_t vf[4] = {__byte_perm(N.wt.x, fv_lo, 0x5410), __byte_perm(N.wt.x, fv_lo, 0x7632), __byte_perm(N.wt.y, fv_hi, 0x5410),
+                            __byte_perm(N.wt.y, fv_hi, 0x7632)};
     const uint32_t gmul = noise ? 0u : 1u << 24;
-    uint32_t mx = add_column<0>(sm, N, fresh_lo, fresh_hi, hs, gmul);
-    mx = max(mx, add_column<-1>(sm, N, fresh_lo, fresh_hi, hs, gmul));
-    mx = max(mx, add_column<1>(sm, N, fresh_lo, fresh_hi, hs, gmul));
-    mx = max(mx, add_column<-2>(sm, N, fresh_lo, fresh_hi, hs, gmul));
-    mx = max(mx, add_column<2>(sm, N, fresh_lo, fresh_hi, hs, gmul));
-    mx = max(mx, add_column<-3>(sm, N, fresh_lo, fresh_hi, hs, gmul));
-    mx = max(mx, add_column<3>(sm, N, fresh_lo, fresh_hi, hs, gmul));
+    uint32_t mx = add_column<0>(sm, N, vf, hs, gmul);
+    mx = max(mx, add_column<-1>(sm, N, vf, hs, gmul));
+    mx = max(mx, add_column<1>(sm, N, vf, hs, gmul));
+    mx = max(mx, add_column<-2>(sm, N, vf, hs, gmul));
+    mx = max(mx, add_column<2>(sm, N, vf, hs, gmul));
+    mx = max(mx, add_column<-3>(sm, N, vf, hs, gmul));
+    mx = max(mx, add_column<3>(sm, N, vf, hs, gmul));
     return (y + 3) * 32 + x + 3 - (int)(mx & 0xffu);   // the winning site from the key's low byte
 }
 
