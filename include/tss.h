@@ -221,7 +221,9 @@ typedef struct tss_search_params {
  * windows with the platforms near window borders frozen, and keeps each window's best (its target_count is not used:
  * the windows search without a target).  n_chains = chains per window
  * (rounded up to a multiple of 4; 0 = 8..16).  Otherwise (AUTO) those grids run the 1x1 window decomposition with a
- * host post-pass.  tss_search_create answers TSS_E_UNSUPPORTED where it does not apply. */
+ * host post-pass.  tss_search_create answers TSS_E_UNSUPPORTED where it does not apply.  With per-type limits
+ * (tss_search_create_with_limits) AUTO selects this search too, and every window's chains run with per-class budgets that
+ * keep the global layout within every limit. */
 #define TSS_KERNEL_WINDOW_PLACEMENTS 5
 
 /* Creates a portfolio on one terrain.  defs must contain 1x1 (encoder.rs:564-566). */
@@ -337,7 +339,8 @@ typedef struct tss_instance_info {
     int32_t w, h, n_defs;            /* terrain size and platform set of the encoding */
     int32_t card_limit_1x1;          /* n of "at most n platforms" (PlatformLimits.card_limits[1x1], main.rs:346), -1 if none */
     int32_t n_other_card_limits;     /* card limits on other platform types (per-type limits: tss_solve_instance steers the search by
-                                        them on grids up to 32x32 when the handle came from tss_instance_find) */
+                                        them on grids up to 32x32, larger ones with tss_engine_window_limits, when the handle came
+                                        from tss_instance_find) */
     int32_t has_weight_limit;
     int64_t weight_limit;            /* PlatformLimits.weight_limit (crates/gui/src/app.rs:235-245) */
     int32_t n_weights;
@@ -377,10 +380,15 @@ int tss_cnf_complete(tss_engine* e, const tss_cnf* c, uint8_t* assignment, int32
  * such instances (grids up to 32x32) take the class-aware LP (tss_lower_bound_lp_limits) instead of the plain one, which is what
  * ends a `solve -l k:v` loop whose optimum the limits moved above the plain bounds.  Each LP bound is cached on the encoding,
  * keyed by the per-type records and the weights.
+ * Instances with per-type limits on grids larger than 32x32 return TSS_UNKNOWN unless tss_engine_window_limits is on: then
+ * tss_solve_with_limits answers them (the window placement search), TSS_SAT with a verified model or TSS_UNKNOWN, never
+ * TSS_UNSAT (there is no class-aware bound at that size; a platform set that search does not take is TSS_UNKNOWN too).
  * tss_engine_certified_unsat switches the bound-based UNSAT answers off (0) or on (non-zero, the default);
- * tss_engine_limit_bounds switches the class-aware LP on (non-zero) or off (0, the default). */
+ * tss_engine_limit_bounds switches the class-aware LP on (non-zero) or off (0, the default);
+ * tss_engine_window_limits switches the answers on grids larger than 32x32 with per-type limits on (non-zero) or off (0, the default). */
 int tss_engine_certified_unsat(tss_engine* e, int enabled);
 int tss_engine_limit_bounds(tss_engine* e, int enabled);
+int tss_engine_window_limits(tss_engine* e, int enabled);
 int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc, const tss_instance_info* info, const int32_t* weights,
                        uint64_t seed, int64_t give_up_steps, uint8_t* assignment);
 
@@ -408,12 +416,26 @@ int tss_card_limit_classes(const tss_dims* defs, int32_t n_defs, const int32_t* 
  * first tss_search_run.  TSS_E_INVALID for a 1x1 record (the platform count is the search's bound: tss_search_set_bound), a
  * negative limit, or after the first run; vacuous records are ignored (on a {1x1}-only set every record is); TSS_E_UNSUPPORTED
  * for a record that is not vacuous on a search other than the placement search on a grid up to 32x32 (the window searches:
- * their windows pick winners independently, which could jointly exceed a limit). */
+ * their windows pick winners independently, which could jointly exceed a limit; tss_search_create_with_limits gives the window
+ * placement search limits it keeps). */
 int tss_search_set_card_limits(tss_search* s, const int32_t* card, int32_t n_card);
+/* tss_search_create with per-type limits fixed at creation.  Records and errors are those of tss_search_set_card_limits (a 1x1
+ * record or a negative limit is TSS_E_INVALID, vacuous records are ignored).  Grids up to 32x32: tss_search_create followed by
+ * tss_search_set_card_limits.  Larger grids with a record that is not vacuous: the window placement search (kernel AUTO or
+ * TSS_KERNEL_WINDOW_PLACEMENTS; tss_search_kernel reports TSS_KERNEL_WINDOW_PLACEMENTS) from the greedy placement cover trimmed
+ * to the limits — its platforms in row-major anchor order, each kept while every class it belongs to has room, then a 1x1 on
+ * every ceiling tile still unsupported, row-major.  In every phase window w's chains run with class budgets
+ * b_{w,j} = m_{w,j} + floor(s_j / N) + [((w - p) mod N) < (s_j mod N)] (m_{w,j} = the window's movable platforms in class j,
+ * s_j = L_j - n_j the slack of the global layout, N windows, p the phase), so the global layout keeps every limit after every
+ * phase whatever each window's winner is.  TSS_E_UNSUPPORTED for a platform set that search does not take (more than 16 dims
+ * keys, or a key beyond 6x6), for another kernel, and on more than one rank. */
+int tss_search_create_with_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
+                                  int32_t n_card, const tss_search_params* params, tss_search** out);
 /* The PlatformLimits-shaped one-shot solve: card = records (def_w, def_h, limit) including the platform count (1x1); with
  * weights (n_weights > 0) the objective is the total weight, bounded by weight_limit (< 0: unbounded), and a 1x1 record is
  * TSS_E_UNSUPPORTED (one objective per search).  Defs in a class with limit 0 are dropped from the set first (as --platforms
- * would), positive limits steer the placement search (tss_search_set_card_limits; grids up to 32x32).  Budgets and the return
+ * would), positive limits steer the placement search (tss_search_set_card_limits on grids up to 32x32; on larger grids the window
+ * placement search with the limits fixed at creation, tss_search_create_with_limits).  Budgets and the return
  * contract are tss_solve_upper_bound's: TSS_SAT with the layout and *out_objective (optional) = its count or weight, TSS_UNKNOWN
  * if none was found, never TSS_UNSAT. */
 int tss_solve_with_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,

@@ -150,6 +150,7 @@ unsafe extern "C" {
     pub fn tss_cnf_complete(e: *mut tss_engine, c: *const tss_cnf, assignment: *mut u8, out_conflict: *mut i32, out_n_falsified: *mut i32) -> c_int;
     pub fn tss_engine_certified_unsat(e: *mut tss_engine, enabled: c_int) -> c_int;
     pub fn tss_engine_limit_bounds(e: *mut tss_engine, enabled: c_int) -> c_int;
+    pub fn tss_engine_window_limits(e: *mut tss_engine, enabled: c_int) -> c_int;
     pub fn tss_solve_instance(
         e: *mut tss_engine, c: *const tss_cnf, enc: *const tss_encoding, info: *const tss_instance_info, weights: *const i32, seed: u64,
         give_up_steps: i64, assignment: *mut u8,
@@ -219,6 +220,10 @@ unsafe extern "C" {
     ) -> c_int;
     pub fn tss_search_set_weights(s: *mut tss_search, weights: *const i32, n_weights: i32) -> c_int;
     pub fn tss_search_set_card_limits(s: *mut tss_search, card: *const i32, n_card: i32) -> c_int;
+    pub fn tss_search_create_with_limits(
+        e: *mut tss_engine, grid: *const u8, w: i32, h: i32, defs: *const tss_dims, n_defs: i32, card: *const i32, n_card: i32,
+        params: *const tss_search_params, out: *mut *mut tss_search,
+    ) -> c_int;
     pub fn tss_card_limit_classes(
         defs: *const tss_dims, n_defs: i32, card: *const i32, n_card: i32, key_mask: *mut i32, class_limit: *mut i32, n_keys: *mut i32,
         n_classes: *mut i32,

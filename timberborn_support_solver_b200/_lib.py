@@ -105,6 +105,7 @@ SIGNATURES = {
     "tss_solve_upper_bound": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32, _u64, _i32, _i64, _P(Platform), _i32, _i32p]),
     "tss_card_limit_classes": (C.c_int, [_P(Dims), _i32, _i32p, _i32, _i32p, _i32p, _i32p, _i32p]),
     "tss_search_set_card_limits": (C.c_int, [_vp, _i32p, _i32]),
+    "tss_search_create_with_limits": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _P(SearchParams), _P(_vp)]),
     "tss_solve_with_limits": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32p, _i32, _i64, _u64, _i32, _i64, _P(Platform), _i32, _i32p, _i64p]),
     "tss_lower_bound": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _u64, _i32, _i32p, _i32, _i32p]),
     "tss_lower_bound_lp": (C.c_int, [_vp, _u8p, _i32, _i32, _P(Dims), _i32, _i32p, _i32, _i32, _i64, _i32p, _i64p, _i64p, _i64p, _i32p]),
@@ -119,6 +120,7 @@ SIGNATURES = {
     "tss_cnf_complete": (C.c_int, [_vp, _vp, _u8p, _i32p, _i32p]),
     "tss_engine_certified_unsat": (C.c_int, [_vp, C.c_int]),
     "tss_engine_limit_bounds": (C.c_int, [_vp, C.c_int]),
+    "tss_engine_window_limits": (C.c_int, [_vp, C.c_int]),
     "tss_measure_peaks": (C.c_int, [_vp, _P(C.c_double), _i32]),
 }
 

@@ -464,17 +464,26 @@ def card_limit_classes(defs, limits: dict):
 class Search:
     """A device-resident SLS portfolio on one terrain (kernel (b))."""
 
-    def __init__(self, engine: "Engine", grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], seed=0, n_chains=0, chain_offset=0, noise_pct=-1, kernel=0):
+    def __init__(self, engine: "Engine", grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], seed=0, n_chains=0, chain_offset=0, noise_pct=-1, kernel=0,
+                 limits: Optional[dict] = None):
         """kernel: KERNEL_AUTO / KERNEL_WARP / KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR (tss.h TSS_KERNEL_*): equivalent SLS kernels
         (KERNEL_PAIR: one chain per thread with two grid rows per word, grids of at most 16x16).  KERNEL_WINDOW_PLACEMENTS: the
         window-decomposed placement search on grids larger than 32x32 with platforms beyond 1x1 (n_chains = chains per window); each
-        run() is a phase that can only improve the global layout, best_layout() returns it (before the first run: the greedy cover)."""
+        run() is a phase that can only improve the global layout, best_layout() returns it (before the first run: the greedy cover).
+        limits ({PlatformDef: limit}, per-type limits without 1x1): fixed at creation (tss_search_create_with_limits).  Up to 32x32
+        that is set_card_limits; on larger grids AUTO selects the window placement search, which starts from the greedy cover
+        trimmed to the limits and keeps them in every phase."""
         self.engine, self.grid = engine, grid
         self._h = C.c_void_p()
         params = _lib.SearchParams(seed, n_chains, chain_offset, noise_pct, kernel)
         defs = list(defs)
-        engine._check(engine.lib.tss_search_create(engine._h, _ptr(grid.data, C.c_uint8), grid.width, grid.height, _defs_array(defs), len(defs),
-                                                   C.byref(params), C.byref(self._h)))
+        common = (engine._h, _ptr(grid.data, C.c_uint8), grid.width, grid.height, _defs_array(defs), len(defs))
+        if limits is None:
+            engine._check(engine.lib.tss_search_create(*common, C.byref(params), C.byref(self._h)))
+        else:
+            card = _card_records(limits)
+            engine._check(engine.lib.tss_search_create_with_limits(*common, _ptr(card, C.c_int32) if len(card) else None, len(card), C.byref(params),
+                                                                   C.byref(self._h)))
         self.n_chains = engine.lib.tss_search_n_chains(self._h)
 
     def close(self):
@@ -665,7 +674,8 @@ class Engine:
     def search(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], **kw) -> Search:
         """A device-resident SLS portfolio; kw: seed, n_chains, chain_offset, noise_pct, kernel (KERNEL_AUTO, or one of KERNEL_WARP /
         KERNEL_HALF_WARP / KERNEL_THREAD / KERNEL_PAIR to pin a variant, or KERNEL_WINDOW_PLACEMENTS for the placement search on
-        grids larger than 32x32; a kernel that does not fit the grid or platform set raises TssError)."""
+        grids larger than 32x32; a kernel that does not fit the grid or platform set raises TssError), limits ({PlatformDef: limit},
+        per-type limits fixed at creation: see Search)."""
         return Search(self, grid, defs, **kw)
 
     def solve_upper_bound(self, grid: WorldGrid, defs=PLATFORMS_DEFAULT[:1], card_limit: Optional[int] = None, seed=0, budget_ms=0, max_steps=0):
@@ -756,6 +766,11 @@ class Engine:
         LP (grids up to 32x32) instead of the bounds of the whole set.  Off by default."""
         self._check(self.lib.tss_engine_limit_bounds(self._h, 1 if enabled else 0))
 
+    def window_limits(self, enabled: bool = True):
+        """tss_engine_window_limits: tss_solve_instance answers instances with per-type limits on grids larger than 32x32 with the
+        window placement search (SAT with a verified model, or unknown; never UNSAT).  Off by default."""
+        self._check(self.lib.tss_engine_window_limits(self._h, 1 if enabled else 0))
+
     def solve_batch(self, grids, seed=0, steps=2048, want_layouts=False, chains_per_terrain=0):
         """grids: uint8[n, h, w] -> counts int32[n] (and packed support rows uint32[n, h] if asked)"""
         g = _u8(grids)
@@ -779,9 +794,12 @@ class GpuBoundSolver:
     solve() returns SAT with a CNF-verified witness when a layout within the instance's bound exists in the budget,
     INTERRUPTED (unknown) otherwise — never UNSAT, only the exact solver proves that (see INTEGRATION.md)."""
 
-    def __init__(self, engine: Engine, encoding: Encoding, limits: PlatformLimits, seed=0, budget_ms=50, max_steps=0):
+    def __init__(self, engine: Engine, encoding: Encoding, limits: PlatformLimits, seed=0, budget_ms=50, max_steps=0, window_limits=False):
+        """window_limits: instances with per-type limits on grids larger than 32x32 are searched (the window placement search)
+        instead of being left to the exact solver."""
         self.engine, self.encoding, self.limits = engine, encoding, limits
         self.seed, self.budget_ms, self.max_steps = seed, budget_ms, max_steps
+        self.window_limits = window_limits
         self._cnf: Optional[Cnf] = None
         self._dev: Optional[DeviceCnf] = None
         self._solution = None
@@ -798,17 +816,23 @@ class GpuBoundSolver:
         """SAT with a CNF-verified witness, or INTERRUPTED = "the GPU could not answer within its budget" (which is also what a
         real interrupt returns).  The search is steered by the 1x1 card limit (= the platform count, what the REPL tightens,
         main.rs:346) or by the weight limit (the GUI's objective, app.rs:235-245), and by limits on other platform types
-        (`solve -l k:v`) on grids up to 32x32; elsewhere such instances go to the exact solver."""
+        (`solve -l k:v`) on grids up to 32x32, larger ones with window_limits; elsewhere such instances go to the exact solver."""
         one = PlatformDef(1, 1)
         bound = self.limits.card_limits.get(one)
         self.engine.clear_interrupt()      # the flag is sticky by design (InterruptSolver::interrupt may fire before solve starts a kernel): one solve, one flag
         weighted = bool(self.limits.weights) and (self.limits.weight_limit is not None or bound is None)
         if any(d != one for d in self.limits.card_limits):
             g = self.encoding._grid
-            if g.width > 32 or g.height > 32 or (weighted and bound is not None):
+            large = g.width > 32 or g.height > 32
+            if (large and not self.window_limits) or (weighted and bound is not None):
                 return INTERRUPTED         # limits the search cannot steer by here: leave the instance to the exact solver
             lim = self.limits if weighted else PlatformLimits(dict(self.limits.card_limits), {}, None)
-            res, layout, _ = self.engine.solve_with_limits(g, self.encoding.defs, lim, self.seed, self.budget_ms, self.max_steps)
+            try:
+                res, layout, _ = self.engine.solve_with_limits(g, self.encoding.defs, lim, self.seed, self.budget_ms, self.max_steps)
+            except TssError as err:        # a platform set the window placement search does not take: the exact solver's instance
+                if not large or err.code != _lib.TSS_E_UNSUPPORTED:
+                    raise
+                return INTERRUPTED
         elif weighted:
             # the GUI's instances: weights always, a weight limit from the second iteration on (app.rs:235-245)
             res, layout, _ = self.engine.solve_min_weight(self.encoding._grid, self.encoding.defs, self.limits.weights, self.limits.weight_limit,
@@ -836,7 +860,7 @@ class GpuBoundSolver:
 
 
 def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, engine: Engine, exact_solver=None, seed=0, budget_ms=None,
-                on_solution=None, use_lower_bound=True, limit_bounds=False):
+                on_solution=None, use_lower_bound=True, limit_bounds=False, window_limits=False):
     """crates/repl/src/main.rs:280-366 with the GPU engine as the SAT side and an optional exact solver
     (`exact_solver(cnf) -> (SAT|UNSAT|INTERRUPTED, assignment)`, Glucose in the reference) for the proof.
 
@@ -850,6 +874,9 @@ def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, en
 
     limit_bounds: loops with per-type limits (`solve -l k:v`) use the bounds as well, the fractional one being the class-aware LP
     that keeps the limits (Engine.lower_bound_lp(..., limits=...)); without it only loops whose sole limit is the count do.
+
+    window_limits: loops with per-type limits on grids larger than 32x32 ask the GPU (the window placement search) instead of going
+    straight to the exact solver; without an exact solver such a loop ends INTERRUPTED once the GPU finds nothing below the count.
 
     Returns dict(best=PlatformLayout|None, proved_optimal=bool, steps=[...], lower_bound=int|None)."""
     one = PlatformDef(1, 1)
@@ -886,9 +913,9 @@ def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, en
         lp_pending = use_lower_bound and not lp_done and best is not None
         first = max(128, give_up // 8) if (budget_ms is None and lp_pending) else give_up
         if budget_ms is None:
-            solver = GpuBoundSolver(engine, encoding, limits, seed=seed, budget_ms=0, max_steps=-first)
+            solver = GpuBoundSolver(engine, encoding, limits, seed=seed, budget_ms=0, max_steps=-first, window_limits=window_limits)
         else:
-            solver = GpuBoundSolver(engine, encoding, limits, seed=seed, budget_ms=budget_ms)
+            solver = GpuBoundSolver(engine, encoding, limits, seed=seed, budget_ms=budget_ms, window_limits=window_limits)
         solver.add_cnf(cnf)                                     # solver_runner.rs:12
         result = solver.solve()
         if result != SAT and lp_pending:
@@ -900,7 +927,8 @@ def solver_loop(project: Project, encoding: Encoding, limits: PlatformLimits, en
                 proved = True
                 break
             if budget_ms is None and first < give_up:           # not refuted: the whole budget, other seeds
-                solver = GpuBoundSolver(engine, encoding, limits, seed=seed ^ 0x9E3779B97F4A7C15, budget_ms=0, max_steps=-give_up)
+                solver = GpuBoundSolver(engine, encoding, limits, seed=seed ^ 0x9E3779B97F4A7C15, budget_ms=0, max_steps=-give_up,
+                                        window_limits=window_limits)
                 solver.add_cnf(cnf)
                 result = solver.solve()
         if result == SAT:

@@ -68,7 +68,8 @@ int lns_chains(const LnsSearch* s);
 // lns_placements.cu — window-decomposed placement search for grids larger than 32x32 (TSS_KERNEL_WINDOW_PLACEMENTS)
 struct LnspSearch;
 int lnsp_create(tss_engine* e, const uint8_t* grid, int w, int h, const uint8_t* anchors, const int2* keys_dev, const int* costs_dev, const int* order_dev,
-                int n_keys, int seeds, uint64_t seed, uint32_t chain_offset, int noise, LnspSearch** out);
+                int n_keys, int seeds, uint64_t seed, uint32_t chain_offset, int noise, const uint32_t* class_mask, const int* class_limit, int n_classes,
+                LnspSearch** out);
 void lnsp_destroy(LnspSearch* s);
 int lnsp_phase(tss_engine* e, LnspSearch* s, long long steps);
 int lnsp_objective(tss_engine* e, LnspSearch* s);
@@ -76,6 +77,7 @@ int lnsp_anchors(tss_engine* e, LnspSearch* s, std::vector<uint8_t>& anchors);
 int lnsp_value(const LnspSearch* s);
 unsigned long long lnsp_total(const LnspSearch* s, int i);
 int lnsp_chains(const LnspSearch* s);
+int lnsp_over_limit(const LnspSearch* s, int* count, int* limit);
 // sls_multi.cu — placements of several platform types
 size_t slsm_state_bytes();
 int slsm_max_keys();
@@ -753,7 +755,7 @@ static int card_limit_classes(const std::vector<int2>& key_dims, const int32_t* 
     return TSS_OK;
 }
 
-static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds);
+static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds, const int32_t* card, int n_card);
 
 // Chains that fill the device: 32 warps per SM for the warp kernels (two chains per warp on grids of <= 16 rows),
 // 3 CTAs of 128 threads per SM for the thread-per-chain kernels.
@@ -764,8 +766,9 @@ static int default_chains(const tss_engine* e, int w, int h, int kernel) {
     return e->prop.multiProcessorCount * per_sm;
 }
 
-int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
-                      const tss_search_params* params, tss_search** out) {
+// tss_search_create; card / n_card: per-type limit records for the window placement search (tss_search_create_with_limits)
+static int search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
+                         const tss_search_params* params, const int32_t* card, int32_t n_card, tss_search** out) {
     if (!e) return TSS_E_INVALID;
     if (!grid || !out || w <= 0 || h <= 0 || (!defs && n_defs > 0)) return e->fail(TSS_E_INVALID, "tss_search_create: bad arguments");
     if (int rc = check_defs(e, defs, n_defs, "tss_search_create", nullptr)) return rc;
@@ -788,7 +791,7 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
         fill = fill < 8 ? 8 : (fill > 16 ? 16 : fill);
         int seeds = (params && params->n_chains > 0) ? ((params->n_chains + 3) / 4) * 4 : fill;
         if (params && params->kernel == TSS_KERNEL_WINDOW_PLACEMENTS) {
-            int rc = window_placements_create(e, s, defs, n_defs, seeds);
+            int rc = window_placements_create(e, s, defs, n_defs, seeds, card, n_card);
             if (rc != TSS_OK) { search_free(s); return rc; }
             *out = s;
             return TSS_OK;
@@ -865,6 +868,46 @@ int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, 
     if (rc != TSS_OK) { search_free(s); return rc; }
     *out = s;
     return TSS_OK;
+}
+
+int tss_search_create(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs,
+                      const tss_search_params* params, tss_search** out) {
+    return search_create(e, grid, w, h, defs, n_defs, params, nullptr, 0, out);
+}
+
+int tss_search_create_with_limits(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h, const tss_dims* defs, int32_t n_defs, const int32_t* card,
+                                  int32_t n_card, const tss_search_params* params, tss_search** out) {
+    if (!e) return TSS_E_INVALID;
+    if (!grid || !out || w <= 0 || h <= 0 || (!defs && n_defs > 0) || n_card < 0 || (n_card > 0 && !card))
+        return e->fail(TSS_E_INVALID, "tss_search_create_with_limits: bad arguments");
+    if (int rc = check_defs(e, defs, n_defs, "tss_search_create_with_limits", nullptr)) return rc;
+    for (int i = 0; i < n_card; i++) {
+        if (card[3 * i] == 1 && card[3 * i + 1] == 1)
+            return e->fail(TSS_E_INVALID, "tss_search_create_with_limits: the platform count (1x1) is the search's bound, not a per-type limit");
+        if (card[3 * i + 2] < 0) return e->fail(TSS_E_INVALID, "tss_search_create_with_limits: negative limit for %dx%d", card[3 * i], card[3 * i + 1]);
+    }
+    if (w <= 32 && h <= 32) {
+        int rc = tss_search_create(e, grid, w, h, defs, n_defs, params, out);
+        if (rc == TSS_OK && (rc = tss_search_set_card_limits(*out, card, n_card)) != TSS_OK) {
+            tss_search_destroy(*out);
+            *out = nullptr;
+        }
+        return rc;
+    }
+    std::vector<int2> kd;
+    std::vector<tss_platform> kp;
+    std::vector<uint32_t> mask;
+    std::vector<int> lim;
+    build_keys(defs, n_defs, kd, kp);
+    int rc = card_limit_classes(kd, card, n_card, mask, lim);
+    if (rc) return e->fail(rc, "tss_search_create_with_limits: bad limit records");
+    if (lim.empty()) return tss_search_create(e, grid, w, h, defs, n_defs, params, out);   // every record vacuous
+    // the limits are fixed here because the window placement search's start layout depends on them
+    tss_search_params p = params ? *params : tss_search_params{0, 0, 0, -1, TSS_KERNEL_AUTO};
+    if (p.kernel != TSS_KERNEL_AUTO && p.kernel != TSS_KERNEL_WINDOW_PLACEMENTS)
+        return e->fail(TSS_E_UNSUPPORTED, "tss_search_create_with_limits: per-type limits on a %dx%d grid need the window placement search (kernel %d)", w, h, p.kernel);
+    p.kernel = TSS_KERNEL_WINDOW_PLACEMENTS;
+    return search_create(e, grid, w, h, defs, n_defs, &p, card, n_card, out);
 }
 
 void tss_search_destroy(tss_search* s) {
@@ -1226,9 +1269,39 @@ static int greedy_layout(tss_engine* e, const tss_search* s, bool anchor_order, 
     return TSS_OK;
 }
 
+// The start layout under per-type limits: the platforms of `plats` in row-major anchor order, each kept only while every class
+// it belongs to has room, then a 1x1 on every ceiling tile (row-major) that is still unsupported.  Such a tile lies under no
+// footprint, and 1x1 is in no class: the layout is complete and keeps every limit.
+static void limit_start_layout(const tss_search* s, const std::vector<uint32_t>& mask, const std::vector<int>& lim, std::vector<tss_platform>& plats) {
+    std::vector<int> n(lim.size(), 0), reach;
+    std::vector<uint8_t> sup((size_t)s->w * s->h, 0);
+    std::vector<tss_platform> kept;
+    auto add = [&](const tss_platform& p) {
+        kept.push_back(p);
+        platform_reach(s->grid, s->w, s->h, p, reach);
+        for (int t : reach) sup[(size_t)t] = 1;
+    };
+    for (const tss_platform& p : plats) {
+        const Dims d = platform_dims(p);
+        uint32_t m = 0;
+        for (size_t k = 0; k < s->key_dims.size(); k++)
+            if (s->key_dims[k].x == d.w && s->key_dims[k].y == d.h) m = mask[k];
+        bool room = true;
+        for (size_t j = 0; j < lim.size(); j++) room = room && !(((m >> j) & 1u) && n[j] >= lim[j]);
+        if (!room) continue;
+        for (size_t j = 0; j < lim.size(); j++) n[j] += (m >> j) & 1u;
+        add(p);
+    }
+    for (int t = 0; t < s->w * s->h; t++)
+        if (s->grid[(size_t)t] && !sup[(size_t)t]) add(tss_platform{t % s->w, t / s->w, 1, 1, 0});
+    plats.swap(kept);
+}
+
 // TSS_KERNEL_WINDOW_PLACEMENTS on a grid larger than 32x32: dims keys, costs and the start layout — the greedy placement cover,
 // redundant platforms pruned, as an anchor grid — on the device, then the search (lns_placements.cu).  seeds = chains per window.
-static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds) {
+// card / n_card: per-type limit records (tss_search_create_with_limits); when they make classes, the start layout is trimmed to
+// keep them (limit_start_layout) and the search keeps them in every phase.
+static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims* defs, int n_defs, int seeds, const int32_t* card, int n_card) {
     build_keys(defs, n_defs, s->key_dims, s->key_proto);
     bool fits = s->key_dims.size() > 1 && (int)s->key_dims.size() <= slsm_max_keys();
     for (auto& kd : s->key_dims) fits = fits && kd.x <= 6 && kd.y <= 6;
@@ -1236,11 +1309,15 @@ static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims
         return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: the window placement search needs a platform set beyond {1x1} with at most %d dims keys, each at most 6x6",
                        slsm_max_keys());
     if (e->comm && comm_world(e->comm) > 1) return e->fail(TSS_E_UNSUPPORTED, "tss_search_create: the window placement search runs on a single rank");
+    std::vector<uint32_t> mask;
+    std::vector<int> lim;
+    if (int rc = card_limit_classes(s->key_dims, card, n_card, mask, lim)) return e->fail(rc, "tss_search_create_with_limits: bad limit records");
     s->kernel = TSS_KERNEL_WINDOW_PLACEMENTS;
     s->key_costs.assign(s->key_dims.size(), 1);
     std::vector<tss_platform> start;
     int rc = greedy_layout(e, s, true, start);
     if (rc) return rc;
+    if (!lim.empty()) limit_start_layout(s, mask, lim, start);
     std::vector<uint8_t> anchors((size_t)s->w * s->h, 0);
     for (auto& p : start) {
         const Dims d = platform_dims(p);
@@ -1256,7 +1333,7 @@ static int window_placements_create(tss_engine* e, tss_search* s, const tss_dims
     if (err == cudaSuccess) err = cudaMemcpy(s->costs_dev + slsm_max_keys(), order.data(), sizeof(int) * nk, cudaMemcpyHostToDevice);
     if (err != cudaSuccess) return e->fail(TSS_E_CUDA, "tss_search_create: %s", cudaGetErrorString(err));
     rc = lnsp_create(e, s->grid.data(), s->w, s->h, anchors.data(), s->keys_dev, s->costs_dev, s->costs_dev + slsm_max_keys(), (int)nk, seeds, s->seed,
-                     s->chain_offset, s->noise, &s->lnsp);
+                     s->chain_offset, s->noise, mask.data(), lim.data(), (int)lim.size(), &s->lnsp);
     if (rc) return rc;
     s->n_chains = lnsp_chains(s->lnsp);
     return TSS_OK;
@@ -1341,6 +1418,9 @@ int tss_search_best_layout(tss_search* s, tss_platform* out, int32_t cap, int32_
                 cost += s->key_costs[(size_t)a - 1];
             }
         if (cost != lnsp_value(s->lnsp)) return e->fail(TSS_E_CUDA, "internal error: layout costs %d, the search reported %d", cost, lnsp_value(s->lnsp));
+        int n_j = 0, l_j = 0;
+        if (const int j = lnsp_over_limit(s->lnsp, &n_j, &l_j); j >= 0)
+            return e->fail(TSS_E_CUDA, "internal error: the layout holds %d platforms of limit class %d, its limit is %d", n_j, j, l_j);
         best = make_int2((int)plats.size(), 0);
     } else if (s->multi) {
         best = s->best_host[0];
@@ -1658,13 +1738,18 @@ static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h
             if (rc != TSS_OK) { search_free(s); return rc; }
         }
     }
+    if (!s && limited && (w > 32 || h > 32)) {   // per-type limits on a large grid: the window placement search, limits fixed at creation
+        p.kernel = TSS_KERNEL_AUTO;
+        rc = tss_search_create_with_limits(e, grid, w, h, defs, n_defs, card, n_card, &p, &s);
+        if (rc) return rc;
+    }
     if (!s) {
         rc = tss_search_create(e, grid, w, h, defs, n_defs, &p, &s);
         if (rc) return rc;
     }
     s->share = false;  // a one-shot solve runs a rank-local number of epochs: no collective inside
     if (n_weights > 0) rc = tss_search_set_weights(s, weights, n_weights);
-    if (rc == TSS_OK && limited) rc = tss_search_set_card_limits(s, card, n_card);
+    if (rc == TSS_OK && limited && !s->lnsp) rc = tss_search_set_card_limits(s, card, n_card);
     if (rc == TSS_OK && card_limit >= 0 && fused_steps == 0) rc = tss_search_set_bound(s, card_limit + 1);   // (the fused epoch took its bound as a parameter)
     const double t0 = now_ms();
     // no budget given: behave like one SAT call (return the first model within the bound), but give up after a
@@ -1676,7 +1761,7 @@ static int solve_search(tss_engine* e, const uint8_t* grid, int32_t w, int32_t h
     // (a placement-search step costs ~5 us of latency: start with short epochs when the first model is all that is asked for)
     int64_t done_steps = fused_steps, epoch = fused_steps ? 2 * fused_steps : ((s->multi && first_model_only) ? 16 : (first_model_only && !s->lns ? 32 : 64));
     int best = fused_best;
-    const bool in_stream_witness = !s->lns && !s->multi && s->n_groups == 1;   // 1x1 supports on a grid up to 32x32
+    const bool in_stream_witness = !s->lns && !s->lnsp && !s->multi && s->n_groups == 1;   // 1x1 supports on a grid up to 32x32
     // First-model mode: chains stop at the first layout within the limit (target = card_limit).  (Queueing several epochs
     // per synchronisation — later ones do nothing once the bound is within the target, sls_spec.hpp — was measured and lost:
     // ~20 us of launch / event / copy calls per queued epoch against ~15 us per synchronisation.)

@@ -48,6 +48,7 @@ struct tss_engine {
     std::atomic<int> interrupt_flag{0};
     bool certified_unsat = true;             // tss_solve_instance may answer TSS_UNSAT from a certified lower bound (tss_engine_certified_unsat)
     bool limit_bounds = false;               // ... and asks the class-aware LP for instances with per-type limits (tss_engine_limit_bounds)
+    bool window_limits = false;              // tss_solve_instance answers per-type instances on grids larger than 32x32 (tss_engine_window_limits)
     struct tss_search* cached_search = nullptr;  // workspace reused by tss_solve_upper_bound (no cudaMalloc per call)
     struct tss_search* cached_batch = nullptr;   // workspace reused by tss_solve_batch
     struct tss_search* cached_multi = nullptr;   // workspace of the placement search (platform sets beyond {1x1}) of a one-shot solve

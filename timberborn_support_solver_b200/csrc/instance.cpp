@@ -156,15 +156,23 @@ int tss_engine_limit_bounds(tss_engine* e, int enabled) {
     return TSS_OK;
 }
 
+int tss_engine_window_limits(tss_engine* e, int enabled) {
+    if (!e) return TSS_E_INVALID;
+    e->window_limits = enabled != 0;
+    return TSS_OK;
+}
+
 int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc, const tss_instance_info* info, const int32_t* weights,
                        uint64_t seed, int64_t give_up_steps, uint8_t* assignment) {
     if (!e) return TSS_E_INVALID;
     if (!c || !enc || !info || !assignment) return e->fail(TSS_E_INVALID, "tss_solve_instance: bad arguments");
     const Encoding& E = enc->d->enc;
-    // per-type limits: the placement search steers by the limits recorded on a handle of tss_instance_find, on grids up to 32x32,
-    // with one objective (the platform count or the total weight); anything else is left to the exact solver
+    // per-type limits: the placement search steers by the limits recorded on a handle of tss_instance_find, on grids up to 32x32
+    // (larger grids: the window placement search, with tss_engine_window_limits), with one objective (the platform count or the
+    // total weight); anything else is left to the exact solver
     const bool per_type = info->n_other_card_limits > 0;
-    if (per_type && (!enc->has_card_limits || E.w > 32 || E.h > 32 || (info->has_weight_limit && info->card_limit_1x1 >= 0))) return TSS_UNKNOWN;
+    const bool large = E.w > 32 || E.h > 32;
+    if (per_type && (!enc->has_card_limits || (large && !e->window_limits) || (info->has_weight_limit && info->card_limit_1x1 >= 0))) return TSS_UNKNOWN;
     std::vector<tss_dims> defs;
     for (const Dims& d : E.defs) defs.push_back(tss_dims{d.w, d.h});
     // A limit below a CERTIFIED lower bound has no model: answer UNSAT without searching.  Only when one objective is limited
@@ -275,6 +283,8 @@ int tss_solve_instance(tss_engine* e, const tss_cnf* c, const tss_encoding* enc,
     const bool two_phase = pending && give_up_steps > first_budget;
     int rc = search(two_phase ? first_budget : give_up_steps, seed);
     if (rc == TSS_SAT) return tss_witness_for_cnf(e, c, enc, plats.data(), n, assignment);
+    // (a platform set the window placement search does not take, e.g. a 1x7 def: the exact solver's instance)
+    if (per_type && large && rc == TSS_E_UNSUPPORTED) return TSS_UNKNOWN;
     if (rc == TSS_UNKNOWN && (count_only || weight_only) && !e->interrupted()) {   // nothing found within the limit: can the fractional bound certify that nothing exists?
         if (lp_refutes()) return TSS_UNSAT;
         if (two_phase) {

@@ -16,6 +16,15 @@
 //   4. per window the chain with the lowest best wins (lowest chain on ties); the window's movable anchors are cleared and
 //      the winner's best placements written back
 //   5. the objective (platform count, or total weight) of the global layout, reduced on the device into pinned memory
+//
+// Per-type limits (tss_search_create_with_limits): class j (tss::card_limit_classes) holds at most L_j platforms.  The windows
+// pick their winners independently, so each window gets a budget per class: with n_j = the platforms of the global layout in
+// class j (kept current on the device), m_{w,j} = the movable platforms of window w in class j, s_j = L_j - n_j >= 0 and N windows,
+// window w's chains run with limits b_{w,j} = m_{w,j} + floor(s_j / N) + [((w - p) mod N) < (s_j mod N)] (the remainder rotates
+// with the phase p).  Every chain starts from the window's movable platforms, which fit b_{w,j}, and the LIMITS step rule keeps
+// every layout of every chain within b_{w,j}; frozen platforms stay.  So after the write-back n_j <= (n_j - sum_w m_{w,j}) +
+// sum_w b_{w,j} = L_j whatever each window's winner is.  n_j is recounted after every write-back and copied to pinned memory next
+// to the objective, for the host to check.
 #include "engine.hpp"
 #include "lns_window.cuh"
 #include "sls_multi.hpp"
@@ -24,7 +33,7 @@
 namespace tss {
 int slsm_run_windows(tss_engine* e, const uint32_t* rows_dev, const slsm::WindowM& wm, const int2* keys_dev, const int* costs_dev, const int* order_dev,
                      int n_keys, slsm::MultiState* states, int n_chains, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev,
-                     int target, int noise_pct, unsigned long long* totals_dev);
+                     int target, int noise_pct, unsigned long long* totals_dev, const slsm::LimitsM& lm);
 
 namespace lnsp {
 
@@ -110,6 +119,39 @@ __global__ void extract_kernel(const uint8_t* __restrict__ A, const uint32_t* __
     }
 }
 
+// one thread per tile: n_j += 1 for every class j of the platform anchored there (counts zeroed before)
+__global__ void count_classes_kernel(const uint8_t* __restrict__ A, int n, const int* __restrict__ mask, int* __restrict__ ncls) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n || !A[t]) return;
+    for (uint32_t m = (uint32_t)mask[A[t] - 1]; m; m &= m - 1) atomicAdd(&ncls[__ffs(m) - 1], 1);
+}
+
+// one warp per window, lane = window row: m_{w,j} = the movable platforms of the window in class j, then lane j writes the
+// window's budget b_{w,j} = m_{w,j} + its share of the slack s_j = L_j - n_j (the remainder rotates with the phase)
+__global__ void budget_kernel(const uint8_t* __restrict__ A, int w, int h, const int2* __restrict__ keys, const int* __restrict__ mask,
+                              const int* __restrict__ limit, const int* __restrict__ ncls, int n_classes, int ox, int oy, int nwx, int n_windows,
+                              int phase, int* __restrict__ budgets) {
+    const int win = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (win >= n_windows) return;
+    const int gx0 = ox + 32 * (win % nwx), gy0 = oy + 32 * (win / nwx), gy = gy0 + lane;
+    const bool row_ok = lane >= CORE_LO && lane < CORE_HI && gy >= 0 && gy < h;
+    int mine = 0;
+    for (int j = 0; j < n_classes; j++) {
+        int n = 0;
+        for (int lx = CORE_LO; row_ok && lx < CORE_HI; lx++) {
+            const int X = gx0 + lx;
+            const int a = (X >= 0 && X < w) ? A[gy * w + X] : 0;
+            if (a && ((mask[a - 1] >> j) & 1) && movable_local(lx, lane, keys[a - 1])) n++;
+        }
+        n = __reduce_add_sync(0xffffffffu, n);
+        if (lane == j) mine = n;
+    }
+    if (lane < n_classes) {
+        const int slack = limit[lane] - ncls[lane], pos = ((win - phase) % n_windows + n_windows) % n_windows;
+        budgets[win * slsm::MAX_KEYS + lane] = mine + slack / n_windows + (pos < slack % n_windows ? 1 : 0);
+    }
+}
+
 // one warp per window: the chain with the lowest best (lowest chain on ties) -> best[win] = (best, chain)
 __global__ void window_best_kernel(const slsm::MultiState* __restrict__ states, int n_windows, int seeds, int2* __restrict__ best) {
     const int win = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -177,13 +219,22 @@ struct LnspSearch {
     int* obj_dev = nullptr;
     int* obj_host = nullptr;                     // pinned
     unsigned long long* totals_host = nullptr;   // pinned [3]
+    // per-type limits (n_classes > 0): class mask per key [MAX_KEYS] then L_j [MAX_KEYS]; budgets [max_windows][MAX_KEYS]; n_j
+    int n_classes = 0;
+    std::vector<int> limit;                      // L_j (host)
+    int* classes = nullptr;
+    int* budgets = nullptr;
+    int* ncls_dev = nullptr;
+    int* ncls_host = nullptr;                    // pinned [MAX_KEYS]: n_j of the current layout
 };
 
 void lnsp_destroy(LnspSearch* s) {
     if (!s) return;
     cudaFree(s->A); cudaFree(s->C); cudaFree(s->F); cudaFree(s->T0); cudaFree(s->T1); cudaFree(s->rows_win); cudaFree(s->need_win); cudaFree(s->occ_win);
     cudaFree(s->box); cudaFree(s->states); cudaFree(s->best); cudaFree(s->bounds); cudaFree(s->totals); cudaFree(s->obj_dev);
+    cudaFree(s->classes); cudaFree(s->budgets); cudaFree(s->ncls_dev);
     if (s->obj_host) cudaFreeHost(s->obj_host);
+    if (s->ncls_host) cudaFreeHost(s->ncls_host);
     if (s->totals_host) cudaFreeHost(s->totals_host);
     delete s;
 }
@@ -198,10 +249,22 @@ int lnsp_objective(tss_engine* e, LnspSearch* s) {
     return TSS_OK;
 }
 
+// n_j of the current layout, in-stream into ncls_dev and pinned memory (read after a synchronisation)
+static int lnsp_count_classes(tss_engine* e, LnspSearch* s) {
+    TSS_CUDA(e, cudaMemsetAsync(s->ncls_dev, 0, sizeof(int) * slsm::MAX_KEYS, e->stream));
+    lnsp::count_classes_kernel<<<(s->w * s->h + 255) / 256, 256, 0, e->stream>>>(s->A, s->w * s->h, s->classes, s->ncls_dev);
+    TSS_CHECK_LAUNCH(e);
+    e->stats.kernel_launches++;
+    TSS_CUDA(e, cudaMemcpyAsync(s->ncls_host, s->ncls_dev, sizeof(int) * slsm::MAX_KEYS, cudaMemcpyDeviceToHost, e->stream));
+    return TSS_OK;
+}
+
 // anchors: the start layout (u8[w*h], 0 or key + 1), complete, footprints in bounds and disjoint.  keys / costs / order stay
-// owned by the caller and must outlive the search.  Synchronises the stream.
+// owned by the caller and must outlive the search.  n_classes > 0: per-type limits, class_mask[n_keys] and class_limit[n_classes]
+// (tss::card_limit_classes), which the start layout keeps.  Synchronises the stream.
 int lnsp_create(tss_engine* e, const uint8_t* grid, int w, int h, const uint8_t* anchors, const int2* keys_dev, const int* costs_dev, const int* order_dev,
-                int n_keys, int seeds, uint64_t seed, uint32_t chain_offset, int noise, LnspSearch** out) {
+                int n_keys, int seeds, uint64_t seed, uint32_t chain_offset, int noise, const uint32_t* class_mask, const int* class_limit, int n_classes,
+                LnspSearch** out) {
     LnspSearch* s = new LnspSearch();
     s->w = w; s->h = h; s->wpr = (w + 31) / 32; s->nw = h * s->wpr; s->seeds = seeds; s->seed = seed; s->chain_offset = chain_offset; s->noise = noise;
     s->keys = keys_dev; s->costs = costs_dev; s->order = order_dev; s->n_keys = n_keys;
@@ -220,9 +283,21 @@ int lnsp_create(tss_engine* e, const uint8_t* grid, int w, int h, const uint8_t*
     if (err == cudaSuccess) err = cudaMemcpyAsync(s->C, bg.rows.data(), nwb, cudaMemcpyHostToDevice, e->stream);
     if (err == cudaSuccess) err = cudaMemcpyAsync(s->A, anchors, (size_t)w * h, cudaMemcpyHostToDevice, e->stream);
     if (err == cudaSuccess) err = cudaMemsetAsync(s->totals, 0, sizeof(unsigned long long) * 3, e->stream);
+    std::vector<int> cls(2 * (size_t)slsm::MAX_KEYS, 0);
+    if (n_classes > 0) {
+        s->n_classes = n_classes;
+        s->limit.assign(class_limit, class_limit + n_classes);
+        for (int k = 0; k < n_keys; k++) cls[(size_t)k] = (int)class_mask[k];
+        for (int j = 0; j < n_classes; j++) cls[(size_t)slsm::MAX_KEYS + j] = class_limit[j];
+        A((void**)&s->classes, sizeof(int) * cls.size()); A((void**)&s->ncls_dev, sizeof(int) * slsm::MAX_KEYS);
+        A((void**)&s->budgets, sizeof(int) * slsm::MAX_KEYS * (size_t)s->max_windows);
+        if (err == cudaSuccess) err = cudaHostAlloc((void**)&s->ncls_host, sizeof(int) * slsm::MAX_KEYS, cudaHostAllocDefault);
+        if (err == cudaSuccess) err = cudaMemcpyAsync(s->classes, cls.data(), sizeof(int) * cls.size(), cudaMemcpyHostToDevice, e->stream);
+    }
     if (err != cudaSuccess) { lnsp_destroy(s); return e->fail(TSS_E_CUDA, "lnsp_create: %s", cudaGetErrorString(err)); }
     s->totals_host[0] = s->totals_host[1] = s->totals_host[2] = 0;
     int rc = lnsp_objective(e, s);
+    if (rc == TSS_OK && s->n_classes > 0) rc = lnsp_count_classes(e, s);
     if (rc == TSS_OK && cudaStreamSynchronize(e->stream) != cudaSuccess) rc = e->fail(TSS_E_CUDA, "lnsp_create: stream sync failed");
     if (rc != TSS_OK) { lnsp_destroy(s); return rc; }
     *out = s;
@@ -245,15 +320,23 @@ int lnsp_phase(tss_engine* e, LnspSearch* s, long long steps) {
                                                       ((uint32_t)s->phase + 1u) << 20, s->rows_win, s->need_win, s->occ_win, s->box, s->states, s->bounds);
     TSS_CHECK_LAUNCH(e);
     e->stats.kernel_launches += 6;
+    if (s->n_classes > 0) {   // (n_j of the current layout is already in ncls_dev: counted at creation and after every write-back)
+        lnsp::budget_kernel<<<gwin, 128, 0, e->stream>>>(s->A, s->w, s->h, s->keys, s->classes, s->classes + slsm::MAX_KEYS, s->ncls_dev, s->n_classes, ox, oy,
+                                                         nwx, n_windows, s->phase, s->budgets);
+        TSS_CHECK_LAUNCH(e);
+        e->stats.kernel_launches++;
+    }
     const slsm::WindowM wm{s->need_win, s->occ_win, s->box, s->seeds};
+    const slsm::LimitsM lm{s->classes, s->budgets, s->n_classes};
     int rc = slsm_run_windows(e, s->rows_win, wm, s->keys, s->costs, s->order, s->n_keys, s->states, n_chains, s->chain_offset, s->seed, steps, s->bounds,
-                              -1, s->noise, s->totals);
+                              -1, s->noise, s->totals, lm);
     if (rc) return rc;
     lnsp::window_best_kernel<<<gwin, 128, 0, e->stream>>>(s->states, n_windows, s->seeds, s->best);
     lnsp::writeback_kernel<<<gwin, 128, 0, e->stream>>>(s->A, s->w, s->h, s->keys, ox, oy, nwx, n_windows, s->best, s->states);
     TSS_CHECK_LAUNCH(e);
     e->stats.kernel_launches += 2;
     rc = lnsp_objective(e, s);
+    if (rc == TSS_OK && s->n_classes > 0) rc = lnsp_count_classes(e, s);
     if (rc) return rc;
     TSS_CUDA(e, cudaMemcpyAsync(s->totals_host, s->totals, sizeof(unsigned long long) * 3, cudaMemcpyDeviceToHost, e->stream));
     s->phase++;
@@ -271,5 +354,11 @@ int lnsp_anchors(tss_engine* e, LnspSearch* s, std::vector<uint8_t>& anchors) {
 int lnsp_value(const LnspSearch* s) { return s->obj_host[0]; }
 unsigned long long lnsp_total(const LnspSearch* s, int i) { return s->totals_host[i]; }
 int lnsp_chains(const LnspSearch* s) { return s->max_windows * s->seeds; }
+// per-type limits: a class whose count in the current layout exceeds its limit (after a synchronisation), or -1
+int lnsp_over_limit(const LnspSearch* s, int* count, int* limit) {
+    for (int j = 0; j < s->n_classes; j++)
+        if (s->ncls_host[j] > s->limit[(size_t)j]) { *count = s->ncls_host[j]; *limit = s->limit[(size_t)j]; return j; }
+    return -1;
+}
 
 }  // namespace tss

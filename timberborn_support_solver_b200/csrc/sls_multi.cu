@@ -181,23 +181,11 @@ struct OneShotM {
                                   // from word 16: the n placement codes as u16
 };
 
-// LIMITS = per-type platform limits (`solve -l k:v`, PlatformLimits.card_limits beyond 1x1; tss_search_set_card_limits): class j
-// of the limits holds the keys whose platforms count towards limit j (tss::card_limit_classes), mask[key] is the set of classes
-// of a key.  Lane j keeps n_j, the platforms of the current layout in class j (recounted from the item list at every launch),
-// and `full` = { j : n_j >= limit[j] } is one ballot after every flip.  An addition whose key lies in a full class is not a
-// candidate, and the swap trigger takes its minimum cost over the keys that are not blocked.  Chains start empty, so every
-// current and every best layout keeps every limit.
-struct LimitsM {
-    const int* mask;              // [n_keys] classes of each key (bit j = class j)
-    const int* limit;             // [n_classes] at most limit[j] platforms in class j (>= 1)
-    int n_classes;                // <= MAX_KEYS
-};
-
 // WINDOW = the window-decomposed placement search on grids larger than 32x32 (lns_placements.cu, see WindowM): chain c works
 // on window c / seeds, `terrain_rows` holds 32 ceiling rows per window and the epoch bound is bounds[window].
 // (WINDOW: at most 4 CTAs per SM, i.e. up to 128 registers — the window's need rows and box do not fit the 96 registers the
 // compiler settles for otherwise without spilling; a phase on 256x256 launches ~1300 chains, 2-3 CTAs per SM.  LIMITS: the
-// same, for the class counters; an epoch launches 16 chains = 4 CTAs per SM)
+// same, for the class counters; an epoch launches 16 chains = 4 CTAs per SM.  WINDOW and LIMITS together fit the same 128)
 template <bool ONESHOT, bool WINDOW, bool LIMITS>
 __global__ void __launch_bounds__(WARPS * 32, (WINDOW || LIMITS) ? 4 : 0) sls_multi_kernel(const uint32_t* __restrict__ terrain_rows, int W, int H,
                                                               const int2* __restrict__ keys_g, const int* __restrict__ costs_g,
@@ -208,7 +196,7 @@ __global__ void __launch_bounds__(WARPS * 32, (WINDOW || LIMITS) ? 4 : 0) sls_mu
                                                               const volatile int* interrupt, unsigned long long* __restrict__ totals,
                                                               const OneShotM os, const WindowM wm, const LimitsM lm) {
     static_assert(!(ONESHOT && WINDOW), "a one-shot solve never runs on windows");
-    static_assert(!LIMITS || (!ONESHOT && !WINDOW), "per-type limits run on the epoch kernel only");
+    static_assert(!LIMITS || !ONESHOT, "per-type limits never run in a one-shot launch");
     __shared__ uint16_t items_all[WARPS][MAX_ITEMS];
     __shared__ int2 keys[MAX_KEYS];
     __shared__ int costs[MAX_KEYS];
@@ -254,7 +242,7 @@ __global__ void __launch_bounds__(WARPS * 32, (WINDOW || LIMITS) ? 4 : 0) sls_mu
     // LIMITS: lane i < n_keys holds key i's class mask and cost, lane j < n_classes holds n_j and limit[j]
     const uint32_t kmask = LIMITS && lane < n_keys ? (uint32_t)lm.mask[lane] : 0u;
     const int kcost = LIMITS && lane < n_keys ? costs[lane] : 0x7fffffff;
-    const int climit = LIMITS && lane < lm.n_classes ? lm.limit[lane] : 0x7fffffff;
+    const int climit = LIMITS && lane < lm.n_classes ? lm.limit[(WINDOW ? win * MAX_KEYS : 0) + lane] : 0x7fffffff;
     int ncls = 0;
     for (int i = 0; i < k; i++) {
         int x, y, w, h;
@@ -512,14 +500,20 @@ int slsm_run_oneshot(tss_engine* e, const uint32_t* rows32_host, int bound, uint
     return TSS_OK;
 }
 // One epoch of every window's chains (the window-decomposed placement search, lns_placements.cu); chains are numbered
-// window * wm.seeds + j.  No best-reduce here: the caller picks a winner per window.
+// window * wm.seeds + j.  No best-reduce here: the caller picks a winner per window.  lm.n_classes > 0: per-window class budgets
+// (slsm::LimitsM).
 int slsm_run_windows(tss_engine* e, const uint32_t* rows_dev, const slsm::WindowM& wm, const int2* keys_dev, const int* costs_dev, const int* order_dev,
                      int n_keys, slsm::MultiState* states, int n_chains, uint32_t chain_offset, uint64_t seed, long long steps, const int* bounds_dev,
-                     int target, int noise_pct, unsigned long long* totals_dev) {
+                     int target, int noise_pct, unsigned long long* totals_dev, const slsm::LimitsM& lm) {
     const int blocks = (n_chains + slsm::WARPS - 1) / slsm::WARPS;
-    slsm::sls_multi_kernel<false, true, false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, 32, 32, keys_dev, costs_dev, order_dev, n_keys, states, n_chains,
-                                                                                         chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
-                                                                                         totals_dev, slsm::OneShotM{}, wm, slsm::LimitsM{});
+    if (lm.n_classes > 0)
+        slsm::sls_multi_kernel<false, true, true><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, 32, 32, keys_dev, costs_dev, order_dev, n_keys, states, n_chains,
+                                                                                            chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
+                                                                                            totals_dev, slsm::OneShotM{}, wm, lm);
+    else
+        slsm::sls_multi_kernel<false, true, false><<<blocks, slsm::WARPS * 32, 0, e->stream>>>(rows_dev, 32, 32, keys_dev, costs_dev, order_dev, n_keys, states, n_chains,
+                                                                                             chain_offset, seed, steps, bounds_dev, target, noise_pct, e->interrupt_dev,
+                                                                                             totals_dev, slsm::OneShotM{}, wm, slsm::LimitsM{});
     TSS_CHECK_LAUNCH(e);
     e->stats.kernel_launches++;
     return TSS_OK;

@@ -32,5 +32,19 @@ struct WindowM {
     int seeds;                    // chains per window: chain c belongs to window c / seeds
 };
 
+// LIMITS = per-type platform limits (`solve -l k:v`, PlatformLimits.card_limits beyond 1x1; tss_search_set_card_limits): class j
+// of the limits holds the keys whose platforms count towards limit j (tss::card_limit_classes), mask[key] is the set of classes
+// of a key.  Lane j keeps n_j, the platforms of the current layout in class j (recounted from the item list at every launch),
+// and `full` = { j : n_j >= limit[j] } is one ballot after every flip.  An addition whose key lies in a full class is not a
+// candidate, and the swap trigger takes its minimum cost over the keys that are not blocked.  Chains start within the limits
+// (empty, or in WINDOW mode from the window's movable platforms, which fit the window's budgets), so every current and every best
+// layout keeps every limit.  WINDOW: limit[] holds one row of MAX_KEYS budgets per window (lns_placements.cu budget_kernel), the
+// masks are shared by all windows.  A limit of 0 is legal: the class is full from the start.
+struct LimitsM {
+    const int* mask;              // [n_keys] classes of each key (bit j = class j)
+    const int* limit;             // [n_classes] at most limit[j] platforms in class j (>= 0); WINDOW: [n_windows][MAX_KEYS]
+    int n_classes;                // <= MAX_KEYS
+};
+
 }  // namespace slsm
 }  // namespace tss

@@ -16,11 +16,14 @@
 // `--limit-bounds` lets tss_solve_instance certify the UNSAT of a `-l` loop with the class-aware LP, which keeps the per-type
 // limits (tss_engine_limit_bounds); `--no-lower-bound` switches every bound off, this one included.
 //
+// `--window-limits` lets tss_solve_instance answer `-l` instances on grids larger than 32x32 with the window placement search
+// (tss_engine_window_limits); it finds layouts, it proves nothing, so without `--exact` such a loop ends "unknown".
+//
 // `--gui` runs the GUI's loop instead (crates/gui/src/app.rs:212-249): the default-8 set with the GUI's default weights
 // (app.rs:53-62), no card limits; after every solution limits.weight_limit = total_weight - 1 (while that is positive), until
 // the solver says Unsat — the weight limit's pseudo-boolean constraint is part of the clauses the witness is checked against.
 //
-//   tss_repl PROJECT.toml [--platforms default|1x1] [-l k:v[,k:v]] [--gui] [--exact "CMD"] [--seed N] [--no-lower-bound] [--limit-bounds] [--quiet] [--repeat N] [--phases]
+//   tss_repl PROJECT.toml [--platforms default|1x1] [-l k:v[,k:v]] [--gui] [--exact "CMD"] [--seed N] [--no-lower-bound] [--limit-bounds] [--window-limits] [--quiet] [--repeat N] [--phases]
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -100,7 +103,7 @@ int main(int argc, char** argv) {
     std::string project, exact_cmd, platforms = "default";
     std::vector<int32_t> card;
     uint64_t seed = 0;
-    bool use_lb = true, limit_lb = false, quiet = false, phases = false, gui = false;
+    bool use_lb = true, limit_lb = false, window_limits = false, quiet = false, phases = false, gui = false;
     int repeat = 1;
     double ph[8] = {};   // --phases: wall ms per call site, summed over the warm repeats
     static const char* const PH[8] = {"encoding_create", "with_limits", "cnf_upload", "instance_find", "solve_instance", "from_assignment", "validate", "destroy"};
@@ -113,12 +116,13 @@ int main(int argc, char** argv) {
         else if (a.rfind("-l", 0) == 0 && a.size() > 2) { if (!parse_limits(a.substr(2), card)) { std::fprintf(stderr, "bad -l argument\n"); return 2; } }
         else if (a == "--no-lower-bound") use_lb = false;
         else if (a == "--limit-bounds") limit_lb = true;
+        else if (a == "--window-limits") window_limits = true;
         else if (a == "--quiet") quiet = true;
         else if (a == "--phases") phases = true;
         else if (a == "--gui") gui = true;
         else if (a == "--repeat" && i + 1 < argc) repeat = std::atoi(argv[++i]) > 0 ? std::atoi(argv[i]) : 1;
         else if (project.empty()) project = a;
-        else { std::fprintf(stderr, "usage: tss_repl PROJECT.toml [--platforms default|1x1] [-l k:v[,k:v]] [--exact CMD] [--seed N] [--no-lower-bound] [--limit-bounds] [--quiet]\n"); return 2; }
+        else { std::fprintf(stderr, "usage: tss_repl PROJECT.toml [--platforms default|1x1] [-l k:v[,k:v]] [--exact CMD] [--seed N] [--no-lower-bound] [--limit-bounds] [--window-limits] [--quiet]\n"); return 2; }
     }
     if (project.empty()) { std::fprintf(stderr, "no project file\n"); return 2; }
     std::ifstream in(project);
@@ -175,6 +179,7 @@ int main(int argc, char** argv) {
         // solve() sees them: this driver, like the REPL's, knows nothing about bounds
         tss_engine_certified_unsat(e, use_lb ? 1 : 0);
         tss_engine_limit_bounds(e, use_lb && limit_lb ? 1 : 0);
+        tss_engine_window_limits(e, window_limits ? 1 : 0);
 
         int64_t give_up = 1024;
         for (;;) {
